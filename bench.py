@@ -13,6 +13,7 @@ __graft_entry__.build() from /root/reference) on the box's host cores, one proce
 the same synthetic frames -- a bounded sample of the same workload, all cores busy.
 
 Launch: python bench.py --gpus N --steps K --warmup W   (N > 1 under torchrun, one rank per GPU).
+--dump-outputs DIR writes the result records of the last timed step as .npy files, to compare two builds output for output.
 """
 import argparse
 import json
@@ -204,6 +205,8 @@ def run_b200(args, rank, world, local_rank, dist):
     k_plan, k_eval, k_lists, k_n = eng.kernel_times()
     eng.kernel_timing(False)
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, vb, d_res, n)
     ms_total = vb.shard.max_over_ranks(ms_total, dist, 'cuda:%d' % local_rank)
 
     e2e_s, e2e_steps, e2e_full_s, e2e_plan_s = float("nan"), 1, float("nan"), float("nan")
@@ -325,6 +328,27 @@ def run_b200(args, rank, world, local_rank, dist):
     if world == 1 and not args.no_bitexact and not args.resident_only:
         out['bitexact'] = bitexact_leg(frames, local_rank)
     emit(out)
+
+
+DUMP_VISITS = 1 << 16      # 46 MB of arrays; all 679 260 records would be 250 MB
+
+
+def dump_outputs(out_dir, eng, vb, d_res, n):
+    """--dump-outputs: the result records of the last timed step, as vvcb_rmd_eval_device hands them to its caller, for a fixed
+    seeded sample of the step's visits.  One float array per field: list lengths (n_rd, n_had, n_final), costs, and the
+    (mip, mrl, mode) triple of every list entry; entries past a list's length are zero, as the kernel writes them."""
+    res = np.empty(n, vb.RESULT_DTYPE)
+    eng.dev_download(res, d_res)
+    idx = np.sort(np.random.default_rng(7).choice(n, min(n, DUMP_VISITS), replace=False))
+    r = res[idx]
+    arrays = {'visit_index': idx.astype(np.float64),
+              'list_lengths': np.stack([r['n_rd'], r['n_had'], r['n_final']], axis=1).astype(np.float64),
+              'rd_cost': r['rd_cost'].astype(np.float64), 'had_cost': r['had_cost'].astype(np.float64)}
+    for f in ('rd_mode', 'had_mode', 'final_mode'):
+        arrays[f] = np.stack([r[f]['mip'], r[f]['mrl'], r[f]['mode']], axis=-1).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def strong_scaling_leg(eng, vb, rank, world, dist, local_rank):
@@ -677,7 +701,12 @@ def main():
     ap.add_argument('--no-strong', action='store_true', help='skip the configs[2] strong-scaling leg (64 x 2160p frames sharded over the ranks)')
     ap.add_argument('--no-bitexact', action='store_true', help='skip the brokered bit-exact encode leg (walker processes + plain reference on the host cores)')
     ap.add_argument('--resident-only', action='store_true', help='profiling aid: only the HBM-resident timed loop (no e2e / TU / CPU legs); not a bench line')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the result records of the last timed step (a fixed sample of %d visits) as DIR/<field>.npy' % DUMP_VISITS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to the b200 arm')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

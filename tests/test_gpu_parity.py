@@ -7,6 +7,7 @@ import pytest
 import vvc_intra_b200 as vb
 from oracle import oracle_py as O
 import golden_util as G
+from make_golden import SERVED_WORKLOADS
 
 pytestmark = pytest.mark.gpu
 
@@ -27,7 +28,18 @@ def eng8():
 def test_golden_fixture_parity(name, bd, eng8, eng10):
     """Every recorded visit of the reference encoder: SAD/SATD of every evaluation, candidate lists with
     exact double costs, and byte-identical result structs versus the oracle."""
-    eng = eng8 if bd == 8 else eng10
+    _check_fixture(name, bd, eng8 if bd == 8 else eng10)
+
+
+@pytest.mark.parametrize('name', sorted(SERVED_WORKLOADS))
+def test_served_workload_visits_match_reference(name, eng8, eng10):
+    """The pictures the reference encoder encodes in the served-encoder tests below (tools/make_golden.py SERVED_WORKLOADS), checked without
+    the reference binaries: sampled rough-mode-decision visits of the reference against the engine, as in test_golden_fixture_parity."""
+    bd = 8 if '_8b_' in name else 10
+    _check_fixture('served/' + name, bd, eng8 if bd == 8 else eng10)
+
+
+def _check_fixture(name, bd, eng):
     visits, _ = G.load_fixture(name)
     orig, reco, arr = G.build_atlas(visits)
     eng.frame_begin(orig)

@@ -18,9 +18,13 @@ FAKE = os.path.join(ROOT, 'tests/fake_engine')
 
 
 @pytest.fixture(scope='module')
-def built():
+def libraries():
     import __graft_entry__ as g
     g.build()
+
+
+@pytest.fixture(scope='module')
+def built(libraries):
     need = [os.path.join(REF, f) for f in ('EncoderApp', 'EncoderAppServe', 'encoder_intra.cfg')] + [os.path.join(FAKE, 'libvvc_intra_b200.so'), os.path.join(FAKE, 'vvcb_broker')]
     if not all(os.path.exists(p) for p in need):
         pytest.skip('oracle/_ref binaries are built only in the container that has /root/reference')
@@ -45,7 +49,7 @@ def run(cmd, cwd, env=None):
     return r.stdout
 
 
-def test_broker_header_symbols_are_exported(built):
+def test_broker_header_symbols_are_exported(libraries):
     hdr = open(os.path.join(ROOT, 'include/vvc_intra_b200_broker.h')).read()
     names = sorted(set(re.findall(r'\b(vvcb_broker_[a-z_]+)\s*\(', hdr)))
     assert names == ['vvcb_broker_read_stats', 'vvcb_broker_serve', 'vvcb_broker_stop']

@@ -119,5 +119,59 @@ def extra_fixtures(which):
             f.write(todo[n](n) + '\n')
 
 
+# The pictures the reference encoder encodes in the served-encoder tests of tests/test_gpu_parity.py (name: w, h, bits, qp, frame).
+SERVED_WORKLOADS = {
+    'rmd_8b_128x64_qp32_f0': (128, 64, 8, 32, 0), 'rmd_10b_128x128_qp27_f0': (128, 128, 10, 27, 0),
+    'rmd_10b_128x128_qp37_f0': (128, 128, 10, 37, 0), 'rmd_10b_128x128_qp22_f0': (128, 128, 10, 22, 0),
+    'rmd_10b_128x64_qp27_f1': (128, 64, 10, 27, 1), 'rmd_10b_128x128_qp32_f2': (128, 128, 10, 32, 2),
+    'rmd_10b_128x64_qp37_f3': (128, 64, 10, 37, 3), 'rmd_10b_128x64_qp32_f2': (128, 64, 10, 32, 2),
+    'rmd_8b_416x240_qp32_f0': (416, 240, 8, 32, 0),
+}
+
+
+def served_fixture(name, keep=10):
+    """tests/golden/served/<name>.bin.gz: the V/R/P/B/L records (reference lines, predictions, SAD/SATD, mode bits, candidate lists)
+    of `keep` evenly spaced ones of every 97th rough-mode-decision visit of one picture; the TU records are dropped to keep the file small."""
+    import struct
+    w, h, bits, qp, frame = SERVED_WORKLOADS[name]
+    tmp = tempfile.mkdtemp(prefix='vvcgold_')
+    try:
+        Y, U, V = synth_yuv(w, h, bits, frame)
+        open(os.path.join(tmp, 'in.yuv'), 'wb').write(Y.tobytes() + U.tobytes() + V.tobytes())
+        open(os.path.join(tmp, 'Time_python.dat'), 'w').close()
+        cfg = os.path.join(ROOT, 'oracle/_ref/encoder_intra.cfg')
+        e = dict(os.environ, VVC_TRACE_OUT=os.path.join(tmp, 'trace.bin'), VVC_TRACE_VISIT_FIRST='0', VVC_TRACE_VISIT_STRIDE='97',
+                 VVC_TRACE_FULL_PRED='0', VVC_TRACE_TU_FIRST='1000000000', VVC_TRACE_TU_STRIDE='1000000000')
+        cmd = [os.path.join(ROOT, 'oracle/_ref/EncoderAppTrace'), '-c', cfg, '-i', 'in.yuv', '-wdt', str(w), '-hgt', str(h), '-q', str(qp),
+               '-f', '1', '-fr', '30', '-b', 'out.bin', '--InputBitDepth=%d' % bits, '--InternalBitDepth=%d' % bits, '--OutputBitDepth=%d' % bits]
+        out = subprocess.run(cmd, cwd=tmp, env=e, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+        if out.returncode:
+            raise SystemExit('reference encoder failed: ' + out.stdout[-2000:])
+        b = open(os.path.join(tmp, 'trace.bin'), 'rb').read()
+        visits, o = [], 0
+        while o < len(b):
+            tag, n = chr(b[o]), struct.unpack_from('<I', b, o + 1)[0]
+            if tag == 'V':
+                visits.append([])
+            if tag in 'VRPBL':
+                visits[-1].append(b[o:o + 5 + n])
+            o += 5 + n
+        pick = np.linspace(0, len(visits) - 1, keep).astype(int)
+        dst = os.path.join(ROOT, 'tests/golden/served', name + '.bin.gz')
+        os.makedirs(os.path.dirname(dst), exist_ok=True)
+        with gzip.GzipFile(dst, 'wb', compresslevel=9, mtime=0) as f:
+            f.write(b''.join(r for i in pick for r in visits[i]))
+        return '%s: %dx%d %d-bit qp%d frame %d, visits %s of %d' % (name, w, h, bits, qp, frame, pick.tolist(), len(visits))
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+
+
 if __name__ == '__main__':
+    if len(sys.argv) > 1 and sys.argv[1] == '--served':
+        from multiprocessing import Pool
+        with Pool(8) as p:
+            lines = p.map(served_fixture, sys.argv[2:] or sorted(SERVED_WORKLOADS))
+        with open(os.path.join(ROOT, 'tests/golden/MANIFEST.txt'), 'a') as f:
+            f.write(''.join('served/' + l + '\n' for l in lines))
+        sys.exit(0)
     sys.exit(main())
