@@ -362,8 +362,10 @@ double vvcb_calc_rd_cost(double lambda, uint64_t frac_bits, uint64_t distortion)
  *     the lines of the whole CU once (fetch_*), every region then predicts with top = cu_w + pred_w, left = cu_h + pred_h samples;
  *   TrQuant::getTrTypes (CL/TrQuant.cpp:752-783) -- ISP blocks take DST-VII in a direction of 4..16 samples, DCT-II otherwise
  *     (DCT-II in both when the SPS switches MTS off: use_mts = sps.getUseMTS()).
- * The evaluation kernels for these blocks (1xN / 2xN / Nx1 / Nx2 transforms, their scans and contexts) are NOT in the library yet:
- * the served encoder hands ISP candidates to the reference code (DESIGN.md 7).                                                         */
+ * vvcb_isp_eval (below) evaluates ISP candidates whose transform blocks are all at least 4x4 (horizontal split: CU height >= 16 or the
+ * 4x8 CU; vertical split: CU width >= 16 or the 8x4 CU).  NOT in the library yet: the 1xN / 2xN / Nx1 / Nx2 blocks (one-dimensional and
+ * 2-point transforms, their scans and contexts, the 4-wide prediction rule) and LFNST with ISP; the served encoder still hands ISP
+ * candidates to the reference code (DESIGN.md 7).                                                                                      */
 #define VVCB_ISP_NONE 0
 #define VVCB_ISP_HOR  1   /* HOR_INTRA_SUBPARTITIONS: blocks stacked top to bottom (TU_1D_HORZ_SPLIT) */
 #define VVCB_ISP_VER  2   /* VER_INTRA_SUBPARTITIONS: blocks side by side (TU_1D_VERT_SPLIT)          */
@@ -395,6 +397,50 @@ typedef struct vvcb_isp_mode {
   uint8_t  pad;
 } vvcb_isp_mode;        /* 8 bytes */
 int vvcb_isp_mode_param(int cu_w, int cu_h, int pred_w, int pred_h, int mode, vvcb_isp_mode* out);
+
+/* Evaluation of ISP candidates: the luma part of IntraSearch::xIntraCodingLumaISP (EL/IntraSearch.cpp:3171) for CUs whose blocks are at
+ * least 4x4.  A candidate is one CU x split x luma mode x quantiser setting; its blocks are coded in order on one estimator, as the
+ * reference does after restoring the CABAC estimator once per candidate: initIntraPatternChTypeISP + predIntraAng of block k from the
+ * reconstruction of block k-1 (CL/IntraPrediction.cpp:1092-1203; lines unfiltered, cubic interpolation, reference line 0),
+ * TrQuant::transformNxN with the implicit DST-VII / DCT-II pair (CL/TrQuant.cpp:752-783), Quant::quant or DepQuant::quant with
+ * cbfDeltaBits of the ISP branch of RateEstimator::xSetLastCoeffOffset (CL/DepQuant.cpp:491-540), invTransformNxN, reconstruction and SSE
+ * (xIntraCodingTUBlock, :2694), then xGetIntraFracBitsQT's cbf bin (Ctx::QtCbf[luma](2 + cbf of the previous block); the last block's cbf
+ * is not coded when every earlier one is 0) and residual_coding, each block priced on the context models the previous block left.
+ * Header bits (mode, ISP flag, LFNST index) stay with the caller, and so do the early exits of the reference's loop (bestCostSoFar): they
+ * never change the value of a block that is computed, so every block is computed and the per-block results let the caller apply them.
+ * Blocks of 1 or 2 samples in one direction, LFNST, transform skip and explicit MTS are not evaluated (vvcb_isp_plan describes them).    */
+typedef struct vvcb_isp_job {
+  uint32_t visit;            /* index into visits[]: the CU (position, size, availability); mpm / rates / sqrt_lambda are not read      */
+  uint8_t  isp_mode;         /* VVCB_ISP_HOR / VVCB_ISP_VER                                                                          */
+  uint8_t  mode;             /* luma mode 0..66                                                                                      */
+  uint8_t  flags;            /* VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE]                                                  */
+  uint8_t  use_mts;          /* sps.getUseMTS(): DST-VII for block sides 4..16                                                       */
+  uint8_t  max_tb_size;      /* sps max TB size (CU::canUseISP)                                                                      */
+  uint8_t  lfnst_idx;        /* must be 0                                                                                            */
+  int16_t  qp_per, qp_rem;   /* as vvcb_tu_job                                                                                       */
+  uint16_t rate_idx;         /* states[rate_idx]: the estimator's models at the start of the candidate                               */
+  uint32_t offset;           /* first sample of this candidate's cu_w*cu_h outputs: its blocks in coding order, each dense w*h      */
+  vvcb_bin_model cbf[2];     /* Ctx::QtCbf[luma] contexts 2 and 3 at the start of the candidate                                      */
+  double   lambda;           /* Quant::m_dLambda (dependent quantisation)                                                            */
+} vvcb_isp_job;              /* 40 bytes */
+typedef struct vvcb_isp_result {
+  vvcb_tu_result part[VVCB_ISP_MAX_PARTS];  /* per block, coding order: abs sums, sse, residual frac_bits (VVCB_TU_RATE)             */
+  uint32_t cbf_bits[VVCB_ISP_MAX_PARTS];    /* fractional bits of the block's cbf bin, 0 when it is inferred                        */
+  uint8_t  cbf[VVCB_ISP_MAX_PARTS];
+  uint8_t  n_parts;                         /* 2 or 4                                                                               */
+  uint8_t  discarded;                       /* the last cbf is inferred but the last block has no level: the reference gives the
+                                               candidate MAX_INT distortion                                                          */
+  uint8_t  pad[2];
+} vvcb_isp_result;                          /* 120 bytes */
+/* visits: HOST, the CUs (availability must be all or nothing on each side: n_left 0 or h/4, n_above 0 or w/4, and no below-left /
+ * above-right without it -- in a tree partition the left and above of a CU's own rows and columns are coded before it, and only then
+ * does the fresh fetch of the device agree with the reference's shifted lines).  level / reco / pred: optional HOST outputs of n_samples.
+ * Needs vvcb_frame_begin (original and reconstruction planes).  Returns VVCB_ERR_ARG for a CU or split without blocks of at least 4x4,
+ * other availability, mode > 66, lfnst_idx != 0, transform-skip / RDOQ flags, a bad rate_idx, lambda <= 0 with VVCB_TU_DEPQUANT, or
+ * outputs outside n_samples.                                                                                                       */
+int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, const vvcb_isp_job* jobs, int n,
+                  const vvcb_ctx_states* states, int n_states, size_t n_samples,
+                  int32_t* level, int16_t* reco, int16_t* pred, vvcb_isp_result* results);
 
 /* ---- texture features (orig-only, trivially parallel) ------------------------------------------------------------
  * vvcb_ctu_hads_islice: EncCu::updateCtuDataISlice (EL/EncCu.cpp:564-675) for every CTU of the frame, as

@@ -1556,6 +1556,279 @@ extern "C" int vvcb_isp_mode_param(int cu_w, int cu_h, int pred_w, int pred_h, i
   return VVCB_OK;
 }
 
+// ISP candidates (include/vvc_intra_b200.h): up to four steps, one per block index k, over the TU kernels; the blocks of every candidate
+// that has a block k run in step k: isp_pred_kernel (lines from block k-1's reconstruction, prediction, residual, cbf of block k-1 and
+// cbfDeltaBits of block k), tu_eval_kernel pass 0, the quantiser (the dependent one priced by rates_from_states_kernel from the models the
+// previous block left), pass 1 (reconstruction into the candidate's buffer), rate_kernel adapting the candidate's carried models in place.
+// A fifth isp_pred_kernel pass codes the cbf of the last block of four-block candidates.
+// One chunk of at most kIspChunk candidates (their TU jobs name the carried snapshots with the 16-bit rate_idx); base: index of the
+// chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
+constexpr int kIspChunk = 65536;
+static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, const vvcb_isp_job* jobs, int n, int base,
+                          const vvcb_ctx_states* states, int n_states, size_t n_samples,
+                          int32_t* level, int16_t* reco, int16_t* pred, vvcb_isp_result* results, bool checkOnly)
+{
+  const unsigned kFlags = VVCB_TU_QUANT | VVCB_TU_DEPQUANT | VVCB_TU_RATE;
+  std::vector<IspCand> cands(n);
+  std::vector<vvcb_tu_job> tj((size_t)4 * n);
+  std::vector<uint8_t> trPair((size_t)4 * n, 0);
+  std::vector<IspState> ist(n);
+  std::vector<vvcb_ctx_states> cst(n);
+  size_t cs = 0;                                   // the chunk's own samples: candidates are packed densely on the device, whatever the caller's offsets
+  for (int i = 0; i < n; i++) {
+    const vvcb_isp_job& j = jobs[i];
+    auto bad = [&](const char* why) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_isp_eval: job %d: %s", base + i, why); return VVCB_ERR_ARG; };
+    if (j.visit >= (uint32_t)n_visits) return bad("visit index out of range");
+    const vvcb_rmd_visit& v = visits[j.visit];
+    const int cuW = 1 << v.log2w, cuH = 1 << v.log2h;
+    vvcb_isp_part parts[VVCB_ISP_MAX_PARTS];
+    const int np = vvcb_isp_plan(cuW, cuH, j.isp_mode, j.max_tb_size, j.use_mts, parts);
+    if (np <= 0) return bad("the CU may not use this split (vvcb_isp_plan)");
+    if (parts[0].w < 4 || parts[0].h < 4) return bad("blocks narrower than 4 samples are not evaluated");
+    // all-or-nothing availability: the fresh fetch of isp_pred_kernel equals the reference's shifted lines only then
+    if ((v.n_left != 0 && v.n_left != cuH / 4) || (v.n_above != 0 && v.n_above != cuW / 4) || (!v.n_left && v.n_below_left) || (!v.n_above && v.n_above_right))
+      return bad("left / above availability is not all or nothing");
+    if (j.mode >= VVCB_NUM_LUMA_MODE) return bad("mode above 66");
+    if (j.lfnst_idx != 0) return bad("LFNST with ISP is not evaluated");
+    if ((j.flags & ~kFlags) || !(j.flags & VVCB_TU_QUANT)) return bad("flags: VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE] only");
+    if (j.qp_rem < 0 || j.qp_rem >= 6 || j.qp_per < 0 || j.qp_per >= 16) return bad("qp_per / qp_rem out of range");
+    const bool dq = (j.flags & VVCB_TU_DEPQUANT) != 0, carried = dq || (j.flags & VVCB_TU_RATE);
+    if (carried && (!states || j.rate_idx >= n_states)) return bad("rate_idx does not name a context snapshot");
+    if (dq && !(j.lambda > 0.0)) return bad("dependent quantisation needs lambda > 0");
+    if ((size_t)j.offset + (size_t)cuW * cuH > n_samples) return bad("outputs outside n_samples");
+    IspCand& c = cands[i];
+    c.x = v.x; c.y = v.y; c.cuW = (int16_t)cuW; c.cuH = (int16_t)cuH; c.bw = parts[0].w; c.bh = parts[0].h;
+    c.topLen = parts[0].top_ref_len; c.leftLen = parts[0].left_ref_len;
+    c.hor = j.isp_mode == VVCB_ISP_HOR; c.nParts = (uint8_t)np; c.availAl = v.avail_al; c.nAbove = v.n_above; c.nAboveRight = v.n_above_right;
+    c.nLeft = v.n_left; c.nBelowLeft = v.n_below_left; c.mode = j.mode; c.offset = (uint32_t)cs;
+    c.p = make_mode_param_isp(cuW, cuH, parts[0].pred_w, parts[0].pred_h, j.mode);
+    memset(&ist[i], 0, sizeof(IspState));
+    ist[i].ctx[0] = j.cbf[0]; ist[i].ctx[1] = j.cbf[1];
+    if (carried) cst[i] = states[j.rate_idx]; else memset(&cst[i], 0, sizeof(vvcb_ctx_states));
+    for (int k = 0; k < np; k++) {
+      vvcb_tu_job& t = tj[(size_t)k * n + i];
+      memset(&t, 0, sizeof(t));
+      t.x = (int16_t)(v.x + parts[k].x); t.y = (int16_t)(v.y + parts[k].y);
+      t.log2w = (uint8_t)vlog2(parts[k].w); t.log2h = (uint8_t)vlog2(parts[k].h);
+      t.mts_idx = 0;
+      t.flags = (uint8_t)((j.flags & VVCB_TU_DEPQUANT) ? (VVCB_TU_QUANT | VVCB_TU_DEPQUANT) : VVCB_TU_QUANT);
+      t.qp_per = j.qp_per; t.qp_rem = j.qp_rem;
+      t.offset = (uint32_t)(cs + (size_t)k * parts[k].w * parts[k].h);
+      t.rate_idx = (uint16_t)i;                        // the candidate's own carried snapshot
+      t.lambda = j.lambda;
+      trPair[(size_t)k * n + i] = (uint8_t)(parts[k].tr_hor | parts[k].tr_ver << 2);
+    }
+    cs += (size_t)cuW * cuH;
+  }
+  if (checkOnly) return VVCB_OK;
+  // per-step work lists (all host-known: the values change, the shapes do not)
+  std::vector<int> predList[5], team[4], dqOrder[4], rateOrder[4];
+  int nSmall[4] = { 0, 0, 0, 0 };
+  for (int k = 0; k <= 4; k++)
+    for (int i = 0; i < n; i++) if (cands[i].nParts > k || (k > 0 && cands[i].nParts == k)) predList[k].push_back(i);
+  for (int k = 0; k < 4; k++) {
+    std::vector<int> large, bySize[9];
+    for (int i = 0; i < n; i++) {
+      if (cands[i].nParts <= k) continue;
+      const vvcb_tu_job& t = tj[(size_t)k * n + i];
+      if (t.log2w + t.log2h <= 8) team[k].push_back(i); else large.push_back(i);
+      if (jobs[i].flags & VVCB_TU_DEPQUANT) dqOrder[k].push_back(i);
+      if (jobs[i].flags & (VVCB_TU_DEPQUANT | VVCB_TU_RATE)) bySize[t.log2w + t.log2h - 4].push_back(i);
+    }
+    nSmall[k] = (int)team[k].size();
+    team[k].insert(team[k].end(), large.begin(), large.end());
+    for (int c = 8; c >= 0; c--) rateOrder[k].insert(rateOrder[k].end(), bySize[c].begin(), bySize[c].end());
+  }
+  // one input arena in page-locked memory: candidates, TU jobs, transform pairs, cbf state, carried models, lists
+  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+  size_t o = 0;
+  auto take = [&](size_t b) { const size_t at = o; o += up16(b); return at; };
+  const size_t iCand = take((size_t)n * sizeof(IspCand)), iJobs = take(tj.size() * sizeof(vvcb_tu_job)), iTr = take(trPair.size()),
+               iState = take((size_t)n * sizeof(IspState)), iCst = take((size_t)n * sizeof(vvcb_ctx_states));
+  size_t iPred[5], iTeam[4], iDq[4], iRate[4];
+  for (int k = 0; k <= 4; k++) iPred[k] = take(predList[k].size() * sizeof(int));
+  for (int k = 0; k < 4; k++) { iTeam[k] = take(team[k].size() * sizeof(int)); iDq[k] = take(dqOrder[k].size() * sizeof(int)); iRate[k] = take(rateOrder[k].size() * sizeof(int)); }
+  const size_t inBytes = o;
+  int rc;
+  if ((rc = pin_buf(ctx, 6, inBytes))) return rc;
+  uint8_t* hin = static_cast<uint8_t*>(ctx->hPin[6]);
+  memcpy(&hin[iCand], cands.data(), (size_t)n * sizeof(IspCand));
+  memcpy(&hin[iJobs], tj.data(), tj.size() * sizeof(vvcb_tu_job));
+  memcpy(&hin[iTr], trPair.data(), trPair.size());
+  memcpy(&hin[iState], ist.data(), (size_t)n * sizeof(IspState));
+  memcpy(&hin[iCst], cst.data(), (size_t)n * sizeof(vvcb_ctx_states));
+  auto put = [&](size_t at, const std::vector<int>& v) { if (!v.empty()) memcpy(&hin[at], v.data(), v.size() * sizeof(int)); };
+  for (int k = 0; k <= 4; k++) put(iPred[k], predList[k]);
+  for (int k = 0; k < 4; k++) { put(iTeam[k], team[k]); put(iDq[k], dqOrder[k]); put(iRate[k], rateOrder[k]); }
+  // work arena: per-step TU results, prediction, residual, reconstruction, levels, dequantised coefficients, derived prices
+  o = 0;
+  const size_t oRes = take((size_t)4 * n * sizeof(vvcb_tu_result)), oPred = take(cs * sizeof(int16_t)), oResi = take(cs * sizeof(int16_t)),
+               oReco = take(cs * sizeof(int16_t)), oLevel = take(cs * sizeof(int32_t)), oDeq = take(cs * sizeof(int32_t)),
+               oRates = take((size_t)n * sizeof(vvcb_dq_rates));
+  const size_t workBytes = o;
+  auto dq_grid = [&](int nDq) { const int g = nDq <= 2048 ? (nDq + kDqThreads / 32 - 1) / (kDqThreads / 32) : (nDq + kDqGroups - 1) / kDqGroups; return std::min(g, ctx->numSms * 4); };
+  int maxDq = 0, maxDqGrid = 0;                                      // the grid is not monotonic in the job count (sparse below 2049 jobs)
+  for (int k = 0; k < 4; k++) { maxDq = std::max(maxDq, (int)dqOrder[k].size()); maxDqGrid = std::max(maxDqGrid, dq_grid((int)dqOrder[k].size())); }
+  CK(cudaSetDevice(ctx->device));
+  if ((rc = tu_buf(ctx, 22, inBytes))) return rc;
+  if ((rc = tu_buf(ctx, 23, workBytes))) return rc;
+  if ((rc = tu_buf(ctx, 7, cs * sizeof(int32_t)))) return rc;
+  if (maxDq) {
+    if ((rc = tu_buf(ctx, 11, (size_t)n * sizeof(DqRateTab)))) return rc;
+    if ((rc = tu_buf(ctx, 12, (size_t)maxDqGrid * kDqGroups * kDqSlotBytes))) return rc;
+    if ((rc = tu_buf(ctx, 13, ((size_t)maxDq * 3 + kDqBins) * sizeof(int)))) return rc;
+  }
+  uint8_t* din = static_cast<uint8_t*>(ctx->dTu[22]);
+  uint8_t* dw = static_cast<uint8_t*>(ctx->dTu[23]);
+  CK(cudaMemcpyAsync(din, hin, inBytes, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(dw + oLevel, 0, oRates - oLevel, ctx->stream));        // levels / dequantised coefficients the quantisers do not reach stay zero
+  const IspCand* dCand = reinterpret_cast<const IspCand*>(din + iCand);
+  vvcb_tu_job* dJobs = reinterpret_cast<vvcb_tu_job*>(din + iJobs);
+  const uint8_t* dTr = din + iTr;
+  IspState* dState = reinterpret_cast<IspState*>(din + iState);
+  vvcb_ctx_states* dCst = reinterpret_cast<vvcb_ctx_states*>(din + iCst);
+  vvcb_tu_result* dRes = reinterpret_cast<vvcb_tu_result*>(dw + oRes);
+  int16_t* dPred = reinterpret_cast<int16_t*>(dw + oPred); int16_t* dResi = reinterpret_cast<int16_t*>(dw + oResi);
+  int16_t* dReco = reinterpret_cast<int16_t*>(dw + oReco);
+  int32_t* dLevel = reinterpret_cast<int32_t*>(dw + oLevel); int32_t* dDeq = reinterpret_cast<int32_t*>(dw + oDeq);
+  vvcb_dq_rates* dRates = reinterpret_cast<vvcb_dq_rates*>(dw + oRates);
+  const bool tm = ctx->timing != 0;
+  struct Events {                                    // per-stage timing of the steps (vvcb_tu_kernel_times); destroyed on every exit
+    cudaEvent_t e[5 * 4] = {};
+    ~Events() { for (auto& x : e) if (x) cudaEventDestroy(x); }
+  } tev;
+  cudaEvent_t* ev = tev.e;
+  if (tm) for (auto& e : tev.e) CK(cudaEventCreate(&e));
+  for (int k = 0; k <= 4; k++) {
+    if (tm && k < 4) CK(cudaEventRecord(ev[5 * k], ctx->stream));
+    if (!predList[k].empty()) {
+      IspPredParams Q;
+      Q.cands = dCand; Q.list = reinterpret_cast<const int*>(din + iPred[k]); Q.n = (int)predList[k].size(); Q.k = k;
+      Q.jobs = dJobs + (size_t)(k < 4 ? k : 3) * n; Q.prev = dRes + (size_t)(k > 0 ? k - 1 : 0) * n; Q.state = dState;
+      Q.pred = dPred; Q.resi = dResi; Q.cuReco = dReco; Q.orig = ctx->bOrig; Q.reco = ctx->bReco; Q.stride = ctx->stride; Q.bd = ctx->bd;
+      Q.rom = ctx->dRom; Q.frac = ctx->dRateRom->binFracBits;
+      const int g = std::min((Q.n + kIspPredWarps - 1) / kIspPredWarps, ctx->numSms * 8);
+      isp_pred_kernel<<<g, kIspPredWarps * 32, 0, ctx->stream>>>(Q);
+      ctx->launches++;
+    }
+    if (k == 4 || team[k].empty()) continue;
+    const int nTeam = (int)team[k].size(), nS = nSmall[k], nL = nTeam - nS, nDq = (int)dqOrder[k].size(), nRate = (int)rateOrder[k].size();
+    const int* dTeam = reinterpret_cast<const int*>(din + iTeam[k]);
+    TuParams P;
+    P.jobs = dJobs + (size_t)k * n; P.list = nullptr; P.n = 0; P.resi = dResi; P.pred = dPred; P.coeff = nullptr; P.level = dLevel; P.reco = dReco;
+    P.results = dRes + (size_t)k * n; P.orig = ctx->bOrig; P.stride = ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
+    P.dqCoeff = static_cast<int32_t*>(ctx->dTu[7]); P.dqDeq = dDeq; P.phase = 0; P.trPair = dTr + (size_t)k * n;
+    auto launch_tu = [&](TuParams Q) {
+      if (nS) { Q.list = dTeam; Q.n = nS; tu_eval_kernel<32><<<std::min((nS + 3) / 4, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
+      if (nL) { Q.list = dTeam + nS; Q.n = nL; tu_eval_kernel<128><<<std::min(nL, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
+    };
+    launch_tu(P);
+    if (tm) CK(cudaEventRecord(ev[5 * k + 1], ctx->stream));
+    if (nDq) {
+      const int* dOrder = reinterpret_cast<const int*>(din + iDq[k]);
+      const long long nPrice = (long long)n * kDqRateModels;
+      rates_from_states_kernel<<<(unsigned)((nPrice + 127) / 128), 128, 0, ctx->stream>>>(dCst, n, ctx->dRateRom, dRates);
+      dq_rate_kernel<<<n, 32, 0, ctx->stream>>>(dRates, n, static_cast<DqRateTab*>(ctx->dTu[11]));
+      int* firstRaw = static_cast<int*>(ctx->dTu[13]);
+      int* orderSorted = firstRaw + nDq;
+      int* firstSorted = firstRaw + 2 * nDq;
+      const int firstGrid = std::min((nDq + kDqGroups - 1) / kDqGroups, ctx->numSms * 8);
+      dq_first_kernel<<<firstGrid, kDqThreads, 0, ctx->stream>>>(P.jobs, dOrder, nDq, P.dqCoeff, ctx->dDqRom, ctx->bd, firstRaw);
+      ctx->launches += 3;
+      const bool sortJobs = nDq > 2048;                            // as tu_eval_impl: sweeps sort by first test position, walks do not
+      if (sortJobs) {
+        int* binCount = firstRaw + 3 * (size_t)nDq;
+        const int sortGrid = (nDq + kDqSortPerBlock - 1) / kDqSortPerBlock;
+        CK(cudaMemsetAsync(binCount, 0, kDqBins * sizeof(int), ctx->stream));
+        dq_hist_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(firstRaw, nDq, binCount);
+        dq_scan_kernel<<<1, 32, 0, ctx->stream>>>(binCount);
+        dq_scatter_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(dOrder, firstRaw, nDq, binCount, orderSorted, firstSorted);
+        ctx->launches += 3;
+      }
+      DqParams D;
+      D.jobs = P.jobs; D.order = sortJobs ? orderSorted : dOrder; D.firstPos = sortJobs ? firstSorted : firstRaw; D.n = nDq;
+      D.coeff = P.dqCoeff; D.level = P.level; D.deq = dDeq; D.results = P.results;
+      D.rates = dRates; D.tabs = static_cast<const DqRateTab*>(ctx->dTu[11]);
+      D.rom = ctx->dDqRom; D.scratch = static_cast<uint8_t*>(ctx->dTu[12]); D.bd = ctx->bd; D.sparse = !sortJobs;
+      dq_kernel<<<dq_grid(nDq), kDqThreads, 0, ctx->stream>>>(D);
+      ctx->launches++;
+    }
+    if (tm) CK(cudaEventRecord(ev[5 * k + 2], ctx->stream));
+    if (nDq) { P.phase = 1; launch_tu(P); }
+    if (tm) CK(cudaEventRecord(ev[5 * k + 3], ctx->stream));
+    if (nRate) {
+      RateParams R;
+      R.jobs = P.jobs; R.order = reinterpret_cast<const int*>(din + iRate[k]); R.n = nRate; R.level = P.level; R.results = P.results;
+      R.states = dCst; R.statesOut = dCst; R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
+      rate_kernel<<<std::min((nRate + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
+      ctx->launches++;
+    }
+    if (tm) CK(cudaEventRecord(ev[5 * k + 4], ctx->stream));
+  }
+  CK(cudaGetLastError());
+  // page-locked output staging: per-step results, cbf state, then the wanted sample outputs of the chunk's densely packed candidates
+  o = 0;
+  const size_t hRes = take((size_t)4 * n * sizeof(vvcb_tu_result)), hSt = take((size_t)n * sizeof(IspState)),
+               hLv = take(level ? cs * sizeof(int32_t) : 0), hRc = take(reco ? cs * sizeof(int16_t) : 0), hPr = take(pred ? cs * sizeof(int16_t) : 0);
+  if ((rc = pin_buf(ctx, 7, o))) return rc;
+  uint8_t* hout = static_cast<uint8_t*>(ctx->hPin[7]);
+  CK(cudaMemcpyAsync(hout + hRes, dRes, (size_t)4 * n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(hout + hSt, dState, (size_t)n * sizeof(IspState), cudaMemcpyDeviceToHost, ctx->stream));
+  if (level) CK(cudaMemcpyAsync(hout + hLv, dLevel, cs * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (reco) CK(cudaMemcpyAsync(hout + hRc, dReco, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (pred) CK(cudaMemcpyAsync(hout + hPr, dPred, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(ctx_sync(ctx));
+  const vvcb_tu_result* res = reinterpret_cast<const vvcb_tu_result*>(hout + hRes);
+  memcpy(ist.data(), hout + hSt, (size_t)n * sizeof(IspState));
+  for (int i = 0; i < n; i++) {                      // each candidate's samples to the caller's offset
+    const size_t from = cands[i].offset, to = jobs[i].offset, m = (size_t)cands[i].cuW * cands[i].cuH;
+    if (level) memcpy(level + to, reinterpret_cast<const int32_t*>(hout + hLv) + from, m * sizeof(int32_t));
+    if (reco) memcpy(reco + to, reinterpret_cast<const int16_t*>(hout + hRc) + from, m * sizeof(int16_t));
+    if (pred) memcpy(pred + to, reinterpret_cast<const int16_t*>(hout + hPr) + from, m * sizeof(int16_t));
+  }
+  if (tm) {
+    for (int k = 0; k < 4; k++) {
+      if (team[k].empty()) continue;
+      for (int i = 0; i < 4; i++) { float ms = 0; CK(cudaEventElapsedTime(&ms, ev[5 * k + i], ev[5 * k + i + 1])); ctx->tuMs[i] += ms; }
+    }
+    ctx->tuTimed++;
+  }
+  for (int i = 0; i < n; i++) {
+    vvcb_isp_result& r = results[i];
+    memset(&r, 0, sizeof(r));
+    const int np = cands[i].nParts;
+    r.n_parts = (uint8_t)np;
+    for (int k = 0; k < np; k++) {
+      r.part[k] = res[(size_t)k * n + i];
+      if (!(jobs[i].flags & VVCB_TU_RATE)) r.part[k].frac_bits = 0;
+      r.cbf_bits[k] = ist[i].cbfBits[k];
+      r.cbf[k] = ist[i].cbf[k];
+    }
+    r.discarded = !ist[i].anyCbf;                                    // the last cbf was inferred (1) but that block has no level either
+  }
+  return VVCB_OK;
+}
+
+extern "C" int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, const vvcb_isp_job* jobs, int n,
+                             const vvcb_ctx_states* states, int n_states, size_t n_samples,
+                             int32_t* level, int16_t* reco, int16_t* pred, vvcb_isp_result* results)
+{
+  if (!ctx) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_isp_eval");
+  if (n < 0 || n_states < 0 || (n > 0 && (!jobs || !results || !visits || n_visits <= 0))) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_isp_eval: bad argument"); return VVCB_ERR_ARG; }
+  if (n == 0) return VVCB_OK;
+  if (!ctx->bOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_isp_eval: vvcb_frame_begin has not been called"); return VVCB_ERR_STATE; }
+  const int rcv = check_visits(ctx, visits, n_visits);
+  if (rcv) return rcv;
+  for (int pass = 0; pass < 2; pass++)                               // every job is validated before anything runs
+    for (int b = 0; b < n; b += kIspChunk) {
+      const int rc = isp_eval_chunk(ctx, visits, n_visits, jobs + b, std::min(kIspChunk, n - b), b, states, n_states, n_samples,
+                                    level, reco, pred, results + b, pass == 0);
+      if (rc) return rc;
+    }
+  return VVCB_OK;
+}
+
 static int feat_buf(vvcb_ctx* ctx, int i, size_t bytes)
 {
   if (bytes > ctx->capFeat[i]) {

@@ -21,6 +21,8 @@ struct RateParams {
   const DqRom* rom;
   const RateRom* rate;
   int depQuant;              // slice->getDepQuantEnabledFlag(): selects the state machine that picks the significance context set
+  vvcb_ctx_states* statesOut = nullptr;   // optional: statesOut[job index] receives the models as the TU has left them (unchanged for an all-zero
+                                          // TU); may be `states` itself when every job has a rate_idx of its own (vvcb_isp_eval)
 };
 
 struct RateEst {
@@ -112,7 +114,15 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
       for (int u = 3; u >= 0; u--) if (idx[u] >= 0 && coeff[idx[u]] != 0) best = base - 32 * u - lane;
       scanPosLast = __reduce_max_sync(0xffffffffu, best);
     }
-    if (scanPosLast < 0) { if (lane == 0) P.results[ji].frac_bits = 0; continue; }
+    if (scanPosLast < 0) {
+      if (lane == 0) P.results[ji].frac_bits = 0;
+      if (P.statesOut) {
+        const vvcb_bin_model* src = reinterpret_cast<const vvcb_bin_model*>(&P.states[job.rate_idx]);
+        vvcb_bin_model* dst = reinterpret_cast<vvcb_bin_model*>(&P.statesOut[ji]);
+        for (int i = lane; i < kRateModels; i += 32) dst[i] = src[i];
+      }
+      continue;
+    }
 
     {                                                            // this TU's private copy of the context models
       const vvcb_bin_model* src = reinterpret_cast<const vvcb_bin_model*>(&P.states[job.rate_idx]);
@@ -310,7 +320,34 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
       }
     }
     __syncwarp();
+    if (P.statesOut) {
+      vvcb_bin_model* dst = reinterpret_cast<vvcb_bin_model*>(&P.statesOut[ji]);
+      for (int i = lane; i < kRateModels; i += 32) {
+        vvcb_bin_model m;
+        m.state[0] = (uint16_t)(models[i].st & 0xffffu); m.state[1] = (uint16_t)(models[i].st >> 16);
+        m.rate = (uint8_t)models[i].rate; m.pad = 0;
+        dst[i] = m;
+      }
+      __syncwarp();
+    }
   }
+}
+
+// vvcb_dq_rates (BinFracBits::intBits of each context, BinProbModel_Std::getFracBitsArray, CL/Contexts.h) of carried model states: the
+// dependent quantiser of an ISP block is priced from the models as the previous block of its CU left them.  The two structs list the
+// same contexts in the same order, vvcb_ctx_states with the MTS index contexts in front.  One thread per (snapshot, context).
+constexpr int kDqRateModels = (int)(sizeof(vvcb_dq_rates) / (2 * sizeof(uint32_t)));
+static_assert(kDqRateModels == kRateModels - 11, "vvcb_dq_rates lists the contexts of vvcb_ctx_states behind mts_idx[11]");
+
+__global__ void __launch_bounds__(128) rates_from_states_kernel(const vvcb_ctx_states* states, int n, const RateRom* rom, vvcb_dq_rates* out)
+{
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (long long)n * kDqRateModels) return;
+  const int s = (int)(t / kDqRateModels), i = (int)(t % kDqRateModels);
+  const vvcb_bin_model m = reinterpret_cast<const vvcb_bin_model*>(&states[s])[11 + i];
+  const int q = ((int)m.state[0] + (int)m.state[1]) >> 8;
+  uint32_t* dst = reinterpret_cast<uint32_t*>(&out[s]) + 2 * i;
+  dst[0] = rom->binFracBits[2 * q]; dst[1] = rom->binFracBits[2 * q + 1];
 }
 
 }  // namespace

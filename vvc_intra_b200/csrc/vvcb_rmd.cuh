@@ -1036,6 +1036,187 @@ __global__ void __launch_bounds__(kTuPredWarps * 32) tu_pred_kernel(TuPredParams
   }
 }
 
+// =====================================================================================================
+// intra sub-partitions (vvcb_isp_eval): prediction of block k of every candidate, one warp per candidate
+// =====================================================================================================
+// A candidate is one ISP CU x split x luma mode x quantiser setting; its blocks (2 or 4, all of one size, at least 4x4) are coded in
+// order and block k is predicted from the reconstruction of block k-1 (EL/IntraSearch.cpp:3171 xIntraCodingLumaISP).  The reference
+// builds the lines of block k > 0 by shifting the side it holds and re-fetching the line block k-1 has just reconstructed
+// (initIntraPatternChTypeISP, CL/IntraPrediction.cpp:1136-1203).  This kernel makes the equivalent fresh fetch: the same padding walk as
+// make_line_geom, with the lengths m_topRefLength / m_leftRefLength of the block and availability derived from the CU's -- which agrees
+// with the shift for all-or-nothing left and above neighbours only (vvcb_isp_eval refuses the rest).  Samples inside the CU come from the
+// candidate's own reconstruction buffer, the others from the picture.
+struct IspCand {                   // host-built (vvcb_api.cu), one per candidate
+  int16_t x, y, cuW, cuH;          // CU in the picture
+  int16_t bw, bh, topLen, leftLen; // block size, reference-line lengths of every block
+  uint8_t hor, nParts, availAl, nAbove, nAboveRight, nLeft, nBelowLeft, mode;
+  uint32_t offset;                 // first sample of the candidate's blocks (coding order, each dense bw*bh)
+  ModeParam p;                     // make_mode_param_isp
+};
+struct IspState {                  // per candidate, carried from step to step
+  vvcb_bin_model ctx[2];           // Ctx::QtCbf[luma] contexts 2, 3
+  uint32_t cbfBits[4];
+  uint8_t cbf[4], anyCbf, pad[3];
+};
+struct IspPredParams {
+  const IspCand* cands;
+  const int* list; int n;          // candidates with a block k, and (k > 0) those whose last block is k - 1
+  int k;
+  vvcb_tu_job* jobs;               // step k's TU jobs, index = candidate: cbf_delta_bits is written here
+  const vvcb_tu_result* prev;      // step k - 1's results
+  IspState* state;
+  int16_t* pred; int16_t* resi;
+  const int16_t* cuReco;           // candidates' reconstructions (coding order, like pred)
+  const int16_t* orig; const int16_t* reco; int stride, bd;
+  const Rom* rom;
+  const uint32_t* frac;            // ProbModelTables::m_binFracBits
+};
+
+// price and adapt one context-coded bin (TBitEstimator::encodeBin; the same arithmetic as rate_bin, vvcb_rate.cuh)
+__device__ __forceinline__ uint32_t isp_code_bin(vvcb_bin_model& m, const uint32_t* frac, unsigned bin)
+{
+  const unsigned rate0 = m.rate >> 4, rate1 = m.rate & 15, s0 = m.state[0], s1 = m.state[1];
+  const uint32_t bits = frac[2 * ((s0 + s1) >> 8) + bin];
+  unsigned n0 = s0 - ((s0 >> rate0) & 0x7fe0u), n1 = s1 - ((s1 >> rate1) & 0x7ffeu);
+  if (bin) { n0 += (0x7fffu >> rate0) & 0x7fe0u; n1 += (0x7fffu >> rate1) & 0x7ffeu; }
+  m.state[0] = (uint16_t)n0; m.state[1] = (uint16_t)n1;
+  return bits;
+}
+
+// [lo, hi) clipped to [0, n); empty -> kNoInterval
+__device__ __forceinline__ void isp_interval(int lo, int hi, int n, int& a, int& b)
+{
+  lo = vmax(lo, 0); hi = vmin(hi, n);
+  if (lo < hi) { a = lo; b = hi; } else { a = kNoInterval; b = kNoInterval; }
+}
+
+constexpr int kIspPredWarps = 4;
+
+__global__ void __launch_bounds__(kIspPredWarps * 32) isp_pred_kernel(IspPredParams P)
+{
+  __shared__ WarpSmem smem[kIspPredWarps];
+  __shared__ int16_t sScratch[kIspPredWarps][kSlotLineWords];
+  __shared__ uint32_t sFilt[64];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  WarpSmem& sm = smem[warp];
+  int16_t* const slotBuf = sScratch[warp];
+  if (threadIdx.x < 64) sFilt[threadIdx.x] = (&P.rom->filt[0][0])[threadIdx.x];
+  __syncthreads();
+  const int k = P.k;
+  for (int q = blockIdx.x * kIspPredWarps + warp; q < P.n; q += gridDim.x * kIspPredWarps) {
+    const int c = P.list[q];
+    const IspCand cd = P.cands[c];
+    // ---- cbf of block k - 1, then cbfDeltaBits of block k (RateEstimator::xSetLastCoeffOffset, CL/DepQuant.cpp:491-540, ISP branch):
+    // block j's cbf is coded with context 2 + cbf of block j - 1, except the last block's when every earlier one is 0 (inferred 1)
+    if (lane == 0) {
+      IspState st = P.state[c];
+      if (k > 0) {
+        const int j = k - 1;
+        const unsigned cbf = P.prev[c].abs_sum_level != 0;
+        const bool inferred = j == cd.nParts - 1 && !st.anyCbf;
+        st.cbfBits[j] = inferred ? 0u : isp_code_bin(st.ctx[j ? st.cbf[j - 1] : 0], P.frac, cbf);
+        st.cbf[j] = (uint8_t)cbf;
+        st.anyCbf |= (uint8_t)cbf;
+      }
+      if (k < cd.nParts) {
+        const bool inferred = k == cd.nParts - 1 && !st.anyCbf;
+        const vvcb_bin_model m = st.ctx[k ? st.cbf[k - 1] : 0];
+        const int qs = ((int)m.state[0] + (int)m.state[1]) >> 8;
+        P.jobs[c].cbf_delta_bits = inferred ? 0 : (int32_t)P.frac[2 * qs + 1] - (int32_t)P.frac[2 * qs];
+      }
+      P.state[c] = st;
+    }
+    if (k >= cd.nParts) continue;                                   // finishing pass of a candidate: its last cbf only
+    const bool hor = cd.hor != 0;
+    const int bx = hor ? 0 : k * cd.bw, by = hor ? k * cd.bh : 0, bs = cd.bw * cd.bh;
+    const int T = cd.topLen, L = cd.leftLen;
+    VVCB_EMUL_ASSERT(T + 2 < kLineMax && L + 2 < kLineMax);          // the lines and their two replicated samples fit the line arrays
+    // ---- walk of block k: left[L] .. left[1], corner, top[1] .. top[T]; availability intervals in walk order
+    LineGeom g;
+    g.w = T; g.h = L; g.mrl = 0; g.n = L + 1 + T;
+    int a, b;
+    if (k == 0 || hor) {                                            // the CU's left column, shifted by the block's row
+      isp_interval(cd.cuH - by, cd.cuH + 4 * cd.nBelowLeft - by, L, a, b); g.lo[0] = a == kNoInterval ? a : L - b; g.hi[0] = a == kNoInterval ? a : L - a;
+      isp_interval(-by, 4 * cd.nLeft - by, L, a, b);                   g.lo[1] = a == kNoInterval ? a : L - b; g.hi[1] = a == kNoInterval ? a : L - a;
+    } else {                                                        // vertical split: block k-1's last column, nothing below the CU
+      g.lo[0] = g.hi[0] = kNoInterval;
+      isp_interval(0, cd.cuH, L, a, b);                               g.lo[1] = L - b; g.hi[1] = L - a;
+    }
+    const bool corner = k == 0 ? cd.availAl != 0 : (hor ? by - 1 < 4 * cd.nLeft : bx - 1 < 4 * cd.nAbove);
+    g.lo[2] = corner ? L : kNoInterval; g.hi[2] = corner ? L + 1 : kNoInterval;
+    if (k == 0 || !hor) {                                           // the CU's above row, shifted by the block's column
+      isp_interval(-bx, 4 * cd.nAbove - bx, T, a, b);                  g.lo[3] = a == kNoInterval ? a : L + 1 + a; g.hi[3] = a == kNoInterval ? a : L + 1 + b;
+      isp_interval(cd.cuW - bx, cd.cuW + 4 * cd.nAboveRight - bx, T, a, b); g.lo[4] = a == kNoInterval ? a : L + 1 + a; g.hi[4] = a == kNoInterval ? a : L + 1 + b;
+    } else {                                                        // horizontal split: block k-1's last row, nothing right of the CU
+      isp_interval(0, cd.cuW, T, a, b);                               g.lo[3] = L + 1 + a; g.hi[3] = L + 1 + b;
+      g.lo[4] = g.hi[4] = kNoInterval;
+    }
+    g.first = -1;
+#pragma unroll
+    for (int t = 4; t >= 0; t--) if (g.lo[t] != kNoInterval) g.first = g.lo[t];
+    const int16_t* cuReco = P.cuReco + cd.offset;
+    __syncwarp();
+    // walk positions, then the two replicated samples past each line's end (CL/IntraPrediction.cpp:717-726, refLength = the ISP lengths)
+    for (int i = lane; i < g.n + 4; i += 32) {
+      const int pos = i < g.n ? i : (i < g.n + 2 ? g.n - 1 : 0);
+      const int src = line_source(g, pos);
+      int val = 1 << (P.bd - 1);
+      if (src >= 0) {
+        const int px = src < L ? bx - 1 : (src == L ? bx - 1 : bx + src - L - 1);   // CU frame
+        const int py = src < L ? by + L - 1 - src : by - 1;
+        if (px >= 0 && py >= 0) {                                    // inside the CU: an earlier block of this candidate
+          const int j = hor ? py / cd.bh : px / cd.bw;
+          val = cuReco[j * bs + (py - (hor ? j * cd.bh : 0)) * cd.bw + px - (hor ? 0 : j * cd.bw)];
+        } else val = P.reco[(size_t)(cd.y + py) * P.stride + cd.x + px];
+      }
+      if (i < L) sm.lines[0][1][L - i] = (int16_t)val;
+      else if (i == L) { sm.lines[0][0][0] = (int16_t)val; sm.lines[0][1][0] = (int16_t)val; }
+      else if (i < g.n) sm.lines[0][0][i - L] = (int16_t)val;
+      else if (i < g.n + 2) sm.lines[0][0][T + 1 + i - g.n] = (int16_t)val;
+      else sm.lines[0][1][L + 1 + i - g.n - 2] = (int16_t)val;
+    }
+    __syncwarp();
+    // ---- prediction of the block: the units of tu_pred_kernel, unfiltered lines, cubic interpolation (make_mode_param_isp)
+    const Shape sh = make_shape(vlog2(cd.bw), vlog2(cd.bh));
+    SlotInfo s;
+    s.mode = cd.mode; s.mrl = 0; s.set = 0; s.p = cd.p;
+    s.kind = s.mode == 0 ? 0 : (s.mode == 1 ? 1 : 2);
+    int dc = 0;
+    if (s.kind == 2) {
+      if (s.p.angle < 0) build_projected_line(slotBuf, sm, s, s.p.is_ver ? sh.w : sh.h, s.p.is_ver ? sh.h : sh.w, lane, 32);
+    } else if (s.kind == 1) {
+      int part = 0;
+      const int16_t* top = sm.lines[0][0] + 1;
+      const int16_t* left = sm.lines[0][1] + 1;
+      if (sh.w >= sh.h) for (int i = lane; i < sh.w; i += 32) part += top[i];
+      if (sh.w <= sh.h) for (int i = lane; i < sh.h; i += 32) part += left[i];
+      for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
+      const int denom = sh.w == sh.h ? 2 * sh.w : vmax(sh.w, sh.h);
+      dc = (part + (denom >> 1)) >> vlog2(denom);
+    }
+    __syncwarp();
+    const bool transposed = s.kind == 2 && !s.p.is_ver;
+    const int16_t* org = P.orig + (size_t)(cd.y + by) * P.stride + cd.x + bx;
+    int16_t* predOut = P.pred + cd.offset + k * bs;
+    int16_t* resiOut = P.resi + cd.offset + k * bs;
+    const int piecesX = sh.w >> 2, pieces = (sh.w * sh.h) >> 4;
+    for (int u = lane; u < pieces; u += 32) {
+      const int x0 = (u % piecesX) * 4, y0 = (u / piecesX) * 4;
+      int qv[4][4];
+      if (s.kind == 2) predict_angular<4, 4>(sm, slotBuf, s, sh, sFilt, P.bd, x0, y0, 0, qv);
+      else pred_planar_dc_unit<4, 4>(sm.lines[0][0], sm.lines[0][1], s.kind, s.p.pdpc, dc, sh.lw, sh.lh, x0, y0, qv);
+#pragma unroll
+      for (int i = 0; i < 4; i++)
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+          const int yy = transposed ? y0 + j : y0 + i, xx = transposed ? x0 + i : x0 + j;
+          predOut[yy * sh.w + xx] = (int16_t)qv[i][j];
+          resiOut[yy * sh.w + xx] = (int16_t)(org[yy * P.stride + xx] - qv[i][j]);
+        }
+    }
+  }
+}
+
 // calls F<TILE, KIND, MODE>(args) for launch b = tile class * kNumKinds + kind
 #define VVCB_FOR_BUCKET(b, PACK, F, ...)                                                                    \
   switch (b) {                                                                                               \

@@ -148,6 +148,9 @@ struct TuParams {
   int32_t* dqCoeff;
   const int32_t* dqDeq;
   int phase;
+  // optional explicit transform pair per job (intra sub-partitions, vvcb_isp_eval): VVCB_TR_* of the horizontal transform | vertical << 2,
+  // read instead of mts_idx, which those jobs keep at 0 (implicit selection: no MTS zero-out or MTS rate semantics downstream)
+  const uint8_t* trPair = nullptr;
 };
 
 __device__ __forceinline__ int clip16(int v) { return vmin(vmax(v, -32768), 32767); }
@@ -189,8 +192,9 @@ __global__ void __launch_bounds__(kTuThreads) tu_eval_kernel(TuParams P)
     const vvcb_tu_job job = P.jobs[ji];
     const int lw = job.log2w, lh = job.log2h, w = 1 << lw, h = 1 << lh, n = w * h;
     const bool ts = job.mts_idx == 1;
-    const int hor = job.mts_idx > 1 ? (((job.mts_idx - 2) & 1) ? 1 : 2) : 0;
-    const int ver = job.mts_idx > 1 ? (((job.mts_idx - 2) >> 1) ? 1 : 2) : 0;
+    int hor = job.mts_idx > 1 ? (((job.mts_idx - 2) & 1) ? 1 : 2) : 0;
+    int ver = job.mts_idx > 1 ? (((job.mts_idx - 2) >> 1) ? 1 : 2) : 0;
+    if (P.trPair) { hor = P.trPair[ji] & 3; ver = P.trPair[ji] >> 2; }
     int wKeep = w - ((hor != 0 && w == 32) ? 16 : (w > 32 ? w - 32 : 0));
     int hKeep = h - ((ver != 0 && h == 32) ? 16 : (h > 32 ? h - 32 : 0));
     const LfnstGeom lf = make_lfnst(rom, w, h, lw, lh, ts, job.lfnst_idx, job.intra_mode);

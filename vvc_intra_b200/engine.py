@@ -81,6 +81,14 @@ ISP_PART_DTYPE = np.dtype([('x', '<i2'), ('y', '<i2'), ('w', '<i2'), ('h', '<i2'
 ISP_MODE_DTYPE = np.dtype([('angle', '<i2'), ('inv_angle', '<u2'), ('is_ver', 'u1'), ('pdpc', 'u1'), ('ang_scale', 'i1'), ('pad', 'u1')])
 ISP_HOR, ISP_VER, TR_DCT2, TR_DCT8, TR_DST7 = 1, 2, 0, 1, 2
 assert CU_AUTO_DTYPE.itemsize == 40
+# vvcb_isp_job / vvcb_isp_result (include/vvc_intra_b200.h): one ISP candidate and its per-block results
+ISP_JOB_DTYPE = np.dtype([('visit', '<u4'), ('isp_mode', 'u1'), ('mode', 'u1'), ('flags', 'u1'), ('use_mts', 'u1'), ('max_tb_size', 'u1'),
+                          ('lfnst_idx', 'u1'), ('qp_per', '<i2'), ('qp_rem', '<i2'), ('rate_idx', '<u2'), ('offset', '<u4'),
+                          ('cbf', BIN_MODEL_DTYPE, 2), ('lambda', '<f8')], align=True)
+ISP_MAX_PARTS = 4
+ISP_RESULT_DTYPE = np.dtype([('part', TU_RESULT_DTYPE, ISP_MAX_PARTS), ('cbf_bits', '<u4', ISP_MAX_PARTS), ('cbf', 'u1', ISP_MAX_PARTS),
+                             ('n_parts', 'u1'), ('discarded', 'u1'), ('pad', 'u1', 2)], align=True)
+assert ISP_JOB_DTYPE.itemsize == 40 and ISP_RESULT_DTYPE.itemsize == 120
 AUTO_FINAL, AUTO_REGULAR = 1, 2
 
 
@@ -139,6 +147,8 @@ def load_library():
         L.vvcb_calc_rd_cost.restype = C.c_double
         L.vvcb_isp_plan.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
         L.vvcb_isp_mode_param.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
+        L.vvcb_isp_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.vvcb_ctu_hads_islice.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.vvcb_features_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.vvcb_frame_bind_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
@@ -400,6 +410,23 @@ class IntraCostEngine:
         self._ck(self._lib.vvcb_tu_eval_pred(self._ctx, _ptr(visits), len(visits), _ptr(src), _ptr(jobs), len(jobs), n_samples,
                                              _ptr(rates) if rates is not None else None, _ptr(states) if states is not None else None, nr,
                                              p('coeff'), p('level'), p('reco'), p('pred'), _ptr(out['results'])))
+        return out
+
+    def isp_eval(self, visits, jobs, n_samples, states=None, want_level=False, want_reco=False, want_pred=False):
+        """vvcb_isp_eval: ISP candidates (ISP_JOB_DTYPE) of the CUs in visits, blocks of at least 4x4.  states: CTX_STATES_DTYPE
+        array indexed by job['rate_idx'].  Returns dict with 'results' (ISP_RESULT_DTYPE) and the wanted flat outputs of n_samples,
+        each candidate's blocks in coding order at job['offset']."""
+        visits = np.ascontiguousarray(visits, VISIT_DTYPE)
+        jobs = np.ascontiguousarray(jobs, ISP_JOB_DTYPE)
+        states = None if states is None else np.ascontiguousarray(states, CTX_STATES_DTYPE)
+        out = dict(results=np.zeros(len(jobs), ISP_RESULT_DTYPE))
+        for key, want, dt in (('level', want_level, np.int32), ('reco', want_reco, np.int16), ('pred', want_pred, np.int16)):
+            if want:
+                out[key] = np.zeros(n_samples, dt)
+        p = lambda k: _ptr(out[k]) if k in out else None
+        self._ck(self._lib.vvcb_isp_eval(self._ctx, _ptr(visits), len(visits), _ptr(jobs), len(jobs),
+                                         _ptr(states) if states is not None else None, 0 if states is None else len(states), n_samples,
+                                         p('level'), p('reco'), p('pred'), _ptr(out['results'])))
         return out
 
     def residual_bits(self, jobs, levels, states):
