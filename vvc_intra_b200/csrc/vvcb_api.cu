@@ -12,6 +12,7 @@
 #include "vvcb_dq.cuh"
 #include "vvcb_rate.cuh"
 #include <vector>
+#include <algorithm>
 #include <time.h>
 #include <thread>
 #include <atomic>
@@ -48,14 +49,23 @@ __global__ void __launch_bounds__(256) int_peak_kernel(const int* in, int* out, 
 // C ABI
 // =====================================================================================================
 constexpr int kSideStreams = 7;
+// Scratch slots of a context: device (vvcb_ctx::dTu, tu_buf) and page-locked (vvcb_ctx::hPin, pin_buf).  The stage-1 arenas of
+// vvcb_cu_eval and the arenas of vvcb_isp_eval share kStageIn / kStageOut: a context serves one call at a time.
+enum TuSlot {
+  kTuIn, kTuOut,                 // tu_eval_impl / vvcb_residual_bits: inputs from the host, outputs (+ dequantised coefficients)
+  kTuResi, kTuCoeff,             // residual, transform coefficients (vvcb_tu_eval's want_coeff)
+  kDqCoeff, kDqTabs, kDqScratch, kDqLists,   // quantiser scratch (quant_scratch)
+  kStageIn, kStageOut,
+  kTuSlots
+};
+enum PinSlot { kPinTuIn, kPinTuOut, kPinStageIn, kPinStageOut, kPinSlots };
 struct vvcb_ctx {
   int device, bd, ctu;
   cudaStream_t stream;
   cudaEvent_t ev0, ev1;
   Rom* dRom;
   TrRom* dTrRom;
-  void* dTu[24]; size_t capTu[24];  // TU scratch: jobs, resi, pred, coeff, level, reco, results; DepQuant: coeff in, dequantised out,
-                                    // job order, context prices, derived rate tables, per-group context memory + trellis
+  void* dTu[kTuSlots]; size_t capTu[kTuSlots];
   DqRom* dDqRom;
   RateRom* dRateRom;
   int depQuant;                     // slice->getDepQuantEnabledFlag() (vvcb_set_option), 1 = the shipped configuration
@@ -83,7 +93,7 @@ struct vvcb_ctx {
   int16_t* wReco;                   // writable reconstruction plane: own (dReco) or another context's (vvcb_frame_share)
   int yieldSync; cudaEvent_t evYield;   // VVCB_OPT_YIELD_SYNC
   void* remote;                     // broker client proxy: VVCB_BROKER was set at vvcb_create (vvcb_broker.inc)
-  void* hPin[10]; size_t capPin[10];  // page-locked staging of vvcb_cu_eval / vvcb_reco_update_rects
+  void* hPin[kPinSlots]; size_t capPin[kPinSlots];
   void* dRect[2]; size_t capRect[2];
   uint64_t launches;
   uint64_t cuNs[8], cuCalls, tuWaitFrom;    // vvcb_cu_eval_phases
@@ -227,11 +237,11 @@ extern "C" void vvcb_destroy(vvcb_ctx* ctx)
   if (ctx->remote) { vvcbc_disconnect(ctx->remote); delete ctx; return; }
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  for (int i = 0; i < 10; i++) if (ctx->hPin[i]) cudaFreeHost(ctx->hPin[i]);
+  for (int i = 0; i < kPinSlots; i++) if (ctx->hPin[i]) cudaFreeHost(ctx->hPin[i]);
   cudaFree(ctx->dRect[0]); cudaFree(ctx->dRect[1]); cudaFree(ctx->dBrief);
   cudaFree(ctx->dRom); cudaFree(ctx->dOrig); cudaFree(ctx->dReco); cudaFree(ctx->dVisits); cudaFree(ctx->dResults); cudaFree(ctx->dDetails); cudaFree(ctx->dScratch);
   cudaFree(ctx->dItems); cudaFree(ctx->dPlan); cudaFree(ctx->dPred); cudaFree(ctx->dTrRom);
-  for (int i = 0; i < 24; i++) cudaFree(ctx->dTu[i]);
+  for (int i = 0; i < kTuSlots; i++) cudaFree(ctx->dTu[i]);
   cudaFree(ctx->dRateRom);
   cudaFree(ctx->dDqRom);
   for (int i = 0; i < 2; i++) cudaFree(ctx->dFeat[i]);
@@ -358,7 +368,7 @@ extern "C" int vvcb_orig_update(vvcb_ctx* ctx, const int16_t* orig, int stride, 
 }
 
 // page-locked staging buffer i of at least `bytes`
-static int pin_buf(vvcb_ctx* ctx, int i, size_t bytes)
+static int pin_buf(vvcb_ctx* ctx, PinSlot i, size_t bytes)
 {
   if (bytes > ctx->capPin[i]) {
     if (ctx->hPin[i]) cudaFreeHost(ctx->hPin[i]);
@@ -369,6 +379,13 @@ static int pin_buf(vvcb_ctx* ctx, int i, size_t bytes)
   }
   return VVCB_OK;
 }
+
+// Layout of one arena of several arrays: take() returns the next array's offset, 16-byte aligned (the kernels' widest access, uint4).
+struct Arena {
+  size_t size = 0;
+  size_t take(size_t bytes) { const size_t at = size; size += (bytes + 15) & ~(size_t)15; return at; }
+};
+template <class T> static T* at(void* base, size_t offset) { return reinterpret_cast<T*>(static_cast<uint8_t*>(base) + offset); }
 
 // one CTA per rectangle: dense w*h block -> the reconstruction plane
 __global__ void __launch_bounds__(128) reco_scatter_kernel(const vvcb_rect* __restrict__ rects, int n, const int16_t* __restrict__ samples, int16_t* __restrict__ plane, int stride)
@@ -914,13 +931,166 @@ static cudaError_t arena_copy(vvcb_ctx* ctx, const void* src, void* dst, size_t 
   return cudaGetLastError();
 }
 
-static int tu_buf(vvcb_ctx* ctx, int i, size_t bytes)
+static int tu_buf(vvcb_ctx* ctx, TuSlot i, size_t bytes)
 {
   if (bytes > ctx->capTu[i]) {
     cudaFree(ctx->dTu[i]); ctx->dTu[i] = nullptr; ctx->capTu[i] = 0;
     CK(cudaMalloc(&ctx->dTu[i], bytes));
     ctx->capTu[i] = bytes;
   }
+  return VVCB_OK;
+}
+
+// The counting sort of the dependent quantiser's jobs by first test position buys warp efficiency for sweeps (eight TUs per warp walk
+// scans of equal length); a walk's batch of a few dozen candidates is latency bound, skips its three launches and runs one TU per warp.
+constexpr int kDqSortAbove = 2048;
+
+static int dq_grid(const vvcb_ctx* ctx, int nDq)
+{
+  const int g = nDq <= kDqSortAbove ? (nDq + kDqThreads / 32 - 1) / (kDqThreads / 32) : (nDq + kDqGroups - 1) / kDqGroups;
+  return std::min(g, ctx->numSms * 4);
+}
+
+// Quantiser scratch of one call whose batches hold `samples` samples, nRates price sets and nDq[0..steps) dependent-quantiser jobs:
+// pass 0's coefficients, the derived rate tables, per-group context memory + trellis, the first-position / sort lists.  Sized once per
+// call, before its first batch: a buffer that grew between two batches would be freed under the previous one's kernels.
+static int quant_scratch(vvcb_ctx* ctx, size_t samples, int nRates, const int* nDq, int steps)
+{
+  int maxDq = 0, maxGrid = 0;                                       // the grid is not monotonic in the job count (sparse, kDqSortAbove)
+  for (int k = 0; k < steps; k++) { maxDq = std::max(maxDq, nDq[k]); maxGrid = std::max(maxGrid, dq_grid(ctx, nDq[k])); }
+  int rc;
+  if ((rc = tu_buf(ctx, kDqCoeff, samples * sizeof(int32_t)))) return rc;
+  if (!maxDq) return VVCB_OK;
+  if ((rc = tu_buf(ctx, kDqTabs, (size_t)nRates * sizeof(DqRateTab)))) return rc;
+  if ((rc = tu_buf(ctx, kDqScratch, (size_t)maxGrid * kDqGroups * kDqSlotBytes))) return rc;
+  return tu_buf(ctx, kDqLists, ((size_t)maxDq * 3 + kDqBins) * sizeof(int));
+}
+
+// job indices of bySize[log2w + log2h - 4], largest TU first
+static std::vector<int> largest_first(const std::vector<int> (&bySize)[9])
+{
+  std::vector<int> out;
+  for (int c = 8; c >= 0; c--) out.insert(out.end(), bySize[c].begin(), bySize[c].end());
+  return out;
+}
+
+// Host work lists of one TU batch over the jobs i < n with part(i):
+// - team: the job list of tu_eval_kernel, the nSmall blocks of up to 256 samples (one warp each) first, then the larger ones;
+// - dq: the dependent quantiser's jobs (sorted on the device by scan length once the coefficients exist);
+// - ts: the transform-skip RDOQ jobs, largest block first (one thread per block: equal chain lengths per warp);
+// - rate: the VVCB_TU_RATE jobs, whose residual bits are wanted, largest TU first.
+struct TuLists { std::vector<int> team, dq, ts, rate; int nSmall; };
+
+template <class Part> static TuLists tu_lists(const vvcb_tu_job* jobs, int n, Part part)
+{
+  TuLists L;
+  L.team.reserve(n); L.dq.reserve(n);
+  std::vector<int> large, tsBySize[9], rateBySize[9];
+  for (int i = 0; i < n; i++) {
+    if (!part(i)) continue;
+    const vvcb_tu_job& j = jobs[i];
+    const int c = j.log2w + j.log2h - 4;
+    const bool q = (j.flags & VVCB_TU_QUANT) != 0;
+    (c <= 4 ? L.team : large).push_back(i);
+    if (q && (j.flags & VVCB_TU_DEPQUANT)) L.dq.push_back(i);
+    else if (q && (j.flags & VVCB_TU_RDOQ_TS)) tsBySize[c].push_back(i);
+    if (q && (j.flags & VVCB_TU_RATE)) rateBySize[c].push_back(i);
+  }
+  L.nSmall = (int)L.team.size();
+  L.team.insert(L.team.end(), large.rbegin(), large.rend());
+  L.ts = largest_first(tsBySize);
+  L.rate = largest_first(rateBySize);
+  return L;
+}
+
+// Device pointers of one TU batch (counts: its TuLists).  The quantiser scratch comes from quant_scratch.
+struct TuChain {
+  const vvcb_tu_job* jobs;
+  const uint8_t* trPair;                                            // optional explicit transform pair per job (TuParams)
+  const int *team, *dq, *ts, *rate;                                 // the TuLists
+  const int16_t *resi, *pred;
+  int32_t* coeff; int32_t* level; int16_t* reco; int32_t* deq; vvcb_tu_result* results;   // coeff, reco optional
+  vvcb_dq_rates* rates; int nRates;                                 // quantiser prices
+  const vvcb_ctx_states* priceFrom;                                 // optional: rates_from_states_kernel fills `rates` from these models first
+  const vvcb_ctx_states* states; vvcb_ctx_states* statesOut;        // rate_kernel's models; statesOut optional
+};
+
+// Launches one TU batch: tu_eval_kernel pass 0 in its two team sizes, the dependent quantiser and / or transform-skip RDOQ, pass 1 for
+// the jobs they quantised, rate_kernel.  ev (optional): ev[1..4] are recorded after pass 0, the quantisers, pass 1 and rate_kernel.
+static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const cudaEvent_t* ev)
+{
+  const int nSmall = L.nSmall, nLarge = (int)L.team.size() - nSmall, nDq = (int)L.dq.size(), nTs = (int)L.ts.size(), nRate = (int)L.rate.size();
+  TuParams P;
+  P.jobs = c.jobs; P.list = nullptr; P.n = 0; P.resi = c.resi; P.pred = c.pred; P.coeff = c.coeff; P.level = c.level; P.reco = c.reco;
+  P.results = c.results; P.orig = ctx->bOrig; P.stride = ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
+  P.dqCoeff = static_cast<int32_t*>(ctx->dTu[kDqCoeff]); P.dqDeq = c.deq; P.phase = 0; P.trPair = c.trPair;
+  auto launch_tu = [&](TuParams Q) {
+    if (nSmall) { Q.list = c.team; Q.n = nSmall; tu_eval_kernel<32><<<std::min((nSmall + 3) / 4, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
+    if (nLarge) { Q.list = c.team + nSmall; Q.n = nLarge; tu_eval_kernel<128><<<std::min(nLarge, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
+  };
+  launch_tu(P);
+  if (ev) CK(cudaEventRecord(ev[1], ctx->stream));
+  // transform-skip RDOQ and dependent quantisation work on disjoint jobs: the former runs on a side stream next to the latter
+  const bool tsAside = nTs && nDq;
+  if (tsAside) {
+    CK(cudaEventRecord(ctx->evPlan, ctx->stream));
+    CK(cudaStreamWaitEvent(ctx->sKind[0], ctx->evPlan, 0));
+  }
+  if (nDq) {
+    if (c.priceFrom) {
+      const long long nPrice = (long long)c.nRates * kDqRateModels;
+      rates_from_states_kernel<<<(unsigned)((nPrice + 127) / 128), 128, 0, ctx->stream>>>(c.priceFrom, c.nRates, ctx->dRateRom, c.rates);
+      ctx->launches++;
+    }
+    dq_rate_kernel<<<c.nRates, 32, 0, ctx->stream>>>(c.rates, c.nRates, static_cast<DqRateTab*>(ctx->dTu[kDqTabs]));
+    int* firstRaw = static_cast<int*>(ctx->dTu[kDqLists]);
+    int* orderSorted = firstRaw + nDq;
+    int* firstSorted = firstRaw + 2 * nDq;
+    dq_first_kernel<<<std::min((nDq + kDqGroups - 1) / kDqGroups, ctx->numSms * 8), kDqThreads, 0, ctx->stream>>>(c.jobs, c.dq, nDq, P.dqCoeff, ctx->dDqRom, ctx->bd, firstRaw);
+    const bool sortJobs = nDq > kDqSortAbove;
+    if (sortJobs) {
+      int* binCount = firstRaw + 3 * (size_t)nDq;
+      const int sortGrid = (nDq + kDqSortPerBlock - 1) / kDqSortPerBlock;
+      CK(cudaMemsetAsync(binCount, 0, kDqBins * sizeof(int), ctx->stream));
+      dq_hist_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(firstRaw, nDq, binCount);
+      dq_scan_kernel<<<1, 32, 0, ctx->stream>>>(binCount);
+      dq_scatter_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(c.dq, firstRaw, nDq, binCount, orderSorted, firstSorted);
+      ctx->launches += 3;
+    }
+    DqParams D;
+    D.jobs = c.jobs; D.order = sortJobs ? orderSorted : c.dq; D.firstPos = sortJobs ? firstSorted : firstRaw; D.n = nDq;
+    D.coeff = P.dqCoeff; D.level = c.level; D.deq = c.deq; D.results = c.results;
+    D.rates = c.rates; D.tabs = static_cast<const DqRateTab*>(ctx->dTu[kDqTabs]);
+    D.rom = ctx->dDqRom; D.scratch = static_cast<uint8_t*>(ctx->dTu[kDqScratch]); D.bd = ctx->bd; D.sparse = !sortJobs;
+    dq_kernel<<<dq_grid(ctx, nDq), kDqThreads, 0, ctx->stream>>>(D);
+    ctx->launches += 3;
+  }
+  if (nTs) {
+    RdoqParams R;
+    R.jobs = c.jobs; R.order = c.ts; R.n = nTs; R.coeff = P.dqCoeff; R.level = c.level;
+    R.deq = c.deq; R.results = c.results; R.rates = c.rates;
+    R.rom = ctx->dDqRom; R.bd = ctx->bd;
+    rdoq_ts_kernel<<<std::min((nTs + kTsWarps - 1) / kTsWarps, 16 * ctx->numSms), kTsThreads, 0, tsAside ? ctx->sKind[0] : ctx->stream>>>(R);
+    ctx->launches++;
+    if (tsAside) {
+      CK(cudaEventRecord(ctx->evKind[0], ctx->sKind[0]));
+      CK(cudaStreamWaitEvent(ctx->stream, ctx->evKind[0], 0));
+    }
+  }
+  if (ev) CK(cudaEventRecord(ev[2], ctx->stream));
+  if (nDq || nTs) {
+    P.phase = 1;
+    launch_tu(P);
+  }
+  if (ev) CK(cudaEventRecord(ev[3], ctx->stream));
+  if (nRate) {                                                     // levels are final: price them (CABACWriter::residual_coding on the estimator)
+    RateParams R;
+    R.jobs = c.jobs; R.order = c.rate; R.n = nRate; R.level = c.level; R.results = c.results;
+    R.states = c.states; R.statesOut = c.statesOut; R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
+    rate_kernel<<<std::min((nRate + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
+    ctx->launches++;
+  }
+  if (ev) CK(cudaEventRecord(ev[4], ctx->stream));
   return VVCB_OK;
 }
 
@@ -971,242 +1141,93 @@ static int tu_eval_impl(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n, const int
     return ok;
   });
   if (badJob >= 0) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_tu_eval: job %d is malformed", badJob); return VVCB_ERR_ARG; }
-  bool anyQuant = false;
-  std::vector<int> order;                 // DepQuant jobs (sorted on the device by scan length once the coefficients exist)
-  std::vector<int> tsBySize[7], rateBySize[9];
-  order.reserve(n);
-  for (int i = 0; i < n; i++) {
-    const bool q = (jobs[i].flags & VVCB_TU_QUANT) != 0;
-    anyQuant = anyQuant || q;
-    if (q && (jobs[i].flags & VVCB_TU_DEPQUANT)) order.push_back(i);
-    else if (q && (jobs[i].flags & VVCB_TU_RDOQ_TS)) tsBySize[jobs[i].log2w + jobs[i].log2h - 4].push_back(i);
-    if (q && (jobs[i].flags & VVCB_TU_RATE)) rateBySize[jobs[i].log2w + jobs[i].log2h - 4].push_back(i);
-  }
-  std::vector<int> rateOrder;             // jobs whose residual bits are wanted, largest TU first
-  for (int c = 8; c >= 0; c--) rateOrder.insert(rateOrder.end(), rateBySize[c].begin(), rateBySize[c].end());
-  const int nRate = (int)rateOrder.size();
-  std::vector<int> tsOrder;               // RDOQ transform-skip jobs, largest block first (one thread per block: equal chain lengths per warp)
-  for (int c = 6; c >= 0; c--) tsOrder.insert(tsOrder.end(), tsBySize[c].begin(), tsBySize[c].end());
-  const int nTs = (int)tsOrder.size();
+  const bool anyQuant = std::any_of(jobs, jobs + n, [](const vvcb_tu_job& j) { return (j.flags & VVCB_TU_QUANT) != 0; });
   if (anyQuant && !pred && !src) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_tu_eval: VVCB_TU_QUANT needs the prediction samples"); return VVCB_ERR_ARG; }
-  const int nDq = (int)order.size();
+  const TuLists L = tu_lists(jobs, n, [](int) { return true; });
+  const int nDq = (int)L.dq.size(), nTs = (int)L.ts.size(), nRate = (int)L.rate.size();
   CK(cudaSetDevice(ctx->device));
   int rc;
   const bool wLevel = walk ? walk->wantLevel : level != nullptr, wReco = walk ? walk->wantReco : reco != nullptr, wPred = walk ? walk->wantPred : pred_out != nullptr;
-  // job index lists of the two team sizes of tu_eval_kernel: blocks of up to 256 samples go to one warp each
-  std::vector<int> teamList(n);
-  int nSmall = 0;
-  {
-    int lo = 0, hi = n;
-    for (int i = 0; i < n; i++) { if (jobs[i].log2w + jobs[i].log2h <= 8) teamList[lo++] = i; else teamList[--hi] = i; }
-    nSmall = lo;
-  }
-  const int nLarge = n - nSmall;
-  int dqGrid = 0;
-  if (nDq) {
-    dqGrid = nDq <= 2048 ? (nDq + kDqThreads / 32 - 1) / (kDqThreads / 32) : (nDq + kDqGroups - 1) / kDqGroups;   // walk-sized batch: one TU per warp
-    if (dqGrid > ctx->numSms * 4) dqGrid = ctx->numSms * 4;
-    if ((rc = tu_buf(ctx, 11, (size_t)n_rates * sizeof(DqRateTab)))) return rc;
-    if ((rc = tu_buf(ctx, 12, (size_t)dqGrid * kDqGroups * kDqSlotBytes))) return rc;
-    if ((rc = tu_buf(ctx, 13, ((size_t)nDq * 3 + kDqBins) * sizeof(int)))) return rc;
-  }
-  if ((rc = tu_buf(ctx, 1, n_samples * sizeof(int16_t)))) return rc;
-  if (coeff && (rc = tu_buf(ctx, 3, n_samples * sizeof(int32_t)))) return rc;
-  if ((nDq || nTs) && (rc = tu_buf(ctx, 7, n_samples * sizeof(int32_t)))) return rc;
-  // device pointers of the host inputs and of the outputs: separate buffers, or (walk mode) offsets into the two arenas
-  const vvcb_tu_job* dJobs; const vvcb_rmd_visit* dVis = nullptr; const vvcb_tu_src* dSrc = nullptr; const int *dTeam, *dOrder = nullptr, *dTsOrder = nullptr, *dRateOrder = nullptr;
-  const vvcb_dq_rates* dRates = nullptr; const vvcb_ctx_states* dStates = nullptr;
-  vvcb_tu_result* dResults; int16_t *dPredBuf, *dRecoBuf = nullptr; int32_t *dLevel = nullptr, *dDeq = nullptr;
   const bool needLevel = wLevel || nDq || nTs || nRate;
-  size_t outBytes = 0;                                              // walk mode: bytes of the output arena that travel back
+  if ((nDq || nTs) && (rc = quant_scratch(ctx, n_samples, n_rates, &nDq, 1))) return rc;
+  if ((rc = tu_buf(ctx, kTuResi, n_samples * sizeof(int16_t)))) return rc;
+  if (coeff && (rc = tu_buf(ctx, kTuCoeff, n_samples * sizeof(int32_t)))) return rc;
+  // the host inputs in one device arena; walk mode stages them in page-locked memory, moved by one copy kernel
+  const size_t ratesBytes = (nDq || nTs) ? (size_t)n_rates * sizeof(vvcb_dq_rates) : 0, statesBytes = nRate ? (size_t)n_rates * sizeof(vvcb_ctx_states) : 0;
+  Arena in;
+  const size_t iJobs = in.take((size_t)n * sizeof(vvcb_tu_job)), iVis = in.take((size_t)n_visits * sizeof(vvcb_rmd_visit)),
+               iSrc = in.take(src ? (size_t)n * sizeof(vvcb_tu_src) : 0), iTeam = in.take((size_t)n * sizeof(int)), iOrder = in.take((size_t)nDq * sizeof(int)),
+               iTs = in.take((size_t)nTs * sizeof(int)), iRates = in.take(ratesBytes), iRateOrder = in.take((size_t)nRate * sizeof(int)), iStates = in.take(statesBytes);
+  uint8_t* hin = nullptr;
   if (walk) {
-    auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
-    size_t o = 0;
-    auto take = [&](size_t b) { const size_t at = o; o += up16(b); return at; };
-    const size_t iJobs = take((size_t)n * sizeof(vvcb_tu_job)), iVis = take((size_t)n_visits * sizeof(vvcb_rmd_visit)), iSrc = take((size_t)n * sizeof(vvcb_tu_src)),
-                 iTeam = take((size_t)n * sizeof(int)), iOrder = take((size_t)nDq * sizeof(int)), iTs = take((size_t)nTs * sizeof(int)),
-                 iRates = take((nDq || nTs) ? (size_t)n_rates * sizeof(vvcb_dq_rates) : 0), iRateOrder = take((size_t)nRate * sizeof(int)),
-                 iStates = take(nRate ? (size_t)n_rates * sizeof(vvcb_ctx_states) : 0);
-    const size_t inBytes = o;
-    if ((rc = pin_buf(ctx, 9, inBytes))) return rc;
-    if ((rc = tu_buf(ctx, 20, inBytes))) return rc;
-    uint8_t* hin = static_cast<uint8_t*>(ctx->hPin[9]);
-    memcpy(hin + iJobs, jobs, (size_t)n * sizeof(vvcb_tu_job));
-    memcpy(hin + iVis, visits, (size_t)n_visits * sizeof(vvcb_rmd_visit));
-    memcpy(hin + iSrc, src, (size_t)n * sizeof(vvcb_tu_src));
-    memcpy(hin + iTeam, teamList.data(), (size_t)n * sizeof(int));
-    if (nDq) memcpy(hin + iOrder, order.data(), (size_t)nDq * sizeof(int));
-    if (nTs) memcpy(hin + iTs, tsOrder.data(), (size_t)nTs * sizeof(int));
-    if (nDq || nTs) memcpy(hin + iRates, rates, (size_t)n_rates * sizeof(vvcb_dq_rates));
-    if (nRate) { memcpy(hin + iRateOrder, rateOrder.data(), (size_t)nRate * sizeof(int)); memcpy(hin + iStates, states, (size_t)n_rates * sizeof(vvcb_ctx_states)); }
-    uint8_t* din = static_cast<uint8_t*>(ctx->dTu[20]);
-    CK(arena_copy(ctx, hin, din, inBytes));
-    dJobs = reinterpret_cast<const vvcb_tu_job*>(din + iJobs); dVis = reinterpret_cast<const vvcb_rmd_visit*>(din + iVis); dSrc = reinterpret_cast<const vvcb_tu_src*>(din + iSrc);
-    dTeam = reinterpret_cast<const int*>(din + iTeam); dOrder = reinterpret_cast<const int*>(din + iOrder); dTsOrder = reinterpret_cast<const int*>(din + iTs);
-    dRates = reinterpret_cast<const vvcb_dq_rates*>(din + iRates); dRateOrder = reinterpret_cast<const int*>(din + iRateOrder); dStates = reinterpret_cast<const vvcb_ctx_states*>(din + iStates);
-    // output arena: results | prediction | reconstruction | levels, then (not travelling) the dequantised coefficients next to the levels
-    o = 0;
-    const size_t oRes = take((size_t)n * sizeof(vvcb_tu_result)), oPred = take(n_samples * sizeof(int16_t)), oReco = take(wReco ? n_samples * sizeof(int16_t) : 0),
-                 oLevel = take(needLevel ? n_samples * sizeof(int32_t) : 0);
-    outBytes = wLevel ? o : (wReco ? oLevel : (wPred ? oReco : oPred));
-    const size_t oDeq = take((nDq || nTs) ? n_samples * sizeof(int32_t) : 0);
-    if ((rc = tu_buf(ctx, 21, o))) return rc;
-    if ((rc = pin_buf(ctx, 8, outBytes))) return rc;
-    uint8_t* dout = static_cast<uint8_t*>(ctx->dTu[21]);
-    uint8_t* hout = static_cast<uint8_t*>(ctx->hPin[8]);
-    dResults = reinterpret_cast<vvcb_tu_result*>(dout + oRes); dPredBuf = reinterpret_cast<int16_t*>(dout + oPred); dRecoBuf = wReco ? reinterpret_cast<int16_t*>(dout + oReco) : nullptr;
-    dLevel = needLevel ? reinterpret_cast<int32_t*>(dout + oLevel) : nullptr; dDeq = (nDq || nTs) ? reinterpret_cast<int32_t*>(dout + oDeq) : nullptr;
-    walk->results = reinterpret_cast<vvcb_tu_result*>(hout + oRes); walk->pred = reinterpret_cast<int16_t*>(hout + oPred);
-    walk->reco = reinterpret_cast<int16_t*>(hout + oReco); walk->level = reinterpret_cast<int32_t*>(hout + oLevel);
-    if (nDq || nTs) CK(cudaMemsetAsync(dLevel, 0, up16(n_samples * sizeof(int32_t)) + n_samples * sizeof(int32_t), ctx->stream));   // levels and dequantised coefficients: adjacent
-  } else {
-    if ((rc = tu_buf(ctx, 0, (size_t)n * sizeof(vvcb_tu_job)))) return rc;
-    if ((rc = tu_buf(ctx, 2, n_samples * sizeof(int16_t)))) return rc;
-    if (needLevel && (rc = tu_buf(ctx, 4, n_samples * sizeof(int32_t)))) return rc;
-    if (nRate && (rc = tu_buf(ctx, 17, (size_t)nRate * sizeof(int)))) return rc;
-    if (nRate && (rc = tu_buf(ctx, 18, (size_t)n_rates * sizeof(vvcb_ctx_states)))) return rc;
-    if (wReco && (rc = tu_buf(ctx, 5, n_samples * sizeof(int16_t)))) return rc;
-    if ((rc = tu_buf(ctx, 6, (size_t)n * sizeof(vvcb_tu_result)))) return rc;
-    if (nDq || nTs) {
-      if ((rc = tu_buf(ctx, 8, n_samples * sizeof(int32_t)))) return rc;
-      if ((rc = tu_buf(ctx, 10, (size_t)n_rates * sizeof(vvcb_dq_rates)))) return rc;
-      if (nTs && (rc = tu_buf(ctx, 16, (size_t)nTs * sizeof(int)))) return rc;
-    }
-    if (nDq && (rc = tu_buf(ctx, 9, (size_t)nDq * sizeof(int)))) return rc;
-    if ((rc = tu_buf(ctx, 19, (size_t)n * sizeof(int)))) return rc;
-    CK(cudaMemcpyAsync(ctx->dTu[0], jobs, (size_t)n * sizeof(vvcb_tu_job), cudaMemcpyHostToDevice, ctx->stream));
-    if (src) {
-      if ((rc = tu_buf(ctx, 14, (size_t)n_visits * sizeof(vvcb_rmd_visit)))) return rc;
-      if ((rc = tu_buf(ctx, 15, (size_t)n * sizeof(vvcb_tu_src)))) return rc;
-      CK(cudaMemcpyAsync(ctx->dTu[14], visits, (size_t)n_visits * sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
-      CK(cudaMemcpyAsync(ctx->dTu[15], src, (size_t)n * sizeof(vvcb_tu_src), cudaMemcpyHostToDevice, ctx->stream));
-      dVis = static_cast<const vvcb_rmd_visit*>(ctx->dTu[14]); dSrc = static_cast<const vvcb_tu_src*>(ctx->dTu[15]);
-    }
-    CK(cudaMemcpyAsync(ctx->dTu[19], teamList.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-    if (nDq || nTs) {
-      CK(cudaMemsetAsync(ctx->dTu[4], 0, n_samples * sizeof(int32_t), ctx->stream));     // levels / dequantised coefficients the
-      CK(cudaMemsetAsync(ctx->dTu[8], 0, n_samples * sizeof(int32_t), ctx->stream));     // quantiser kernels do not reach stay zero
-      if (nDq) CK(cudaMemcpyAsync(ctx->dTu[9], order.data(), (size_t)nDq * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-      if (nTs) CK(cudaMemcpyAsync(ctx->dTu[16], tsOrder.data(), (size_t)nTs * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-      CK(cudaMemcpyAsync(ctx->dTu[10], rates, (size_t)n_rates * sizeof(vvcb_dq_rates), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    if (nRate) {
-      CK(cudaMemcpyAsync(ctx->dTu[17], rateOrder.data(), (size_t)nRate * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-      CK(cudaMemcpyAsync(ctx->dTu[18], states, (size_t)n_rates * sizeof(vvcb_ctx_states), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    dJobs = static_cast<const vvcb_tu_job*>(ctx->dTu[0]); dTeam = static_cast<const int*>(ctx->dTu[19]);
-    dOrder = static_cast<const int*>(ctx->dTu[9]); dTsOrder = static_cast<const int*>(ctx->dTu[16]); dRateOrder = static_cast<const int*>(ctx->dTu[17]);
-    dRates = static_cast<const vvcb_dq_rates*>(ctx->dTu[10]); dStates = static_cast<const vvcb_ctx_states*>(ctx->dTu[18]);
-    dResults = static_cast<vvcb_tu_result*>(ctx->dTu[6]); dPredBuf = static_cast<int16_t*>(ctx->dTu[2]); dRecoBuf = wReco ? static_cast<int16_t*>(ctx->dTu[5]) : nullptr;
-    dLevel = needLevel ? static_cast<int32_t*>(ctx->dTu[4]) : nullptr; dDeq = static_cast<int32_t*>(ctx->dTu[8]);
+    if ((rc = pin_buf(ctx, kPinTuIn, in.size))) return rc;
+    hin = static_cast<uint8_t*>(ctx->hPin[kPinTuIn]);
   }
+  if ((rc = tu_buf(ctx, kTuIn, in.size))) return rc;
+  void* din = ctx->dTu[kTuIn];
+  auto put = [&](size_t o, const void* p, size_t bytes) {
+    if (!bytes) return cudaSuccess;
+    if (walk) { memcpy(hin + o, p, bytes); return cudaSuccess; }
+    return cudaMemcpyAsync(at<uint8_t>(din, o), p, bytes, cudaMemcpyHostToDevice, ctx->stream);
+  };
+  CK(put(iJobs, jobs, (size_t)n * sizeof(vvcb_tu_job)));
+  if (src) { CK(put(iVis, visits, (size_t)n_visits * sizeof(vvcb_rmd_visit))); CK(put(iSrc, src, (size_t)n * sizeof(vvcb_tu_src))); }
+  CK(put(iTeam, L.team.data(), (size_t)n * sizeof(int)));
+  CK(put(iOrder, L.dq.data(), (size_t)nDq * sizeof(int)));
+  CK(put(iTs, L.ts.data(), (size_t)nTs * sizeof(int)));
+  CK(put(iRates, rates, ratesBytes));
+  CK(put(iRateOrder, L.rate.data(), (size_t)nRate * sizeof(int)));
+  CK(put(iStates, states, statesBytes));
+  if (walk) CK(arena_copy(ctx, hin, din, in.size));
+  // the outputs in one device arena: results | prediction | reconstruction | levels, then the dequantised coefficients next to the levels
+  Arena out;
+  const size_t oRes = out.take((size_t)n * sizeof(vvcb_tu_result)), oPred = out.take(n_samples * sizeof(int16_t)),
+               oReco = out.take(wReco ? n_samples * sizeof(int16_t) : 0), oLevel = out.take(needLevel ? n_samples * sizeof(int32_t) : 0);
+  const size_t outBytes = wLevel ? out.size : (wReco ? oLevel : (wPred ? oReco : oPred));   // walk mode: what travels back
+  const size_t oDeq = out.take((nDq || nTs) ? n_samples * sizeof(int32_t) : 0);
+  if ((rc = tu_buf(ctx, kTuOut, out.size))) return rc;
+  void* dout = ctx->dTu[kTuOut];
+  if (walk) {
+    if ((rc = pin_buf(ctx, kPinTuOut, outBytes))) return rc;
+    void* hout = ctx->hPin[kPinTuOut];
+    walk->results = at<vvcb_tu_result>(hout, oRes); walk->pred = at<int16_t>(hout, oPred);
+    walk->reco = at<int16_t>(hout, oReco); walk->level = at<int32_t>(hout, oLevel);
+  }
+  TuChain c = {};
+  c.jobs = at<const vvcb_tu_job>(din, iJobs);
+  c.team = at<const int>(din, iTeam); c.dq = at<const int>(din, iOrder); c.ts = at<const int>(din, iTs); c.rate = at<const int>(din, iRateOrder);
+  int16_t* dPred = at<int16_t>(dout, oPred);
+  c.resi = static_cast<const int16_t*>(ctx->dTu[kTuResi]); c.pred = dPred;
+  c.coeff = coeff ? static_cast<int32_t*>(ctx->dTu[kTuCoeff]) : nullptr;
+  c.level = needLevel ? at<int32_t>(dout, oLevel) : nullptr; c.reco = wReco ? at<int16_t>(dout, oReco) : nullptr;
+  c.deq = (nDq || nTs) ? at<int32_t>(dout, oDeq) : nullptr; c.results = at<vvcb_tu_result>(dout, oRes);
+  c.rates = at<vvcb_dq_rates>(din, iRates); c.nRates = n_rates; c.states = at<const vvcb_ctx_states>(din, iStates);
+  if (nDq || nTs) CK(cudaMemsetAsync(c.level, 0, oDeq - oLevel + n_samples * sizeof(int32_t), ctx->stream));   // levels and dequantised coefficients
+                                                                                                               // the quantisers do not reach stay zero
   const bool tm = ctx->timing != 0;
   if (src) {
     if (tm) CK(cudaEventRecord(ctx->tev[0], ctx->stream));
     TuPredParams Q;
-    Q.visits = dVis; Q.src = dSrc; Q.jobs = dJobs; Q.n = n;
-    Q.pred = dPredBuf; Q.resi = static_cast<int16_t*>(ctx->dTu[1]);
+    Q.visits = at<const vvcb_rmd_visit>(din, iVis); Q.src = at<const vvcb_tu_src>(din, iSrc); Q.jobs = c.jobs; Q.n = n;
+    Q.pred = dPred; Q.resi = static_cast<int16_t*>(ctx->dTu[kTuResi]);
     Q.orig = ctx->bOrig; Q.reco = ctx->bReco; Q.stride = ctx->stride; Q.bd = ctx->bd; Q.ctu = ctx->ctu; Q.rom = ctx->dRom;
     const int pg = (n + kTuPredWarps - 1) / kTuPredWarps < ctx->numSms * 8 ? (n + kTuPredWarps - 1) / kTuPredWarps : ctx->numSms * 8;
     tu_pred_kernel<<<pg, kTuPredWarps * 32, 0, ctx->stream>>>(Q);
     ctx->launches++;
   } else {
-    CK(cudaMemcpyAsync(ctx->dTu[1], resi, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
-    if (pred) CK(cudaMemcpyAsync(dPredBuf, pred, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->dTu[kTuResi], resi, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
+    if (pred) CK(cudaMemcpyAsync(dPred, pred, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
+    if (tm) CK(cudaEventRecord(ctx->tev[0], ctx->stream));
   }
-  TuParams P;
-  P.jobs = dJobs; P.list = nullptr; P.n = 0;
-  P.resi = static_cast<const int16_t*>(ctx->dTu[1]); P.pred = dPredBuf;
-  P.coeff = coeff ? static_cast<int32_t*>(ctx->dTu[3]) : nullptr;
-  P.level = dLevel;
-  P.reco = dRecoBuf;
-  P.results = dResults;
-  P.orig = ctx->bOrig; P.stride = ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
-  P.dqCoeff = static_cast<int32_t*>(ctx->dTu[7]); P.dqDeq = dDeq; P.phase = 0;
-  auto launch_tu = [&](TuParams Q) {
-    if (nSmall) {
-      Q.list = dTeam; Q.n = nSmall;
-      const int g = (nSmall + 3) / 4 < ctx->numSms * 8 ? (nSmall + 3) / 4 : ctx->numSms * 8;
-      tu_eval_kernel<32><<<g, kTuThreads, 0, ctx->stream>>>(Q);
-      ctx->launches++;
-    }
-    if (nLarge) {
-      Q.list = dTeam + nSmall; Q.n = nLarge;
-      const int g = nLarge < ctx->numSms * 8 ? nLarge : ctx->numSms * 8;
-      tu_eval_kernel<128><<<g, kTuThreads, 0, ctx->stream>>>(Q);
-      ctx->launches++;
-    }
-  };
-  if (tm && !src) CK(cudaEventRecord(ctx->tev[0], ctx->stream));
-  launch_tu(P);
-  if (tm) CK(cudaEventRecord(ctx->tev[1], ctx->stream));
-  // transform-skip RDOQ and dependent quantisation work on disjoint jobs: the former runs on a side stream next to the latter
-  const bool tsAside = nTs && nDq;
-  if (tsAside) {
-    CK(cudaEventRecord(ctx->evPlan, ctx->stream));
-    CK(cudaStreamWaitEvent(ctx->sKind[0], ctx->evPlan, 0));
-  }
-  if (nDq) {
-    dq_rate_kernel<<<n_rates, 32, 0, ctx->stream>>>(dRates, n_rates, static_cast<DqRateTab*>(ctx->dTu[11]));
-    DqParams D;
-    int* firstRaw = static_cast<int*>(ctx->dTu[13]);
-    int* orderSorted = firstRaw + nDq;
-    int* firstSorted = firstRaw + 2 * nDq;
-    const int firstGrid = (nDq + kDqGroups - 1) / kDqGroups < ctx->numSms * 8 ? (nDq + kDqGroups - 1) / kDqGroups : ctx->numSms * 8;
-    dq_first_kernel<<<firstGrid, kDqThreads, 0, ctx->stream>>>(P.jobs, dOrder, nDq, P.dqCoeff, ctx->dDqRom, ctx->bd, firstRaw);
-    // The counting sort by first test position buys warp efficiency for sweeps (eight TUs per warp walk scans of equal length); a walk's batch
-    // of a few dozen candidates is latency bound and skips its three launches.
-    const bool sortJobs = nDq > 2048;
-    if (sortJobs) {
-      int* binCount = firstRaw + 3 * (size_t)nDq;
-      const int sortGrid = (nDq + kDqSortPerBlock - 1) / kDqSortPerBlock;
-      CK(cudaMemsetAsync(binCount, 0, kDqBins * sizeof(int), ctx->stream));
-      dq_hist_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(firstRaw, nDq, binCount);
-      dq_scan_kernel<<<1, 32, 0, ctx->stream>>>(binCount);
-      dq_scatter_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(dOrder, firstRaw, nDq, binCount, orderSorted, firstSorted);
-      ctx->launches += 3;
-    }
-    D.jobs = P.jobs; D.order = sortJobs ? orderSorted : dOrder; D.firstPos = sortJobs ? firstSorted : firstRaw; D.n = nDq;
-    D.coeff = P.dqCoeff; D.level = P.level; D.deq = dDeq; D.results = P.results;
-    D.rates = dRates; D.tabs = static_cast<const DqRateTab*>(ctx->dTu[11]);
-    D.rom = ctx->dDqRom; D.scratch = static_cast<uint8_t*>(ctx->dTu[12]); D.bd = ctx->bd; D.sparse = !sortJobs;
-    dq_kernel<<<dqGrid, kDqThreads, 0, ctx->stream>>>(D);
-    ctx->launches += 3;
-  }
-  if (nTs) {
-    RdoqParams R;
-    R.jobs = P.jobs; R.order = dTsOrder; R.n = nTs; R.coeff = P.dqCoeff; R.level = P.level;
-    R.deq = dDeq; R.results = P.results; R.rates = dRates;
-    R.rom = ctx->dDqRom; R.bd = ctx->bd;
-    rdoq_ts_kernel<<<std::min((nTs + kTsWarps - 1) / kTsWarps, 16 * ctx->numSms), kTsThreads, 0, tsAside ? ctx->sKind[0] : ctx->stream>>>(R);
-    ctx->launches++;
-    if (tsAside) {
-      CK(cudaEventRecord(ctx->evKind[0], ctx->sKind[0]));
-      CK(cudaStreamWaitEvent(ctx->stream, ctx->evKind[0], 0));
-    }
-  }
-  if (tm) CK(cudaEventRecord(ctx->tev[2], ctx->stream));
-  if (nDq || nTs) {
-    P.phase = 1;
-    launch_tu(P);
-  }
-  if (tm) CK(cudaEventRecord(ctx->tev[3], ctx->stream));
-  if (nRate) {                                                     // levels are final: price them (CABACWriter::residual_coding on the estimator)
-    RateParams R;
-    R.jobs = P.jobs; R.order = dRateOrder; R.n = nRate; R.level = P.level; R.results = P.results;
-    R.states = dStates; R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
-    rate_kernel<<<std::min((nRate + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
-    ctx->launches++;
-  }
-  if (tm) CK(cudaEventRecord(ctx->tev[4], ctx->stream));
+  if ((rc = run_tu_chain(ctx, c, L, tm ? ctx->tev : nullptr))) return rc;
   CK(cudaGetLastError());
-  if (coeff) CK(cudaMemcpyAsync(coeff, ctx->dTu[3], n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (walk) CK(arena_copy(ctx, ctx->dTu[21], ctx->hPin[8], outBytes));
+  if (coeff) CK(cudaMemcpyAsync(coeff, c.coeff, n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (walk) CK(arena_copy(ctx, dout, ctx->hPin[kPinTuOut], outBytes));
   else {
-    if (level) CK(cudaMemcpyAsync(level, dLevel, n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if (reco) CK(cudaMemcpyAsync(reco, dRecoBuf, n_samples * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-    if (pred_out) CK(cudaMemcpyAsync(pred_out, dPredBuf, n_samples * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(results, dResults, (size_t)n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
+    if (level) CK(cudaMemcpyAsync(level, c.level, n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (reco) CK(cudaMemcpyAsync(reco, c.reco, n_samples * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (pred_out) CK(cudaMemcpyAsync(pred_out, dPred, n_samples * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(results, c.results, (size_t)n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
   }
   if (ctx->cuSpan) CK(cudaEventRecord(ctx->cev[3], ctx->stream));
   ctx->tuWaitFrom = host_ns();
@@ -1286,17 +1307,17 @@ extern "C" int vvcb_cu_eval(vvcb_ctx* ctx, vvcb_cu_request* reqs, int n)
   ctx->cuSpan = true;
   CK(cudaEventRecord(ctx->cev[0], ctx->stream));
   // ---- inputs of the first stage: rectangles | their samples | visits, one page-locked arena, moved by a copy kernel (see TuWalk) ----
-  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
-  const size_t iSmp = up16(nRects * sizeof(vvcb_rect)), iVis = iSmp + up16(nRectSamples * sizeof(int16_t)), inBytes = iVis + up16((size_t)nRmd * sizeof(vvcb_rmd_visit));
+  Arena in;
+  const size_t iRects = in.take(nRects * sizeof(vvcb_rect)), iSmp = in.take(nRectSamples * sizeof(int16_t)), iVis = in.take((size_t)nRmd * sizeof(vvcb_rmd_visit));
   vvcb_rmd_result* hRes = nullptr; vvcb_rmd_detail* hDet = nullptr;
-  if (inBytes) {
-    if ((rc = pin_buf(ctx, 0, inBytes))) return rc;
-    if ((rc = tu_buf(ctx, 22, inBytes))) return rc;
-    uint8_t* hin = static_cast<uint8_t*>(ctx->hPin[0]);
-    uint8_t* din = static_cast<uint8_t*>(ctx->dTu[22]);
-    vvcb_rect* hr = reinterpret_cast<vvcb_rect*>(hin);
-    int16_t* hs = reinterpret_cast<int16_t*>(hin + iSmp);
-    vvcb_rmd_visit* hv = reinterpret_cast<vvcb_rmd_visit*>(hin + iVis);
+  if (in.size) {
+    if ((rc = pin_buf(ctx, kPinStageIn, in.size))) return rc;
+    if ((rc = tu_buf(ctx, kStageIn, in.size))) return rc;
+    void* hin = ctx->hPin[kPinStageIn];
+    void* din = ctx->dTu[kStageIn];
+    vvcb_rect* hr = at<vvcb_rect>(hin, iRects);
+    int16_t* hs = at<int16_t>(hin, iSmp);
+    vvcb_rmd_visit* hv = at<vvcb_rmd_visit>(hin, iVis);
     size_t ri = 0, so = 0;
     int vi = 0;
     for (int i = 0; i < n; i++) {
@@ -1308,26 +1329,27 @@ extern "C" int vvcb_cu_eval(vvcb_ctx* ctx, vvcb_cu_request* reqs, int n)
       so += q.n_rect_samples;
     }
     if (nRmd && (rc = check_visits(ctx, hv, nRmd))) return rc;
-    CK(arena_copy(ctx, hin, din, inBytes));
+    CK(arena_copy(ctx, hin, din, in.size));
     // ---- reconstruction rectangles ----
     if (nRects) {
-      reco_scatter_kernel<<<(int)nRects < ctx->numSms * 8 ? (int)nRects : ctx->numSms * 8, 128, 0, ctx->stream>>>(reinterpret_cast<const vvcb_rect*>(din), (int)nRects,
-                                                                                                          reinterpret_cast<const int16_t*>(din + iSmp), ctx->wReco, ctx->stride);
+      reco_scatter_kernel<<<(int)nRects < ctx->numSms * 8 ? (int)nRects : ctx->numSms * 8, 128, 0, ctx->stream>>>(at<const vvcb_rect>(din, iRects), (int)nRects,
+                                                                                                          at<const int16_t>(din, iSmp), ctx->wReco, ctx->stride);
       ctx->launches++;
       CK(cudaGetLastError());
     }
     // ---- rough mode decision ----
     if (nRmd) {
-      const size_t oDet = up16((size_t)nRmd * sizeof(vvcb_rmd_result)), outBytes = oDet + (anyDetail ? (size_t)nRmd * sizeof(vvcb_rmd_detail) : 0);
-      if ((rc = tu_buf(ctx, 23, outBytes))) return rc;
-      if ((rc = pin_buf(ctx, 3, outBytes))) return rc;
-      uint8_t* dout = static_cast<uint8_t*>(ctx->dTu[23]);
-      uint8_t* hout = static_cast<uint8_t*>(ctx->hPin[3]);
-      hRes = reinterpret_cast<vvcb_rmd_result*>(hout);
-      hDet = anyDetail ? reinterpret_cast<vvcb_rmd_detail*>(hout + oDet) : nullptr;
-      if ((rc = launch_rmd(ctx, reinterpret_cast<const vvcb_rmd_visit*>(din + iVis), nRmd, reinterpret_cast<vvcb_rmd_result*>(dout),
-                           anyDetail ? reinterpret_cast<vvcb_rmd_detail*>(dout + oDet) : nullptr, nullptr, hv))) return rc;
-      CK(arena_copy(ctx, dout, hout, outBytes));
+      Arena out;
+      const size_t oRes = out.take((size_t)nRmd * sizeof(vvcb_rmd_result)), oDet = out.take(anyDetail ? (size_t)nRmd * sizeof(vvcb_rmd_detail) : 0);
+      if ((rc = tu_buf(ctx, kStageOut, out.size))) return rc;
+      if ((rc = pin_buf(ctx, kPinStageOut, out.size))) return rc;
+      void* dout = ctx->dTu[kStageOut];
+      void* hout = ctx->hPin[kPinStageOut];
+      hRes = at<vvcb_rmd_result>(hout, oRes);
+      hDet = anyDetail ? at<vvcb_rmd_detail>(hout, oDet) : nullptr;
+      if ((rc = launch_rmd(ctx, at<const vvcb_rmd_visit>(din, iVis), nRmd, at<vvcb_rmd_result>(dout, oRes),
+                           anyDetail ? at<vvcb_rmd_detail>(dout, oDet) : nullptr, nullptr, hv))) return rc;
+      CK(arena_copy(ctx, dout, hout, out.size));
     }
   }
   if (nRmd) {
@@ -1446,27 +1468,28 @@ extern "C" int vvcb_residual_bits(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n,
   if (bad >= 0) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_residual_bits: job %d is malformed", bad); return VVCB_ERR_ARG; }
   CK(cudaSetDevice(ctx->device));
   int rc;
-  if ((rc = tu_buf(ctx, 0, (size_t)n * sizeof(vvcb_tu_job)))) return rc;
-  if ((rc = tu_buf(ctx, 4, n_samples * sizeof(int32_t)))) return rc;
-  if ((rc = tu_buf(ctx, 6, (size_t)n * sizeof(vvcb_tu_result)))) return rc;
-  if ((rc = tu_buf(ctx, 17, (size_t)n * sizeof(int)))) return rc;
-  if ((rc = tu_buf(ctx, 18, (size_t)n_states * sizeof(vvcb_ctx_states)))) return rc;
-  std::vector<int> bySize[9], order;
+  std::vector<int> bySize[9];
   for (int i = 0; i < n; i++) bySize[jobs[i].log2w + jobs[i].log2h - 4].push_back(i);
-  for (int c = 8; c >= 0; c--) order.insert(order.end(), bySize[c].begin(), bySize[c].end());
-  CK(cudaMemcpyAsync(ctx->dTu[0], jobs, (size_t)n * sizeof(vvcb_tu_job), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->dTu[4], levels, n_samples * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->dTu[17], order.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->dTu[18], states, (size_t)n_states * sizeof(vvcb_ctx_states), cudaMemcpyHostToDevice, ctx->stream));
+  const std::vector<int> order = largest_first(bySize);
+  Arena in;
+  const size_t iJobs = in.take((size_t)n * sizeof(vvcb_tu_job)), iLevel = in.take(n_samples * sizeof(int32_t)), iOrder = in.take((size_t)n * sizeof(int)),
+               iStates = in.take((size_t)n_states * sizeof(vvcb_ctx_states));
+  if ((rc = tu_buf(ctx, kTuIn, in.size))) return rc;
+  if ((rc = tu_buf(ctx, kTuOut, (size_t)n * sizeof(vvcb_tu_result)))) return rc;
+  void* din = ctx->dTu[kTuIn];
+  CK(cudaMemcpyAsync(at<uint8_t>(din, iJobs), jobs, (size_t)n * sizeof(vvcb_tu_job), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(at<uint8_t>(din, iLevel), levels, n_samples * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(at<uint8_t>(din, iOrder), order.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(at<uint8_t>(din, iStates), states, (size_t)n_states * sizeof(vvcb_ctx_states), cudaMemcpyHostToDevice, ctx->stream));
   RateParams R;
-  R.jobs = static_cast<const vvcb_tu_job*>(ctx->dTu[0]); R.order = static_cast<const int*>(ctx->dTu[17]); R.n = n;
-  R.level = static_cast<const int32_t*>(ctx->dTu[4]); R.results = static_cast<vvcb_tu_result*>(ctx->dTu[6]);
-  R.states = static_cast<const vvcb_ctx_states*>(ctx->dTu[18]); R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
+  R.jobs = at<const vvcb_tu_job>(din, iJobs); R.order = at<const int>(din, iOrder); R.n = n;
+  R.level = at<const int32_t>(din, iLevel); R.results = static_cast<vvcb_tu_result*>(ctx->dTu[kTuOut]);
+  R.states = at<const vvcb_ctx_states>(din, iStates); R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
   rate_kernel<<<std::min((n + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
   ctx->launches++;
   CK(cudaGetLastError());
   std::vector<vvcb_tu_result> res(n);
-  CK(cudaMemcpyAsync(res.data(), ctx->dTu[6], (size_t)n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(res.data(), R.results, (size_t)n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (int i = 0; i < n; i++) bits[i] = res[i].frac_bits;
   return VVCB_OK;
@@ -1611,7 +1634,7 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
       t.x = (int16_t)(v.x + parts[k].x); t.y = (int16_t)(v.y + parts[k].y);
       t.log2w = (uint8_t)vlog2(parts[k].w); t.log2h = (uint8_t)vlog2(parts[k].h);
       t.mts_idx = 0;
-      t.flags = (uint8_t)((j.flags & VVCB_TU_DEPQUANT) ? (VVCB_TU_QUANT | VVCB_TU_DEPQUANT) : VVCB_TU_QUANT);
+      t.flags = (uint8_t)(j.flags | (carried ? VVCB_TU_RATE : 0));   // rate_kernel adapts the carried models of DEPQUANT candidates too
       t.qp_per = j.qp_per; t.qp_rem = j.qp_rem;
       t.offset = (uint32_t)(cs + (size_t)k * parts[k].w * parts[k].h);
       t.rate_idx = (uint16_t)i;                        // the candidate's own carried snapshot
@@ -1622,76 +1645,50 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
   }
   if (checkOnly) return VVCB_OK;
   // per-step work lists (all host-known: the values change, the shapes do not)
-  std::vector<int> predList[5], team[4], dqOrder[4], rateOrder[4];
-  int nSmall[4] = { 0, 0, 0, 0 };
+  std::vector<int> predList[5];
+  TuLists L[4];
   for (int k = 0; k <= 4; k++)
     for (int i = 0; i < n; i++) if (cands[i].nParts > k || (k > 0 && cands[i].nParts == k)) predList[k].push_back(i);
-  for (int k = 0; k < 4; k++) {
-    std::vector<int> large, bySize[9];
-    for (int i = 0; i < n; i++) {
-      if (cands[i].nParts <= k) continue;
-      const vvcb_tu_job& t = tj[(size_t)k * n + i];
-      if (t.log2w + t.log2h <= 8) team[k].push_back(i); else large.push_back(i);
-      if (jobs[i].flags & VVCB_TU_DEPQUANT) dqOrder[k].push_back(i);
-      if (jobs[i].flags & (VVCB_TU_DEPQUANT | VVCB_TU_RATE)) bySize[t.log2w + t.log2h - 4].push_back(i);
-    }
-    nSmall[k] = (int)team[k].size();
-    team[k].insert(team[k].end(), large.begin(), large.end());
-    for (int c = 8; c >= 0; c--) rateOrder[k].insert(rateOrder[k].end(), bySize[c].begin(), bySize[c].end());
-  }
+  for (int k = 0; k < 4; k++) L[k] = tu_lists(&tj[(size_t)k * n], n, [&](int i) { return cands[i].nParts > k; });
   // one input arena in page-locked memory: candidates, TU jobs, transform pairs, cbf state, carried models, lists
-  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
-  size_t o = 0;
-  auto take = [&](size_t b) { const size_t at = o; o += up16(b); return at; };
-  const size_t iCand = take((size_t)n * sizeof(IspCand)), iJobs = take(tj.size() * sizeof(vvcb_tu_job)), iTr = take(trPair.size()),
-               iState = take((size_t)n * sizeof(IspState)), iCst = take((size_t)n * sizeof(vvcb_ctx_states));
+  Arena in;
+  const size_t iCand = in.take((size_t)n * sizeof(IspCand)), iJobs = in.take(tj.size() * sizeof(vvcb_tu_job)), iTr = in.take(trPair.size()),
+               iState = in.take((size_t)n * sizeof(IspState)), iCst = in.take((size_t)n * sizeof(vvcb_ctx_states));
   size_t iPred[5], iTeam[4], iDq[4], iRate[4];
-  for (int k = 0; k <= 4; k++) iPred[k] = take(predList[k].size() * sizeof(int));
-  for (int k = 0; k < 4; k++) { iTeam[k] = take(team[k].size() * sizeof(int)); iDq[k] = take(dqOrder[k].size() * sizeof(int)); iRate[k] = take(rateOrder[k].size() * sizeof(int)); }
-  const size_t inBytes = o;
+  for (int k = 0; k <= 4; k++) iPred[k] = in.take(predList[k].size() * sizeof(int));
+  for (int k = 0; k < 4; k++) { iTeam[k] = in.take(L[k].team.size() * sizeof(int)); iDq[k] = in.take(L[k].dq.size() * sizeof(int)); iRate[k] = in.take(L[k].rate.size() * sizeof(int)); }
   int rc;
-  if ((rc = pin_buf(ctx, 6, inBytes))) return rc;
-  uint8_t* hin = static_cast<uint8_t*>(ctx->hPin[6]);
-  memcpy(&hin[iCand], cands.data(), (size_t)n * sizeof(IspCand));
-  memcpy(&hin[iJobs], tj.data(), tj.size() * sizeof(vvcb_tu_job));
-  memcpy(&hin[iTr], trPair.data(), trPair.size());
-  memcpy(&hin[iState], ist.data(), (size_t)n * sizeof(IspState));
-  memcpy(&hin[iCst], cst.data(), (size_t)n * sizeof(vvcb_ctx_states));
-  auto put = [&](size_t at, const std::vector<int>& v) { if (!v.empty()) memcpy(&hin[at], v.data(), v.size() * sizeof(int)); };
+  if ((rc = pin_buf(ctx, kPinStageIn, in.size))) return rc;
+  void* hin = ctx->hPin[kPinStageIn];
+  memcpy(at<IspCand>(hin, iCand), cands.data(), (size_t)n * sizeof(IspCand));
+  memcpy(at<vvcb_tu_job>(hin, iJobs), tj.data(), tj.size() * sizeof(vvcb_tu_job));
+  memcpy(at<uint8_t>(hin, iTr), trPair.data(), trPair.size());
+  memcpy(at<IspState>(hin, iState), ist.data(), (size_t)n * sizeof(IspState));
+  memcpy(at<vvcb_ctx_states>(hin, iCst), cst.data(), (size_t)n * sizeof(vvcb_ctx_states));
+  auto put = [&](size_t o, const std::vector<int>& v) { if (!v.empty()) memcpy(at<int>(hin, o), v.data(), v.size() * sizeof(int)); };
   for (int k = 0; k <= 4; k++) put(iPred[k], predList[k]);
-  for (int k = 0; k < 4; k++) { put(iTeam[k], team[k]); put(iDq[k], dqOrder[k]); put(iRate[k], rateOrder[k]); }
+  for (int k = 0; k < 4; k++) { put(iTeam[k], L[k].team); put(iDq[k], L[k].dq); put(iRate[k], L[k].rate); }
   // work arena: per-step TU results, prediction, residual, reconstruction, levels, dequantised coefficients, derived prices
-  o = 0;
-  const size_t oRes = take((size_t)4 * n * sizeof(vvcb_tu_result)), oPred = take(cs * sizeof(int16_t)), oResi = take(cs * sizeof(int16_t)),
-               oReco = take(cs * sizeof(int16_t)), oLevel = take(cs * sizeof(int32_t)), oDeq = take(cs * sizeof(int32_t)),
-               oRates = take((size_t)n * sizeof(vvcb_dq_rates));
-  const size_t workBytes = o;
-  auto dq_grid = [&](int nDq) { const int g = nDq <= 2048 ? (nDq + kDqThreads / 32 - 1) / (kDqThreads / 32) : (nDq + kDqGroups - 1) / kDqGroups; return std::min(g, ctx->numSms * 4); };
-  int maxDq = 0, maxDqGrid = 0;                                      // the grid is not monotonic in the job count (sparse below 2049 jobs)
-  for (int k = 0; k < 4; k++) { maxDq = std::max(maxDq, (int)dqOrder[k].size()); maxDqGrid = std::max(maxDqGrid, dq_grid((int)dqOrder[k].size())); }
+  Arena work;
+  const size_t oRes = work.take((size_t)4 * n * sizeof(vvcb_tu_result)), oPred = work.take(cs * sizeof(int16_t)), oResi = work.take(cs * sizeof(int16_t)),
+               oReco = work.take(cs * sizeof(int16_t)), oLevel = work.take(cs * sizeof(int32_t)), oDeq = work.take(cs * sizeof(int32_t)),
+               oRates = work.take((size_t)n * sizeof(vvcb_dq_rates));
+  const int nDq[4] = { (int)L[0].dq.size(), (int)L[1].dq.size(), (int)L[2].dq.size(), (int)L[3].dq.size() };
   CK(cudaSetDevice(ctx->device));
-  if ((rc = tu_buf(ctx, 22, inBytes))) return rc;
-  if ((rc = tu_buf(ctx, 23, workBytes))) return rc;
-  if ((rc = tu_buf(ctx, 7, cs * sizeof(int32_t)))) return rc;
-  if (maxDq) {
-    if ((rc = tu_buf(ctx, 11, (size_t)n * sizeof(DqRateTab)))) return rc;
-    if ((rc = tu_buf(ctx, 12, (size_t)maxDqGrid * kDqGroups * kDqSlotBytes))) return rc;
-    if ((rc = tu_buf(ctx, 13, ((size_t)maxDq * 3 + kDqBins) * sizeof(int)))) return rc;
-  }
-  uint8_t* din = static_cast<uint8_t*>(ctx->dTu[22]);
-  uint8_t* dw = static_cast<uint8_t*>(ctx->dTu[23]);
-  CK(cudaMemcpyAsync(din, hin, inBytes, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemsetAsync(dw + oLevel, 0, oRates - oLevel, ctx->stream));        // levels / dequantised coefficients the quantisers do not reach stay zero
-  const IspCand* dCand = reinterpret_cast<const IspCand*>(din + iCand);
-  vvcb_tu_job* dJobs = reinterpret_cast<vvcb_tu_job*>(din + iJobs);
-  const uint8_t* dTr = din + iTr;
-  IspState* dState = reinterpret_cast<IspState*>(din + iState);
-  vvcb_ctx_states* dCst = reinterpret_cast<vvcb_ctx_states*>(din + iCst);
-  vvcb_tu_result* dRes = reinterpret_cast<vvcb_tu_result*>(dw + oRes);
-  int16_t* dPred = reinterpret_cast<int16_t*>(dw + oPred); int16_t* dResi = reinterpret_cast<int16_t*>(dw + oResi);
-  int16_t* dReco = reinterpret_cast<int16_t*>(dw + oReco);
-  int32_t* dLevel = reinterpret_cast<int32_t*>(dw + oLevel); int32_t* dDeq = reinterpret_cast<int32_t*>(dw + oDeq);
-  vvcb_dq_rates* dRates = reinterpret_cast<vvcb_dq_rates*>(dw + oRates);
+  if ((rc = tu_buf(ctx, kStageIn, in.size))) return rc;
+  if ((rc = tu_buf(ctx, kStageOut, work.size))) return rc;
+  if ((rc = quant_scratch(ctx, cs, n, nDq, 4))) return rc;
+  void* din = ctx->dTu[kStageIn];
+  void* dw = ctx->dTu[kStageOut];
+  CK(cudaMemcpyAsync(din, hin, in.size, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(at<uint8_t>(dw, oLevel), 0, oRates - oLevel, ctx->stream));        // levels / dequantised coefficients the quantisers do not reach stay zero
+  const IspCand* dCand = at<const IspCand>(din, iCand);
+  vvcb_tu_job* dJobs = at<vvcb_tu_job>(din, iJobs);
+  IspState* dState = at<IspState>(din, iState);
+  vvcb_ctx_states* dCst = at<vvcb_ctx_states>(din, iCst);
+  vvcb_tu_result* dRes = at<vvcb_tu_result>(dw, oRes);
+  int16_t* dPred = at<int16_t>(dw, oPred); int16_t* dResi = at<int16_t>(dw, oResi);
+  int16_t* dReco = at<int16_t>(dw, oReco); int32_t* dLevel = at<int32_t>(dw, oLevel);
   const bool tm = ctx->timing != 0;
   struct Events {                                    // per-stage timing of the steps (vvcb_tu_kernel_times); destroyed on every exit
     cudaEvent_t e[5 * 4] = {};
@@ -1703,7 +1700,7 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
     if (tm && k < 4) CK(cudaEventRecord(ev[5 * k], ctx->stream));
     if (!predList[k].empty()) {
       IspPredParams Q;
-      Q.cands = dCand; Q.list = reinterpret_cast<const int*>(din + iPred[k]); Q.n = (int)predList[k].size(); Q.k = k;
+      Q.cands = dCand; Q.list = at<const int>(din, iPred[k]); Q.n = (int)predList[k].size(); Q.k = k;
       Q.jobs = dJobs + (size_t)(k < 4 ? k : 3) * n; Q.prev = dRes + (size_t)(k > 0 ? k - 1 : 0) * n; Q.state = dState;
       Q.pred = dPred; Q.resi = dResi; Q.cuReco = dReco; Q.orig = ctx->bOrig; Q.reco = ctx->bReco; Q.stride = ctx->stride; Q.bd = ctx->bd;
       Q.rom = ctx->dRom; Q.frac = ctx->dRateRom->binFracBits;
@@ -1711,84 +1708,39 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
       isp_pred_kernel<<<g, kIspPredWarps * 32, 0, ctx->stream>>>(Q);
       ctx->launches++;
     }
-    if (k == 4 || team[k].empty()) continue;
-    const int nTeam = (int)team[k].size(), nS = nSmall[k], nL = nTeam - nS, nDq = (int)dqOrder[k].size(), nRate = (int)rateOrder[k].size();
-    const int* dTeam = reinterpret_cast<const int*>(din + iTeam[k]);
-    TuParams P;
-    P.jobs = dJobs + (size_t)k * n; P.list = nullptr; P.n = 0; P.resi = dResi; P.pred = dPred; P.coeff = nullptr; P.level = dLevel; P.reco = dReco;
-    P.results = dRes + (size_t)k * n; P.orig = ctx->bOrig; P.stride = ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
-    P.dqCoeff = static_cast<int32_t*>(ctx->dTu[7]); P.dqDeq = dDeq; P.phase = 0; P.trPair = dTr + (size_t)k * n;
-    auto launch_tu = [&](TuParams Q) {
-      if (nS) { Q.list = dTeam; Q.n = nS; tu_eval_kernel<32><<<std::min((nS + 3) / 4, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
-      if (nL) { Q.list = dTeam + nS; Q.n = nL; tu_eval_kernel<128><<<std::min(nL, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
-    };
-    launch_tu(P);
-    if (tm) CK(cudaEventRecord(ev[5 * k + 1], ctx->stream));
-    if (nDq) {
-      const int* dOrder = reinterpret_cast<const int*>(din + iDq[k]);
-      const long long nPrice = (long long)n * kDqRateModels;
-      rates_from_states_kernel<<<(unsigned)((nPrice + 127) / 128), 128, 0, ctx->stream>>>(dCst, n, ctx->dRateRom, dRates);
-      dq_rate_kernel<<<n, 32, 0, ctx->stream>>>(dRates, n, static_cast<DqRateTab*>(ctx->dTu[11]));
-      int* firstRaw = static_cast<int*>(ctx->dTu[13]);
-      int* orderSorted = firstRaw + nDq;
-      int* firstSorted = firstRaw + 2 * nDq;
-      const int firstGrid = std::min((nDq + kDqGroups - 1) / kDqGroups, ctx->numSms * 8);
-      dq_first_kernel<<<firstGrid, kDqThreads, 0, ctx->stream>>>(P.jobs, dOrder, nDq, P.dqCoeff, ctx->dDqRom, ctx->bd, firstRaw);
-      ctx->launches += 3;
-      const bool sortJobs = nDq > 2048;                            // as tu_eval_impl: sweeps sort by first test position, walks do not
-      if (sortJobs) {
-        int* binCount = firstRaw + 3 * (size_t)nDq;
-        const int sortGrid = (nDq + kDqSortPerBlock - 1) / kDqSortPerBlock;
-        CK(cudaMemsetAsync(binCount, 0, kDqBins * sizeof(int), ctx->stream));
-        dq_hist_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(firstRaw, nDq, binCount);
-        dq_scan_kernel<<<1, 32, 0, ctx->stream>>>(binCount);
-        dq_scatter_kernel<<<sortGrid, kDqSortThreads, 0, ctx->stream>>>(dOrder, firstRaw, nDq, binCount, orderSorted, firstSorted);
-        ctx->launches += 3;
-      }
-      DqParams D;
-      D.jobs = P.jobs; D.order = sortJobs ? orderSorted : dOrder; D.firstPos = sortJobs ? firstSorted : firstRaw; D.n = nDq;
-      D.coeff = P.dqCoeff; D.level = P.level; D.deq = dDeq; D.results = P.results;
-      D.rates = dRates; D.tabs = static_cast<const DqRateTab*>(ctx->dTu[11]);
-      D.rom = ctx->dDqRom; D.scratch = static_cast<uint8_t*>(ctx->dTu[12]); D.bd = ctx->bd; D.sparse = !sortJobs;
-      dq_kernel<<<dq_grid(nDq), kDqThreads, 0, ctx->stream>>>(D);
-      ctx->launches++;
-    }
-    if (tm) CK(cudaEventRecord(ev[5 * k + 2], ctx->stream));
-    if (nDq) { P.phase = 1; launch_tu(P); }
-    if (tm) CK(cudaEventRecord(ev[5 * k + 3], ctx->stream));
-    if (nRate) {
-      RateParams R;
-      R.jobs = P.jobs; R.order = reinterpret_cast<const int*>(din + iRate[k]); R.n = nRate; R.level = P.level; R.results = P.results;
-      R.states = dCst; R.statesOut = dCst; R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
-      rate_kernel<<<std::min((nRate + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
-      ctx->launches++;
-    }
-    if (tm) CK(cudaEventRecord(ev[5 * k + 4], ctx->stream));
+    if (k == 4 || L[k].team.empty()) continue;
+    TuChain c = {};
+    c.jobs = dJobs + (size_t)k * n; c.trPair = at<const uint8_t>(din, iTr) + (size_t)k * n;
+    c.team = at<const int>(din, iTeam[k]); c.dq = at<const int>(din, iDq[k]); c.rate = at<const int>(din, iRate[k]);
+    c.resi = dResi; c.pred = dPred; c.level = dLevel; c.reco = dReco; c.deq = at<int32_t>(dw, oDeq); c.results = dRes + (size_t)k * n;
+    c.rates = at<vvcb_dq_rates>(dw, oRates); c.nRates = n; c.priceFrom = dCst;
+    c.states = dCst; c.statesOut = dCst;                             // the block's models adapted in place for the next block
+    if ((rc = run_tu_chain(ctx, c, L[k], tm ? ev + 5 * k : nullptr))) return rc;
   }
   CK(cudaGetLastError());
   // page-locked output staging: per-step results, cbf state, then the wanted sample outputs of the chunk's densely packed candidates
-  o = 0;
-  const size_t hRes = take((size_t)4 * n * sizeof(vvcb_tu_result)), hSt = take((size_t)n * sizeof(IspState)),
-               hLv = take(level ? cs * sizeof(int32_t) : 0), hRc = take(reco ? cs * sizeof(int16_t) : 0), hPr = take(pred ? cs * sizeof(int16_t) : 0);
-  if ((rc = pin_buf(ctx, 7, o))) return rc;
-  uint8_t* hout = static_cast<uint8_t*>(ctx->hPin[7]);
-  CK(cudaMemcpyAsync(hout + hRes, dRes, (size_t)4 * n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(hout + hSt, dState, (size_t)n * sizeof(IspState), cudaMemcpyDeviceToHost, ctx->stream));
-  if (level) CK(cudaMemcpyAsync(hout + hLv, dLevel, cs * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (reco) CK(cudaMemcpyAsync(hout + hRc, dReco, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (pred) CK(cudaMemcpyAsync(hout + hPr, dPred, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  Arena out;
+  const size_t hRes = out.take((size_t)4 * n * sizeof(vvcb_tu_result)), hSt = out.take((size_t)n * sizeof(IspState)),
+               hLv = out.take(level ? cs * sizeof(int32_t) : 0), hRc = out.take(reco ? cs * sizeof(int16_t) : 0), hPr = out.take(pred ? cs * sizeof(int16_t) : 0);
+  if ((rc = pin_buf(ctx, kPinStageOut, out.size))) return rc;
+  void* hout = ctx->hPin[kPinStageOut];
+  CK(cudaMemcpyAsync(at<uint8_t>(hout, hRes), dRes, (size_t)4 * n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(at<uint8_t>(hout, hSt), dState, (size_t)n * sizeof(IspState), cudaMemcpyDeviceToHost, ctx->stream));
+  if (level) CK(cudaMemcpyAsync(at<uint8_t>(hout, hLv), dLevel, cs * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (reco) CK(cudaMemcpyAsync(at<uint8_t>(hout, hRc), dReco, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (pred) CK(cudaMemcpyAsync(at<uint8_t>(hout, hPr), dPred, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
   CK(ctx_sync(ctx));
-  const vvcb_tu_result* res = reinterpret_cast<const vvcb_tu_result*>(hout + hRes);
-  memcpy(ist.data(), hout + hSt, (size_t)n * sizeof(IspState));
+  const vvcb_tu_result* res = at<const vvcb_tu_result>(hout, hRes);
+  memcpy(ist.data(), at<IspState>(hout, hSt), (size_t)n * sizeof(IspState));
   for (int i = 0; i < n; i++) {                      // each candidate's samples to the caller's offset
     const size_t from = cands[i].offset, to = jobs[i].offset, m = (size_t)cands[i].cuW * cands[i].cuH;
-    if (level) memcpy(level + to, reinterpret_cast<const int32_t*>(hout + hLv) + from, m * sizeof(int32_t));
-    if (reco) memcpy(reco + to, reinterpret_cast<const int16_t*>(hout + hRc) + from, m * sizeof(int16_t));
-    if (pred) memcpy(pred + to, reinterpret_cast<const int16_t*>(hout + hPr) + from, m * sizeof(int16_t));
+    if (level) memcpy(level + to, at<const int32_t>(hout, hLv) + from, m * sizeof(int32_t));
+    if (reco) memcpy(reco + to, at<const int16_t>(hout, hRc) + from, m * sizeof(int16_t));
+    if (pred) memcpy(pred + to, at<const int16_t>(hout, hPr) + from, m * sizeof(int16_t));
   }
   if (tm) {
     for (int k = 0; k < 4; k++) {
-      if (team[k].empty()) continue;
+      if (L[k].team.empty()) continue;
       for (int i = 0; i < 4; i++) { float ms = 0; CK(cudaEventElapsedTime(&ms, ev[5 * k + i], ev[5 * k + i + 1])); ctx->tuMs[i] += ms; }
     }
     ctx->tuTimed++;
