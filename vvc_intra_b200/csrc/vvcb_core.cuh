@@ -79,6 +79,24 @@ VHD int add_halves_u16x2(uint32_t w, int acc)
 #endif
 }
 
+// c + the signed int16 pair a times the signed int8 pair in bytes 0, 1 (lo) or 2, 3 (hi) of b: one IDP.2A.S16.S8 on the device
+VHD int dot2_s16_s8_lo(uint32_t a, uint32_t b, int c)
+{
+#if defined(__CUDA_ARCH__)
+  return __dp2a_lo((int)a, (int)b, c);
+#else
+  return c + (int)(int16_t)(a & 0xffffu) * (int)(int8_t)(b & 0xffu) + (int)(int16_t)(a >> 16) * (int)(int8_t)((b >> 8) & 0xffu);
+#endif
+}
+VHD int dot2_s16_s8_hi(uint32_t a, uint32_t b, int c)
+{
+#if defined(__CUDA_ARCH__)
+  return __dp2a_hi((int)a, (int)b, c);
+#else
+  return c + (int)(int16_t)(a & 0xffffu) * (int)(int8_t)((b >> 16) & 0xffu) + (int)(int16_t)(a >> 16) * (int)(int8_t)(b >> 24);
+#endif
+}
+
 // Per (shape, mode) prediction parameters, precomputed on the host at context creation.
 struct ModeParam {
   int16_t  angle;        // intraPredAngle (signed)
@@ -250,13 +268,24 @@ VHD void line_pos(const LineGeom& g, int i, bool& isLeft, int& k, int& dx, int& 
   else           { isLeft = false; k = i - nLeft;  dx = -1 - g.mrl + k; dy = -1 - g.mrl; }
 }
 
+// ---- MIP matrices for IDP.2A ---------------------------------------------------------------------------
+// Per matrix family (0: 4x4, 18 modes of 16 rows x 4 weights; 1: 8x8, 10 modes of 16 x 8; 2: 16x16, 6 modes of 64 x 7) and mode: its rows
+// as packed int8 weights, one word (family 0) or two words (1, 2) per row, then one header row whose first word is shift | offset << 8.
+// The 16x16 family's 7 columns get a zero weight in front, standing for its first input, which that family drops (and which the input
+// vector holds as 0), so a row is the dot product of the 4 or 8 inputs with two or four IDP.2A.  The header row also staggers the modes
+// over the shared-memory banks (mode stride = odd number of rows): the lanes of a warp iteration reading the same row of different modes
+// hit different banks.  The weights are 0..123, so they read the same as signed bytes.
+VHD int mip_mode_words(int family) { return family == 0 ? 17 : (family == 1 ? 34 : 130); }
+VHD int mip_family_words(int family) { return family == 0 ? 18 * 17 : (family == 1 ? 10 * 34 : 6 * 130); }
+VHD int mip_family_base(int family) { return family == 0 ? 0 : (family == 1 ? 18 * 17 : 18 * 17 + 10 * 34); }
+constexpr int kMipRomWords = 18 * 17 + 10 * 34 + 6 * 130;   // 5 704 bytes
+
 // ---- 4-tap filter tables (packed int8 x4, one word per fractional position) -------------------------
 struct Rom {
   uint32_t filt[2][32];                    // [0] cubic (CL/InterpolationFilter.cpp:100), [1] Gaussian (CL/IntraPrediction.cpp:76)
   ModeParam mode[6][6][VVCB_NUM_LUMA_MODE];  // [log2w-2][log2h-2][mode], reference line 0
   uint8_t angOrder[6][6][65];              // angular modes 2..66 ordered by (hor/ver, PDPC class) so that the lanes of a warp agree
-  uint8_t mip4[18 * 16 * 4], mip8[10 * 16 * 8], mip16[6 * 64 * 7];
-  uint8_t mipOff4[18], mipSh4[18], mipOff8[10], mipSh8[10], mipOff16[6], mipSh16[6];
+  alignas(16) uint32_t mip[kMipRomWords];  // MIP matrices, shifts and offsets in the layout above (two-word rows read as one 8-byte load)
 };
 
 // ---- register-resident Walsh-Hadamard pieces -------------------------------------------------------
@@ -439,7 +468,7 @@ template <int R, int C> VHD void pred_planar_dc_unit(const int16_t* top, const i
 
 // ---- MIP --------------------------------------------------------------------------------------------
 struct MipGeom {
-  int numModes, small, bsz, redW, redH, upH, upV, grid, cols;
+  int numModes, small, bsz, redW, redH, upH, upV, grid;
   int lgRedW, lgUpH, lgUpV;
   int family;            // 0: 4x4 matrices (4 inputs), 1: 8x8 matrices (8 inputs), 2: 16x16 matrices (7 inputs, first column dropped)
 };
@@ -454,7 +483,6 @@ VHD MipGeom make_mip_geom(int w, int h)
   g.redH  = g.small ? 4 : vmin(h, 8);
   g.upH   = w / g.redW; g.upV = h / g.redH;
   g.grid  = g.small ? 4 : 8;
-  g.cols  = (w == 4 && h == 4) ? 4 : (g.small ? 8 : 7);
   g.lgRedW = vlog2(g.redW); g.lgUpH = vlog2(g.upH); g.lgUpV = vlog2(g.upV);
   g.family = (w == 4 && h == 4) ? 0 : (g.small ? 1 : 2);
   return g;
@@ -462,28 +490,47 @@ VHD MipGeom make_mip_geom(int w, int h)
 
 // Everything one MIP mode needs besides the visit's boundary (CL/MatrixIntraPrediction.cpp:211-254, 570-591)
 struct MipSlot {
-  const uint8_t* mat;
+  const uint32_t* mat;   // the mode's rows in Rom::mip's layout
   int shift, off, inOff;
   bool transpose;
-  int in[8];             // rebased reduced boundary (zero padded); in[0] == 0 for the 16x16 family
+  uint32_t in[4];        // rebased reduced boundary (zero padded) as int16 pairs; input 0 is 0 for the 16x16 family
 };
 
-// mipIn[t][i]: rebased input vector of orientation t (0 normal, 1 transposed); mipAux: {inOff[0], inOff[1], sum[0], sum[1]}
-VHD MipSlot make_mip_slot(const Rom& rom, const MipGeom& g, const int16_t (*mipIn)[8], const int* mipAux, int mode)
+// famRom: g.family's part of Rom::mip (in global memory or a shared-memory copy); mipIn[t][i]: rebased input vector of orientation t
+// (0 normal, 1 transposed), word aligned; mipAux: {inOff[0], inOff[1], sum[0], sum[1]}
+VHD MipSlot make_mip_slot(const uint32_t* famRom, const MipGeom& g, const int16_t (*mipIn)[8], const int* mipAux, int mode)
 {
   MipSlot m;
   m.transpose = mode > g.numModes / 2;
   const int widx = m.transpose ? mode - g.numModes / 2 : mode;
-  int offs;
-  if (g.family == 0)      { m.mat = rom.mip4 + widx * 64;   m.shift = rom.mipSh4[widx];  offs = rom.mipOff4[widx]; }
-  else if (g.family == 1) { m.mat = rom.mip8 + widx * 128;  m.shift = rom.mipSh8[widx];  offs = rom.mipOff8[widx]; }
-  else                    { m.mat = rom.mip16 + widx * 448; m.shift = rom.mipSh16[widx]; offs = rom.mipOff16[widx]; }
+  m.mat = famRom + widx * mip_mode_words(g.family);
+  const uint32_t head = m.mat[g.family == 2 ? 128 : (g.family == 1 ? 32 : 16)];
+  m.shift = (int)(head & 0xffu);
   const int t = m.transpose ? 1 : 0;
+  const uint32_t* in2 = reinterpret_cast<const uint32_t*>(mipIn[t]);
 #pragma unroll
-  for (int i = 0; i < 8; i++) m.in[i] = mipIn[t][i];
+  for (int i = 0; i < 4; i++) m.in[i] = in2[i];
   m.inOff = mipAux[t];
-  m.off = (1 << (m.shift - 1)) - offs * mipAux[2 + t];
+  m.off = (1 << (m.shift - 1)) - (int)(head >> 8) * mipAux[2 + t];
   return m;
+}
+
+// Reduced sample of matrix row `row`: WIDE = 8 inputs (8x8 and 16x16 families), else 4 (4x4 family)
+template <bool WIDE> VHD int mip_row_sample(const MipSlot& m, int row, int maxv)
+{
+  int acc;
+  if (WIDE) {
+    const uint2 w = reinterpret_cast<const uint2*>(m.mat)[row];
+    acc = dot2_s16_s8_lo(m.in[0], w.x, m.off);
+    acc = dot2_s16_s8_hi(m.in[1], w.x, acc);
+    acc = dot2_s16_s8_lo(m.in[2], w.y, acc);
+    acc = dot2_s16_s8_hi(m.in[3], w.y, acc);
+  } else {
+    const uint32_t w = m.mat[row];
+    acc = dot2_s16_s8_lo(m.in[0], w, m.off);
+    acc = dot2_s16_s8_hi(m.in[1], w, acc);
+  }
+  return clip_bd((acc >> m.shift) + m.inOff, maxv);
 }
 
 // One sample of the reduced prediction at logical position (rx, ry), CL/MatrixIntraPrediction.cpp:637-741.
@@ -493,19 +540,7 @@ VHD int mip_reduced_sample(const MipSlot& m, const MipGeom& g, int w, int h, int
   int xx = rx, yy = ry, iw = g.redW;
   if (m.transpose) { const bool t = lho; lho = lvo; lvo = t; xx = ry; yy = rx; iw = g.redH; }
   const int row = (lvo ? 2 * yy : yy) * (g.small ? iw : g.grid) + (lho ? 2 * xx : xx);
-  const uint8_t* wgt = m.mat + row * g.cols;
-  int acc = m.off;
-  if (g.family == 0) {
-#pragma unroll
-    for (int i = 0; i < 4; i++) acc += m.in[i] * wgt[i];
-  } else if (g.family == 1) {
-#pragma unroll
-    for (int i = 0; i < 8; i++) acc += m.in[i] * wgt[i];
-  } else {
-#pragma unroll
-    for (int i = 1; i < 8; i++) acc += m.in[i] * wgt[i - 1];
-  }
-  return clip_bd((acc >> m.shift) + m.inOff, maxv);
+  return g.family == 0 ? mip_row_sample<false>(m, row, maxv) : mip_row_sample<true>(m, row, maxv);
 }
 
 // ---- mode bits (lists kernel) -----------------------------------------------------------------------

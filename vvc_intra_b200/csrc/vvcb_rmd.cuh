@@ -556,7 +556,7 @@ template <class SM>
 __device__ void build_mip_planes(int16_t* red, int16_t* plane, const Rom& rom, const SM& sm, const MipGeom& mg, const Shape& sh,
                                  int bd, int mode, int gl, int gsize)
 {
-  const MipSlot ms = make_mip_slot(rom, mg, sm.mipIn, sm.mipAux, mode);
+  const MipSlot ms = make_mip_slot(rom.mip + mip_family_base(mg.family), mg, sm.mipIn, sm.mipAux, mode);
   const int nRed = mg.redW * mg.redH, maxv = (1 << bd) - 1;
   for (int i = gl; i < nRed; i += gsize)
     red[i] = (int16_t)mip_reduced_sample(ms, mg, sh.w, sh.h, maxv, i & (mg.redW - 1), i >> mg.lgRedW);
@@ -623,6 +623,63 @@ __device__ __forceinline__ void predict_mip(const SM& sm, const int16_t* plane, 
   }
 }
 
+// MIP prediction of piece k of a slot that one lane owns: the packed 4x4, 8x4, 4x8 and 8x8 shapes, one per tile class TILE 0..3
+// (4x4 matrices for 4x4, 8x8 matrices for the others; a 4 x 4 reduced block).  The reduced samples the piece needs are computed in
+// registers and up-sampled there (CL/MatrixIntraPrediction.cpp:469-567), with no plane in shared memory and no pass for an identity
+// direction.  Pieces come in order k = 0, 1 (4x4: k = 0 only): 8x4 takes reduced columns 2k, 2k + 1, 4x8 and 8x8 reduced rows 2k, 2k + 1;
+// `carry` hands piece 1 the last reduced column / row of piece 0, the sample before its first one.
+template <int TILE, int R, int C, class SM>
+__device__ __forceinline__ void predict_mip_lane(const SM& sm, const MipSlot& ms, int k, int maxv, int (&carry)[4], int (&q)[R][C])
+{
+  const int16_t* top = sm.lines[0][0];
+  const int16_t* left = sm.lines[0][1];
+  // matrix row of reduced sample (ry, rx): ry * 4 + rx, transposed modes rx * 4 + ry
+  const int stepY = ms.transpose ? 1 : 4, stepX = ms.transpose ? 4 : 1;
+  if constexpr (TILE == 0) {
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+#pragma unroll
+      for (int j = 0; j < 4; j++) q[i][j] = mip_row_sample<false>(ms, i * stepY + j * stepX, maxv);
+  } else if constexpr (TILE == 1) {
+    // 8x4: the vertical pass is the identity; horizontal up-sampling by 2 from the left boundary
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      const int b  = k ? carry[i] : left[1 + i];
+      const int r0 = mip_row_sample<true>(ms, i * stepY + 2 * k * stepX, maxv);
+      const int r1 = mip_row_sample<true>(ms, i * stepY + (2 * k + 1) * stepX, maxv);
+      q[i][0] = (b + r0 + 1) >> 1; q[i][1] = r0; q[i][2] = (r0 + r1 + 1) >> 1; q[i][3] = r1;
+      carry[i] = r1;
+    }
+  } else {
+    // 4x8, 8x8: vertical up-sampling by 2 from the top boundary (at the reduced columns), then for 8x8 horizontal by 2 from the left one
+    int v[4][4];
+#pragma unroll
+    for (int rx = 0; rx < 4; rx++) {
+      const int b  = k ? carry[rx] : top[TILE == 3 ? 2 + 2 * rx : 1 + rx];
+      const int r0 = mip_row_sample<true>(ms, 2 * k * stepY + rx * stepX, maxv);
+      const int r1 = mip_row_sample<true>(ms, (2 * k + 1) * stepY + rx * stepX, maxv);
+      v[0][rx] = (b + r0 + 1) >> 1; v[1][rx] = r0; v[2][rx] = (r0 + r1 + 1) >> 1; v[3][rx] = r1;
+      carry[rx] = r1;
+    }
+    if constexpr (TILE == 2) {
+#pragma unroll
+      for (int i = 0; i < 4; i++)
+#pragma unroll
+        for (int j = 0; j < 4; j++) q[i][j] = v[i][j];
+    } else {
+#pragma unroll
+      for (int i = 0; i < 4; i++) {
+        const int l = left[1 + 4 * k + i];
+#pragma unroll
+        for (int rx = 0; rx < 4; rx++) {
+          q[i][2 * rx]     = ((rx ? v[i][rx - 1] : l) + v[i][rx] + 1) >> 1;
+          q[i][2 * rx + 1] = v[i][rx];
+        }
+      }
+    }
+  }
+}
+
 // =====================================================================================================
 // the evaluation kernel, one instantiation per (SATD tile class, prediction kind)
 // =====================================================================================================
@@ -660,14 +717,25 @@ template <bool PACK> struct EvalShared {
   uint32_t sFilt[64];
 };
 
+// MIP slots that one lane owns (4x4, 8x4, 4x8, 8x8) are predicted in registers (predict_mip_lane), with the matrices of their family
+// (4x4 for the 4x4 class, 8x8 for the others) copied to shared memory: at most 1 360 bytes, which fit under the 48 KB of static shared
+// memory beside EvalShared; the slots of larger shapes read theirs from the ROM in global memory.  The lane-owned shapes come in packed
+// items, and in plain items only for the prediction-output kernels (MODE 2).
+template <int TILE, int KIND, int MODE> constexpr bool kLaneMip = KIND == KIND_MIP && TILE < 4 && MODE != 0;
+constexpr int kMipLaneWords = 10 * 34;       // the larger of mip_family_words(0), mip_family_words(1)
+
+// sMip: kMipLaneWords of shared memory when kLaneMip<TILE, KIND, MODE>
 template <int TILE, int KIND, int MODE>
-__device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MODE == 1>& shm)
+__device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MODE == 1>& shm, uint32_t* sMip)
 {
   constexpr bool PACK = MODE == 1, WITH_PRED = MODE == 2;
   using Cfg = EvalCfg<PACK>;
   using SM = typename Cfg::Smem;
   constexpr int S = TILE < 3 ? 4 : 8;
   constexpr int V = Cfg::kVisits;
+  constexpr bool LANE_MIP = kLaneMip<TILE, KIND, MODE>;
+  constexpr bool ONLY_LANE_MIP = LANE_MIP && PACK && (TILE == 0 || TILE == 3);    // the packed 4x4 and 8x8 classes hold nothing else
+  constexpr int MIP_FAMILY = TILE == 0 ? 0 : 1;
   auto& smem = shm.smem;
   auto& sScratch = shm.sScratch;
   auto& sVisit = shm.sVisit;
@@ -676,6 +744,8 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
   auto& sFilt = shm.sFilt;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if (threadIdx.x < 64) sFilt[threadIdx.x] = (&P.rom->filt[0][0])[threadIdx.x];
+  if (LANE_MIP)
+    for (int i = threadIdx.x; i < mip_family_words(MIP_FAMILY); i += Cfg::kThreads) sMip[i] = P.rom->mip[mip_family_base(MIP_FAMILY) + i];
   __syncthreads();
   const Rom& rom = *P.rom;
 
@@ -778,10 +848,11 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
       // ---- per-slot scratch built by the slot's lanes
       __syncwarp();
       int dc = 0;
+      const bool laneMip = ONLY_LANE_MIP || (LANE_MIP && lanes == 1);     // uniform over the warp: one shape per item
       if (KIND == KIND_ANG) {
         if (s.p.angle < 0) build_projected_line(scratch, sm, s, s.p.is_ver ? sh.w : sh.h, s.p.is_ver ? sh.h : sh.w, gl, gsize);
       } else if (KIND == KIND_MIP) {
-        build_mip_planes(scratch, scratch + mip_plane_offset(mg, sh), rom, sm, mg, sh, P.bd, s.mode, gl, gsize);
+        if (!laneMip) build_mip_planes(scratch, scratch + mip_plane_offset(mg, sh), rom, sm, mg, sh, P.bd, s.mode, gl, gsize);
       } else {
         // DC value (CL/IntraPrediction.cpp:248-285), summed by the slot's lanes
         int part = 0;
@@ -799,6 +870,9 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
 
       int sad = 0, satd = 0;
       const bool transposed = KIND == KIND_ANG && !s.p.is_ver;
+      MipSlot ms = {};
+      int mipCarry[4] = {};
+      if (laneMip) ms = make_mip_slot(sMip, mg, sm.mipIn, sm.mipAux, s.mode);
       if constexpr (S == 8) {
         // An 8x8 unit is processed as two 4x8 halves by the same loop body (kept rolled: the fully unrolled unit was
         // > 64 KB of code and instruction-fetch bound, profiles/r1m_summary.md history).  Rows and the first two column stages of the
@@ -816,6 +890,7 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
           int q[4][8], d[4][8];
           const int hx = transposed ? x0 + 4 * k : x0, hy = transposed ? y0 : y0 + 4 * k;   // picture origin of the half
           if (KIND == KIND_ANG)      predict_angular<4, 8>(sm, scratch, s, sh, sFilt, P.bd, x0, y0, 4 * k, q);
+          else if (KIND == KIND_MIP && laneMip) predict_mip_lane<TILE, 4, 8>(sm, ms, k, (1 << P.bd) - 1, mipCarry, q);
           else if (KIND == KIND_MIP) predict_mip<4, 8>(sm, scratch + mip_plane_offset(mg, sh), mg, sh, hx, hy, q);
           else pred_planar_dc_unit<4, 8>(sm.lines[s.set][0], sm.lines[s.set][1], s.kind, s.p.pdpc, dc, sh.lw, sh.lh, hx, hy, q);
           if (WITH_PRED && P.predOut && act) store_pred<4, 8>(P.predOut + (size_t)slot * sh.w * sh.h, sh.w, hx, hy, transposed, q);
@@ -860,6 +935,7 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
           const int y0 = ty * (TILE == 2 ? 8 : 4) + (TILE == 2 ? 4 * k : 0);
           int q[4][4], d[4][4];
           if (KIND == KIND_ANG)      predict_angular<4, 4>(sm, scratch, s, sh, sFilt, P.bd, x0, y0, 0, q);
+          else if (KIND == KIND_MIP && laneMip) predict_mip_lane<TILE, 4, 4>(sm, ms, k, (1 << P.bd) - 1, mipCarry, q);
           else if (KIND == KIND_MIP) predict_mip<4, 4>(sm, scratch + mip_plane_offset(mg, sh), mg, sh, x0, y0, q);
           else pred_planar_dc_unit<4, 4>(sm.lines[s.set][0], sm.lines[s.set][1], s.kind, s.p.pdpc, dc, sh.lw, sh.lh, x0, y0, q);
           if (WITH_PRED && P.predOut && act) store_pred<4, 4>(P.predOut + (size_t)slot * sh.w * sh.h, sh.w, x0, y0, transposed, q);
@@ -922,7 +998,10 @@ template <int TILE, int KIND, int MODE>
 __global__ void __launch_bounds__(EvalCfg<MODE == 1>::kThreads, EvalCfg<MODE == 1>::kMinCtas) rmd_eval_kernel(EvalParams P)
 {
   __shared__ EvalShared<MODE == 1> shm;
-  rmd_eval_body<TILE, KIND, MODE>(P, shm);
+  if constexpr (kLaneMip<TILE, KIND, MODE>) {
+    alignas(16) __shared__ uint32_t sMip[kMipLaneWords];
+    rmd_eval_body<TILE, KIND, MODE>(P, shm, sMip);
+  } else rmd_eval_body<TILE, KIND, MODE>(P, shm, nullptr);
 }
 
 // One launch for every bucket a walk-sized batch occupies (vvcb_cu_eval: a few dozen visits of mixed shapes): the CTAs of the grid are dealt
@@ -938,15 +1017,16 @@ template <int MODE>
 __global__ void __launch_bounds__(EvalCfg<MODE == 1>::kThreads, EvalCfg<MODE == 1>::kMinCtas) rmd_eval_any_kernel(EvalParams P, EvalAny A)
 {
   __shared__ EvalShared<MODE == 1> shm;
+  alignas(16) __shared__ uint32_t sMip[MODE == 0 ? 1 : kMipLaneWords];
   int k = 0;
   while (k + 1 < A.n && (int)blockIdx.x >= A.firstCta[k + 1]) k++;
   switch (A.bucket[k]) {
-    case 0:  rmd_eval_body<0, 0, MODE>(P, shm); break;  case 1:  rmd_eval_body<0, 1, MODE>(P, shm); break;  case 2:  rmd_eval_body<0, 2, MODE>(P, shm); break;
-    case 3:  rmd_eval_body<1, 0, MODE>(P, shm); break;  case 4:  rmd_eval_body<1, 1, MODE>(P, shm); break;  case 5:  rmd_eval_body<1, 2, MODE>(P, shm); break;
-    case 6:  rmd_eval_body<2, 0, MODE>(P, shm); break;  case 7:  rmd_eval_body<2, 1, MODE>(P, shm); break;  case 8:  rmd_eval_body<2, 2, MODE>(P, shm); break;
-    case 9:  rmd_eval_body<3, 0, MODE>(P, shm); break;  case 10: rmd_eval_body<3, 1, MODE>(P, shm); break;  case 11: rmd_eval_body<3, 2, MODE>(P, shm); break;
-    case 12: rmd_eval_body<4, 0, MODE>(P, shm); break;  case 13: rmd_eval_body<4, 1, MODE>(P, shm); break;  case 14: rmd_eval_body<4, 2, MODE>(P, shm); break;
-    case 15: rmd_eval_body<5, 0, MODE>(P, shm); break;  case 16: rmd_eval_body<5, 1, MODE>(P, shm); break;  case 17: rmd_eval_body<5, 2, MODE>(P, shm); break;
+    case 0:  rmd_eval_body<0, 0, MODE>(P, shm, sMip); break;  case 1:  rmd_eval_body<0, 1, MODE>(P, shm, sMip); break;  case 2:  rmd_eval_body<0, 2, MODE>(P, shm, sMip); break;
+    case 3:  rmd_eval_body<1, 0, MODE>(P, shm, sMip); break;  case 4:  rmd_eval_body<1, 1, MODE>(P, shm, sMip); break;  case 5:  rmd_eval_body<1, 2, MODE>(P, shm, sMip); break;
+    case 6:  rmd_eval_body<2, 0, MODE>(P, shm, sMip); break;  case 7:  rmd_eval_body<2, 1, MODE>(P, shm, sMip); break;  case 8:  rmd_eval_body<2, 2, MODE>(P, shm, sMip); break;
+    case 9:  rmd_eval_body<3, 0, MODE>(P, shm, sMip); break;  case 10: rmd_eval_body<3, 1, MODE>(P, shm, sMip); break;  case 11: rmd_eval_body<3, 2, MODE>(P, shm, sMip); break;
+    case 12: rmd_eval_body<4, 0, MODE>(P, shm, sMip); break;  case 13: rmd_eval_body<4, 1, MODE>(P, shm, sMip); break;  case 14: rmd_eval_body<4, 2, MODE>(P, shm, sMip); break;
+    case 15: rmd_eval_body<5, 0, MODE>(P, shm, sMip); break;  case 16: rmd_eval_body<5, 1, MODE>(P, shm, sMip); break;  case 17: rmd_eval_body<5, 2, MODE>(P, shm, sMip); break;
   }
 }
 

@@ -1,5 +1,6 @@
-// Host-side construction of the device ROM (filter words, per-shape mode parameters, MIP matrices).
+// Host-side construction of the device ROM (filter words, per-shape mode parameters, MIP matrices in IDP.2A form).
 #pragma once
+#include <stdlib.h>
 #include <string.h>
 #include "vvcb_core.cuh"
 #include "vvc_rom_tables.h"
@@ -26,12 +27,24 @@ inline void fill_rom(Rom& r)
           if (p.is_ver * 3 + cls == key) r.angOrder[lw - 2][lh - 2][n++] = (uint8_t)m;
         }
     }
-  memcpy(r.mip4, kMipMatrix4x4, sizeof(r.mip4));
-  memcpy(r.mip8, kMipMatrix8x8, sizeof(r.mip8));
-  memcpy(r.mip16, kMipMatrix16x16, sizeof(r.mip16));
-  memcpy(r.mipOff4, kMipOffset4x4, 18); memcpy(r.mipSh4, kMipShift4x4, 18);
-  memcpy(r.mipOff8, kMipOffset8x8, 10); memcpy(r.mipSh8, kMipShift8x8, 10);
-  memcpy(r.mipOff16, kMipOffset16x16, 6); memcpy(r.mipSh16, kMipShift16x16, 6);
+  // MIP matrices in Rom::mip's layout: rows of 4 or 8 int8 weights (the 16x16 family's 7 behind a zero), then the header row
+  static const uint8_t* const mat[3] = { kMipMatrix4x4, kMipMatrix8x8, kMipMatrix16x16 };
+  static const uint8_t* const off[3] = { kMipOffset4x4, kMipOffset8x8, kMipOffset16x16 };
+  static const uint8_t* const sh[3] = { kMipShift4x4, kMipShift8x8, kMipShift16x16 };
+  static const int modes[3] = { 18, 10, 6 }, rows[3] = { 16, 16, 64 }, cols[3] = { 4, 8, 7 };
+  for (int f = 0; f < 3; f++)
+    for (int m = 0; m < modes[f]; m++) {
+      uint32_t* dst = r.mip + mip_family_base(f) + m * mip_mode_words(f);
+      const int rowWords = f ? 2 : 1;
+      for (int y = 0; y < rows[f]; y++)
+        for (int c = 0; c < cols[f]; c++) {
+          const uint8_t wgt = mat[f][(m * rows[f] + y) * cols[f] + c];
+          if (wgt > 127) abort();                    // read as a signed byte by IDP.2A
+          const int k = c + (f == 2 ? 1 : 0);
+          dst[y * rowWords + (k >> 2)] |= (uint32_t)wgt << (8 * (k & 3));
+        }
+      dst[rows[f] * rowWords] = (uint32_t)sh[f][m] | ((uint32_t)off[f][m] << 8);
+    }
 }
 
 }  // namespace vvcb
