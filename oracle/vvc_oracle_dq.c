@@ -192,7 +192,10 @@ static void init_quant(dq_quant* q, int bd, int w, int h, int qp, double lambda)
   dfShift = ceil_log2_u64((uint64_t)pow2dfShift);
   q->distShift = 62 + q->qShift - 2 * 15 - dfShift;
   q->distAdd = ((int64_t)1 << q->distShift) >> 1;
-  q->distStepAdd = (int64_t)(nomDistFactor * (double)((int64_t)1 << (q->distShift + q->qShift)) + .5);
+  /* distShift + qShift reaches 64..73 on 4x4 blocks at QP >= 48.  The reference's shift is then undefined in C++; x86 masks the count
+     to its low six bits, which is written out here.  The device shift gives 0 instead; both round f * 2^(count - 64) + .5 down to 0 as
+     long as that product stays below .5 (tests/test_tu_range_limits.py checks it over the QP range). */
+  q->distStepAdd = (int64_t)(nomDistFactor * (double)((int64_t)1 << ((q->distShift + q->qShift) & 63)) + .5);
   q->distOrgFact = (int64_t)(nomDistFactor * (double)((int64_t)1 << (q->distShift + 1)) + .5);
 }
 

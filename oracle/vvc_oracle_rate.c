@@ -204,11 +204,12 @@ uint64_t orc_residual_bits(const int32_t* coeff, int w, int h, int mts_idx, int 
   int scanPosLast = -1, pos, sb, state = 0, regBins;
   const int stateTab = dep_quant ? 32040 : 0;
   build_res_scan(&sc, w, h);
-  mts_coding(&e, &c, mts_idx, ts_allowed, mts_allowed);
-  if (mts_idx == 1) { residual_ts(&e, &c, &sc, coeff); return e.bits; }
   memset(sigGroup, 0, sizeof(sigGroup)); memset(coded, 0, sizeof(coded));
   for (pos = 0; pos < sc.numCoeff; pos++) if (coeff[sc.idx[pos]]) { scanPosLast = pos; sigGroup[pos >> 4] = 1; }
+  /* residual_coding runs only for a coded block (cbf 1): an all-zero block costs nothing, transform skip included */
   if (scanPosLast < 0) return 0;
+  mts_coding(&e, &c, mts_idx, ts_allowed, mts_allowed);
+  if (mts_idx == 1) { residual_ts(&e, &c, &sc, coeff); return e.bits; }
   {                                                              /* last_sig_coeff */
     int px = sc.x[scanPosLast], py = sc.y[scanPosLast];
     const int gX = kGroupIdx[px], gY = kGroupIdx[py], lw = ilog2(w), lh = ilog2(h);

@@ -293,6 +293,28 @@ def test_device_matches_oracle_chain(lib, bd, dq):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize('bd', (8, 9, 10))
+def test_device_matches_oracle_chain_at_extreme_qps(lib, bd):
+    """internal QPs 0..11 and 52..63 + 6 (bitDepth - 8), lambda 0.57 * 2^((QP - 12) / 3) x1/4 / x1 / x4, scalar and dependent quantisation,
+    every in-scope shape x split with flat, +-max checkerboard and noise pictures"""
+    rng = np.random.default_rng(300 + bd)
+    qps = list(range(0, 12)) + list(range(52, 64 + 6 * (bd - 8)))
+    cases = []
+    for w, h, isp, n in in_scope():
+        avs = availabilities(w, h, rng)
+        for mode in (0, 1, 18, 50, int(rng.integers(2, 67))):
+            cases.append((w, h, isp, mode, qps[len(cases) % len(qps)], avs[int(rng.integers(0, len(avs)))]))
+    fr, jobs, states, ns = make_batch(rng, bd, cases, [i % 2 for i in range(len(cases))])
+    qp = 6 * jobs['qp_per'].astype(np.int64) + jobs['qp_rem']
+    jobs['lambda'] = np.array((0.25, 1.0, 4.0))[np.arange(len(jobs)) % 3] * 0.57 * 2.0 ** ((qp - 12) / 3.0)
+    assert set(qp.tolist()) == set(qps) and len(cases) > 2 * len(qps)
+    dev = run_device(fr, jobs, states, ns)
+    ora = oracle_batch(lib, fr, jobs, states, ns)
+    compare(dev, ora, bd)
+    assert (dev['results']['part']['abs_sum_level'][qp < 12] > 0).any()
+
+
+@pytest.mark.gpu
 def test_mixed_batch_matches_oracle_chain(lib):
     """one batch mixing scalar and dependent quantisation, candidates with and without VVCB_TU_RATE and with and without MTS (DCT-II in
     both directions), every in-scope shape x split: pass 1 skips the scalar candidates and only some candidates carry models"""
@@ -428,7 +450,9 @@ def test_refusals():
     cases = [edit(set_('isp_mode', 0)), edit(set_('isp_mode', 3)),
              edit(set_('mode', 67)),
              edit(set_('lfnst_idx', 1)), edit(set_('flags', 1 | 4)), edit(set_('flags', 1 | 8)), edit(set_('flags', 1 | 16)), edit(set_('flags', 2)),
-             edit(set_('rate_idx', 2)), edit(set_('lambda', 0.0)), edit(set_('visit', 5)), edit(set_('max_tb_size', 8)),
+             edit(set_('rate_idx', 2)), edit(set_('lambda', 0.0)), edit(set_('lambda', np.inf)), edit(set_('lambda', np.nan)),
+             edit(lambda j: j[0].__setitem__('qp_per', 12) or j[0].__setitem__('qp_rem', 4)),      # internal QP 76 > 75, the 10-bit maximum
+             edit(set_('visit', 5)), edit(set_('max_tb_size', 8)),
              edit(lambda j: None, n_samples=ns - 1), edit(lambda j: None, st=None)]
     bv = bad_visits.copy(); bv[0]['n_left'] = 2
     cases.append(edit(lambda j: None, visits=bv))
@@ -440,6 +464,9 @@ def test_refusals():
         eng.frame_begin(fr.orig)
         eng.reco_update(fr.reco)
         eng.isp_eval(fr.visits, jobs, ns, states=states)                   # the unedited batch is accepted
+        top = jobs.copy()
+        top['qp_per'], top['qp_rem'] = 12, 3                               # internal QP 75, the 10-bit maximum
+        eng.isp_eval(fr.visits, top, ns, states=states)
         for j, visits, n_samples, st in cases:
             with pytest.raises(vb.engine.EngineError):
                 eng.isp_eval(visits, j, n_samples, states=st)

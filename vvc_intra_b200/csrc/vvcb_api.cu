@@ -634,6 +634,11 @@ static int launch_rmd(vvcb_ctx* ctx, const vvcb_rmd_visit* dVisits, int n, vvcb_
   return VVCB_OK;
 }
 
+// The largest internal QP (6 * qp_per + qp_rem) of a luma block: 63 + QpBdOffset, QpBdOffset = 6 * (bitDepth - 8).
+static int max_qp(int bd) { return 63 + 6 * (bd - 8); }
+// lambda of the RD quantisers: the dependent quantiser derives shift counts from it (vvcb_dq.cuh, dq_init_quant), so +inf is refused too.
+static bool lambda_ok(double l) { return l > 0.0 && isfinite(l); }
+
 // Host-side validation of large batches runs on a few threads: returns the smallest index for which ok(i) is false, or -1.
 template <class F> static int first_bad_index(int n, F ok)
 {
@@ -1130,12 +1135,12 @@ static int tu_eval_impl(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n, const int
     const bool q = (j.flags & VVCB_TU_QUANT) != 0;
     const bool dq = q && (j.flags & VVCB_TU_DEPQUANT);
     bool ok = j.log2w >= 2 && j.log2w <= 6 && j.log2h >= 2 && j.log2h <= 6 && j.mts_idx <= 5 && (size_t)j.offset + sz <= n_samples &&
-              j.qp_rem >= 0 && j.qp_rem < 6 && j.qp_per >= 0 && j.qp_per < 16;
+              j.qp_rem >= 0 && j.qp_rem < 6 && j.qp_per >= 0 && 6 * j.qp_per + j.qp_rem <= max_qp(ctx->bd);
     if (j.mts_idx == 1) ok = ok && j.log2w <= 5 && j.log2h <= 5;                 // TU::isTSAllowed, CL/UnitTools.cpp:4524
     if (j.mts_idx > 1)  ok = ok && j.log2w <= 5 && j.log2h <= 5;                 // TU::isMTSAllowed, :4549
     if (q) ok = ok && ctx->bOrig && j.x >= 0 && j.y >= 0 && j.x + (1 << j.log2w) <= ctx->width && j.y + (1 << j.log2h) <= ctx->height;
-    if (dq) ok = ok && j.mts_idx != 1 && rates && j.rate_idx < n_rates && j.lfnst_idx <= 2 && j.lambda > 0.0;   // CL/DepQuant.cpp:1757: TS goes to RDOQ
-    if (j.flags & VVCB_TU_RDOQ_TS) ok = ok && q && !dq && j.mts_idx == 1 && rates && j.rate_idx < n_rates && j.lambda > 0.0;
+    if (dq) ok = ok && j.mts_idx != 1 && rates && j.rate_idx < n_rates && j.lfnst_idx <= 2 && lambda_ok(j.lambda);   // CL/DepQuant.cpp:1757: TS goes to RDOQ
+    if (j.flags & VVCB_TU_RDOQ_TS) ok = ok && q && !dq && j.mts_idx == 1 && rates && j.rate_idx < n_rates && lambda_ok(j.lambda);
     ok = ok && j.lfnst_idx <= 2 && (j.lfnst_idx == 0 || j.intra_mode < VVCB_NUM_LUMA_MODE);
     if (j.flags & VVCB_TU_RATE) ok = ok && q && states && j.rate_idx < n_rates;
     return ok;
@@ -1463,9 +1468,11 @@ extern "C" int vvcb_residual_bits(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n,
     bool ok = j.log2w >= 2 && j.log2w <= 6 && j.log2h >= 2 && j.log2h <= 6 && j.mts_idx <= 5 && j.rate_idx < n_states &&
               (size_t)j.offset + ((size_t)1 << (j.log2w + j.log2h)) <= n_samples;
     if (j.mts_idx >= 1) ok = ok && j.log2w <= 5 && j.log2h <= 5;
+    // levels are 16-bit (entropyCodingMinimum / entropyCodingMaximum with maxLog2TrDynamicRange 15, CL/Quant.cpp)
+    if (ok) ok = std::all_of(levels + j.offset, levels + j.offset + ((size_t)1 << (j.log2w + j.log2h)), [](int32_t v) { return v >= -32768 && v <= 32767; });
     return ok;
   });
-  if (bad >= 0) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_residual_bits: job %d is malformed", bad); return VVCB_ERR_ARG; }
+  if (bad >= 0) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_residual_bits: job %d is malformed (geometry, rate_idx, or a level outside [-32768, 32767])", bad); return VVCB_ERR_ARG; }
   CK(cudaSetDevice(ctx->device));
   int rc;
   std::vector<int> bySize[9];
@@ -1614,10 +1621,10 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
     if (j.mode >= VVCB_NUM_LUMA_MODE) return bad("mode above 66");
     if (j.lfnst_idx != 0) return bad("LFNST with ISP is not evaluated");
     if ((j.flags & ~kFlags) || !(j.flags & VVCB_TU_QUANT)) return bad("flags: VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE] only");
-    if (j.qp_rem < 0 || j.qp_rem >= 6 || j.qp_per < 0 || j.qp_per >= 16) return bad("qp_per / qp_rem out of range");
+    if (j.qp_rem < 0 || j.qp_rem >= 6 || j.qp_per < 0 || 6 * j.qp_per + j.qp_rem > max_qp(ctx->bd)) return bad("qp_per / qp_rem out of range");
     const bool dq = (j.flags & VVCB_TU_DEPQUANT) != 0, carried = dq || (j.flags & VVCB_TU_RATE);
     if (carried && (!states || j.rate_idx >= n_states)) return bad("rate_idx does not name a context snapshot");
-    if (dq && !(j.lambda > 0.0)) return bad("dependent quantisation needs lambda > 0");
+    if (dq && !lambda_ok(j.lambda)) return bad("dependent quantisation needs a finite lambda > 0");
     if ((size_t)j.offset + (size_t)cuW * cuH > n_samples) return bad("outputs outside n_samples");
     IspCand& c = cands[i];
     c.x = v.x; c.y = v.y; c.cuW = (int16_t)cuW; c.cuH = (int16_t)cuH; c.bw = parts[0].w; c.bh = parts[0].h;
