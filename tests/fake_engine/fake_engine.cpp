@@ -41,7 +41,7 @@ const char* vvcb_last_error(const vvcb_ctx* ctx) { return ctx ? ctx->err : g_cre
 
 int vvcb_create(vvcb_ctx** out, int device, int bit_depth, int ctu_size)
 {
-  if (!out || bit_depth < 8 || bit_depth > 12 || ctu_size < 32 || (ctu_size & (ctu_size - 1))) { snprintf(g_createErr, sizeof(g_createErr), "vvcb_create: bad argument"); return VVCB_ERR_ARG; }
+  if (!out || bit_depth < 8 || bit_depth > 10 || ctu_size < 32 || ctu_size > 128 || (ctu_size & (ctu_size - 1))) { snprintf(g_createErr, sizeof(g_createErr), "vvcb_create: bad argument"); return VVCB_ERR_ARG; }
   vvcb_ctx* ctx = new vvcb_ctx();
   ctx->bd = bit_depth; ctx->ctu = ctu_size; ctx->depQuant = 1; ctx->width = ctx->height = 0; ctx->remote = nullptr; ctx->err[0] = 0;
   ctx->origP = &ctx->origOwn; ctx->recoP = &ctx->recoOwn;

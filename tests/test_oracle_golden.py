@@ -91,7 +91,7 @@ def test_rmd_visit_lists(name):
 def test_satd_normalisation_shortcut_is_exact():
     """The CUDA kernel replaces (int)(s / sqrt(N) * 2) (CL/RdCost.cpp:2452,2662) by one multiply with a
     reciprocal; prove it over the whole reachable range of s.  By Parseval the sum of the 128 absolute Hadamard coefficients of a
-    16x8 tile is at most 128 * sqrt(128) * max|residual|: < 1.5e6 for 10-bit residuals, < 6e6 for the 12 bits vvcb_create accepts."""
+    16x8 tile is at most 128 * sqrt(128) * max|residual|: < 1.5e6 for 10-bit residuals, < 6e6 even for 12-bit ones."""
     s = np.arange(0, 1 << 23, dtype=np.int64)
     for n in (128.0, 32.0):
         ref = (s / np.sqrt(n) * 2).astype(np.int64)

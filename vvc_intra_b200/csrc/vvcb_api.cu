@@ -145,9 +145,9 @@ extern "C" void vvcb_destroy(vvcb_ctx* ctx);
 extern "C" int vvcb_create(vvcb_ctx** out, int device, int bit_depth, int ctu_size)
 {
   // bit depths above 10 would need the negative transform-skip shift branch of TrQuant::xTransformSkip (CL/TrQuant.cpp:1394) and have no
-  // golden coverage: refused rather than computed differently
-  if (!out || bit_depth < 8 || bit_depth > 10 || ctu_size < 32 || (ctu_size & (ctu_size - 1))) {
-    snprintf(g_createErr, sizeof(g_createErr), "vvcb_create: bad argument (bit depth 8..10, CTU size a power of two >= 32)");
+  // golden coverage: refused rather than computed differently.  H.266 caps CtbSizeY at 128 (sps_log2_ctu_size_minus5 <= 2).
+  if (!out || bit_depth < 8 || bit_depth > 10 || ctu_size < 32 || ctu_size > 128 || (ctu_size & (ctu_size - 1))) {
+    snprintf(g_createErr, sizeof(g_createErr), "vvcb_create: bad argument (bit depth 8..10, CTU size 32, 64 or 128)");
     return VVCB_ERR_ARG;
   }
   *out = nullptr;
@@ -899,7 +899,15 @@ static int rmd_pred_impl(vvcb_ctx* ctx, const vvcb_rmd_visit* visit, int slot, i
   rc = launch_rmd(ctx, ctx->dVisits, 1, ctx->dResults, nullptr, ctx->dPred);
   if (rc) return rc;
   if (slot >= 0) CK(cudaMemcpyAsync(pred, ctx->dPred + (size_t)slot * w * h, (size_t)w * h * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-  else           CK(cudaMemcpyAsync(pred, ctx->dPred, need * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  else {
+    // only the slots the visit evaluates: the device buffer holds an earlier visit's samples in the others, and the caller's copy of
+    // those is left untouched (vvc_intra_b200.h)
+    const int spans[3][2] = { { 0, VVCB_SLOT_MRL1 }, { VVCB_SLOT_MRL1, mrlAllowed ? VVCB_SLOT_MIP : VVCB_SLOT_MRL1 }, { VVCB_SLOT_MIP, VVCB_SLOT_MIP + numMip } };
+    for (const auto& s : spans)
+      if (s[1] > s[0])
+        CK(cudaMemcpyAsync(pred + (size_t)s[0] * w * h, ctx->dPred + (size_t)s[0] * w * h, (size_t)(s[1] - s[0]) * w * h * sizeof(int16_t),
+                           cudaMemcpyDeviceToHost, ctx->stream));
+  }
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
