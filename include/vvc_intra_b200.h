@@ -442,6 +442,55 @@ int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, con
                   const vvcb_ctx_states* states, int n_states, size_t n_samples,
                   int32_t* level, int16_t* reco, int16_t* pred, vvcb_isp_result* results);
 
+/* ---- chroma intra candidates (4:2:0, separate tree): prediction + SAD / SATD of Cb and Cr ------------------------------------------
+ * The data-parallel half of IntraSearch::estIntraPredChromaQT (EL/IntraSearch.cpp:1382), which every chroma CU of the separate tree of an
+ * all-intra picture runs (EL/EncCu.cpp:519-536): the candidates of PU::getIntraChromaCandModes (CL/UnitTools.cpp) predicted for Cb and
+ * Cr -- planar / DC / angular with the chroma rules of initPredIntraParams and xPredIntraAng (CL/IntraPrediction.cpp:487-618, 633-935:
+ * parameters from the chroma block's own shape, reference lines never smoothed, the 2-tap linear interpolation) and the cross-component
+ * modes (CL/IntraPrediction.cpp:1665-2150: xGetLumaRecPixels with the [1 2 1; 1 2 1] / 8 down-sampling of sps_cclm_colocated_chroma
+ * = 0, xGetLMParameters, predIntraChromaLM) -- and measured with RdCost::xGetSAD / xGetHADs on the chroma block.  No ordering or
+ * pruning of the candidates: that is the caller's.  Chroma TU coding (chroma QP mapping, joint Cb-Cr) is not in the library.
+ * Restated from H.266 and the cited reference lines; not compared with the reference encoder's own chroma output.                   */
+#define VVCB_CHROMA_CANDS 8
+#define VVCB_LM_CHROMA   67   /* LM_CHROMA_IDX: CCLM from the above and left neighbours */
+#define VVCB_MDLM_L      68   /* MDLM_L_IDX: left and below-left only                    */
+#define VVCB_MDLM_T      69   /* MDLM_T_IDX: above and above-right only                  */
+#define VVCB_DM_CHROMA   70   /* DM_CHROMA_IDX: the derived luma mode (vvcb_chroma_visit::dm_mode) */
+
+/* Chroma planes of the picture given to vvcb_frame_begin: Cb / Cr originals, their reconstructions cleared.  cw = width / 2,
+ * ch = height / 2 (4:2:0); bit depth = the context's.  The CCLM modes read the context's luma reconstruction (vvcb_reco_update /
+ * vvcb_reco_update_rects): in the separate tree the whole luma CTU is coded before its chroma.                                   */
+int vvcb_chroma_frame_begin(vvcb_ctx* ctx, const int16_t* cb, const int16_t* cr, int stride, int cw, int ch);
+/* the rectangle (chroma samples) of both reconstructions the host has just decided */
+int vvcb_chroma_reco_update(vvcb_ctx* ctx, const int16_t* cb, const int16_t* cr, int stride, int x, int y, int w, int h);
+
+/* One chroma CU of the separate tree. */
+typedef struct vvcb_chroma_visit {
+  int16_t x, y;              /* chroma position, even                                                                           */
+  uint8_t log2w, log2h;      /* 2..5 (2xN / Nx2 are not evaluated)                                                              */
+  /* reference-sample availability in the reference's chroma units of 2 samples (pcv.minCUWidth >> scaleX), prefix counts as for
+   * vvcb_rmd_visit: avail_al 0/1, n_above / n_above_right 0..w/2, n_left / n_below_left 0..h/2.  CCLM takes a side only when it is
+   * whole (n_above == w/2, n_left == h/2), and the above-right / below-left only with their side.                                   */
+  uint8_t avail_al, n_above, n_above_right, n_left, n_below_left;
+  uint8_t dm_mode;           /* the derived luma mode 0..66 (PLANAR when the collocated luma CU is MIP), kept by the caller's walk */
+  uint8_t cclm;              /* 1: the LM modes are evaluated (PU::isLMCModeEnabled, the caller's decision)                        */
+  uint8_t pad[3];
+} vvcb_chroma_visit;         /* 16 bytes */
+
+/* The 8 candidates in the reference's order: PLANAR, VER (50), HOR (18), DC, LM, MDLM_L, MDLM_T, DM; the first of the four regular ones
+ * that equals dm_mode is VDIA (66) instead.  sad / satd [candidate][0 Cb, 1 Cr]; VVCB_SAT_NONE: not evaluated (LM modes without cclm). */
+typedef struct vvcb_chroma_result {
+  uint8_t  mode[VVCB_CHROMA_CANDS];        /* 0..66, VVCB_LM_CHROMA / VVCB_MDLM_L / VVCB_MDLM_T, VVCB_DM_CHROMA (predicts dm_mode) */
+  uint32_t sad[VVCB_CHROMA_CANDS][2];
+  uint32_t satd[VVCB_CHROMA_CANDS][2];
+} vvcb_chroma_result;        /* 136 bytes */
+
+/* visits / results: HOST arrays of n.  pred_out (optional, HOST): per visit, in order, 8 x 2 x w*h int16 -- [candidate][Cb, Cr][h][w]
+ * (the blocks of LM candidates that are not evaluated are zero).  VVCB_ERR_ARG for sides outside 4..32, odd positions,
+ * counts above their maximum, dm_mode > 66, a CU or neighbour outside the chroma picture; VVCB_ERR_STATE before
+ * vvcb_chroma_frame_begin and through the broker.                                                                                 */
+int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n, int16_t* pred_out, vvcb_chroma_result* results);
+
 /* ---- texture features (orig-only, trivially parallel) ------------------------------------------------------------
  * vvcb_ctu_hads_islice: EncCu::updateCtuDataISlice (EL/EncCu.cpp:564-675) for every CTU of the frame, as
  * EncSlice::calCostSliceI calls it (EL/EncSlice.cpp:1276-1298): sum over the complete 8x8 blocks of the CTU's

@@ -11,6 +11,7 @@
 #include "vvcb_feat.cuh"
 #include "vvcb_dq.cuh"
 #include "vvcb_rate.cuh"
+#include "vvcb_chroma.cuh"
 #include <vector>
 #include <algorithm>
 #include <time.h>
@@ -99,6 +100,9 @@ struct vvcb_ctx {
   uint64_t cuNs[8], cuCalls, tuWaitFrom;    // vvcb_cu_eval_phases
   cudaEvent_t cev[4]; bool cuSpan;          // device spans of the two stages of vvcb_cu_eval
   int timing; int timedLaunches; float kms[3]; cudaEvent_t kev[4];
+  int16_t* dChroma; size_t capChroma;       // vvcb_chroma_frame_begin: Cb, Cr originals, then Cb, Cr reconstructions, cstride * ch each
+  int cw, ch, cstride;                      // 0 until vvcb_chroma_frame_begin
+  void* dChromaIo; size_t capChromaIo;      // vvcb_chroma_eval: visits, results, prediction offsets, predictions
   char err[512];
 };
 
@@ -241,6 +245,7 @@ extern "C" void vvcb_destroy(vvcb_ctx* ctx)
   cudaFree(ctx->dRect[0]); cudaFree(ctx->dRect[1]); cudaFree(ctx->dBrief);
   cudaFree(ctx->dRom); cudaFree(ctx->dOrig); cudaFree(ctx->dReco); cudaFree(ctx->dVisits); cudaFree(ctx->dResults); cudaFree(ctx->dDetails); cudaFree(ctx->dScratch);
   cudaFree(ctx->dItems); cudaFree(ctx->dPlan); cudaFree(ctx->dPred); cudaFree(ctx->dTrRom);
+  cudaFree(ctx->dChroma); cudaFree(ctx->dChromaIo);
   for (int i = 0; i < kTuSlots; i++) cudaFree(ctx->dTu[i]);
   cudaFree(ctx->dRateRom);
   cudaFree(ctx->dDqRom);
@@ -1793,6 +1798,119 @@ extern "C" int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_
                                     level, reco, pred, results + b, pass == 0);
       if (rc) return rc;
     }
+  return VVCB_OK;
+}
+
+// =====================================================================================================
+// chroma intra candidates (vvcb_chroma.cuh)
+// =====================================================================================================
+extern "C" int vvcb_chroma_frame_begin(vvcb_ctx* ctx, const int16_t* cb, const int16_t* cr, int stride, int cw, int ch)
+{
+  if (!ctx) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_chroma_frame_begin");
+  if (!ctx->dOrig || ctx->bOrig != ctx->dOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_frame_begin: vvcb_frame_begin has not been called"); return VVCB_ERR_STATE; }
+  if (!cb || !cr || cw != ctx->width / 2 || ch != ctx->height / 2 || stride < cw) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_frame_begin: bad argument (4:2:0 planes of %d x %d)", ctx->width / 2, ctx->height / 2);
+    return VVCB_ERR_ARG;
+  }
+  CK(cudaSetDevice(ctx->device));
+  const int pitch = (cw + 63) & ~63;
+  const size_t plane = (size_t)pitch * ch;
+  if (4 * plane > ctx->capChroma) {
+    cudaFree(ctx->dChroma); ctx->dChroma = nullptr; ctx->capChroma = 0;
+    CK(cudaMalloc(&ctx->dChroma, 4 * plane * sizeof(int16_t)));
+    ctx->capChroma = 4 * plane;
+  }
+  ctx->cw = cw; ctx->ch = ch; ctx->cstride = pitch;
+  const int16_t* src[2] = { cb, cr };
+  for (int c = 0; c < 2; c++)
+    CK(cudaMemcpy2DAsync(ctx->dChroma + c * plane, pitch * sizeof(int16_t), src[c], stride * sizeof(int16_t), cw * sizeof(int16_t), ch,
+                         cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(ctx->dChroma + 2 * plane, 0, 2 * plane * sizeof(int16_t), ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return VVCB_OK;
+}
+
+extern "C" int vvcb_chroma_reco_update(vvcb_ctx* ctx, const int16_t* cb, const int16_t* cr, int stride, int x, int y, int w, int h)
+{
+  if (!ctx) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_chroma_reco_update");
+  if (!ctx->cw) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_reco_update: vvcb_chroma_frame_begin has not been called"); return VVCB_ERR_STATE; }
+  if (!cb || !cr || x < 0 || y < 0 || w <= 0 || h <= 0 || x + w > ctx->cw || y + h > ctx->ch || stride < w) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_reco_update: rectangle outside the chroma picture");
+    return VVCB_ERR_ARG;
+  }
+  CK(cudaSetDevice(ctx->device));
+  const size_t plane = (size_t)ctx->cstride * ctx->ch;
+  const int16_t* src[2] = { cb, cr };
+  for (int c = 0; c < 2; c++)
+    CK(cudaMemcpy2DAsync(ctx->dChroma + (2 + c) * plane + (size_t)y * ctx->cstride + x, ctx->cstride * sizeof(int16_t), src[c],
+                         stride * sizeof(int16_t), w * sizeof(int16_t), h, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return VVCB_OK;
+}
+
+// why a chroma visit may not be evaluated, nullptr when it may
+static const char* chroma_visit_error(const vvcb_ctx* ctx, const vvcb_chroma_visit& v)
+{
+  if (v.log2w < 2 || v.log2w > 5 || v.log2h < 2 || v.log2h > 5) return "sides must be 4..32";
+  const int w = 1 << v.log2w, h = 1 << v.log2h;
+  if (v.avail_al > 1 || v.n_above > w / 2 || v.n_above_right > w / 2 || v.n_left > h / 2 || v.n_below_left > h / 2 || v.cclm > 1)
+    return "availability count above its maximum (units of 2 samples) or cclm not 0/1";
+  if (v.dm_mode > 66) return "dm_mode above 66";
+  if (v.x < 0 || v.y < 0 || (v.x & 1) || (v.y & 1) || v.x + w > ctx->cw || v.y + h > ctx->ch) return "CU outside the chroma picture or at an odd position";
+  if (((v.avail_al || v.n_left || v.n_below_left) && v.x == 0) || ((v.avail_al || v.n_above || v.n_above_right) && v.y == 0) ||
+      v.x + w + 2 * v.n_above_right > ctx->cw || v.y + h + 2 * v.n_below_left > ctx->ch)
+    return "available neighbours outside the chroma picture";
+  return nullptr;
+}
+
+extern "C" int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n, int16_t* pred_out, vvcb_chroma_result* results)
+{
+  if (!ctx) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_chroma_eval");
+  if (n < 0 || (n > 0 && (!visits || !results))) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_eval: bad argument"); return VVCB_ERR_ARG; }
+  if (!ctx->cw || ctx->cw != ctx->width / 2 || ctx->ch != ctx->height / 2 || !ctx->bReco) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_eval: vvcb_chroma_frame_begin has not been called for this picture");
+    return VVCB_ERR_STATE;
+  }
+  std::vector<uint32_t> off((size_t)n);
+  size_t total = 0;
+  for (int i = 0; i < n; i++) {
+    if (const char* why = chroma_visit_error(ctx, visits[i])) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_eval: visit %d: %s", i, why); return VVCB_ERR_ARG; }
+    off[i] = (uint32_t)total;
+    total += (size_t)VVCB_CHROMA_CANDS * 2 << (visits[i].log2w + visits[i].log2h);
+  }
+  if (n == 0) return VVCB_OK;
+  if (pred_out && total > 0xFFFFFFFFu) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_eval: prediction output above 2^32 samples: split the batch"); return VVCB_ERR_ARG; }
+  CK(cudaSetDevice(ctx->device));
+  Arena ar;
+  const size_t oVis = ar.take(sizeof(vvcb_chroma_visit) * n), oRes = ar.take(sizeof(vvcb_chroma_result) * n);
+  const size_t oOff = pred_out ? ar.take(sizeof(uint32_t) * n) : 0, oPred = pred_out ? ar.take(sizeof(int16_t) * total) : 0;
+  if (ar.size > ctx->capChromaIo) {
+    cudaFree(ctx->dChromaIo); ctx->dChromaIo = nullptr; ctx->capChromaIo = 0;
+    CK(cudaMalloc(&ctx->dChromaIo, ar.size));
+    ctx->capChromaIo = ar.size;
+  }
+  void* io = ctx->dChromaIo;
+  CK(cudaMemcpyAsync(at<void>(io, oVis), visits, sizeof(vvcb_chroma_visit) * n, cudaMemcpyHostToDevice, ctx->stream));
+  if (pred_out) {
+    CK(cudaMemcpyAsync(at<void>(io, oOff), off.data(), sizeof(uint32_t) * n, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(at<void>(io, oPred), 0, sizeof(int16_t) * total, ctx->stream));    // the blocks of LM candidates that are not evaluated
+  }
+  const size_t plane = (size_t)ctx->cstride * ctx->ch;
+  ChromaParams P;
+  P.visits = at<const vvcb_chroma_visit>(io, oVis); P.n = n; P.results = at<vvcb_chroma_result>(io, oRes);
+  P.predOut = pred_out ? at<int16_t>(io, oPred) : nullptr; P.predOff = pred_out ? at<const uint32_t>(io, oOff) : nullptr;
+  P.orig[0] = ctx->dChroma; P.orig[1] = ctx->dChroma + plane; P.reco[0] = ctx->dChroma + 2 * plane; P.reco[1] = ctx->dChroma + 3 * plane;
+  P.cstride = ctx->cstride; P.luma = ctx->bReco; P.lstride = ctx->stride; P.bd = ctx->bd; P.ctu = ctx->ctu; P.rom = ctx->dRom;
+  const int blocks = std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16);
+  chroma_eval_kernel<<<blocks, kChromaWarps * 32, 0, ctx->stream>>>(P);
+  ctx->launches++;
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(results, P.results, sizeof(vvcb_chroma_result) * n, cudaMemcpyDeviceToHost, ctx->stream));
+  if (pred_out) CK(cudaMemcpyAsync(pred_out, P.predOut, sizeof(int16_t) * total, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(ctx_sync(ctx));
   return VVCB_OK;
 }
 

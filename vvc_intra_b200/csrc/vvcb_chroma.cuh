@@ -1,0 +1,333 @@
+// vvc_intra_b200 -- chroma intra candidates (vvcb_chroma_eval): prediction of Cb and Cr under the 8 candidates of
+// PU::getIntraChromaCandModes and their SAD / SATD, 4:2:0.  Included by vvcb_api.cu and, through the CUDA-on-pthreads shim, by
+// tests/host_emul/emul_chroma.cpp.
+//
+// One warp per visit (a chroma CU of the separate tree), warps striding over the batch:
+//   1. the Cb and Cr reference lines into shared memory -- the luma padding walk (build_line_set) with a unit of 2 samples, line 0 only,
+//      never smoothed -- and the block's originals;
+//   2. with the LM modes enabled, the down-sampled luma of the block and of its neighbours, shared by Cb and Cr, then the (a, k, b) of
+//      the three LM modes for both components; the DC values; the projected main reference of DM when its angle is negative;
+//   3. the 16 evaluations (8 candidates x Cb / Cr) as lane tasks: a lane predicts one 8x8 unit (both sides >= 8) or one SATD tile (a side
+//      of 4) into registers and takes residual, SAD and Walsh-Hadamard SATD with the luma tile functions; the tile follows from the
+//      block's shape as xGetHADs chooses it (make_shape), the 16x8 / 8x16 tiles butterfly with the partner lane.
+// Restated from H.266 and CL/IntraPrediction.cpp:487-618, 633-935, 1215-1468, 1665-2150; parity with the reference encoder's own chroma
+// output is unpinned.
+#pragma once
+#include "vvcb_rmd.cuh"
+
+namespace {
+
+constexpr int kChromaWarps = 4;
+constexpr int kChromaMax   = 32;           // largest chroma side evaluated
+constexpr int kChromaLine  = 72;           // 2 * 32 + 1 samples + the 2 replicated ones of positive angles, rounded up to whole words
+
+struct ChromaSmem {                        // one visit, one warp
+  int16_t lines[2][2][kChromaLine];        // [0 Cb, 1 Cr][0 top / 1 left][index]: build_line_set's layout with one "set" per component
+  alignas(8) int16_t org[2][kChromaMax * kChromaMax];   // the block's originals, dense w*h (residual_unit reads 4 samples at a time)
+  int16_t ds[kChromaMax * kChromaMax];     // down-sampled luma of the block, dense w*h
+  int16_t dsTop[2 * kChromaMax], dsLeft[2 * kChromaMax];
+  alignas(4) int16_t proj[2][kChromaLine]; // DM's main reference with its projected part (build_projected_line), negative angles only
+  int lm[3][2][3];                         // [LM, MDLM_L, MDLM_T][Cb, Cr]: a, k, b
+  int dc[2];
+};
+
+struct ChromaParams {
+  const vvcb_chroma_visit* visits;
+  int n;
+  vvcb_chroma_result* results;
+  int16_t* predOut;                        // optional: per visit 8 x 2 blocks of w*h at predOff[visit]
+  const uint32_t* predOff;
+  const int16_t* orig[2];                  // Cb, Cr
+  const int16_t* reco[2];
+  int cstride;
+  const int16_t* luma;                     // luma reconstruction
+  int lstride;
+  int bd, ctu;
+  const Rom* rom;
+};
+
+// PU::getIntraChromaCandModes: PLANAR, VER, HOR, DC, LM, MDLM_L, MDLM_T, DM; the first regular one equal to DM becomes VDIA
+__host__ __device__ __forceinline__ int chroma_cand_code(int c, int dm)
+{
+  const int base = c == 0 ? 0 : c == 1 ? 50 : c == 2 ? 18 : c == 3 ? 1 : VVCB_LM_CHROMA + c - 4;
+  if (c < 4) {
+    const int first = dm == 0 ? 0 : dm == 50 ? 1 : dm == 18 ? 2 : dm == 1 ? 3 : 4;
+    if (first == c) return 66;
+  }
+  return base;
+}
+
+// xGetLMParameters for one LM mode (0 LM, 1 MDLM_L, 2 MDLM_T) and component
+__device__ __forceinline__ void chroma_lm_params(const ChromaSmem& sm, int lm, int comp, int w, int h, int bd, bool availT, bool availL,
+                                                 int nAr, int nBl, int (&out)[3])
+{
+  const int16_t* cTop = sm.lines[comp][0] + 1;
+  const int16_t* cLeft = sm.lines[comp][1] + 1;
+  int numT = w, numL = h;
+  if (lm == 2) { availL = false; numT = w + vmin(nAr, h); }
+  if (lm == 1) { availT = false; numL = h + vmin(nBl, w); }
+  if (!availT && !availL) { out[0] = 0; out[1] = 0; out[2] = 1 << (bd - 1); return; }
+  int selY[4] = { 0, 0, 0, 0 }, selC[4] = { 0, 0, 0, 0 };
+  int cntT = 0, cntL = 0;
+  if (availT) {
+    const int is4 = availL ? 0 : 1;
+    const int start = numT >> (2 + is4), step = vmax(1, numT >> (1 + is4));
+    cntT = vmin(numT, (1 + is4) << 1);
+    for (int i = 0; i < cntT; i++) { selY[i] = sm.dsTop[start + i * step]; selC[i] = cTop[start + i * step]; }
+  }
+  if (availL) {
+    const int is4 = availT ? 0 : 1;
+    const int start = numL >> (2 + is4), step = vmax(1, numL >> (1 + is4));
+    cntL = vmin(numL, (1 + is4) << 1);
+    for (int i = 0; i < cntL; i++) { selY[cntT + i] = sm.dsLeft[start + i * step]; selC[cntT + i] = cLeft[start + i * step]; }
+  }
+  if (cntT + cntL == 2) {
+    selY[3] = selY[0]; selC[3] = selC[0]; selY[2] = selY[1]; selC[2] = selC[1];
+    selY[0] = selY[1]; selC[0] = selC[1]; selY[1] = selY[3]; selC[1] = selC[3];
+  }
+  int mn0 = 0, mn1 = 2, mx0 = 1, mx1 = 3, t;
+  if (selY[mn0] > selY[mn1]) { t = mn0; mn0 = mn1; mn1 = t; }
+  if (selY[mx0] > selY[mx1]) { t = mx0; mx0 = mx1; mx1 = t; }
+  if (selY[mn0] > selY[mx1]) { t = mn0; mn0 = mx0; mx0 = t; t = mn1; mn1 = mx1; mx1 = t; }
+  if (selY[mn1] > selY[mx0]) { t = mn1; mn1 = mx0; mx0 = t; }
+  const int minY = (selY[mn0] + selY[mn1] + 1) >> 1, minC = (selC[mn0] + selC[mn1] + 1) >> 1;
+  const int maxY = (selY[mx0] + selY[mx1] + 1) >> 1, maxC = (selC[mx0] + selC[mx1] + 1) >> 1;
+  const int diff = maxY - minY;
+  if (diff <= 0) { out[0] = 0; out[1] = 0; out[2] = minC; return; }
+  const int divSig[16] = { 0, 7, 6, 5, 5, 4, 4, 3, 3, 2, 2, 1, 1, 1, 1, 0 };
+  const int diffC = maxC - minC;
+  int x = vlog2(diff);
+  const int normDiff = ((diff << 4) >> x) & 15;
+  const int v = divSig[normDiff] | 8;
+  x += normDiff != 0;
+  const int y = diffC ? vlog2(vabs(diffC)) + 1 : 0;
+  int a = (diffC * v + (1 << y >> 1)) >> y;
+  int k = 3 + x - y;
+  if (k < 1) { k = 1; a = a == 0 ? 0 : (a < 0 ? -15 : 15); }
+  out[0] = a; out[1] = k; out[2] = minC - ((a * minY) >> k);
+}
+
+// one candidate of one component, as the lane tasks see it
+struct ChromaCand {
+  int kind;               // 0 planar, 1 DC, 2 angular, 3 LM
+  int comp;
+  ModeParam p;
+  int a, k, b, dc;
+};
+
+// the R x C piece of the block at (x0, y0), block orientation
+template <int R, int C>
+__device__ __forceinline__ void chroma_predict_piece(const ChromaSmem& sm, const ChromaCand& cd, const Shape& sh, const uint32_t* filt, int maxv,
+                                                     int x0, int y0, int (&q)[R][C])
+{
+  const int16_t* top = sm.lines[cd.comp][0];
+  const int16_t* left = sm.lines[cd.comp][1];
+  if (cd.kind == 3) {
+#pragma unroll
+    for (int i = 0; i < R; i++)
+#pragma unroll
+      for (int j = 0; j < C; j++) q[i][j] = clip_bd(((sm.ds[(y0 + i) * sh.w + x0 + j] * cd.a) >> cd.k) + cd.b, maxv);
+  } else if (cd.kind < 2) {
+    pred_planar_dc_unit<R, C>(top, left, cd.kind, cd.p.pdpc, cd.dc, sh.lw, sh.lh, x0, y0, q);
+  } else if (cd.p.is_ver) {
+    const int16_t* ml = cd.p.angle < 0 ? sm.proj[cd.comp] + sh.h : top;
+    pred_angular_unit<R, C, true>(ml, left, cd.p, 0, sh.w, sh.h, x0, y0, filt, maxv, q);
+  } else {
+    int t[C][R];                                           // main/side frame of a horizontal mode: t[i][j] is block sample (y0 + j, x0 + i)
+    const int16_t* ml = cd.p.angle < 0 ? sm.proj[cd.comp] + sh.w : left;
+    pred_angular_unit<C, R, true>(ml, top, cd.p, 0, sh.h, sh.w, y0, x0, filt, maxv, t);
+#pragma unroll
+    for (int i = 0; i < R; i++)
+#pragma unroll
+      for (int j = 0; j < C; j++) q[i][j] = t[j][i];
+  }
+}
+
+__global__ void __launch_bounds__(kChromaWarps * 32) chroma_eval_kernel(ChromaParams P)
+{
+  __shared__ ChromaSmem smem[kChromaWarps];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  ChromaSmem& sm = smem[warp];
+  const Rom& rom = *P.rom;
+  const uint32_t* filt = &rom.filt[0][0];        // not read by the linear interpolation; a valid address for pred_angular_unit's table pointer
+  const int maxv = (1 << P.bd) - 1;
+  for (int vi = blockIdx.x * kChromaWarps + warp; vi < P.n; vi += gridDim.x * kChromaWarps) {
+    const vvcb_chroma_visit cv = P.visits[vi];
+    const Shape sh = make_shape(cv.log2w, cv.log2h);
+    const int w = sh.w, h = sh.h;
+    vvcb_rmd_visit lv = {};                                // the walk's view of the visit (position, size, availability)
+    lv.x = cv.x; lv.y = cv.y; lv.log2w = cv.log2w; lv.log2h = cv.log2h;
+    lv.avail_al = cv.avail_al; lv.n_above = cv.n_above; lv.n_above_right = cv.n_above_right; lv.n_left = cv.n_left; lv.n_below_left = cv.n_below_left;
+    const bool availT = cv.n_above == (w >> 1), availL = cv.n_left == (h >> 1);
+    const int nAr = availT ? 2 * cv.n_above_right : 0, nBl = availL ? 2 * cv.n_below_left : 0;
+    const int dm = cv.dm_mode;
+    ModeParam dmp = rom.mode[sh.lw - 2][sh.lh - 2][dm];
+    __syncwarp();
+    // ---- 1. reference lines and originals
+#pragma unroll 1
+    for (int c = 0; c < 2; c++) build_line_set<2>(sm, c, 0, lv, sh, P.reco[c], P.cstride, P.bd, lane);
+    for (int i = lane; i < 2 * w * h; i += 32) {
+      const int c = i >> (sh.lw + sh.lh), s = i & (w * h - 1);
+      sm.org[c][s] = P.orig[c][(size_t)(cv.y + (s >> sh.lw)) * P.cstride + cv.x + (s & (w - 1))];
+    }
+    // ---- 2. down-sampled luma (xGetLumaRecPixels, 4:2:0, [1 2 1; 1 2 1] / 8; one row [1 2 1] / 4 above a CTU's first row)
+    if (cv.cclm) {
+      const int16_t* Y = P.luma + (size_t)(2 * cv.y) * P.lstride + 2 * cv.x;
+      const int ls = P.lstride;
+      const bool ctuTop = (cv.y & ((P.ctu >> 1) - 1)) == 0;
+      const int nTop = availT ? w + vmin(nAr, h) : 0, nLeft = availL ? h + vmin(nBl, w) : 0;
+      for (int i = lane; i < w * h + nTop + nLeft; i += 32) {
+        int v;
+        if (i < w * h + nTop) {
+          const int x = i < w * h ? i & (w - 1) : i - w * h;
+          const int xl = 2 * x - (x == 0 && !availL ? 0 : 1);      // no left neighbours: column -1 padded from column 0
+          const int16_t* r0 = i < w * h ? Y + (size_t)(2 * (i >> sh.lw)) * ls : Y - 2 * ls;
+          if (i >= w * h && ctuTop) v = (2 * r0[ls + 2 * x] + r0[ls + 2 * x + 1] + r0[ls + xl] + 2) >> 2;
+          else v = (2 * r0[2 * x] + r0[2 * x + 1] + r0[xl] + 2 * r0[ls + 2 * x] + r0[ls + 2 * x + 1] + r0[ls + xl] + 4) >> 3;
+          if (i < w * h) sm.ds[i] = (int16_t)v;
+          else sm.dsTop[x] = (int16_t)v;
+        } else {
+          const int j = i - w * h - nTop;
+          const int16_t* r0 = Y + (size_t)(2 * j) * ls - 3;
+          sm.dsLeft[j] = (int16_t)((2 * r0[1] + r0[2] + r0[0] + 2 * r0[ls + 1] + r0[ls + 2] + r0[ls] + 4) >> 3);
+        }
+      }
+    }
+    __syncwarp();
+    // LM parameters (lanes 0..5), DC values (lanes 6, 7), DM's projected main reference (every lane)
+    if (cv.cclm && lane < 6) {
+      int o[3];
+      chroma_lm_params(sm, lane >> 1, lane & 1, w, h, P.bd, availT, availL, nAr, nBl, o);
+      sm.lm[lane >> 1][lane & 1][0] = o[0]; sm.lm[lane >> 1][lane & 1][1] = o[1]; sm.lm[lane >> 1][lane & 1][2] = o[2];
+    } else if (lane == 6 || lane == 7) {
+      const int c = lane - 6;
+      int sum = 0;
+      if (w >= h) for (int i = 0; i < w; i++) sum += sm.lines[c][0][1 + i];
+      if (w <= h) for (int i = 0; i < h; i++) sum += sm.lines[c][1][1 + i];
+      const int denom = w == h ? 2 * w : vmax(w, h);
+      sm.dc[c] = (sum + (denom >> 1)) >> vlog2(denom);
+    }
+    if (dm > 1 && dmp.angle < 0) {
+      SlotInfo s = {};
+      s.kind = 2; s.mode = dm; s.p = dmp;
+#pragma unroll 1
+      for (int c = 0; c < 2; c++) {
+        s.set = c;
+        build_projected_line(sm.proj[c], sm, s, dmp.is_ver ? w : h, dmp.is_ver ? h : w, lane, 32);
+      }
+    }
+    __syncwarp();
+
+    // ---- 3. evaluations: task = (candidate * 2 + component) * lanes + unit
+    const int lanes = sh.lanes, lgL = sh.lgLanes;
+    int16_t* pout = P.predOut ? P.predOut + P.predOff[vi] : nullptr;
+#pragma unroll 1
+    for (int base = 0; base < (16 << lgL); base += 32) {
+      const int task = base + lane;
+      const int e = vmin(task >> lgL, 15), u = task & (lanes - 1);
+      const int c = e >> 1, comp = e & 1;
+      const int code = chroma_cand_code(c, dm);
+      const int mode = code == VVCB_DM_CHROMA ? dm : code;
+      const bool act = (task >> lgL) < 16 && (mode < VVCB_LM_CHROMA || cv.cclm);
+      ChromaCand cd;
+      cd.comp = comp;
+      cd.kind = mode == 0 ? 0 : mode == 1 ? 1 : mode < VVCB_LM_CHROMA ? 2 : 3;
+      cd.p = rom.mode[sh.lw - 2][sh.lh - 2][mode < VVCB_LM_CHROMA ? mode : 0];
+      cd.dc = sm.dc[comp];
+      const int lm = vmin(vmax(mode - VVCB_LM_CHROMA, 0), 2);
+      cd.a = sm.lm[lm][comp][0]; cd.k = sm.lm[lm][comp][1]; cd.b = sm.lm[lm][comp][2];
+      if (cd.kind == 3 && !cv.cclm) { cd.a = 0; cd.k = 0; cd.b = 0; }   // not evaluated: shadow values, nothing is stored
+      const int16_t* org = sm.org[comp];
+      int16_t* outBlk = pout ? pout + (size_t)e * w * h : nullptr;
+      int sad = 0, satd = 0;
+      if (sh.S == 8) {
+        // an 8x8 unit as two 4x8 halves (the luma evaluation kernels' scheme): rows and the first two column stages inside a half, the
+        // stage across the halves folded into the absolute sum, the 16x8 / 8x16 stage across units a butterfly with the partner lane
+        const int ux = u & (sh.unitsX - 1), uy = u >> sh.lgTilesX;
+        const int x0 = ux * 8, y0 = uy * 8;
+        const int partnerMask = sh.tile == 4 ? 1 : sh.unitsX;
+        const bool owner = sh.tile == 4 ? (ux & 1) == 0 : (uy & 1) == 0;
+        uint32_t c0[4][4];
+        int t = 0;
+#pragma unroll 1
+        for (int k = 0; k < 2; k++) {
+          int q[4][8], d[4][8];
+          chroma_predict_piece<4, 8>(sm, cd, sh, filt, maxv, x0, y0 + 4 * k, q);
+          if (outBlk && act) store_pred<4, 8>(outBlk, w, x0, y0 + 4 * k, false, q);
+          residual_unit<4, 8, false>(org + (y0 + 4 * k) * w + x0, w, q, d, sad);
+          wht_rows_rc<4, 8>(d);
+          wht_cols_rc<4, 8>(d);
+          if (sh.tile != 3) {
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+#pragma unroll
+              for (int j = 0; j < 8; j++) {
+                const int other = __shfl_xor_sync(0xffffffffu, d[i][j], partnerMask);
+                d[i][j] = owner ? d[i][j] + other : d[i][j] - other;
+              }
+          }
+          if (k == 0) {
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+#pragma unroll
+              for (int j = 0; j < 4; j++) c0[i][j] = pack_u16x2(vabs(d[i][2 * j]), vabs(d[i][2 * j + 1]));
+          } else {
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+#pragma unroll
+              for (int j = 0; j < 4; j++) t = add_halves_u16x2(max_u16x2(c0[i][j], pack_u16x2(vabs(d[i][2 * j]), vabs(d[i][2 * j + 1]))), t);
+          }
+        }
+        if (sh.tile == 3) satd = (2 * t + 2) >> 2;                              // CL/RdCost.cpp:2306
+        else {
+          t += __shfl_xor_sync(0xffffffffu, t, partnerMask);
+          satd = owner ? satd_norm_rect(2 * t, true) : 0;                        // CL/RdCost.cpp:2452, :2589
+        }
+      } else {
+        // a side of 4: a lane owns one SATD tile, one (4x4) or two (8x4, 4x8) 4x4 pieces
+        const int tx = u & ((1 << sh.lgTilesX) - 1), ty = u >> sh.lgTilesX;
+        uint32_t c0[4][2];
+        int t = 0;
+#pragma unroll 1
+        for (int k = 0; k < (sh.tile == 0 ? 1 : 2); k++) {
+          const int x0 = tx * (sh.tile == 1 ? 8 : 4) + (sh.tile == 1 ? 4 * k : 0);
+          const int y0 = ty * (sh.tile == 2 ? 8 : 4) + (sh.tile == 2 ? 4 * k : 0);
+          int q[4][4], d[4][4];
+          chroma_predict_piece<4, 4>(sm, cd, sh, filt, maxv, x0, y0, q);
+          if (outBlk && act) store_pred<4, 4>(outBlk, w, x0, y0, false, q);
+          residual_unit<4, 4, false>(org + y0 * w + x0, w, q, d, sad);
+          wht_rows<4>(d);
+          if (sh.tile == 0) {
+            satd = (wht_cols_abs_sum<4>(d) + 1) >> 1;                            // CL/RdCost.cpp:2209
+          } else {
+            wht_cols<4>(d);
+            if (k == 0) {
+#pragma unroll
+              for (int i = 0; i < 4; i++)
+#pragma unroll
+                for (int j = 0; j < 2; j++) c0[i][j] = pack_u16x2(vabs(d[i][2 * j]), vabs(d[i][2 * j + 1]));
+            } else {
+#pragma unroll
+              for (int i = 0; i < 4; i++)
+#pragma unroll
+                for (int j = 0; j < 2; j++) t = add_halves_u16x2(max_u16x2(c0[i][j], pack_u16x2(vabs(d[i][2 * j]), vabs(d[i][2 * j + 1]))), t);
+            }
+          }
+        }
+        if (sh.tile != 0) satd = satd_norm_rect(2 * t, false);                  // CL/RdCost.cpp:2662, :2741
+      }
+      for (int o = lanes >> 1; o > 0; o >>= 1) {
+        sad  += __shfl_xor_sync(0xffffffffu, sad, o);
+        satd += __shfl_xor_sync(0xffffffffu, satd, o);
+      }
+      if (u == 0 && (task >> lgL) < 16) {
+        vvcb_chroma_result& r = P.results[vi];
+        r.sad[c][comp]  = act ? (uint32_t)sad : VVCB_SAT_NONE;
+        r.satd[c][comp] = act ? (uint32_t)satd : VVCB_SAT_NONE;
+        if (comp == 0) r.mode[c] = (uint8_t)code;
+      }
+    }
+  }
+}
+
+}  // namespace

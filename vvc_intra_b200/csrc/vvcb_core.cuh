@@ -225,6 +225,7 @@ struct WorkItem {            // 8 bytes
 // ---- reference lines ------------------------------------------------------------------------------
 // Availability is a set of at most five intervals on the walk bottom-left -> corner -> top-right; an
 // unavailable sample takes the nearest earlier available sample on the walk, or the first available one.
+// UNIT: samples per availability count, 4 for luma, 2 for 4:2:0 chroma (pcv.minCUWidth >> scaleX).
 struct LineGeom {
   int w, h, mrl, n;          // n = walk length
   int lo[5], hi[5];          // available intervals [lo, hi) in walk order: below-left, left, corner, above, above-right; an absent
@@ -233,17 +234,17 @@ struct LineGeom {
 };
 constexpr int kNoInterval = 0x3fffffff;
 
-VHD LineGeom make_line_geom(const vvcb_rmd_visit& v, int w, int h, int mrl)
+template <int UNIT = 4> VHD LineGeom make_line_geom(const vvcb_rmd_visit& v, int w, int h, int mrl)
 {
   LineGeom g;
   g.w = w; g.h = h; g.mrl = mrl;
   const int C = 2 * h + 2 * mrl + 1;
   g.n = C + 2 * w;
-  g.lo[0] = v.n_below_left  ? h - 4 * v.n_below_left : kNoInterval;  g.hi[0] = h;
-  g.lo[1] = v.n_left        ? 2 * h - 4 * v.n_left   : kNoInterval;  g.hi[1] = 2 * h;
-  g.lo[2] = v.avail_al      ? 2 * h                  : kNoInterval;  g.hi[2] = C;
-  g.lo[3] = v.n_above       ? C                      : kNoInterval;  g.hi[3] = C + 4 * v.n_above;
-  g.lo[4] = v.n_above_right ? C + w                  : kNoInterval;  g.hi[4] = C + w + 4 * v.n_above_right;
+  g.lo[0] = v.n_below_left  ? h - UNIT * v.n_below_left : kNoInterval;  g.hi[0] = h;
+  g.lo[1] = v.n_left        ? 2 * h - UNIT * v.n_left   : kNoInterval;  g.hi[1] = 2 * h;
+  g.lo[2] = v.avail_al      ? 2 * h                     : kNoInterval;  g.hi[2] = C;
+  g.lo[3] = v.n_above       ? C                         : kNoInterval;  g.hi[3] = C + UNIT * v.n_above;
+  g.lo[4] = v.n_above_right ? C + w                     : kNoInterval;  g.hi[4] = C + w + UNIT * v.n_above_right;
   g.first = -1;
 #pragma unroll
   for (int k = 4; k >= 0; k--) if (g.lo[k] != kNoInterval) g.first = g.lo[k];
@@ -374,8 +375,9 @@ VHD int clip_bd(int v, int maxv)
 
 // Angular prediction of the unit whose origin is (c0, r0) in the main/side frame.  ml points at the
 // slot's main line so that ml[t] == refMain0[t] (may be indexed with negative t); side points at
-// refSide0.  Output in the main/side frame: q[r][c].
-template <int R, int C> VHD void pred_angular_unit(const int16_t* ml, const int16_t* side, const ModeParam& p, int mrl,
+// refSide0.  Output in the main/side frame: q[r][c].  LINEAR: the 2-tap linear interpolation of chroma blocks
+// ((32 - f) * refMain[x + dInt + 1] + f * refMain[x + dInt + 2] + 16) >> 5 instead of the 4-tap luma filters (filt must still point at the table; its taps are unused).
+template <int R, int C, bool LINEAR = false> VHD void pred_angular_unit(const int16_t* ml, const int16_t* side, const ModeParam& p, int mrl,
                                                    int mw, int mh, int c0, int r0, const uint32_t* filt, int maxv, int (&q)[R][C])
 {
   const int angle = p.angle;
@@ -393,8 +395,10 @@ template <int R, int C> VHD void pred_angular_unit(const int16_t* ml, const int1
 #pragma unroll
     for (int j = 0; j < C + 3; j++) t[j] = m[j];
 #pragma unroll
-    for (int j = 0; j < C; j++)
-      q[i][j] = clip_bd((f0 * t[j] + f1 * t[j + 1] + f2 * t[j + 2] + f3 * t[j + 3] + 32) >> 6, maxv);
+    for (int j = 0; j < C; j++) {
+      if constexpr (LINEAR) q[i][j] = ((32 - dFrac) * t[j + 1] + dFrac * t[j + 2] + 16) >> 5;
+      else q[i][j] = clip_bd((f0 * t[j] + f1 * t[j + 1] + f2 * t[j + 2] + f3 * t[j + 3] + 32) >> 6, maxv);
+    }
   }
   #ifdef VVCB_EXP_NO_PDPC
   if (false) {

@@ -294,10 +294,10 @@ __global__ void __launch_bounds__(256) rmd_plan_small(const vvcb_rmd_visit* visi
 // The load is issued here; the caller stores it with store_line_entry once all the loads of its batch are in flight.
 struct LineCtx { LineGeom g; int extTop, extLeft, nTop, nLeft, total; };
 
-__device__ __forceinline__ LineCtx make_line_ctx(const vvcb_rmd_visit& v, const Shape& sh, int mrl)
+template <int UNIT = 4> __device__ __forceinline__ LineCtx make_line_ctx(const vvcb_rmd_visit& v, const Shape& sh, int mrl)
 {
   LineCtx c;
-  c.g = make_line_geom(v, sh.w, sh.h, mrl);
+  c.g = make_line_geom<UNIT>(v, sh.w, sh.h, mrl);
   // tails: the main reference of positive angles is extended by replication (CL/IntraPrediction.cpp:717-726)
   c.extTop = (mrl << vmax(0, sh.lw - sh.lh)) + 2; c.extLeft = (mrl << vmax(0, sh.lh - sh.lw)) + 2;
   c.nTop = 2 * sh.w + 1 + mrl; c.nLeft = 2 * sh.h + 1 + mrl;
@@ -372,12 +372,12 @@ __device__ void build_line_sets(SM& sm, const vvcb_rmd_visit& v, const Shape& sh
   }
 }
 
-// one line set (TU prediction kernel: a job needs line 0 and at most one more)
-template <class SM>
+// one line set (TU prediction kernel: a job needs line 0 and at most one more); UNIT as make_line_geom
+template <int UNIT = 4, class SM>
 __device__ void build_line_set(SM& sm, int set, int mrl, const vvcb_rmd_visit& v, const Shape& sh,
                                const int16_t* reco, int stride, int bd, int lane)
 {
-  const LineCtx c = make_line_ctx(v, sh, mrl);
+  const LineCtx c = make_line_ctx<UNIT>(v, sh, mrl);
   const int16_t* base = reco + (size_t)v.y * stride + v.x;
   for (int i = lane; i < c.total; i += 32) store_line_entry(sm, set, c, i, load_line_entry(c, base, stride, bd, i));
 }

@@ -90,6 +90,12 @@ ISP_RESULT_DTYPE = np.dtype([('part', TU_RESULT_DTYPE, ISP_MAX_PARTS), ('cbf_bit
                              ('n_parts', 'u1'), ('discarded', 'u1'), ('pad', 'u1', 2)], align=True)
 assert ISP_JOB_DTYPE.itemsize == 40 and ISP_RESULT_DTYPE.itemsize == 120
 AUTO_FINAL, AUTO_REGULAR = 1, 2
+# vvcb_chroma_visit / vvcb_chroma_result (include/vvc_intra_b200.h): one chroma CU of the separate tree, its 8 candidates' distortions
+CHROMA_CANDS, LM_CHROMA, MDLM_L, MDLM_T, DM_CHROMA = 8, 67, 68, 69, 70
+CHROMA_VISIT_DTYPE = np.dtype([('x', '<i2'), ('y', '<i2'), ('log2w', 'u1'), ('log2h', 'u1'), ('avail_al', 'u1'), ('n_above', 'u1'),
+                               ('n_above_right', 'u1'), ('n_left', 'u1'), ('n_below_left', 'u1'), ('dm_mode', 'u1'), ('cclm', 'u1'), ('pad', 'u1', 3)])
+CHROMA_RESULT_DTYPE = np.dtype([('mode', 'u1', CHROMA_CANDS), ('sad', '<u4', (CHROMA_CANDS, 2)), ('satd', '<u4', (CHROMA_CANDS, 2))], align=True)
+assert CHROMA_VISIT_DTYPE.itemsize == 16 and CHROMA_RESULT_DTYPE.itemsize == 136
 
 
 class EngineError(RuntimeError):
@@ -149,6 +155,9 @@ def load_library():
         L.vvcb_isp_mode_param.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
         L.vvcb_isp_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.vvcb_chroma_frame_begin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
+        L.vvcb_chroma_reco_update.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.vvcb_chroma_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.vvcb_ctu_hads_islice.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.vvcb_features_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.vvcb_frame_bind_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
@@ -428,6 +437,37 @@ class IntraCostEngine:
                                          _ptr(states) if states is not None else None, 0 if states is None else len(states), n_samples,
                                          p('level'), p('reco'), p('pred'), _ptr(out['results'])))
         return out
+
+    # ---- chroma intra candidates (4:2:0)
+    def chroma_frame_begin(self, cb, cr):
+        """vvcb_chroma_frame_begin: Cb / Cr originals of the picture given to frame_begin (half its width and height); reconstructions cleared."""
+        cb, cr = np.ascontiguousarray(cb, np.int16), np.ascontiguousarray(cr, np.int16)
+        if cb.shape != cr.shape:
+            raise ValueError('cb and cr must have the same shape')
+        self._ck(self._lib.vvcb_chroma_frame_begin(self._ctx, _ptr(cb), _ptr(cr), cb.shape[1], cb.shape[1], cb.shape[0]))
+
+    def chroma_reco_update(self, cb, cr, x=0, y=0):
+        """vvcb_chroma_reco_update: the rectangle of both chroma reconstructions at (x, y), chroma samples."""
+        cb, cr = np.ascontiguousarray(cb, np.int16), np.ascontiguousarray(cr, np.int16)
+        if cb.shape != cr.shape:
+            raise ValueError('cb and cr must have the same shape')
+        self._ck(self._lib.vvcb_chroma_reco_update(self._ctx, _ptr(cb), _ptr(cr), cb.shape[1], x, y, cb.shape[1], cb.shape[0]))
+
+    def chroma_eval(self, visits, want_pred=False):
+        """vvcb_chroma_eval: the 8 chroma candidates of every visit (CHROMA_VISIT_DTYPE) with SAD / SATD of Cb and Cr.  Returns the
+        CHROMA_RESULT_DTYPE array, or (results, pred) with want_pred: pred is a list of (8, 2, h, w) int16 arrays, one per visit."""
+        visits = np.ascontiguousarray(visits, CHROMA_VISIT_DTYPE)
+        out = np.zeros(len(visits), CHROMA_RESULT_DTYPE)
+        sizes = [2 * CHROMA_CANDS << (int(v['log2w']) + int(v['log2h'])) for v in visits] if want_pred else []
+        pred = np.zeros(sum(sizes), np.int16) if want_pred else None
+        self._ck(self._lib.vvcb_chroma_eval(self._ctx, _ptr(visits), len(visits), _ptr(pred) if want_pred else None, _ptr(out)))
+        if not want_pred:
+            return out
+        blocks, at = [], 0
+        for v, n in zip(visits, sizes):
+            blocks.append(pred[at:at + n].reshape(CHROMA_CANDS, 2, 1 << int(v['log2h']), 1 << int(v['log2w'])))
+            at += n
+        return out, blocks
 
     def residual_bits(self, jobs, levels, states):
         """vvcb_residual_bits: fractional bits of residual_coding for the given levels (flat int32 indexed by job['offset'])."""
