@@ -449,7 +449,8 @@ int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, con
  * parameters from the chroma block's own shape, reference lines never smoothed, the 2-tap linear interpolation) and the cross-component
  * modes (CL/IntraPrediction.cpp:1665-2150: xGetLumaRecPixels with the [1 2 1; 1 2 1] / 8 down-sampling of sps_cclm_colocated_chroma
  * = 0, xGetLMParameters, predIntraChromaLM) -- and measured with RdCost::xGetSAD / xGetHADs on the chroma block.  No ordering or
- * pruning of the candidates: that is the caller's.  Chroma TU coding (chroma QP mapping, joint Cb-Cr) is not in the library.
+ * pruning of the candidates: that is the caller's.  vvcb_chroma_tu_eval (below) codes the TUs of these candidates, Cb and Cr
+ * separately with DCT-II; joint Cb-Cr, chroma transform skip and the chroma QP mapping are not in the library.
  * Restated from H.266 and the cited reference lines; not compared with the reference encoder's own chroma output.                   */
 #define VVCB_CHROMA_CANDS 8
 #define VVCB_LM_CHROMA   67   /* LM_CHROMA_IDX: CCLM from the above and left neighbours */
@@ -490,6 +491,58 @@ typedef struct vvcb_chroma_result {
  * counts above their maximum, dm_mode > 66, a CU or neighbour outside the chroma picture; VVCB_ERR_STATE before
  * vvcb_chroma_frame_begin and through the broker.                                                                                 */
 int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n, int16_t* pred_out, vvcb_chroma_result* results);
+
+/* ---- chroma TU coding of the candidates (4:2:0, separate tree, Cb and Cr coded separately) -------------------------------------
+ * The chroma part of IntraSearch::xRecurIntraChromaCodingQT (EL/IntraSearch.cpp) for a TU that covers its chroma CU -- xIntraCodingTUBlock
+ * (:2694) of Cb, then of Cr -- and the chroma bins of xGetIntraFracBitsQT (:2566), for the candidates estIntraPredChromaQT prices on their
+ * full RD cost.  A job is one chroma CU (visit), one of its 8 candidates and one quantiser setting:
+ *   - prediction: exactly what vvcb_chroma_eval predicts for (visit, cand), the LM modes from the context's luma reconstruction;
+ *     residual = original - prediction, from the planes of vvcb_chroma_frame_begin;
+ *   - TrQuant::transformNxN with DCT-II in both directions, Quant::quant (scalar, intra rounding) or, with VVCB_TU_DEPQUANT,
+ *     DepQuant::quant on the chroma context sets and per-position offsets of H.266 9.3.4.2.5-9.3.4.2.8: significance context
+ *     36 + 8 * max(0, state - 1) + min((sumAbs1 + 1) >> 1, 3) + (d < 2 ? 4 : 0), greater-than / parity context
+ *     min(sumAbs1 - numPos, 4) + 1 + (d == 0 ? 5 : 0) (d = x + y), last-position prefix contexts from offset 20 with shift
+ *     Clip3(0, 2, side >> 3), coded-sub-block flag contexts 2..3; then the dequantiser, invTransformNxN, reconstruction and RdCost::xGetSSE;
+ *   - cbfDeltaBits (RateEstimator::xSetLastCoeffOffset, CL/DepQuant.cpp:491-540): Cb's from Ctx::QtCbf[Cb](0), Cr's from Ctx::QtCbf[Cr]
+ *     selected by Cb's final cbf (prevCbf); so Cr is quantised after Cb's levels are final.  Both quantisers are priced on the
+ *     candidate's starting snapshot states[rate_idx];
+ *   - with VVCB_TU_RATE: the chroma bins of transform_unit on ONE carried copy of states[rate_idx], in coding order -- tu_cb_coded_flag
+ *     (context 0), tu_cr_coded_flag (context = Cb's cbf), residual_coding of Cb, residual_coding of Cr (priced on the models Cb's
+ *     residual left); each bin priced, then its model adapted.  Sign hiding is not modelled (as for luma).
+ * Restated from H.266 and the cited reference lines, as the ISP and chroma-prediction entries are: parity with the reference encoder's
+ * own chroma coding is unpinned.  NOT in the library: joint Cb-Cr, chroma transform skip (its transform_skip_flag bin has contexts of
+ * its own and stays with the caller), LFNST for chroma, the chroma QP mapping (the caller passes QpParam per component, its mapping
+ * table and offsets applied), chroma distortion weighting (the caller applies m_distortionWeight to sse), 2xN blocks, 4:2:2 / 4:4:4,
+ * ISP-coupled chroma.                                                                                                              */
+typedef struct vvcb_chroma_ctx_states {   /* the estimator's chroma models at the start of the chroma TU (as vvcb_ctx_states)       */
+  vvcb_bin_model cbf_cb[2], cbf_cr[3];   /* Ctx::QtCbf[Cb] / [Cr] (tu_cb_coded_flag: 2 contexts, tu_cr_coded_flag: 3)           */
+  vvcb_bin_model sig_sbb[2];             /* Ctx::SigCoeffGroup[CHANNEL_TYPE_CHROMA]                                              */
+  vvcb_bin_model sig[3][8];              /* Ctx::SigFlag[1], [3], [5]: one set per quantiser-state class                          */
+  vvcb_bin_model par[11], gt1[11], gt2[11];   /* Ctx::ParFlag[chroma], GtxFlag[3], GtxFlag[1]                                   */
+  vvcb_bin_model last_x[3], last_y[3];   /* Ctx::LastX / LastY[chroma]                                                           */
+} vvcb_chroma_ctx_states;                /* 70 models, 420 bytes */
+typedef struct vvcb_chroma_tu_job {
+  uint32_t visit;              /* index into visits[]                                                                            */
+  uint8_t  cand;               /* 0..7, the candidate order of vvcb_chroma_result, the DM -> VDIA substitution included          */
+  uint8_t  flags;              /* VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE]                                            */
+  uint16_t rate_idx;           /* states[rate_idx]: the models at the start of the candidate (DEPQUANT or RATE)                  */
+  int16_t  qp_per[2], qp_rem[2];   /* QpParam(tu, COMPONENT_Cb / Cr): the caller's chroma QP mapping and offsets applied          */
+  uint32_t offset;             /* first sample of this candidate's outputs: Cb w*h, then Cr w*h                                  */
+  uint32_t pad;
+  double   lambda[2];          /* Quant::m_dLambda while Cb / Cr are quantised (DEPQUANT)                                        */
+} vvcb_chroma_tu_job;          /* 40 bytes */
+typedef struct vvcb_chroma_tu_result {
+  vvcb_tu_result comp[2];      /* Cb, Cr: abs sums, unweighted sse (xGetSSE), residual frac_bits (VVCB_TU_RATE, 0 without a level) */
+  uint32_t cbf_bits[2];        /* VVCB_TU_RATE: fractional bits of tu_cb_coded_flag / tu_cr_coded_flag                           */
+  uint8_t  cbf[2], pad[6];
+} vvcb_chroma_tu_result;       /* 64 bytes */
+/* visits, jobs, states: HOST arrays (n_visits, n, n_states; states may be NULL when no job has DEPQUANT or RATE).  level / reco / pred:
+ * optional HOST outputs of n_samples.  VVCB_ERR_ARG for a visit vvcb_chroma_eval refuses, cand > 7, an LM candidate of a visit with
+ * cclm == 0, other flags, per / rem out of range for the bit depth, a bad rate_idx, lambda <= 0 with DEPQUANT, or outputs outside
+ * n_samples; VVCB_ERR_STATE before vvcb_chroma_frame_begin and through the broker.                                                 */
+int vvcb_chroma_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_tu_job* jobs, int n,
+                        const vvcb_chroma_ctx_states* states, int n_states, size_t n_samples,
+                        int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_tu_result* results);
 
 /* ---- texture features (orig-only, trivially parallel) ------------------------------------------------------------
  * vvcb_ctu_hads_islice: EncCu::updateCtuDataISlice (EL/EncCu.cpp:564-675) for every CTU of the frame, as

@@ -1031,6 +1031,10 @@ struct TuChain {
   vvcb_dq_rates* rates; int nRates;                                 // quantiser prices
   const vvcb_ctx_states* priceFrom;                                 // optional: rates_from_states_kernel fills `rates` from these models first
   const vvcb_ctx_states* states; vvcb_ctx_states* statesOut;        // rate_kernel's models; statesOut optional
+  // chroma jobs (vvcb_chroma_tu_eval): the chroma instantiations of the quantiser and rate kernels run, and priceFrom / states / statesOut
+  // point at vvcb_chroma_ctx_states
+  bool chroma;
+  const int16_t* orig; int stride;                                  // the original plane the jobs' x / y address; nullptr: the luma plane
 };
 
 // Launches one TU batch: tu_eval_kernel pass 0 in its two team sizes, the dependent quantiser and / or transform-skip RDOQ, pass 1 for
@@ -1040,7 +1044,7 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
   const int nSmall = L.nSmall, nLarge = (int)L.team.size() - nSmall, nDq = (int)L.dq.size(), nTs = (int)L.ts.size(), nRate = (int)L.rate.size();
   TuParams P;
   P.jobs = c.jobs; P.list = nullptr; P.n = 0; P.resi = c.resi; P.pred = c.pred; P.coeff = c.coeff; P.level = c.level; P.reco = c.reco;
-  P.results = c.results; P.orig = ctx->bOrig; P.stride = ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
+  P.results = c.results; P.orig = c.orig ? c.orig : ctx->bOrig; P.stride = c.orig ? c.stride : ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
   P.dqCoeff = static_cast<int32_t*>(ctx->dTu[kDqCoeff]); P.dqDeq = c.deq; P.phase = 0; P.trPair = c.trPair;
   auto launch_tu = [&](TuParams Q) {
     if (nSmall) { Q.list = c.team; Q.n = nSmall; tu_eval_kernel<32><<<std::min((nSmall + 3) / 4, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
@@ -1055,7 +1059,12 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
     CK(cudaStreamWaitEvent(ctx->sKind[0], ctx->evPlan, 0));
   }
   if (nDq) {
-    if (c.priceFrom) {
+    if (c.priceFrom && c.chroma) {
+      const long long nPrice = (long long)c.nRates * kChromaResidualModels;
+      chroma_rates_from_states_kernel<<<(unsigned)((nPrice + 127) / 128), 128, 0, ctx->stream>>>(
+          reinterpret_cast<const vvcb_chroma_ctx_states*>(c.priceFrom), c.nRates, ctx->dRateRom, c.rates);
+      ctx->launches++;
+    } else if (c.priceFrom) {
       const long long nPrice = (long long)c.nRates * kDqRateModels;
       rates_from_states_kernel<<<(unsigned)((nPrice + 127) / 128), 128, 0, ctx->stream>>>(c.priceFrom, c.nRates, ctx->dRateRom, c.rates);
       ctx->launches++;
@@ -1080,7 +1089,8 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
     D.coeff = P.dqCoeff; D.level = c.level; D.deq = c.deq; D.results = c.results;
     D.rates = c.rates; D.tabs = static_cast<const DqRateTab*>(ctx->dTu[kDqTabs]);
     D.rom = ctx->dDqRom; D.scratch = static_cast<uint8_t*>(ctx->dTu[kDqScratch]); D.bd = ctx->bd; D.sparse = !sortJobs;
-    dq_kernel<<<dq_grid(ctx, nDq), kDqThreads, 0, ctx->stream>>>(D);
+    if (c.chroma) dq_kernel<true><<<dq_grid(ctx, nDq), kDqThreads, 0, ctx->stream>>>(D);
+    else dq_kernel<false><<<dq_grid(ctx, nDq), kDqThreads, 0, ctx->stream>>>(D);
     ctx->launches += 3;
   }
   if (nTs) {
@@ -1105,7 +1115,9 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
     RateParams R;
     R.jobs = c.jobs; R.order = c.rate; R.n = nRate; R.level = c.level; R.results = c.results;
     R.states = c.states; R.statesOut = c.statesOut; R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
-    rate_kernel<<<std::min((nRate + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
+    const int g = std::min((nRate + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms);
+    if (c.chroma) rate_kernel<true><<<g, kRateThreads, 0, ctx->stream>>>(R);
+    else rate_kernel<false><<<g, kRateThreads, 0, ctx->stream>>>(R);
     ctx->launches++;
   }
   if (ev) CK(cudaEventRecord(ev[4], ctx->stream));
@@ -1911,6 +1923,181 @@ extern "C" int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, 
   CK(cudaMemcpyAsync(results, P.results, sizeof(vvcb_chroma_result) * n, cudaMemcpyDeviceToHost, ctx->stream));
   if (pred_out) CK(cudaMemcpyAsync(pred_out, P.predOut, sizeof(int16_t) * total, cudaMemcpyDeviceToHost, ctx->stream));
   CK(ctx_sync(ctx));
+  return VVCB_OK;
+}
+
+// Chroma TU coding (include/vvc_intra_b200.h): two steps over the TU kernels, Cb then Cr, because Cr's cbfDeltaBits depend on Cb's final cbf.
+//   chroma_tu_pred_kernel        prediction and residual of both components of every candidate, Cb's cbfDeltaBits;
+//   run_tu_chain (Cb jobs)       pass 0, the dependent quantiser priced by chroma_rates_from_states_kernel from the candidates' starting
+//                                models, pass 1 (reconstruction, SSE), rate_kernel_chroma adapting each candidate's carried models in place;
+//   chroma_cbf_kernel step 1     Cb's cbf bin, Cr's cbfDeltaBits;
+//   run_tu_chain (Cr jobs)       the same kernels on the Cr plane, the quantiser on the prices of step 0, the rate on the models Cb left;
+//   chroma_cbf_kernel step 2     Cr's cbf bin.
+// One chunk of at most kChromaTuChunk candidates (their TU jobs name the carried snapshots with the 16-bit rate_idx); base: index of the
+// chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
+constexpr int kChromaTuChunk = 65536;
+static int chroma_tu_chunk(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_tu_job* jobs, int n, int base,
+                           const vvcb_chroma_ctx_states* states, int n_states, size_t n_samples,
+                           int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_tu_result* results, bool checkOnly)
+{
+  const unsigned kFlags = VVCB_TU_QUANT | VVCB_TU_DEPQUANT | VVCB_TU_RATE;
+  std::vector<vvcb_tu_job> tj((size_t)2 * n);       // [Cb jobs | Cr jobs]
+  std::vector<vvcb_chroma_ctx_states> cst(n);
+  std::vector<uint32_t> from(n);
+  size_t cs = 0;                                   // the chunk's own samples: candidates are packed densely on the device, whatever the caller's offsets
+  for (int i = 0; i < n; i++) {
+    const vvcb_chroma_tu_job& j = jobs[i];
+    auto bad = [&](const char* why) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: job %d: %s", base + i, why); return VVCB_ERR_ARG; };
+    if (j.visit >= (uint32_t)n_visits) return bad("visit index out of range");
+    const vvcb_chroma_visit& v = visits[j.visit];
+    if (j.cand >= VVCB_CHROMA_CANDS) return bad("cand above 7");
+    const int code = chroma_cand_code(j.cand, v.dm_mode);
+    if (code >= VVCB_LM_CHROMA && code <= VVCB_MDLM_T && !v.cclm) return bad("LM candidate of a visit without cclm");
+    if ((j.flags & ~kFlags) || !(j.flags & VVCB_TU_QUANT)) return bad("flags: VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE] only");
+    for (int c = 0; c < 2; c++)
+      if (j.qp_rem[c] < 0 || j.qp_rem[c] >= 6 || j.qp_per[c] < 0 || 6 * j.qp_per[c] + j.qp_rem[c] > max_qp(ctx->bd)) return bad("qp_per / qp_rem out of range");
+    const bool dq = (j.flags & VVCB_TU_DEPQUANT) != 0, carried = dq || (j.flags & VVCB_TU_RATE);
+    if (carried && (!states || j.rate_idx >= n_states)) return bad("rate_idx does not name a context snapshot");
+    if (dq && (!lambda_ok(j.lambda[0]) || !lambda_ok(j.lambda[1]))) return bad("dependent quantisation needs finite lambdas > 0");
+    const size_t m = (size_t)1 << (v.log2w + v.log2h);
+    if ((size_t)j.offset + 2 * m > n_samples) return bad("outputs outside n_samples");
+    if (carried) cst[i] = states[j.rate_idx]; else memset(&cst[i], 0, sizeof(vvcb_chroma_ctx_states));
+    from[i] = (uint32_t)cs;
+    for (int c = 0; c < 2; c++) {
+      vvcb_tu_job& t = tj[(size_t)c * n + i];
+      memset(&t, 0, sizeof(t));
+      t.x = v.x; t.y = v.y; t.log2w = v.log2w; t.log2h = v.log2h;
+      t.flags = j.flags; t.qp_per = j.qp_per[c]; t.qp_rem = j.qp_rem[c];
+      t.offset = (uint32_t)(cs + c * m);
+      t.rate_idx = (uint16_t)i;                        // the candidate's own carried snapshot
+      t.lambda = j.lambda[c];
+    }
+    cs += 2 * m;
+  }
+  if (checkOnly) return VVCB_OK;
+  TuLists L[2];
+  for (int c = 0; c < 2; c++) L[c] = tu_lists(&tj[(size_t)c * n], n, [](int) { return true; });
+  // one input arena in page-locked memory: visits, candidates, TU jobs, carried models, lists
+  Arena in;
+  const size_t iVis = in.take((size_t)n_visits * sizeof(vvcb_chroma_visit)), iJob = in.take((size_t)n * sizeof(vvcb_chroma_tu_job)),
+               iTj = in.take(tj.size() * sizeof(vvcb_tu_job)), iCst = in.take((size_t)n * sizeof(vvcb_chroma_ctx_states));
+  size_t iTeam[2], iDq[2], iRate[2];
+  for (int c = 0; c < 2; c++) { iTeam[c] = in.take(L[c].team.size() * sizeof(int)); iDq[c] = in.take(L[c].dq.size() * sizeof(int)); iRate[c] = in.take(L[c].rate.size() * sizeof(int)); }
+  int rc;
+  if ((rc = pin_buf(ctx, kPinStageIn, in.size))) return rc;
+  void* hin = ctx->hPin[kPinStageIn];
+  memcpy(at<vvcb_chroma_visit>(hin, iVis), visits, (size_t)n_visits * sizeof(vvcb_chroma_visit));
+  memcpy(at<vvcb_chroma_tu_job>(hin, iJob), jobs, (size_t)n * sizeof(vvcb_chroma_tu_job));
+  memcpy(at<vvcb_tu_job>(hin, iTj), tj.data(), tj.size() * sizeof(vvcb_tu_job));
+  memcpy(at<vvcb_chroma_ctx_states>(hin, iCst), cst.data(), (size_t)n * sizeof(vvcb_chroma_ctx_states));
+  auto put = [&](size_t o, const std::vector<int>& v) { if (!v.empty()) memcpy(at<int>(hin, o), v.data(), v.size() * sizeof(int)); };
+  for (int c = 0; c < 2; c++) { put(iTeam[c], L[c].team); put(iDq[c], L[c].dq); put(iRate[c], L[c].rate); }
+  // work arena: TU results, prediction, residual, reconstruction, levels, dequantised coefficients, derived prices, cbf flags and bits
+  Arena work;
+  const size_t oRes = work.take((size_t)2 * n * sizeof(vvcb_tu_result)), oPred = work.take(cs * sizeof(int16_t)), oResi = work.take(cs * sizeof(int16_t)),
+               oReco = work.take(cs * sizeof(int16_t)), oLevel = work.take(cs * sizeof(int32_t)), oDeq = work.take(cs * sizeof(int32_t)),
+               oRates = work.take((size_t)n * sizeof(vvcb_dq_rates)), oCbf = work.take((size_t)2 * n), oCbfBits = work.take((size_t)2 * n * sizeof(uint32_t));
+  const int nDq[2] = { (int)L[0].dq.size(), (int)L[1].dq.size() };
+  CK(cudaSetDevice(ctx->device));
+  if ((rc = tu_buf(ctx, kStageIn, in.size))) return rc;
+  if ((rc = tu_buf(ctx, kStageOut, work.size))) return rc;
+  if ((rc = quant_scratch(ctx, cs, n, nDq, 2))) return rc;
+  void* din = ctx->dTu[kStageIn];
+  void* dw = ctx->dTu[kStageOut];
+  CK(cudaMemcpyAsync(din, hin, in.size, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemsetAsync(at<uint8_t>(dw, oLevel), 0, oRates - oLevel, ctx->stream));        // levels / dequantised coefficients the quantisers do not reach stay zero
+  CK(cudaMemsetAsync(at<uint8_t>(dw, oCbf), 0, work.size - oCbf, ctx->stream));
+  vvcb_tu_job* dTj = at<vvcb_tu_job>(din, iTj);
+  vvcb_chroma_ctx_states* dCst = at<vvcb_chroma_ctx_states>(din, iCst);
+  vvcb_tu_result* dRes = at<vvcb_tu_result>(dw, oRes);
+  int16_t* dPred = at<int16_t>(dw, oPred); int16_t* dResi = at<int16_t>(dw, oResi);
+  int16_t* dReco = at<int16_t>(dw, oReco); int32_t* dLevel = at<int32_t>(dw, oLevel);
+  uint8_t* dCbf = at<uint8_t>(dw, oCbf); uint32_t* dCbfBits = at<uint32_t>(dw, oCbfBits);
+  const size_t plane = (size_t)ctx->cstride * ctx->ch;
+  {
+    ChromaTuPredParams Q = {};
+    ChromaParams& B = Q.planes;
+    B.visits = at<const vvcb_chroma_visit>(din, iVis); B.n = n_visits;
+    B.orig[0] = ctx->dChroma; B.orig[1] = ctx->dChroma + plane; B.reco[0] = ctx->dChroma + 2 * plane; B.reco[1] = ctx->dChroma + 3 * plane;
+    B.cstride = ctx->cstride; B.luma = ctx->bReco; B.lstride = ctx->stride; B.bd = ctx->bd; B.ctu = ctx->ctu; B.rom = ctx->dRom;
+    Q.jobs = at<const vvcb_chroma_tu_job>(din, iJob); Q.n = n; Q.cbJobs = dTj; Q.states = dCst;
+    Q.pred = dPred; Q.resi = dResi; Q.frac = ctx->dRateRom->binFracBits;
+    chroma_tu_pred_kernel<<<std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16), kChromaWarps * 32, 0, ctx->stream>>>(Q);
+    ctx->launches++;
+  }
+  for (int c = 0; c < 2; c++) {
+    TuChain t = {};
+    t.jobs = dTj + (size_t)c * n;
+    t.team = at<const int>(din, iTeam[c]); t.dq = at<const int>(din, iDq[c]); t.rate = at<const int>(din, iRate[c]);
+    t.resi = dResi; t.pred = dPred; t.level = dLevel; t.reco = dReco; t.deq = at<int32_t>(dw, oDeq); t.results = dRes + (size_t)c * n;
+    t.rates = at<vvcb_dq_rates>(dw, oRates); t.nRates = n;
+    t.priceFrom = c == 0 ? reinterpret_cast<const vvcb_ctx_states*>(dCst) : nullptr;      // both quantisers on the starting models
+    t.states = reinterpret_cast<const vvcb_ctx_states*>(dCst); t.statesOut = reinterpret_cast<vvcb_ctx_states*>(dCst);
+    t.chroma = true; t.orig = ctx->dChroma + c * plane; t.stride = ctx->cstride;
+    if ((rc = run_tu_chain(ctx, t, L[c], nullptr))) return rc;
+    ChromaCbfParams F;
+    F.n = n; F.step = c + 1; F.res = dRes + (size_t)c * n; F.crJobs = dTj + n; F.states = dCst; F.cbf = dCbf; F.cbfBits = dCbfBits;
+    F.frac = ctx->dRateRom->binFracBits;
+    chroma_cbf_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(F);
+    ctx->launches++;
+  }
+  CK(cudaGetLastError());
+  // page-locked output staging: TU results, cbf flags and bits, then the wanted sample outputs of the chunk's densely packed candidates
+  Arena out;
+  const size_t hRes = out.take((size_t)2 * n * sizeof(vvcb_tu_result)), hCbf = out.take((size_t)2 * n), hBits = out.take((size_t)2 * n * sizeof(uint32_t)),
+               hLv = out.take(level ? cs * sizeof(int32_t) : 0), hRc = out.take(reco ? cs * sizeof(int16_t) : 0), hPr = out.take(pred ? cs * sizeof(int16_t) : 0);
+  if ((rc = pin_buf(ctx, kPinStageOut, out.size))) return rc;
+  void* hout = ctx->hPin[kPinStageOut];
+  CK(cudaMemcpyAsync(at<uint8_t>(hout, hRes), dRes, (size_t)2 * n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(at<uint8_t>(hout, hCbf), dCbf, (size_t)2 * n, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(at<uint8_t>(hout, hBits), dCbfBits, (size_t)2 * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (level) CK(cudaMemcpyAsync(at<uint8_t>(hout, hLv), dLevel, cs * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (reco) CK(cudaMemcpyAsync(at<uint8_t>(hout, hRc), dReco, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (pred) CK(cudaMemcpyAsync(at<uint8_t>(hout, hPr), dPred, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(ctx_sync(ctx));
+  const vvcb_tu_result* res = at<const vvcb_tu_result>(hout, hRes);
+  const uint8_t* cbf = at<const uint8_t>(hout, hCbf);
+  const uint32_t* bits = at<const uint32_t>(hout, hBits);
+  for (int i = 0; i < n; i++) {
+    const size_t m = (size_t)2 << (visits[jobs[i].visit].log2w + visits[jobs[i].visit].log2h), to = jobs[i].offset;
+    if (level) memcpy(level + to, at<const int32_t>(hout, hLv) + from[i], m * sizeof(int32_t));
+    if (reco) memcpy(reco + to, at<const int16_t>(hout, hRc) + from[i], m * sizeof(int16_t));
+    if (pred) memcpy(pred + to, at<const int16_t>(hout, hPr) + from[i], m * sizeof(int16_t));
+    vvcb_chroma_tu_result& r = results[i];
+    memset(&r, 0, sizeof(r));
+    const bool rate = (jobs[i].flags & VVCB_TU_RATE) != 0;
+    for (int c = 0; c < 2; c++) {
+      r.comp[c] = res[(size_t)c * n + i];
+      if (!rate) r.comp[c].frac_bits = 0;
+      r.cbf[c] = cbf[2 * i + c];
+      r.cbf_bits[c] = rate ? bits[2 * i + c] : 0;
+    }
+  }
+  return VVCB_OK;
+}
+
+extern "C" int vvcb_chroma_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_tu_job* jobs, int n,
+                                   const vvcb_chroma_ctx_states* states, int n_states, size_t n_samples,
+                                   int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_tu_result* results)
+{
+  if (!ctx) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_chroma_tu_eval");
+  if (n < 0 || n_states < 0 || n_visits < 0 || (n > 0 && (!jobs || !results || !visits || n_visits == 0))) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: bad argument"); return VVCB_ERR_ARG;
+  }
+  if (!ctx->cw || ctx->cw != ctx->width / 2 || ctx->ch != ctx->height / 2 || !ctx->bReco) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: vvcb_chroma_frame_begin has not been called for this picture");
+    return VVCB_ERR_STATE;
+  }
+  if (n == 0) return VVCB_OK;
+  for (int i = 0; i < n_visits; i++)
+    if (const char* why = chroma_visit_error(ctx, visits[i])) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: visit %d: %s", i, why); return VVCB_ERR_ARG; }
+  for (int pass = 0; pass < 2; pass++)                               // every job is validated before anything runs
+    for (int b = 0; b < n; b += kChromaTuChunk) {
+      const int rc = chroma_tu_chunk(ctx, visits, n_visits, jobs + b, std::min(kChromaTuChunk, n - b), b, states, n_states, n_samples,
+                                     level, reco, pred, results + b, pass == 0);
+      if (rc) return rc;
+    }
   return VVCB_OK;
 }
 

@@ -1,6 +1,6 @@
 // vvc_intra_b200 -- chroma intra candidates (vvcb_chroma_eval): prediction of Cb and Cr under the 8 candidates of
 // PU::getIntraChromaCandModes and their SAD / SATD, 4:2:0.  Included by vvcb_api.cu and, through the CUDA-on-pthreads shim, by
-// tests/host_emul/emul_chroma.cpp.
+// tests/host_emul/emul_chroma.cpp and emul_chroma_tu.cpp.
 //
 // One warp per visit (a chroma CU of the separate tree), warps striding over the batch:
 //   1. the Cb and Cr reference lines into shared memory -- the luma padding walk (build_line_set) with a unit of 2 samples, line 0 only,
@@ -143,6 +143,92 @@ __device__ __forceinline__ void chroma_predict_piece(const ChromaSmem& sm, const
   }
 }
 
+// Steps 1 and 2 for one visit, the whole warp: reference lines, originals, down-sampled luma, LM parameters, DC values, DM's projected
+// main reference into sm.  Returns the block's shape; sm is complete for every lane on return.
+__device__ __forceinline__ Shape chroma_visit_setup(ChromaSmem& sm, const ChromaParams& P, const Rom& rom, const vvcb_chroma_visit& cv, int lane)
+{
+  const Shape sh = make_shape(cv.log2w, cv.log2h);
+  const int w = sh.w, h = sh.h;
+  vvcb_rmd_visit lv = {};                                // the walk's view of the visit (position, size, availability)
+  lv.x = cv.x; lv.y = cv.y; lv.log2w = cv.log2w; lv.log2h = cv.log2h;
+  lv.avail_al = cv.avail_al; lv.n_above = cv.n_above; lv.n_above_right = cv.n_above_right; lv.n_left = cv.n_left; lv.n_below_left = cv.n_below_left;
+  const bool availT = cv.n_above == (w >> 1), availL = cv.n_left == (h >> 1);
+  const int nAr = availT ? 2 * cv.n_above_right : 0, nBl = availL ? 2 * cv.n_below_left : 0;
+  const int dm = cv.dm_mode;
+  ModeParam dmp = rom.mode[sh.lw - 2][sh.lh - 2][dm];
+  __syncwarp();
+  // ---- 1. reference lines and originals
+#pragma unroll 1
+  for (int c = 0; c < 2; c++) build_line_set<2>(sm, c, 0, lv, sh, P.reco[c], P.cstride, P.bd, lane);
+  for (int i = lane; i < 2 * w * h; i += 32) {
+    const int c = i >> (sh.lw + sh.lh), s = i & (w * h - 1);
+    sm.org[c][s] = P.orig[c][(size_t)(cv.y + (s >> sh.lw)) * P.cstride + cv.x + (s & (w - 1))];
+  }
+  // ---- 2. down-sampled luma (xGetLumaRecPixels, 4:2:0, [1 2 1; 1 2 1] / 8; one row [1 2 1] / 4 above a CTU's first row)
+  if (cv.cclm) {
+    const int16_t* Y = P.luma + (size_t)(2 * cv.y) * P.lstride + 2 * cv.x;
+    const int ls = P.lstride;
+    const bool ctuTop = (cv.y & ((P.ctu >> 1) - 1)) == 0;
+    const int nTop = availT ? w + vmin(nAr, h) : 0, nLeft = availL ? h + vmin(nBl, w) : 0;
+    for (int i = lane; i < w * h + nTop + nLeft; i += 32) {
+      int v;
+      if (i < w * h + nTop) {
+        const int x = i < w * h ? i & (w - 1) : i - w * h;
+        const int xl = 2 * x - (x == 0 && !availL ? 0 : 1);      // no left neighbours: column -1 padded from column 0
+        const int16_t* r0 = i < w * h ? Y + (size_t)(2 * (i >> sh.lw)) * ls : Y - 2 * ls;
+        if (i >= w * h && ctuTop) v = (2 * r0[ls + 2 * x] + r0[ls + 2 * x + 1] + r0[ls + xl] + 2) >> 2;
+        else v = (2 * r0[2 * x] + r0[2 * x + 1] + r0[xl] + 2 * r0[ls + 2 * x] + r0[ls + 2 * x + 1] + r0[ls + xl] + 4) >> 3;
+        if (i < w * h) sm.ds[i] = (int16_t)v;
+        else sm.dsTop[x] = (int16_t)v;
+      } else {
+        const int j = i - w * h - nTop;
+        const int16_t* r0 = Y + (size_t)(2 * j) * ls - 3;
+        sm.dsLeft[j] = (int16_t)((2 * r0[1] + r0[2] + r0[0] + 2 * r0[ls + 1] + r0[ls + 2] + r0[ls] + 4) >> 3);
+      }
+    }
+  }
+  __syncwarp();
+  // LM parameters (lanes 0..5), DC values (lanes 6, 7), DM's projected main reference (every lane)
+  if (cv.cclm && lane < 6) {
+    int o[3];
+    chroma_lm_params(sm, lane >> 1, lane & 1, w, h, P.bd, availT, availL, nAr, nBl, o);
+    sm.lm[lane >> 1][lane & 1][0] = o[0]; sm.lm[lane >> 1][lane & 1][1] = o[1]; sm.lm[lane >> 1][lane & 1][2] = o[2];
+  } else if (lane == 6 || lane == 7) {
+    const int c = lane - 6;
+    int sum = 0;
+    if (w >= h) for (int i = 0; i < w; i++) sum += sm.lines[c][0][1 + i];
+    if (w <= h) for (int i = 0; i < h; i++) sum += sm.lines[c][1][1 + i];
+    const int denom = w == h ? 2 * w : vmax(w, h);
+    sm.dc[c] = (sum + (denom >> 1)) >> vlog2(denom);
+  }
+  if (dm > 1 && dmp.angle < 0) {
+    SlotInfo s = {};
+    s.kind = 2; s.mode = dm; s.p = dmp;
+#pragma unroll 1
+    for (int c = 0; c < 2; c++) {
+      s.set = c;
+      build_projected_line(sm.proj[c], sm, s, dmp.is_ver ? w : h, dmp.is_ver ? h : w, lane, 32);
+    }
+  }
+  __syncwarp();
+  return sh;
+}
+
+// candidate `mode` (0..66 or an LM mode, DM resolved) of component comp, as chroma_predict_piece reads it.  LM modes of a visit without
+// cclm get shadow parameters (nothing of theirs is stored).
+__device__ __forceinline__ ChromaCand chroma_make_cand(const ChromaSmem& sm, const Rom& rom, const Shape& sh, int mode, int comp, bool cclm)
+{
+  ChromaCand cd;
+  cd.comp = comp;
+  cd.kind = mode == 0 ? 0 : mode == 1 ? 1 : mode < VVCB_LM_CHROMA ? 2 : 3;
+  cd.p = rom.mode[sh.lw - 2][sh.lh - 2][mode < VVCB_LM_CHROMA ? mode : 0];
+  cd.dc = sm.dc[comp];
+  const int lm = vmin(vmax(mode - VVCB_LM_CHROMA, 0), 2);
+  cd.a = sm.lm[lm][comp][0]; cd.k = sm.lm[lm][comp][1]; cd.b = sm.lm[lm][comp][2];
+  if (cd.kind == 3 && !cclm) { cd.a = 0; cd.k = 0; cd.b = 0; }
+  return cd;
+}
+
 __global__ void __launch_bounds__(kChromaWarps * 32) chroma_eval_kernel(ChromaParams P)
 {
   __shared__ ChromaSmem smem[kChromaWarps];
@@ -153,70 +239,8 @@ __global__ void __launch_bounds__(kChromaWarps * 32) chroma_eval_kernel(ChromaPa
   const int maxv = (1 << P.bd) - 1;
   for (int vi = blockIdx.x * kChromaWarps + warp; vi < P.n; vi += gridDim.x * kChromaWarps) {
     const vvcb_chroma_visit cv = P.visits[vi];
-    const Shape sh = make_shape(cv.log2w, cv.log2h);
-    const int w = sh.w, h = sh.h;
-    vvcb_rmd_visit lv = {};                                // the walk's view of the visit (position, size, availability)
-    lv.x = cv.x; lv.y = cv.y; lv.log2w = cv.log2w; lv.log2h = cv.log2h;
-    lv.avail_al = cv.avail_al; lv.n_above = cv.n_above; lv.n_above_right = cv.n_above_right; lv.n_left = cv.n_left; lv.n_below_left = cv.n_below_left;
-    const bool availT = cv.n_above == (w >> 1), availL = cv.n_left == (h >> 1);
-    const int nAr = availT ? 2 * cv.n_above_right : 0, nBl = availL ? 2 * cv.n_below_left : 0;
-    const int dm = cv.dm_mode;
-    ModeParam dmp = rom.mode[sh.lw - 2][sh.lh - 2][dm];
-    __syncwarp();
-    // ---- 1. reference lines and originals
-#pragma unroll 1
-    for (int c = 0; c < 2; c++) build_line_set<2>(sm, c, 0, lv, sh, P.reco[c], P.cstride, P.bd, lane);
-    for (int i = lane; i < 2 * w * h; i += 32) {
-      const int c = i >> (sh.lw + sh.lh), s = i & (w * h - 1);
-      sm.org[c][s] = P.orig[c][(size_t)(cv.y + (s >> sh.lw)) * P.cstride + cv.x + (s & (w - 1))];
-    }
-    // ---- 2. down-sampled luma (xGetLumaRecPixels, 4:2:0, [1 2 1; 1 2 1] / 8; one row [1 2 1] / 4 above a CTU's first row)
-    if (cv.cclm) {
-      const int16_t* Y = P.luma + (size_t)(2 * cv.y) * P.lstride + 2 * cv.x;
-      const int ls = P.lstride;
-      const bool ctuTop = (cv.y & ((P.ctu >> 1) - 1)) == 0;
-      const int nTop = availT ? w + vmin(nAr, h) : 0, nLeft = availL ? h + vmin(nBl, w) : 0;
-      for (int i = lane; i < w * h + nTop + nLeft; i += 32) {
-        int v;
-        if (i < w * h + nTop) {
-          const int x = i < w * h ? i & (w - 1) : i - w * h;
-          const int xl = 2 * x - (x == 0 && !availL ? 0 : 1);      // no left neighbours: column -1 padded from column 0
-          const int16_t* r0 = i < w * h ? Y + (size_t)(2 * (i >> sh.lw)) * ls : Y - 2 * ls;
-          if (i >= w * h && ctuTop) v = (2 * r0[ls + 2 * x] + r0[ls + 2 * x + 1] + r0[ls + xl] + 2) >> 2;
-          else v = (2 * r0[2 * x] + r0[2 * x + 1] + r0[xl] + 2 * r0[ls + 2 * x] + r0[ls + 2 * x + 1] + r0[ls + xl] + 4) >> 3;
-          if (i < w * h) sm.ds[i] = (int16_t)v;
-          else sm.dsTop[x] = (int16_t)v;
-        } else {
-          const int j = i - w * h - nTop;
-          const int16_t* r0 = Y + (size_t)(2 * j) * ls - 3;
-          sm.dsLeft[j] = (int16_t)((2 * r0[1] + r0[2] + r0[0] + 2 * r0[ls + 1] + r0[ls + 2] + r0[ls] + 4) >> 3);
-        }
-      }
-    }
-    __syncwarp();
-    // LM parameters (lanes 0..5), DC values (lanes 6, 7), DM's projected main reference (every lane)
-    if (cv.cclm && lane < 6) {
-      int o[3];
-      chroma_lm_params(sm, lane >> 1, lane & 1, w, h, P.bd, availT, availL, nAr, nBl, o);
-      sm.lm[lane >> 1][lane & 1][0] = o[0]; sm.lm[lane >> 1][lane & 1][1] = o[1]; sm.lm[lane >> 1][lane & 1][2] = o[2];
-    } else if (lane == 6 || lane == 7) {
-      const int c = lane - 6;
-      int sum = 0;
-      if (w >= h) for (int i = 0; i < w; i++) sum += sm.lines[c][0][1 + i];
-      if (w <= h) for (int i = 0; i < h; i++) sum += sm.lines[c][1][1 + i];
-      const int denom = w == h ? 2 * w : vmax(w, h);
-      sm.dc[c] = (sum + (denom >> 1)) >> vlog2(denom);
-    }
-    if (dm > 1 && dmp.angle < 0) {
-      SlotInfo s = {};
-      s.kind = 2; s.mode = dm; s.p = dmp;
-#pragma unroll 1
-      for (int c = 0; c < 2; c++) {
-        s.set = c;
-        build_projected_line(sm.proj[c], sm, s, dmp.is_ver ? w : h, dmp.is_ver ? h : w, lane, 32);
-      }
-    }
-    __syncwarp();
+    const Shape sh = chroma_visit_setup(sm, P, rom, cv, lane);
+    const int w = sh.w, h = sh.h, dm = cv.dm_mode;
 
     // ---- 3. evaluations: task = (candidate * 2 + component) * lanes + unit
     const int lanes = sh.lanes, lgL = sh.lgLanes;
@@ -229,14 +253,7 @@ __global__ void __launch_bounds__(kChromaWarps * 32) chroma_eval_kernel(ChromaPa
       const int code = chroma_cand_code(c, dm);
       const int mode = code == VVCB_DM_CHROMA ? dm : code;
       const bool act = (task >> lgL) < 16 && (mode < VVCB_LM_CHROMA || cv.cclm);
-      ChromaCand cd;
-      cd.comp = comp;
-      cd.kind = mode == 0 ? 0 : mode == 1 ? 1 : mode < VVCB_LM_CHROMA ? 2 : 3;
-      cd.p = rom.mode[sh.lw - 2][sh.lh - 2][mode < VVCB_LM_CHROMA ? mode : 0];
-      cd.dc = sm.dc[comp];
-      const int lm = vmin(vmax(mode - VVCB_LM_CHROMA, 0), 2);
-      cd.a = sm.lm[lm][comp][0]; cd.k = sm.lm[lm][comp][1]; cd.b = sm.lm[lm][comp][2];
-      if (cd.kind == 3 && !cv.cclm) { cd.a = 0; cd.k = 0; cd.b = 0; }   // not evaluated: shadow values, nothing is stored
+      const ChromaCand cd = chroma_make_cand(sm, rom, sh, mode, comp, cv.cclm);
       const int16_t* org = sm.org[comp];
       int16_t* outBlk = pout ? pout + (size_t)e * w * h : nullptr;
       int sad = 0, satd = 0;
@@ -327,6 +344,92 @@ __global__ void __launch_bounds__(kChromaWarps * 32) chroma_eval_kernel(ChromaPa
         if (comp == 0) r.mode[c] = (uint8_t)code;
       }
     }
+  }
+}
+
+// ---- chroma TU coding (vvcb_chroma_tu_eval) ----------------------------------------------------------------------------------------
+// Prediction and residual of one candidate per warp, both components, into the candidate's dense blocks (Cb at the Cb TU job's offset,
+// Cr behind it): the visit setup and chroma_predict_piece of chroma_eval_kernel, a lane per 4x4 piece.  Lane 0 also writes Cb's
+// cbfDeltaBits (Ctx::QtCbf[Cb](0) of the candidate's snapshot) into its TU job.
+struct ChromaTuPredParams {
+  ChromaParams planes;                     // visits, planes, bit depth, CTU size, ROM (results / predOut are not used)
+  const vvcb_chroma_tu_job* jobs; int n;
+  vvcb_tu_job* cbJobs;                     // the Cb TU job of each candidate (offset read, cbf_delta_bits written)
+  const vvcb_chroma_ctx_states* states;    // the candidate's snapshot (carried copy)
+  int16_t* pred; int16_t* resi;
+  const uint32_t* frac;                    // ProbModelTables::m_binFracBits
+};
+
+__device__ __forceinline__ int32_t chroma_cbf_delta_bits(const vvcb_bin_model& m, const uint32_t* frac)
+{
+  const int q = ((int)m.state[0] + (int)m.state[1]) >> 8;
+  return (int32_t)frac[2 * q + 1] - (int32_t)frac[2 * q];
+}
+
+__global__ void __launch_bounds__(kChromaWarps * 32) chroma_tu_pred_kernel(ChromaTuPredParams P)
+{
+  __shared__ ChromaSmem smem[kChromaWarps];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  ChromaSmem& sm = smem[warp];
+  const Rom& rom = *P.planes.rom;
+  const uint32_t* filt = &rom.filt[0][0];
+  const int maxv = (1 << P.planes.bd) - 1;
+  for (int q = blockIdx.x * kChromaWarps + warp; q < P.n; q += gridDim.x * kChromaWarps) {
+    const vvcb_chroma_tu_job job = P.jobs[q];
+    const vvcb_chroma_visit cv = P.planes.visits[job.visit];
+    const Shape sh = chroma_visit_setup(sm, P.planes, rom, cv, lane);
+    const int w = sh.w, n = sh.w * sh.h;
+    const int code = chroma_cand_code(job.cand, cv.dm_mode), mode = code == VVCB_DM_CHROMA ? cv.dm_mode : code;
+    const size_t off = P.cbJobs[q].offset;
+#pragma unroll 1
+    for (int comp = 0; comp < 2; comp++) {
+      const ChromaCand cd = chroma_make_cand(sm, rom, sh, mode, comp, cv.cclm);
+      int16_t* pred = P.pred + off + (size_t)comp * n;
+      int16_t* resi = P.resi + off + (size_t)comp * n;
+      for (int u = lane; u < (n >> 4); u += 32) {
+        const int x0 = (u & ((w >> 2) - 1)) << 2, y0 = (u >> (sh.lw - 2)) << 2;
+        int v[4][4];
+        chroma_predict_piece<4, 4>(sm, cd, sh, filt, maxv, x0, y0, v);
+#pragma unroll
+        for (int i = 0; i < 4; i++)
+#pragma unroll
+          for (int j = 0; j < 4; j++) {
+            const int s = (y0 + i) * w + x0 + j;
+            pred[s] = (int16_t)v[i][j];
+            resi[s] = (int16_t)(sm.org[comp][s] - v[i][j]);
+          }
+      }
+    }
+    if (lane == 0) P.cbJobs[q].cbf_delta_bits = chroma_cbf_delta_bits(P.states[q].cbf_cb[0], P.frac);
+    __syncwarp();
+  }
+}
+
+// The cbf bins of xGetIntraFracBitsQT (CABACWriter::cbf_comp, context DeriveCtx::CtxQtCbf) on the candidate's carried models, one thread
+// per candidate.  Step 1, after Cb's levels are final: Cb's cbf, its bin (context 0), and Cr's cbfDeltaBits from the Cr context that cbf
+// selects.  Step 2, after Cr's: Cr's cbf and its bin.
+struct ChromaCbfParams {
+  int n, step;
+  const vvcb_tu_result* res;               // the step's TU results (Cb for step 1, Cr for step 2)
+  vvcb_tu_job* crJobs;                     // step 1: cbf_delta_bits of Cr written
+  vvcb_chroma_ctx_states* states;          // carried models: the cbf contexts adapt
+  uint8_t* cbf; uint32_t* cbfBits;         // [candidate][Cb, Cr]
+  const uint32_t* frac;
+};
+
+__global__ void __launch_bounds__(128) chroma_cbf_kernel(ChromaCbfParams P)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n) return;
+  vvcb_chroma_ctx_states& st = P.states[i];
+  const unsigned cbf = P.res[i].abs_sum_level != 0;
+  if (P.step == 1) {
+    P.cbfBits[2 * i] = isp_code_bin(st.cbf_cb[0], P.frac, cbf);
+    P.cbf[2 * i] = (uint8_t)cbf;
+    P.crJobs[i].cbf_delta_bits = chroma_cbf_delta_bits(st.cbf_cr[cbf], P.frac);
+  } else {
+    P.cbfBits[2 * i + 1] = isp_code_bin(st.cbf_cr[P.cbf[2 * i]], P.frac, cbf);
+    P.cbf[2 * i + 1] = (uint8_t)cbf;
   }
 }
 

@@ -249,6 +249,10 @@ __device__ __forceinline__ uint32_t dq_pack(int absLevel, int prevId) { return (
 #ifndef VVCB_DQ_MIN_CTAS
 #define VVCB_DQ_MIN_CTAS 4
 #endif
+// C: chroma (vvcb_chroma_tu_eval): the chroma context sets and per-position offsets of H.266 9.3.4.2.5-9.3.4.2.8 -- significance offset
+// d < 2 ? 4 : 0 into 8 contexts per state class, greater-than offset d == 0 ? 6 : 1, last-position contexts from the start of the chroma
+// arrays with shift Clip3(0, 2, side >> 3) -- on prices laid out by chroma_rates_from_states_kernel (vvcb_rate.cuh).
+template <bool C = false>
 __global__ void __launch_bounds__(kDqThreads, VVCB_DQ_MIN_CTAS) dq_kernel(DqParams P)
 {
   __shared__ DqGroupSmem smem[kDqGroups];
@@ -305,8 +309,8 @@ __global__ void __launch_bounds__(kDqThreads, VVCB_DQ_MIN_CTAS) dq_kernel(DqPara
     if (k < 2) {                                                   // RateEstimator::xSetLastCoeffOffset :541-567
       const int size = k ? h : w, lg = k ? lh : lw;
       const uint32_t (*ctx)[2] = k ? P.rates[job.rate_idx].last_y : P.rates[job.rate_idx].last_x;
-      const int prefix = lg == 2 ? 0 : lg == 3 ? 3 : lg == 4 ? 6 : lg == 5 ? 10 : 15;
-      const int lastShift = (lg + 1) >> 2, bitOffset = k ? job.cbf_delta_bits : 0;
+      const int prefix = C ? 0 : lg == 2 ? 0 : lg == 3 ? 3 : lg == 4 ? 6 : lg == 5 ? 10 : 15;
+      const int lastShift = C ? vmin(2, size >> 3) : (lg + 1) >> 2, bitOffset = k ? job.cbf_delta_bits : 0;
       const int maxCtxId = rom.groupIdx[vmin(32, size) - 1];
       int32_t* out = k ? sm.lastY : sm.lastX;
       uint32_t sum = 0;
@@ -421,8 +425,8 @@ __global__ void __launch_bounds__(kDqThreads, VVCB_DQ_MIN_CTAS) dq_kernel(DqPara
         if (scanIdx) {
           DqState& cs = sm.st[curr * 4 + k];
           const int diag = nx.x + nx.y;
-          const int sigOff = diag < 2 ? 8 : diag < 5 ? 4 : 0;
-          const int gtxOff = diag < 1 ? 16 : diag < 3 ? 11 : diag < 10 ? 6 : 1;
+          const int sigOff = C ? (diag < 2 ? 4 : 0) : diag < 2 ? 8 : diag < 5 ? 4 : 0;
+          const int gtxOff = C ? (diag < 1 ? 6 : 1) : diag < 1 ? 16 : diag < 3 ? 11 : diag < 10 ? 6 : 1;
           const int nextInside = (scanIdx - 1) & 15;
           if ((scanIdx & 15) == 0) {
             // ---- State::updateStateEOS :1275-1315 + CommonCtx::update :1317-1397 (after m_commonCtx.swap())

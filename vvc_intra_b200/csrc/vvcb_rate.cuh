@@ -17,7 +17,7 @@ struct RateParams {
   int n;
   const int32_t* level;      // final levels, dense per job at job.offset
   vvcb_tu_result* results;   // frac_bits is written here
-  const vvcb_ctx_states* states;
+  const vvcb_ctx_states* states;         // the chroma instantiation reads vvcb_chroma_ctx_states here (and in statesOut)
   const DqRom* rom;
   const RateRom* rate;
   int depQuant;              // slice->getDepQuantEnabledFlag(): selects the state machine that picks the significance context set
@@ -42,6 +42,14 @@ constexpr int kMdlMts = VVCB_MODEL_AT(mts_idx), kMdlSigSbb = VVCB_MODEL_AT(sig_s
 #undef VVCB_MODEL_AT
 constexpr int kRateModels = (int)(sizeof(vvcb_ctx_states) / sizeof(vvcb_bin_model));
 static_assert(sizeof(vvcb_ctx_states) == kRateModels * sizeof(vvcb_bin_model) && sizeof(vvcb_bin_model) == 6, "vvcb_ctx_states is an array of 6-byte models");
+// the same for the chroma models (vvcb_chroma_tu_eval)
+#define VVCB_CMODEL_AT(field) ((int)(offsetof(vvcb_chroma_ctx_states, field) / sizeof(vvcb_bin_model)))
+constexpr int kCMdlCbfCb = VVCB_CMODEL_AT(cbf_cb), kCMdlCbfCr = VVCB_CMODEL_AT(cbf_cr), kCMdlSigSbb = VVCB_CMODEL_AT(sig_sbb),
+              kCMdlSig = VVCB_CMODEL_AT(sig), kCMdlPar = VVCB_CMODEL_AT(par), kCMdlGt1 = VVCB_CMODEL_AT(gt1), kCMdlGt2 = VVCB_CMODEL_AT(gt2),
+              kCMdlLastX = VVCB_CMODEL_AT(last_x), kCMdlLastY = VVCB_CMODEL_AT(last_y);
+#undef VVCB_CMODEL_AT
+constexpr int kChromaRateModels = (int)(sizeof(vvcb_chroma_ctx_states) / sizeof(vvcb_bin_model));
+static_assert(sizeof(vvcb_chroma_ctx_states) == kChromaRateModels * sizeof(vvcb_bin_model) && kChromaRateModels == 70, "vvcb_chroma_ctx_states is an array of 70 models");
 
 // TBitEstimator::encodeBin: price, then BinProbModel_Std::update (MASK_0 0x7fe0, MASK_1 0x7ffe)
 __device__ __forceinline__ void rate_bin(RateEst& e, RateModel* models, int ctx, unsigned bin)
@@ -83,6 +91,9 @@ constexpr int kRateThreads = 32 * kRateWarps;
 //                                 Rice parameter of a remainder after regular bins (2) << 25 | min(sum of the template, 31) (5) << 27
 // packed word, transform skip:    modified level (17) | non-zero (1) << 17 | negative (1) << 18 | coded neighbours 0..2 (2) << 19 |
 //                                 sign context 0..2 (2) << 21 | Rice parameter (2) << 23
+// C: chroma (vvcb_chroma_ctx_states models, the chroma context derivations of H.266 9.3.4.2.5-9.3.4.2.8; chroma jobs never carry
+// transform skip or MTS, so the mts_coding and transform-skip branches are not reached).
+template <bool C = false>
 __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
 {
   __shared__ uint32_t sFrac[512];
@@ -117,16 +128,19 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
     if (scanPosLast < 0) {
       if (lane == 0) P.results[ji].frac_bits = 0;
       if (P.statesOut) {
-        const vvcb_bin_model* src = reinterpret_cast<const vvcb_bin_model*>(&P.states[job.rate_idx]);
-        vvcb_bin_model* dst = reinterpret_cast<vvcb_bin_model*>(&P.statesOut[ji]);
-        for (int i = lane; i < kRateModels; i += 32) dst[i] = src[i];
+        const vvcb_bin_model* src = C ? reinterpret_cast<const vvcb_bin_model*>(P.states) + (size_t)job.rate_idx * kChromaRateModels
+                                      : reinterpret_cast<const vvcb_bin_model*>(&P.states[job.rate_idx]);
+        vvcb_bin_model* dst = C ? reinterpret_cast<vvcb_bin_model*>(P.statesOut) + (size_t)ji * kChromaRateModels
+                                : reinterpret_cast<vvcb_bin_model*>(&P.statesOut[ji]);
+        for (int i = lane; i < (C ? kChromaRateModels : kRateModels); i += 32) dst[i] = src[i];
       }
       continue;
     }
 
     {                                                            // this TU's private copy of the context models
-      const vvcb_bin_model* src = reinterpret_cast<const vvcb_bin_model*>(&P.states[job.rate_idx]);
-      for (int i = lane; i < kRateModels; i += 32) {
+      const vvcb_bin_model* src = C ? reinterpret_cast<const vvcb_bin_model*>(P.states) + (size_t)job.rate_idx * kChromaRateModels
+                                    : reinterpret_cast<const vvcb_bin_model*>(&P.states[job.rate_idx]);
+      for (int i = lane; i < (C ? kChromaRateModels : kRateModels); i += 32) {
         const vvcb_bin_model m = src[i];
         models[i].st = (uint32_t)m.state[0] | ((uint32_t)m.state[1] << 16);
         models[i].rate = m.rate;
@@ -163,8 +177,8 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
           if (sp.y < h - 1) { VVCB_T(p[w]); if (sp.y < h - 2) VVCB_T(p[2 * w]); }
 #undef VVCB_T
           const int diag = sp.x + sp.y;
-          const int sigCtx = vmin((sumAbs1 + 1) >> 1, 3) + (diag < 2 ? 4 : 0) + (diag < 5 ? 4 : 0);
-          const int ctxOff = vmin(sumAbs1 - numPos, 4) + 1 + (diag == 0 ? 15 : diag < 3 ? 10 : diag < 10 ? 5 : 0);
+          const int sigCtx = vmin((sumAbs1 + 1) >> 1, 3) + (diag < 2 ? 4 : 0) + (!C && diag < 5 ? 4 : 0);
+          const int ctxOff = vmin(sumAbs1 - numPos, 4) + 1 + (C ? (diag == 0 ? 5 : 0) : (diag == 0 ? 15 : diag < 3 ? 10 : diag < 10 ? 5 : 0));
           word = (uint32_t)vmin(vabs(v), 0xffff) | ((uint32_t)sigCtx << 16) | ((uint32_t)ctxOff << 20) |
                  ((uint32_t)rom.goRicePars[vmax(vmin(sumAbs - 20, 31), 0)] << 25) | ((uint32_t)vmin(sumAbs, 31) << 27);
         }
@@ -242,12 +256,13 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
           const int gX = rom.groupIdx[lp.x], gY = rom.groupIdx[lp.y];
           int maxX = rom.groupIdx[vmin(32, w) - 1], maxY = rom.groupIdx[vmin(32, h) - 1];
           if (mts > 1) { if (w == 32) maxX = rom.groupIdx[15]; if (h == 32) maxY = rom.groupIdx[15]; }
-          const int offX = lw == 2 ? 0 : lw == 3 ? 3 : lw == 4 ? 6 : lw == 5 ? 10 : 15, offY = lh == 2 ? 0 : lh == 3 ? 3 : lh == 4 ? 6 : lh == 5 ? 10 : 15;
-          const int shX = (lw + 1) >> 2, shY = (lh + 1) >> 2;
-          for (int k = 0; k < gX; k++) rate_bin(e, models, kMdlLastX + offX + (k >> shX), 1);
-          if (gX < maxX) rate_bin(e, models, kMdlLastX + offX + (gX >> shX), 0);
-          for (int k = 0; k < gY; k++) rate_bin(e, models, kMdlLastY + offY + (k >> shY), 1);
-          if (gY < maxY) rate_bin(e, models, kMdlLastY + offY + (gY >> shY), 0);
+          const int offX = C ? 0 : lw == 2 ? 0 : lw == 3 ? 3 : lw == 4 ? 6 : lw == 5 ? 10 : 15, offY = C ? 0 : lh == 2 ? 0 : lh == 3 ? 3 : lh == 4 ? 6 : lh == 5 ? 10 : 15;
+          const int shX = C ? vmin(2, w >> 3) : (lw + 1) >> 2, shY = C ? vmin(2, h >> 3) : (lh + 1) >> 2;
+          const int mX = C ? kCMdlLastX : kMdlLastX, mY = C ? kCMdlLastY : kMdlLastY;
+          for (int k = 0; k < gX; k++) rate_bin(e, models, mX + offX + (k >> shX), 1);
+          if (gX < maxX) rate_bin(e, models, mX + offX + (gX >> shX), 0);
+          for (int k = 0; k < gY; k++) rate_bin(e, models, mY + offY + (k >> shY), 1);
+          if (gY < maxY) rate_bin(e, models, mY + offY + (gY >> shY), 0);
           if (gX > 3) e.bits += (unsigned long long)((gX - 2) >> 1) << 15;
           if (gY > 3) e.bits += (unsigned long long)((gY - 2) >> 1) << 15;
         }
@@ -270,7 +285,7 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
           if (!isLast && sb != 0) {
             const int sigRight = sx + 1 < shp.widthInSbb ? (int)((coded >> (sbPos + 1)) & 1) : 0;
             const int sigLower = sy + 1 < shp.heightInSbb ? (int)((coded >> (sbPos + shp.widthInSbb)) & 1) : 0;
-            rate_bin(e, models, kMdlSigSbb + (sigRight | sigLower), sig);
+            rate_bin(e, models, (C ? kCMdlSigSbb : kMdlSigSbb) + (sigRight | sigLower), sig);
             if (!sig) continue;
           }
           const int firstSigPos = isLast ? scanPosLast : minSub + 15;
@@ -280,7 +295,7 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
             const uint32_t x = info[next];
             const int a = (int)(x & 0xffffu);
             if (numNonZero || next != inferSigPos) {
-              rate_bin(e, models, kMdlSig + 12 * vmax(0, state - 1) + (int)((x >> 16) & 15), a != 0);
+              rate_bin(e, models, (C ? kCMdlSig + 8 * vmax(0, state - 1) : kMdlSig + 12 * vmax(0, state - 1)) + (int)((x >> 16) & 15), a != 0);
               regBins--;
             }
             if (a) {
@@ -288,14 +303,14 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
               const int ctxOff = next != scanPosLast ? (int)((x >> 20) & 31) : 0;
               int rem = a - 1;
               numNonZero++; signBins++;
-              rate_bin(e, models, kMdlGt1 + ctxOff, rem != 0);
+              rate_bin(e, models, (C ? kCMdlGt1 : kMdlGt1) + ctxOff, rem != 0);
               regBins--;
               if (rem) {
                 rem -= 1;
-                rate_bin(e, models, kMdlPar + ctxOff, rem & 1);
+                rate_bin(e, models, (C ? kCMdlPar : kMdlPar) + ctxOff, rem & 1);
                 rem >>= 1;
                 regBins--;
-                rate_bin(e, models, kMdlGt2 + ctxOff, rem != 0);
+                rate_bin(e, models, (C ? kCMdlGt2 : kMdlGt2) + ctxOff, rem != 0);
                 regBins--;
               }
             }
@@ -321,8 +336,9 @@ __global__ void __launch_bounds__(kRateThreads) rate_kernel(RateParams P)
     }
     __syncwarp();
     if (P.statesOut) {
-      vvcb_bin_model* dst = reinterpret_cast<vvcb_bin_model*>(&P.statesOut[ji]);
-      for (int i = lane; i < kRateModels; i += 32) {
+      vvcb_bin_model* dst = C ? reinterpret_cast<vvcb_bin_model*>(P.statesOut) + (size_t)ji * kChromaRateModels
+                              : reinterpret_cast<vvcb_bin_model*>(&P.statesOut[ji]);
+      for (int i = lane; i < (C ? kChromaRateModels : kRateModels); i += 32) {
         vvcb_bin_model m;
         m.state[0] = (uint16_t)(models[i].st & 0xffffu); m.state[1] = (uint16_t)(models[i].st >> 16);
         m.rate = (uint8_t)models[i].rate; m.pad = 0;
@@ -347,6 +363,25 @@ __global__ void __launch_bounds__(128) rates_from_states_kernel(const vvcb_ctx_s
   const vvcb_bin_model m = reinterpret_cast<const vvcb_bin_model*>(&states[s])[11 + i];
   const int q = ((int)m.state[0] + (int)m.state[1]) >> 8;
   uint32_t* dst = reinterpret_cast<uint32_t*>(&out[s]) + 2 * i;
+  dst[0] = rom->binFracBits[2 * q]; dst[1] = rom->binFracBits[2 * q + 1];
+}
+
+// The chroma models' prices in vvcb_dq_rates, for the chroma instantiation of dq_kernel: each chroma array at the start of its luma
+// counterpart (sig_sbb[0..1], sig[set][0..7], par / gt1 / gt2[0..10], last_x / last_y[0..2]); dq_rate_kernel then derives the same
+// DqRateTab layout, of which the chroma kernel reads those entries only.  One thread per (snapshot, residual context).
+constexpr int kChromaResidualModels = kChromaRateModels - kCMdlSigSbb;
+
+__global__ void __launch_bounds__(128) chroma_rates_from_states_kernel(const vvcb_chroma_ctx_states* states, int n, const RateRom* rom, vvcb_dq_rates* out)
+{
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (long long)n * kChromaResidualModels) return;
+  const int s = (int)(t / kChromaResidualModels), i = kCMdlSigSbb + (int)(t % kChromaResidualModels);
+  const vvcb_bin_model m = reinterpret_cast<const vvcb_bin_model*>(&states[s])[i];
+  const int q = ((int)m.state[0] + (int)m.state[1]) >> 8;
+  vvcb_dq_rates& r = out[s];
+  uint32_t* dst = i < kCMdlSig ? r.sig_sbb[i - kCMdlSigSbb] : i < kCMdlPar ? r.sig[(i - kCMdlSig) >> 3][(i - kCMdlSig) & 7]
+                : i < kCMdlGt1 ? r.par[i - kCMdlPar] : i < kCMdlGt2 ? r.gt1[i - kCMdlGt1] : i < kCMdlLastX ? r.gt2[i - kCMdlGt2]
+                : i < kCMdlLastY ? r.last_x[i - kCMdlLastX] : r.last_y[i - kCMdlLastY];
   dst[0] = rom->binFracBits[2 * q]; dst[1] = rom->binFracBits[2 * q + 1];
 }
 

@@ -96,6 +96,14 @@ CHROMA_VISIT_DTYPE = np.dtype([('x', '<i2'), ('y', '<i2'), ('log2w', 'u1'), ('lo
                                ('n_above_right', 'u1'), ('n_left', 'u1'), ('n_below_left', 'u1'), ('dm_mode', 'u1'), ('cclm', 'u1'), ('pad', 'u1', 3)])
 CHROMA_RESULT_DTYPE = np.dtype([('mode', 'u1', CHROMA_CANDS), ('sad', '<u4', (CHROMA_CANDS, 2)), ('satd', '<u4', (CHROMA_CANDS, 2))], align=True)
 assert CHROMA_VISIT_DTYPE.itemsize == 16 and CHROMA_RESULT_DTYPE.itemsize == 136
+# vvcb_chroma_ctx_states / vvcb_chroma_tu_job / vvcb_chroma_tu_result (include/vvc_intra_b200.h): chroma TU coding of the candidates
+CHROMA_CTX_STATES_DTYPE = np.dtype([('cbf_cb', BIN_MODEL_DTYPE, 2), ('cbf_cr', BIN_MODEL_DTYPE, 3), ('sig_sbb', BIN_MODEL_DTYPE, 2),
+                                    ('sig', BIN_MODEL_DTYPE, (3, 8)), ('par', BIN_MODEL_DTYPE, 11), ('gt1', BIN_MODEL_DTYPE, 11),
+                                    ('gt2', BIN_MODEL_DTYPE, 11), ('last_x', BIN_MODEL_DTYPE, 3), ('last_y', BIN_MODEL_DTYPE, 3)])
+CHROMA_TU_JOB_DTYPE = np.dtype([('visit', '<u4'), ('cand', 'u1'), ('flags', 'u1'), ('rate_idx', '<u2'), ('qp_per', '<i2', 2), ('qp_rem', '<i2', 2),
+                                ('offset', '<u4'), ('pad', '<u4'), ('lambda', '<f8', 2)], align=True)
+CHROMA_TU_RESULT_DTYPE = np.dtype([('comp', TU_RESULT_DTYPE, 2), ('cbf_bits', '<u4', 2), ('cbf', 'u1', 2), ('pad', 'u1', 6)], align=True)
+assert CHROMA_CTX_STATES_DTYPE.itemsize == 420 and CHROMA_TU_JOB_DTYPE.itemsize == 40 and CHROMA_TU_RESULT_DTYPE.itemsize == 64
 
 
 class EngineError(RuntimeError):
@@ -158,6 +166,8 @@ def load_library():
         L.vvcb_chroma_frame_begin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
         L.vvcb_chroma_reco_update.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
         L.vvcb_chroma_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+        L.vvcb_chroma_tu_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.vvcb_ctu_hads_islice.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.vvcb_features_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.vvcb_frame_bind_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
@@ -468,6 +478,23 @@ class IntraCostEngine:
             blocks.append(pred[at:at + n].reshape(CHROMA_CANDS, 2, 1 << int(v['log2h']), 1 << int(v['log2w'])))
             at += n
         return out, blocks
+
+    def chroma_tu_eval(self, visits, jobs, n_samples, states=None, want_level=False, want_reco=False, want_pred=False):
+        """vvcb_chroma_tu_eval: the Cb and Cr TUs of chroma candidates (CHROMA_TU_JOB_DTYPE) of the visits (CHROMA_VISIT_DTYPE).
+        states: CHROMA_CTX_STATES_DTYPE array indexed by job['rate_idx'] (needed by DEPQUANT / RATE jobs).  Returns dict with 'results'
+        (CHROMA_TU_RESULT_DTYPE) and the wanted flat outputs of n_samples: per candidate Cb w*h, then Cr w*h, at job['offset']."""
+        visits = np.ascontiguousarray(visits, CHROMA_VISIT_DTYPE)
+        jobs = np.ascontiguousarray(jobs, CHROMA_TU_JOB_DTYPE)
+        states = None if states is None else np.ascontiguousarray(states, CHROMA_CTX_STATES_DTYPE)
+        out = dict(results=np.zeros(len(jobs), CHROMA_TU_RESULT_DTYPE))
+        for key, want, dt in (('level', want_level, np.int32), ('reco', want_reco, np.int16), ('pred', want_pred, np.int16)):
+            if want:
+                out[key] = np.zeros(n_samples, dt)
+        p = lambda k: _ptr(out[k]) if k in out else None
+        self._ck(self._lib.vvcb_chroma_tu_eval(self._ctx, _ptr(visits), len(visits), _ptr(jobs), len(jobs),
+                                               _ptr(states) if states is not None else None, 0 if states is None else len(states), n_samples,
+                                               p('level'), p('reco'), p('pred'), _ptr(out['results'])))
+        return out
 
     def residual_bits(self, jobs, levels, states):
         """vvcb_residual_bits: fractional bits of residual_coding for the given levels (flat int32 indexed by job['offset'])."""
