@@ -50,59 +50,57 @@ __global__ void __launch_bounds__(256) int_peak_kernel(const int* in, int* out, 
 // C ABI
 // =====================================================================================================
 constexpr int kSideStreams = 7;
-// Scratch slots of a context: device (vvcb_ctx::dTu, tu_buf) and page-locked (vvcb_ctx::hPin, pin_buf).  The stage-1 arenas of
-// vvcb_cu_eval and the arenas of vvcb_isp_eval share kStageIn / kStageOut: a context serves one call at a time.
-enum TuSlot {
+// Grow-only scratch memory of a context (vvcb_ctx::mem; grow sizes a slot, buf reads it): device slots, then page-locked ones (kPinTuIn on).
+// The stage-1 arenas of vvcb_cu_eval and the staged candidate calls (vvcb_isp_eval, vvcb_chroma_tu_eval) share kStageIn / kStageOut and
+// their page-locked twins: a context serves one call at a time.
+enum Slot {
   kTuIn, kTuOut,                 // tu_eval_impl / vvcb_residual_bits: inputs from the host, outputs (+ dequantised coefficients)
   kTuResi, kTuCoeff,             // residual, transform coefficients (vvcb_tu_eval's want_coeff)
   kDqCoeff, kDqTabs, kDqScratch, kDqLists,   // quantiser scratch (quant_scratch)
   kStageIn, kStageOut,
-  kTuSlots
+  kOrig, kReco,                  // the planes the context owns (vvcb_frame_begin / vvcb_frame_alloc)
+  kVisits, kResults, kDetails,   // the host-pointer RMD calls: visits, result lists, detail tables
+  kBrief,                        // brief records of the un-pipelined path (the pipeline re-uses dResP)
+  kSadSatd,                      // SAD / SATD scratch: two planes of n * VVCB_NUM_SLOTS words, visit-major (scratch_at, vvcb_rmd.cuh)
+  kItems,                        // work items of the RMD plan
+  kPred,                         // vvcb_rmd_pred: every slot's prediction
+  kRects, kRectSamples,          // vvcb_reco_update_rects
+  kFeatIn, kFeatOut,             // feature scratch: jobs / per-CTU sums, results
+  kChroma,                       // vvcb_chroma_frame_begin: Cb, Cr originals, then Cb, Cr reconstructions, cstride * ch each
+  kChromaIo,                     // vvcb_chroma_eval: visits, results, prediction offsets, predictions
+  kPinTuIn, kPinTuOut, kPinStageIn, kPinStageOut,
+  kSlots
 };
-enum PinSlot { kPinTuIn, kPinTuOut, kPinStageIn, kPinStageOut, kPinSlots };
+struct Scratch { void* p; size_t cap; bool pinned; };
 struct vvcb_ctx {
   int device, bd, ctu;
   cudaStream_t stream;
   cudaEvent_t ev0, ev1;
   Rom* dRom;
   TrRom* dTrRom;
-  void* dTu[kTuSlots]; size_t capTu[kTuSlots];
+  Scratch mem[kSlots];
   DqRom* dDqRom;
   RateRom* dRateRom;
   int depQuant;                     // slice->getDepQuantEnabledFlag() (vvcb_set_option), 1 = the shipped configuration
   float tuMs[4]; int tuTimed; cudaEvent_t tev[5];   // per-kernel timing of vvcb_tu_eval: transform pass, dependent quantisation, reconstruction pass
-  void* dFeat[2]; size_t capFeat[2]; // feature scratch: jobs / per-CTU sums, results
   // copy/compute pipeline of vvcb_rmd_eval for large host batches
   cudaStream_t sIn, sOut; cudaEvent_t evIn[2], evComp[2], evOut[2];
   cudaStream_t sKind[kSideStreams]; cudaEvent_t evPlan, evKind[kSideStreams];   // evaluation launches are dealt over the main stream and these: the CTAs of the next kernels fill the tail of each one
   int evalStreams;                  // streams in use (1 + side streams), VVCB_EVAL_STREAMS for A/B runs
   vvcb_rmd_visit* dVisP[2]; vvcb_rmd_result* dResP[2]; bool pipeReady;
-  vvcb_rmd_brief* dBrief; size_t capBrief;   // brief records of the un-pipelined path (the pipeline re-uses dResP)
   int trusted;                      // VVCB_OPT_TRUSTED_VISITS
-  int16_t* dOrig; int16_t* dReco;
   const int16_t* bOrig; const int16_t* bReco;   // planes in use (own or bound)
   int width, height, stride;        // planes share one pitch (in samples)
-  size_t planeSamples;
-  // scratch for the host-pointer API
-  vvcb_rmd_visit* dVisits; vvcb_rmd_result* dResults; size_t capVisits;
-  vvcb_rmd_detail* dDetails; size_t capDetails;
-  uint32_t* dScratch; size_t capScratch;   // SAD / SATD scratch: two planes of n * VVCB_NUM_SLOTS words, visit-major (scratch_at, vvcb_rmd.cuh)
-  WorkItem* dItems; size_t capItems;
   PlanState* dPlan;
-  int16_t* dPred; size_t capPred;
   int numSms;
-  int16_t* wReco;                   // writable reconstruction plane: own (dReco) or another context's (vvcb_frame_share)
+  int16_t* wReco;                   // writable reconstruction plane: own (kReco) or another context's (vvcb_frame_share)
   int yieldSync; cudaEvent_t evYield;   // VVCB_OPT_YIELD_SYNC
   void* remote;                     // broker client proxy: VVCB_BROKER was set at vvcb_create (vvcb_broker.inc)
-  void* hPin[kPinSlots]; size_t capPin[kPinSlots];
-  void* dRect[2]; size_t capRect[2];
   uint64_t launches;
   uint64_t cuNs[8], cuCalls, tuWaitFrom;    // vvcb_cu_eval_phases
   cudaEvent_t cev[4]; bool cuSpan;          // device spans of the two stages of vvcb_cu_eval
   int timing; int timedLaunches; float kms[3]; cudaEvent_t kev[4];
-  int16_t* dChroma; size_t capChroma;       // vvcb_chroma_frame_begin: Cb, Cr originals, then Cb, Cr reconstructions, cstride * ch each
   int cw, ch, cstride;                      // 0 until vvcb_chroma_frame_begin
-  void* dChromaIo; size_t capChromaIo;      // vvcb_chroma_eval: visits, results, prediction offsets, predictions
   char err[512];
 };
 
@@ -116,6 +114,27 @@ static char g_createErr[512] = "";
       return VVCB_ERR_CUDA;                                                                               \
     }                                                                                                     \
   } while (0)
+
+template <class T = void> static T* buf(const vvcb_ctx* ctx, Slot s) { return static_cast<T*>(ctx->mem[s].p); }
+
+static void release(Scratch& b)
+{
+  if (b.p) { if (b.pinned) cudaFreeHost(b.p); else cudaFree(b.p); }
+  b.p = nullptr; b.cap = 0;
+}
+
+// Slot s holds at least `need` bytes.  A slot that must grow is freed first (its contents are not kept) and reallocated with `headroom`
+// bytes more.  After a failed allocation the slot is empty, and the next call tries again.
+static int grow(vvcb_ctx* ctx, Slot s, size_t need, size_t headroom = 0)
+{
+  Scratch& b = ctx->mem[s];
+  if (need <= b.cap) return VVCB_OK;
+  release(b);
+  void* p = nullptr;
+  CK(b.pinned ? cudaHostAlloc(&p, need + headroom, cudaHostAllocDefault) : cudaMalloc(&p, need + headroom));
+  b.p = p; b.cap = need + headroom;
+  return VVCB_OK;
+}
 
 // wait for the context's stream: polling (default) or, with VVCB_OPT_YIELD_SYNC, sleeping on a blocking event
 static inline uint64_t host_ns() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return (uint64_t)ts.tv_sec * 1000000000ull + (uint64_t)ts.tv_nsec; }
@@ -176,6 +195,7 @@ extern "C" int vvcb_create(vvcb_ctx** out, int device, int bit_depth, int ctu_si
   if (!ctx) return VVCB_ERR_ARG;
   memset(ctx, 0, sizeof(*ctx));
   ctx->device = device; ctx->bd = bit_depth; ctx->ctu = ctu_size; ctx->depQuant = 1;
+  for (int s = kPinTuIn; s < kSlots; s++) ctx->mem[s].pinned = true;
   auto fail = [&](const char* what, cudaError_t err) {
     snprintf(g_createErr, sizeof(g_createErr), "vvcb_create: %s: %s", what, cudaGetErrorString(err));
     vvcb_destroy(ctx);                       // releases whatever was created so far (the context is zero-initialised)
@@ -241,15 +261,8 @@ extern "C" void vvcb_destroy(vvcb_ctx* ctx)
   if (ctx->remote) { vvcbc_disconnect(ctx->remote); delete ctx; return; }
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  for (int i = 0; i < kPinSlots; i++) if (ctx->hPin[i]) cudaFreeHost(ctx->hPin[i]);
-  cudaFree(ctx->dRect[0]); cudaFree(ctx->dRect[1]); cudaFree(ctx->dBrief);
-  cudaFree(ctx->dRom); cudaFree(ctx->dOrig); cudaFree(ctx->dReco); cudaFree(ctx->dVisits); cudaFree(ctx->dResults); cudaFree(ctx->dDetails); cudaFree(ctx->dScratch);
-  cudaFree(ctx->dItems); cudaFree(ctx->dPlan); cudaFree(ctx->dPred); cudaFree(ctx->dTrRom);
-  cudaFree(ctx->dChroma); cudaFree(ctx->dChromaIo);
-  for (int i = 0; i < kTuSlots; i++) cudaFree(ctx->dTu[i]);
-  cudaFree(ctx->dRateRom);
-  cudaFree(ctx->dDqRom);
-  for (int i = 0; i < 2; i++) cudaFree(ctx->dFeat[i]);
+  for (Scratch& b : ctx->mem) release(b);
+  cudaFree(ctx->dRom); cudaFree(ctx->dPlan); cudaFree(ctx->dTrRom); cudaFree(ctx->dRateRom); cudaFree(ctx->dDqRom);
   if (ctx->pipeReady) {
     cudaStreamSynchronize(ctx->sIn); cudaStreamSynchronize(ctx->sOut);
     for (int i = 0; i < 2; i++) { cudaFree(ctx->dVisP[i]); cudaFree(ctx->dResP[i]); cudaEventDestroy(ctx->evIn[i]); cudaEventDestroy(ctx->evComp[i]); cudaEventDestroy(ctx->evOut[i]); }
@@ -278,6 +291,18 @@ extern "C" int vvcb_set_option(vvcb_ctx* ctx, int option, int value)
   return VVCB_ERR_ARG;
 }
 
+// the context's own planes (kOrig, kReco) sized for width x height and bound as its frame; the pitch is a multiple of 64 samples
+static int own_planes(vvcb_ctx* ctx, int width, int height)
+{
+  const int pitch = (width + 63) & ~63;
+  const size_t bytes = (size_t)pitch * height * sizeof(int16_t);
+  int rc;
+  if ((rc = grow(ctx, kOrig, bytes)) || (rc = grow(ctx, kReco, bytes))) return rc;
+  ctx->width = width; ctx->height = height; ctx->stride = pitch;
+  ctx->bOrig = buf<int16_t>(ctx, kOrig); ctx->bReco = ctx->wReco = buf<int16_t>(ctx, kReco);
+  return VVCB_OK;
+}
+
 extern "C" int vvcb_frame_begin(vvcb_ctx* ctx, const int16_t* orig, int stride, int width, int height)
 {
   if (!ctx) return VVCB_ERR_ARG;
@@ -287,20 +312,11 @@ extern "C" int vvcb_frame_begin(vvcb_ctx* ctx, const int16_t* orig, int stride, 
   }
   if (ctx->remote) return vvcbc_frame_begin(ctx->remote, orig, stride, width, height, ctx->err, sizeof(ctx->err));
   CK(cudaSetDevice(ctx->device));
-  const int pitch = (width + 63) & ~63;
-  const size_t samples = (size_t)pitch * height;
-  if (samples > ctx->planeSamples) {
-    cudaFree(ctx->dOrig); cudaFree(ctx->dReco);
-    ctx->dOrig = ctx->dReco = nullptr; ctx->planeSamples = 0;
-    CK(cudaMalloc(&ctx->dOrig, samples * sizeof(int16_t)));
-    CK(cudaMalloc(&ctx->dReco, samples * sizeof(int16_t)));
-    ctx->planeSamples = samples;
-  }
-  ctx->width = width; ctx->height = height; ctx->stride = pitch;
-  ctx->bOrig = ctx->dOrig; ctx->bReco = ctx->dReco; ctx->wReco = ctx->dReco;
-  CK(cudaMemcpy2DAsync(ctx->dOrig, pitch * sizeof(int16_t), orig, stride * sizeof(int16_t), width * sizeof(int16_t), height,
+  int rc;
+  if ((rc = own_planes(ctx, width, height))) return rc;
+  CK(cudaMemcpy2DAsync(buf(ctx, kOrig), ctx->stride * sizeof(int16_t), orig, stride * sizeof(int16_t), width * sizeof(int16_t), height,
                        cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemsetAsync(ctx->dReco, 0, samples * sizeof(int16_t), ctx->stream));
+  CK(cudaMemsetAsync(buf(ctx, kReco), 0, (size_t)ctx->stride * height * sizeof(int16_t), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
@@ -314,19 +330,10 @@ extern "C" int vvcb_frame_alloc(vvcb_ctx* ctx, int width, int height)
   REMOTE_UNAVAILABLE("vvcb_frame_alloc");
   if (width <= 0 || height <= 0 || (width & 3) || (height & 3)) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_frame_alloc: bad argument"); return VVCB_ERR_ARG; }
   CK(cudaSetDevice(ctx->device));
-  const int pitch = (width + 63) & ~63;
-  const size_t samples = (size_t)pitch * height;
-  if (samples > ctx->planeSamples) {
-    cudaFree(ctx->dOrig); cudaFree(ctx->dReco);
-    ctx->dOrig = ctx->dReco = nullptr; ctx->planeSamples = 0;
-    CK(cudaMalloc(&ctx->dOrig, samples * sizeof(int16_t)));
-    CK(cudaMalloc(&ctx->dReco, samples * sizeof(int16_t)));
-    ctx->planeSamples = samples;
-  }
-  ctx->width = width; ctx->height = height; ctx->stride = pitch;
-  ctx->bOrig = ctx->dOrig; ctx->bReco = ctx->dReco; ctx->wReco = ctx->dReco;
-  CK(cudaMemsetAsync(ctx->dOrig, 0, samples * sizeof(int16_t), ctx->stream));
-  CK(cudaMemsetAsync(ctx->dReco, 0, samples * sizeof(int16_t), ctx->stream));
+  int rc;
+  if ((rc = own_planes(ctx, width, height))) return rc;
+  CK(cudaMemsetAsync(buf(ctx, kOrig), 0, (size_t)ctx->stride * height * sizeof(int16_t), ctx->stream));
+  CK(cudaMemsetAsync(buf(ctx, kReco), 0, (size_t)ctx->stride * height * sizeof(int16_t), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
@@ -335,10 +342,10 @@ extern "C" int vvcb_reco_from_orig(vvcb_ctx* ctx)
 {
   if (!ctx) return VVCB_ERR_ARG;
   REMOTE_UNAVAILABLE("vvcb_reco_from_orig");
-  if (!ctx->dReco || ctx->bReco != ctx->dReco || ctx->bOrig != ctx->dOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_reco_from_orig: no frame owned by the context"); return VVCB_ERR_STATE; }
+  if (!buf(ctx, kReco) || ctx->bReco != buf(ctx, kReco) || ctx->bOrig != buf(ctx, kOrig)) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_reco_from_orig: no frame owned by the context"); return VVCB_ERR_STATE; }
   CK(cudaSetDevice(ctx->device));
   // stream ordered: every later launch of this context (the pipelined path's kernels included) runs behind it
-  CK(cudaMemcpyAsync(ctx->dReco, ctx->dOrig, (size_t)ctx->stride * ctx->height * sizeof(int16_t), cudaMemcpyDeviceToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(buf(ctx, kReco), buf(ctx, kOrig), (size_t)ctx->stride * ctx->height * sizeof(int16_t), cudaMemcpyDeviceToDevice, ctx->stream));
   return VVCB_OK;
 }
 
@@ -347,11 +354,11 @@ extern "C" int vvcb_frame_share(vvcb_ctx* dst, vvcb_ctx* src)
   if (!dst) return VVCB_ERR_ARG;
   vvcb_ctx* ctx = dst;
   REMOTE_UNAVAILABLE("vvcb_frame_share");
-  if (!src || src->remote || !src->dOrig || src->bOrig != src->dOrig || src->device != dst->device) {
+  if (!src || src->remote || !buf(src, kOrig) || src->bOrig != buf(src, kOrig) || src->device != dst->device) {
     snprintf(ctx->err, sizeof(ctx->err), "vvcb_frame_share: the source context owns no frame on this device");
     return VVCB_ERR_STATE;
   }
-  dst->bOrig = src->dOrig; dst->bReco = src->dReco; dst->wReco = src->dReco;
+  dst->bOrig = buf<int16_t>(src, kOrig); dst->bReco = dst->wReco = buf<int16_t>(src, kReco);
   dst->width = src->width; dst->height = src->height; dst->stride = src->stride;
   return VVCB_OK;
 }
@@ -360,28 +367,15 @@ extern "C" int vvcb_orig_update(vvcb_ctx* ctx, const int16_t* orig, int stride, 
 {
   if (!ctx) return VVCB_ERR_ARG;
   REMOTE_UNAVAILABLE("vvcb_orig_update");
-  if (!ctx->dOrig || ctx->bOrig != ctx->dOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_orig_update: no frame owned by the context"); return VVCB_ERR_STATE; }
+  if (!buf(ctx, kOrig) || ctx->bOrig != buf(ctx, kOrig)) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_orig_update: no frame owned by the context"); return VVCB_ERR_STATE; }
   if (!orig || x < 0 || y < 0 || w <= 0 || h <= 0 || x + w > ctx->width || y + h > ctx->height || stride < w) {
     snprintf(ctx->err, sizeof(ctx->err), "vvcb_orig_update: rectangle outside the picture");
     return VVCB_ERR_ARG;
   }
   CK(cudaSetDevice(ctx->device));
-  CK(cudaMemcpy2DAsync(ctx->dOrig + (size_t)y * ctx->stride + x, ctx->stride * sizeof(int16_t), orig, stride * sizeof(int16_t),
+  CK(cudaMemcpy2DAsync(buf<int16_t>(ctx, kOrig) + (size_t)y * ctx->stride + x, ctx->stride * sizeof(int16_t), orig, stride * sizeof(int16_t),
                        w * sizeof(int16_t), h, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  return VVCB_OK;
-}
-
-// page-locked staging buffer i of at least `bytes`
-static int pin_buf(vvcb_ctx* ctx, PinSlot i, size_t bytes)
-{
-  if (bytes > ctx->capPin[i]) {
-    if (ctx->hPin[i]) cudaFreeHost(ctx->hPin[i]);
-    ctx->hPin[i] = nullptr; ctx->capPin[i] = 0;
-    const size_t cap = bytes + bytes / 2 + 4096;
-    CK(cudaHostAlloc(&ctx->hPin[i], cap, cudaHostAllocDefault));
-    ctx->capPin[i] = cap;
-  }
   return VVCB_OK;
 }
 
@@ -391,6 +385,30 @@ struct Arena {
   size_t take(size_t bytes) { const size_t at = size; size += (bytes + 15) & ~(size_t)15; return at; }
 };
 template <class T> static T* at(void* base, size_t offset) { return reinterpret_cast<T*>(static_cast<uint8_t*>(base) + offset); }
+
+// Host or device pieces of one arena, laid out in order by Arena: add() returns a piece's offset.
+struct Pieces {
+  struct Piece { const void* p; size_t at, bytes; };
+  Arena layout;
+  std::vector<Piece> list;
+  size_t add(const void* p, size_t bytes) { list.push_back({ p, layout.size, bytes }); return layout.take(bytes); }
+  template <class T> size_t add(const std::vector<T>& v) { return add(v.data(), v.size() * sizeof(T)); }
+};
+
+// Sizes device slot `dev` for an arena of host pieces and brings them there: with a page-locked slot `pin` they are filled into it and the
+// caller moves that arena in one step; without one (kSlots) each piece is copied directly.
+static int stage_in(vvcb_ctx* ctx, const Pieces& in, Slot dev, Slot pin)
+{
+  const size_t size = in.layout.size;
+  int rc;
+  if ((rc = grow(ctx, dev, size)) || (pin != kSlots && (rc = grow(ctx, pin, size, size / 2 + 4096)))) return rc;
+  for (const Pieces::Piece& q : in.list) {
+    if (!q.bytes) continue;
+    if (pin != kSlots) memcpy(buf<uint8_t>(ctx, pin) + q.at, q.p, q.bytes);
+    else CK(cudaMemcpyAsync(buf<uint8_t>(ctx, dev) + q.at, q.p, q.bytes, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  return VVCB_OK;
+}
 
 // one CTA per rectangle: dense w*h block -> the reconstruction plane
 __global__ void __launch_bounds__(128) reco_scatter_kernel(const vvcb_rect* __restrict__ rects, int n, const int16_t* __restrict__ samples, int16_t* __restrict__ plane, int stride)
@@ -408,17 +426,12 @@ __global__ void __launch_bounds__(128) reco_scatter_kernel(const vvcb_rect* __re
 static int launch_reco_rects(vvcb_ctx* ctx, const vvcb_rect* rects, int n, const int16_t* samples, size_t n_samples)
 {
   if (n == 0) return VVCB_OK;
-  for (int i = 0; i < 2; i++) {
-    const size_t need = i == 0 ? (size_t)n * sizeof(vvcb_rect) : n_samples * sizeof(int16_t);
-    if (need > ctx->capRect[i]) {
-      cudaFree(ctx->dRect[i]); ctx->dRect[i] = nullptr; ctx->capRect[i] = 0;
-      CK(cudaMalloc(&ctx->dRect[i], need * 2));
-      ctx->capRect[i] = need * 2;
-    }
-  }
-  CK(cudaMemcpyAsync(ctx->dRect[0], rects, (size_t)n * sizeof(vvcb_rect), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(ctx->dRect[1], samples, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
-  reco_scatter_kernel<<<n < ctx->numSms * 8 ? n : ctx->numSms * 8, 128, 0, ctx->stream>>>(static_cast<const vvcb_rect*>(ctx->dRect[0]), n, static_cast<const int16_t*>(ctx->dRect[1]), ctx->wReco, ctx->stride);
+  const size_t rectBytes = (size_t)n * sizeof(vvcb_rect), sampleBytes = n_samples * sizeof(int16_t);
+  int rc;
+  if ((rc = grow(ctx, kRects, rectBytes, rectBytes)) || (rc = grow(ctx, kRectSamples, sampleBytes, sampleBytes))) return rc;
+  CK(cudaMemcpyAsync(buf(ctx, kRects), rects, rectBytes, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(buf(ctx, kRectSamples), samples, sampleBytes, cudaMemcpyHostToDevice, ctx->stream));
+  reco_scatter_kernel<<<n < ctx->numSms * 8 ? n : ctx->numSms * 8, 128, 0, ctx->stream>>>(buf<const vvcb_rect>(ctx, kRects), n, buf<const int16_t>(ctx, kRectSamples), ctx->wReco, ctx->stride);
   ctx->launches++;
   CK(cudaGetLastError());
   return VVCB_OK;
@@ -459,13 +472,13 @@ extern "C" int vvcb_reco_update(vvcb_ctx* ctx, const int16_t* reco, int stride, 
     const vvcb_rect rc = { (int16_t)x, (int16_t)y, (int16_t)w, (int16_t)h, 0 };
     return vvcb_reco_update_rects(ctx, &rc, 1, dense.data(), dense.size());
   }
-  if (!ctx->dReco || ctx->bReco != ctx->dReco) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_reco_update: no frame owned by the context"); return VVCB_ERR_STATE; }
+  if (!buf(ctx, kReco) || ctx->bReco != buf(ctx, kReco)) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_reco_update: no frame owned by the context"); return VVCB_ERR_STATE; }
   if (!reco || x < 0 || y < 0 || w <= 0 || h <= 0 || x + w > ctx->width || y + h > ctx->height || stride < w) {
     snprintf(ctx->err, sizeof(ctx->err), "vvcb_reco_update: rectangle outside the picture");
     return VVCB_ERR_ARG;
   }
   CK(cudaSetDevice(ctx->device));
-  CK(cudaMemcpy2DAsync(ctx->dReco + (size_t)y * ctx->stride + x, ctx->stride * sizeof(int16_t), reco, stride * sizeof(int16_t),
+  CK(cudaMemcpy2DAsync(buf<int16_t>(ctx, kReco) + (size_t)y * ctx->stride + x, ctx->stride * sizeof(int16_t), reco, stride * sizeof(int16_t),
                        w * sizeof(int16_t), h, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
@@ -503,28 +516,6 @@ extern "C" int vvcb_kernel_times(vvcb_ctx* ctx, float ms[3], int* launches)
   return VVCB_OK;
 }
 
-static int ensure_items(vvcb_ctx* ctx, int n)
-{
-  static_assert(kItemTasks >= 128, "the item bound below assumes at least 128 lane-tasks per plain work item");
-  const size_t need = (size_t)n * 60 + 8; // worst case 64x64: three kinds, ceil(slots * 64 lanes / kItemTasks) items each
-  if (need > ctx->capItems) {
-    cudaFree(ctx->dItems); ctx->dItems = nullptr; ctx->capItems = 0;
-    CK(cudaMalloc(&ctx->dItems, need * sizeof(WorkItem)));
-    ctx->capItems = need;
-  }
-  return VVCB_OK;
-}
-
-static int ensure_details(vvcb_ctx* ctx, int n)
-{
-  if ((size_t)n > ctx->capDetails) {
-    cudaFree(ctx->dDetails); ctx->dDetails = nullptr; ctx->capDetails = 0;
-    CK(cudaMalloc(&ctx->dDetails, (size_t)n * sizeof(vvcb_rmd_detail)));
-    ctx->capDetails = (size_t)n;
-  }
-  return VVCB_OK;
-}
-
 template <int TILE, int KIND, int MODE> static void launch_eval_bucket(const EvalParams& P, int numSms, long long maxWarps, cudaStream_t stream)
 {
   using Cfg = EvalCfg<MODE == 1>;
@@ -542,13 +533,12 @@ static int launch_rmd(vvcb_ctx* ctx, const vvcb_rmd_visit* dVisits, int n, vvcb_
 {
   if (!ctx->bOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_rmd_eval: vvcb_frame_begin has not been called"); return VVCB_ERR_STATE; }
   if (n == 0) return VVCB_OK;
-  int rc = ensure_items(ctx, n);
-  if (rc) return rc;
-  if ((size_t)n > ctx->capScratch) {
-    cudaFree(ctx->dScratch); ctx->dScratch = nullptr; ctx->capScratch = 0;
-    CK(cudaMalloc(&ctx->dScratch, (size_t)n * 2 * VVCB_NUM_SLOTS * sizeof(uint32_t)));
-    ctx->capScratch = (size_t)n;
-  }
+  static_assert(kItemTasks >= 128, "the item bound below assumes at least 128 lane-tasks per plain work item");
+  // worst case 64x64: three kinds, ceil(slots * 64 lanes / kItemTasks) items each
+  int rc;
+  if ((rc = grow(ctx, kItems, ((size_t)n * 60 + 8) * sizeof(WorkItem))) || (rc = grow(ctx, kSadSatd, (size_t)n * 2 * VVCB_NUM_SLOTS * sizeof(uint32_t)))) return rc;
+  WorkItem* dItems = buf<WorkItem>(ctx, kItems);
+  uint32_t* dScratch = buf<uint32_t>(ctx, kSadSatd);
   const bool smallPlan = hostVisits && n <= 4096;         // walk-sized batch: one planning launch (rmd_plan_small), the plan state is written whole
   if (!smallPlan) CK(cudaMemsetAsync(ctx->dPlan, 0, sizeof(PlanState), ctx->stream));
   const bool tm = ctx->timing != 0;
@@ -567,17 +557,17 @@ static int launch_rmd(vvcb_ctx* ctx, const vvcb_rmd_visit* dVisits, int n, vvcb_
       if (mip) { need[packed][sh.tile * kNumKinds + KIND_MIP] = true; inBucket[packed][sh.tile * kNumKinds + KIND_MIP]++; }
     }
   int evalLaunches = 0;
-  if (smallPlan) rmd_plan_small<<<1, 256, 0, ctx->stream>>>(dVisits, n, ctx->ctu, ctx->dPlan, ctx->dItems, pack);
+  if (smallPlan) rmd_plan_small<<<1, 256, 0, ctx->stream>>>(dVisits, n, ctx->ctu, ctx->dPlan, dItems, pack);
   else {
     rmd_plan_count<<<(n + 255) / 256, 256, 0, ctx->stream>>>(dVisits, n, ctx->ctu, ctx->dPlan, pack);
     rmd_plan_scan<<<1, 32, 0, ctx->stream>>>(ctx->dPlan);
-    rmd_plan_fill<<<(n + 255) / 256, 256, 0, ctx->stream>>>(dVisits, n, ctx->ctu, ctx->dPlan, ctx->dItems, pack);
+    rmd_plan_fill<<<(n + 255) / 256, 256, 0, ctx->stream>>>(dVisits, n, ctx->ctu, ctx->dPlan, dItems, pack);
   }
   if (tm) CK(cudaEventRecord(ctx->kev[1], ctx->stream));
   EvalParams P;
-  P.visits = dVisits; P.items = ctx->dItems; P.plan = ctx->dPlan;
+  P.visits = dVisits; P.items = dItems; P.plan = ctx->dPlan;
   // without detail tables the lists only need min(2 * SAD, SATD): one scratch plane instead of two
-  P.sadSM = ctx->dScratch; P.satdSM = (dDetails || dPred) ? ctx->dScratch + (size_t)VVCB_NUM_SLOTS * n : nullptr; P.nVisits = n;
+  P.sadSM = dScratch; P.satdSM = (dDetails || dPred) ? dScratch + (size_t)VVCB_NUM_SLOTS * n : nullptr; P.nVisits = n;
   P.orig = ctx->bOrig; P.reco = ctx->bReco; P.stride = ctx->stride; P.bd = ctx->bd; P.ctu = ctx->ctu; P.rom = ctx->dRom;
   P.predOut = dPred;
   const long long maxWarps = (long long)n * 8;          // no point in more warps than work items
@@ -639,8 +629,8 @@ static int launch_rmd(vvcb_ctx* ctx, const vvcb_rmd_visit* dVisits, int n, vvcb_
   return VVCB_OK;
 }
 
-// The largest internal QP (6 * qp_per + qp_rem) of a luma block: 63 + QpBdOffset, QpBdOffset = 6 * (bitDepth - 8).
-static int max_qp(int bd) { return 63 + 6 * (bd - 8); }
+// QpParam::per / rem of a block: the internal QP 6 * qp_per + qp_rem goes up to 63 + QpBdOffset, QpBdOffset = 6 * (bitDepth - 8).
+static bool qp_ok(const vvcb_ctx* ctx, int per, int rem) { return rem >= 0 && rem < 6 && per >= 0 && 6 * per + rem <= 63 + 6 * (ctx->bd - 8); }
 // lambda of the RD quantisers: the dependent quantiser derives shift counts from it (vvcb_dq.cuh, dq_init_quant), so +inf is refused too.
 static bool lambda_ok(double l) { return l > 0.0 && isfinite(l); }
 
@@ -696,18 +686,6 @@ static int check_visits(vvcb_ctx* ctx, const vvcb_rmd_visit* v, int n, int first
   if (badIdx >= 0) {
     snprintf(ctx->err, sizeof(ctx->err), "vvcb_rmd_eval: visit %d is malformed (position/size/availability outside the picture)", first + badIdx);
     return VVCB_ERR_ARG;
-  }
-  return VVCB_OK;
-}
-
-static int ensure_visit_buffers(vvcb_ctx* ctx, int n)
-{
-  if ((size_t)n > ctx->capVisits) {
-    cudaFree(ctx->dVisits); cudaFree(ctx->dResults);
-    ctx->dVisits = nullptr; ctx->dResults = nullptr; ctx->capVisits = 0;
-    CK(cudaMalloc(&ctx->dVisits, (size_t)n * sizeof(vvcb_rmd_visit)));
-    CK(cudaMalloc(&ctx->dResults, (size_t)n * sizeof(vvcb_rmd_result)));
-    ctx->capVisits = (size_t)n;
   }
   return VVCB_OK;
 }
@@ -814,17 +792,13 @@ extern "C" int vvcb_rmd_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n,
   if (n > pipe_chunk() && !details) return rmd_eval_pipelined(ctx, visits, n, results);
   int rc = check_visits(ctx, visits, n);
   if (rc) return rc;
-  rc = ensure_visit_buffers(ctx, n);
+  if ((rc = grow(ctx, kVisits, (size_t)n * sizeof(vvcb_rmd_visit))) || (rc = grow(ctx, kResults, (size_t)n * sizeof(vvcb_rmd_result)))) return rc;
+  CK(cudaMemcpyAsync(buf(ctx, kVisits), visits, (size_t)n * sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
+  if (details && (rc = grow(ctx, kDetails, (size_t)n * sizeof(vvcb_rmd_detail)))) return rc;
+  rc = launch_rmd(ctx, buf<vvcb_rmd_visit>(ctx, kVisits), n, buf<vvcb_rmd_result>(ctx, kResults), details ? buf<vvcb_rmd_detail>(ctx, kDetails) : nullptr, nullptr);
   if (rc) return rc;
-  CK(cudaMemcpyAsync(ctx->dVisits, visits, (size_t)n * sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
-  if (details) {
-    rc = ensure_details(ctx, n);
-    if (rc) return rc;
-  }
-  rc = launch_rmd(ctx, ctx->dVisits, n, ctx->dResults, details ? ctx->dDetails : nullptr, nullptr);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(results, ctx->dResults, (size_t)n * sizeof(vvcb_rmd_result), cudaMemcpyDeviceToHost, ctx->stream));
-  if (details) CK(cudaMemcpyAsync(details, ctx->dDetails, (size_t)n * sizeof(vvcb_rmd_detail), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(results, buf(ctx, kResults), (size_t)n * sizeof(vvcb_rmd_result), cudaMemcpyDeviceToHost, ctx->stream));
+  if (details) CK(cudaMemcpyAsync(details, buf(ctx, kDetails), (size_t)n * sizeof(vvcb_rmd_detail), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
@@ -840,15 +814,11 @@ extern "C" int vvcb_rmd_eval_brief(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, 
   if (n > pipe_chunk()) return rmd_eval_pipelined(ctx, visits, n, nullptr, out);
   int rc = check_visits(ctx, visits, n);
   if (rc) return rc;
-  if ((rc = ensure_visit_buffers(ctx, n))) return rc;
-  if ((size_t)n > ctx->capBrief) {
-    cudaFree(ctx->dBrief); ctx->dBrief = nullptr; ctx->capBrief = 0;
-    CK(cudaMalloc(&ctx->dBrief, (size_t)n * sizeof(vvcb_rmd_brief)));
-    ctx->capBrief = (size_t)n;
-  }
-  CK(cudaMemcpyAsync(ctx->dVisits, visits, (size_t)n * sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
-  if ((rc = launch_rmd(ctx, ctx->dVisits, n, nullptr, nullptr, nullptr, nullptr, ctx->dBrief))) return rc;
-  CK(cudaMemcpyAsync(out, ctx->dBrief, (size_t)n * sizeof(vvcb_rmd_brief), cudaMemcpyDeviceToHost, ctx->stream));
+  if ((rc = grow(ctx, kVisits, (size_t)n * sizeof(vvcb_rmd_visit))) || (rc = grow(ctx, kResults, (size_t)n * sizeof(vvcb_rmd_result))) ||
+      (rc = grow(ctx, kBrief, (size_t)n * sizeof(vvcb_rmd_brief)))) return rc;
+  CK(cudaMemcpyAsync(buf(ctx, kVisits), visits, (size_t)n * sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = launch_rmd(ctx, buf<vvcb_rmd_visit>(ctx, kVisits), n, nullptr, nullptr, nullptr, nullptr, buf<vvcb_rmd_brief>(ctx, kBrief)))) return rc;
+  CK(cudaMemcpyAsync(out, buf(ctx, kBrief), (size_t)n * sizeof(vvcb_rmd_brief), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
@@ -892,25 +862,20 @@ static int rmd_pred_impl(vvcb_ctx* ctx, const vvcb_rmd_visit* visit, int slot, i
     if (!evaluated) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_rmd_pred: slot %d is not evaluated for this visit", slot); return VVCB_ERR_ARG; }
   }
   CK(cudaSetDevice(ctx->device));
-  rc = ensure_visit_buffers(ctx, 1);
+  if ((rc = grow(ctx, kVisits, sizeof(vvcb_rmd_visit))) || (rc = grow(ctx, kResults, sizeof(vvcb_rmd_result))) ||
+      (rc = grow(ctx, kPred, (size_t)VVCB_NUM_SLOTS * w * h * sizeof(int16_t)))) return rc;
+  int16_t* dPred = buf<int16_t>(ctx, kPred);
+  CK(cudaMemcpyAsync(buf(ctx, kVisits), visit, sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
+  rc = launch_rmd(ctx, buf<vvcb_rmd_visit>(ctx, kVisits), 1, buf<vvcb_rmd_result>(ctx, kResults), nullptr, dPred);
   if (rc) return rc;
-  const size_t need = (size_t)VVCB_NUM_SLOTS * w * h;
-  if (need > ctx->capPred) {
-    cudaFree(ctx->dPred); ctx->dPred = nullptr; ctx->capPred = 0;
-    CK(cudaMalloc(&ctx->dPred, need * sizeof(int16_t)));
-    ctx->capPred = need;
-  }
-  CK(cudaMemcpyAsync(ctx->dVisits, visit, sizeof(vvcb_rmd_visit), cudaMemcpyHostToDevice, ctx->stream));
-  rc = launch_rmd(ctx, ctx->dVisits, 1, ctx->dResults, nullptr, ctx->dPred);
-  if (rc) return rc;
-  if (slot >= 0) CK(cudaMemcpyAsync(pred, ctx->dPred + (size_t)slot * w * h, (size_t)w * h * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (slot >= 0) CK(cudaMemcpyAsync(pred, dPred + (size_t)slot * w * h, (size_t)w * h * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
   else {
     // only the slots the visit evaluates: the device buffer holds an earlier visit's samples in the others, and the caller's copy of
     // those is left untouched (vvc_intra_b200.h)
     const int spans[3][2] = { { 0, VVCB_SLOT_MRL1 }, { VVCB_SLOT_MRL1, mrlAllowed ? VVCB_SLOT_MIP : VVCB_SLOT_MRL1 }, { VVCB_SLOT_MIP, VVCB_SLOT_MIP + numMip } };
     for (const auto& s : spans)
       if (s[1] > s[0])
-        CK(cudaMemcpyAsync(pred + (size_t)s[0] * w * h, ctx->dPred + (size_t)s[0] * w * h, (size_t)(s[1] - s[0]) * w * h * sizeof(int16_t),
+        CK(cudaMemcpyAsync(pred + (size_t)s[0] * w * h, dPred + (size_t)s[0] * w * h, (size_t)(s[1] - s[0]) * w * h * sizeof(int16_t),
                            cudaMemcpyDeviceToHost, ctx->stream));
   }
   CK(cudaStreamSynchronize(ctx->stream));
@@ -949,16 +914,6 @@ static cudaError_t arena_copy(vvcb_ctx* ctx, const void* src, void* dst, size_t 
   return cudaGetLastError();
 }
 
-static int tu_buf(vvcb_ctx* ctx, TuSlot i, size_t bytes)
-{
-  if (bytes > ctx->capTu[i]) {
-    cudaFree(ctx->dTu[i]); ctx->dTu[i] = nullptr; ctx->capTu[i] = 0;
-    CK(cudaMalloc(&ctx->dTu[i], bytes));
-    ctx->capTu[i] = bytes;
-  }
-  return VVCB_OK;
-}
-
 // The counting sort of the dependent quantiser's jobs by first test position buys warp efficiency for sweeps (eight TUs per warp walk
 // scans of equal length); a walk's batch of a few dozen candidates is latency bound, skips its three launches and runs one TU per warp.
 constexpr int kDqSortAbove = 2048;
@@ -977,11 +932,11 @@ static int quant_scratch(vvcb_ctx* ctx, size_t samples, int nRates, const int* n
   int maxDq = 0, maxGrid = 0;                                       // the grid is not monotonic in the job count (sparse, kDqSortAbove)
   for (int k = 0; k < steps; k++) { maxDq = std::max(maxDq, nDq[k]); maxGrid = std::max(maxGrid, dq_grid(ctx, nDq[k])); }
   int rc;
-  if ((rc = tu_buf(ctx, kDqCoeff, samples * sizeof(int32_t)))) return rc;
+  if ((rc = grow(ctx, kDqCoeff, samples * sizeof(int32_t)))) return rc;
   if (!maxDq) return VVCB_OK;
-  if ((rc = tu_buf(ctx, kDqTabs, (size_t)nRates * sizeof(DqRateTab)))) return rc;
-  if ((rc = tu_buf(ctx, kDqScratch, (size_t)maxGrid * kDqGroups * kDqSlotBytes))) return rc;
-  return tu_buf(ctx, kDqLists, ((size_t)maxDq * 3 + kDqBins) * sizeof(int));
+  if ((rc = grow(ctx, kDqTabs, (size_t)nRates * sizeof(DqRateTab)))) return rc;
+  if ((rc = grow(ctx, kDqScratch, (size_t)maxGrid * kDqGroups * kDqSlotBytes))) return rc;
+  return grow(ctx, kDqLists, ((size_t)maxDq * 3 + kDqBins) * sizeof(int));
 }
 
 // job indices of bySize[log2w + log2h - 4], largest TU first
@@ -1045,7 +1000,7 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
   TuParams P;
   P.jobs = c.jobs; P.list = nullptr; P.n = 0; P.resi = c.resi; P.pred = c.pred; P.coeff = c.coeff; P.level = c.level; P.reco = c.reco;
   P.results = c.results; P.orig = c.orig ? c.orig : ctx->bOrig; P.stride = c.orig ? c.stride : ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
-  P.dqCoeff = static_cast<int32_t*>(ctx->dTu[kDqCoeff]); P.dqDeq = c.deq; P.phase = 0; P.trPair = c.trPair;
+  P.dqCoeff = buf<int32_t>(ctx, kDqCoeff); P.dqDeq = c.deq; P.phase = 0; P.trPair = c.trPair;
   auto launch_tu = [&](TuParams Q) {
     if (nSmall) { Q.list = c.team; Q.n = nSmall; tu_eval_kernel<32><<<std::min((nSmall + 3) / 4, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
     if (nLarge) { Q.list = c.team + nSmall; Q.n = nLarge; tu_eval_kernel<128><<<std::min(nLarge, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
@@ -1069,8 +1024,8 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
       rates_from_states_kernel<<<(unsigned)((nPrice + 127) / 128), 128, 0, ctx->stream>>>(c.priceFrom, c.nRates, ctx->dRateRom, c.rates);
       ctx->launches++;
     }
-    dq_rate_kernel<<<c.nRates, 32, 0, ctx->stream>>>(c.rates, c.nRates, static_cast<DqRateTab*>(ctx->dTu[kDqTabs]));
-    int* firstRaw = static_cast<int*>(ctx->dTu[kDqLists]);
+    dq_rate_kernel<<<c.nRates, 32, 0, ctx->stream>>>(c.rates, c.nRates, buf<DqRateTab>(ctx, kDqTabs));
+    int* firstRaw = buf<int>(ctx, kDqLists);
     int* orderSorted = firstRaw + nDq;
     int* firstSorted = firstRaw + 2 * nDq;
     dq_first_kernel<<<std::min((nDq + kDqGroups - 1) / kDqGroups, ctx->numSms * 8), kDqThreads, 0, ctx->stream>>>(c.jobs, c.dq, nDq, P.dqCoeff, ctx->dDqRom, ctx->bd, firstRaw);
@@ -1087,8 +1042,8 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
     DqParams D;
     D.jobs = c.jobs; D.order = sortJobs ? orderSorted : c.dq; D.firstPos = sortJobs ? firstSorted : firstRaw; D.n = nDq;
     D.coeff = P.dqCoeff; D.level = c.level; D.deq = c.deq; D.results = c.results;
-    D.rates = c.rates; D.tabs = static_cast<const DqRateTab*>(ctx->dTu[kDqTabs]);
-    D.rom = ctx->dDqRom; D.scratch = static_cast<uint8_t*>(ctx->dTu[kDqScratch]); D.bd = ctx->bd; D.sparse = !sortJobs;
+    D.rates = c.rates; D.tabs = buf<const DqRateTab>(ctx, kDqTabs);
+    D.rom = ctx->dDqRom; D.scratch = buf<uint8_t>(ctx, kDqScratch); D.bd = ctx->bd; D.sparse = !sortJobs;
     if (c.chroma) dq_kernel<true><<<dq_grid(ctx, nDq), kDqThreads, 0, ctx->stream>>>(D);
     else dq_kernel<false><<<dq_grid(ctx, nDq), kDqThreads, 0, ctx->stream>>>(D);
     ctx->launches += 3;
@@ -1159,8 +1114,7 @@ static int tu_eval_impl(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n, const int
     const size_t sz = (size_t)1 << (j.log2w + j.log2h);
     const bool q = (j.flags & VVCB_TU_QUANT) != 0;
     const bool dq = q && (j.flags & VVCB_TU_DEPQUANT);
-    bool ok = j.log2w >= 2 && j.log2w <= 6 && j.log2h >= 2 && j.log2h <= 6 && j.mts_idx <= 5 && (size_t)j.offset + sz <= n_samples &&
-              j.qp_rem >= 0 && j.qp_rem < 6 && j.qp_per >= 0 && 6 * j.qp_per + j.qp_rem <= max_qp(ctx->bd);
+    bool ok = j.log2w >= 2 && j.log2w <= 6 && j.log2h >= 2 && j.log2h <= 6 && j.mts_idx <= 5 && (size_t)j.offset + sz <= n_samples && qp_ok(ctx, j.qp_per, j.qp_rem);
     if (j.mts_idx == 1) ok = ok && j.log2w <= 5 && j.log2h <= 5;                 // TU::isTSAllowed, CL/UnitTools.cpp:4524
     if (j.mts_idx > 1)  ok = ok && j.log2w <= 5 && j.log2h <= 5;                 // TU::isMTSAllowed, :4549
     if (q) ok = ok && ctx->bOrig && j.x >= 0 && j.y >= 0 && j.x + (1 << j.log2w) <= ctx->width && j.y + (1 << j.log2h) <= ctx->height;
@@ -1180,46 +1134,28 @@ static int tu_eval_impl(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n, const int
   const bool wLevel = walk ? walk->wantLevel : level != nullptr, wReco = walk ? walk->wantReco : reco != nullptr, wPred = walk ? walk->wantPred : pred_out != nullptr;
   const bool needLevel = wLevel || nDq || nTs || nRate;
   if ((nDq || nTs) && (rc = quant_scratch(ctx, n_samples, n_rates, &nDq, 1))) return rc;
-  if ((rc = tu_buf(ctx, kTuResi, n_samples * sizeof(int16_t)))) return rc;
-  if (coeff && (rc = tu_buf(ctx, kTuCoeff, n_samples * sizeof(int32_t)))) return rc;
+  if ((rc = grow(ctx, kTuResi, n_samples * sizeof(int16_t)))) return rc;
+  if (coeff && (rc = grow(ctx, kTuCoeff, n_samples * sizeof(int32_t)))) return rc;
   // the host inputs in one device arena; walk mode stages them in page-locked memory, moved by one copy kernel
-  const size_t ratesBytes = (nDq || nTs) ? (size_t)n_rates * sizeof(vvcb_dq_rates) : 0, statesBytes = nRate ? (size_t)n_rates * sizeof(vvcb_ctx_states) : 0;
-  Arena in;
-  const size_t iJobs = in.take((size_t)n * sizeof(vvcb_tu_job)), iVis = in.take((size_t)n_visits * sizeof(vvcb_rmd_visit)),
-               iSrc = in.take(src ? (size_t)n * sizeof(vvcb_tu_src) : 0), iTeam = in.take((size_t)n * sizeof(int)), iOrder = in.take((size_t)nDq * sizeof(int)),
-               iTs = in.take((size_t)nTs * sizeof(int)), iRates = in.take(ratesBytes), iRateOrder = in.take((size_t)nRate * sizeof(int)), iStates = in.take(statesBytes);
-  uint8_t* hin = nullptr;
-  if (walk) {
-    if ((rc = pin_buf(ctx, kPinTuIn, in.size))) return rc;
-    hin = static_cast<uint8_t*>(ctx->hPin[kPinTuIn]);
-  }
-  if ((rc = tu_buf(ctx, kTuIn, in.size))) return rc;
-  void* din = ctx->dTu[kTuIn];
-  auto put = [&](size_t o, const void* p, size_t bytes) {
-    if (!bytes) return cudaSuccess;
-    if (walk) { memcpy(hin + o, p, bytes); return cudaSuccess; }
-    return cudaMemcpyAsync(at<uint8_t>(din, o), p, bytes, cudaMemcpyHostToDevice, ctx->stream);
-  };
-  CK(put(iJobs, jobs, (size_t)n * sizeof(vvcb_tu_job)));
-  if (src) { CK(put(iVis, visits, (size_t)n_visits * sizeof(vvcb_rmd_visit))); CK(put(iSrc, src, (size_t)n * sizeof(vvcb_tu_src))); }
-  CK(put(iTeam, L.team.data(), (size_t)n * sizeof(int)));
-  CK(put(iOrder, L.dq.data(), (size_t)nDq * sizeof(int)));
-  CK(put(iTs, L.ts.data(), (size_t)nTs * sizeof(int)));
-  CK(put(iRates, rates, ratesBytes));
-  CK(put(iRateOrder, L.rate.data(), (size_t)nRate * sizeof(int)));
-  CK(put(iStates, states, statesBytes));
-  if (walk) CK(arena_copy(ctx, hin, din, in.size));
+  Pieces in;
+  const size_t iJobs = in.add(jobs, (size_t)n * sizeof(vvcb_tu_job)), iVis = in.add(visits, (size_t)n_visits * sizeof(vvcb_rmd_visit)),
+               iSrc = in.add(src, src ? (size_t)n * sizeof(vvcb_tu_src) : 0), iTeam = in.add(L.team), iOrder = in.add(L.dq), iTs = in.add(L.ts),
+               iRates = in.add(rates, (nDq || nTs) ? (size_t)n_rates * sizeof(vvcb_dq_rates) : 0), iRateOrder = in.add(L.rate),
+               iStates = in.add(states, nRate ? (size_t)n_rates * sizeof(vvcb_ctx_states) : 0);
+  if ((rc = stage_in(ctx, in, kTuIn, walk ? kPinTuIn : kSlots))) return rc;
+  void* din = buf(ctx, kTuIn);
+  if (walk) CK(arena_copy(ctx, buf(ctx, kPinTuIn), din, in.layout.size));
   // the outputs in one device arena: results | prediction | reconstruction | levels, then the dequantised coefficients next to the levels
   Arena out;
   const size_t oRes = out.take((size_t)n * sizeof(vvcb_tu_result)), oPred = out.take(n_samples * sizeof(int16_t)),
                oReco = out.take(wReco ? n_samples * sizeof(int16_t) : 0), oLevel = out.take(needLevel ? n_samples * sizeof(int32_t) : 0);
   const size_t outBytes = wLevel ? out.size : (wReco ? oLevel : (wPred ? oReco : oPred));   // walk mode: what travels back
   const size_t oDeq = out.take((nDq || nTs) ? n_samples * sizeof(int32_t) : 0);
-  if ((rc = tu_buf(ctx, kTuOut, out.size))) return rc;
-  void* dout = ctx->dTu[kTuOut];
+  if ((rc = grow(ctx, kTuOut, out.size))) return rc;
+  void* dout = buf(ctx, kTuOut);
   if (walk) {
-    if ((rc = pin_buf(ctx, kPinTuOut, outBytes))) return rc;
-    void* hout = ctx->hPin[kPinTuOut];
+    if ((rc = grow(ctx, kPinTuOut, outBytes, outBytes / 2 + 4096))) return rc;
+    void* hout = buf(ctx, kPinTuOut);
     walk->results = at<vvcb_tu_result>(hout, oRes); walk->pred = at<int16_t>(hout, oPred);
     walk->reco = at<int16_t>(hout, oReco); walk->level = at<int32_t>(hout, oLevel);
   }
@@ -1227,8 +1163,8 @@ static int tu_eval_impl(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n, const int
   c.jobs = at<const vvcb_tu_job>(din, iJobs);
   c.team = at<const int>(din, iTeam); c.dq = at<const int>(din, iOrder); c.ts = at<const int>(din, iTs); c.rate = at<const int>(din, iRateOrder);
   int16_t* dPred = at<int16_t>(dout, oPred);
-  c.resi = static_cast<const int16_t*>(ctx->dTu[kTuResi]); c.pred = dPred;
-  c.coeff = coeff ? static_cast<int32_t*>(ctx->dTu[kTuCoeff]) : nullptr;
+  c.resi = buf<const int16_t>(ctx, kTuResi); c.pred = dPred;
+  c.coeff = coeff ? buf<int32_t>(ctx, kTuCoeff) : nullptr;
   c.level = needLevel ? at<int32_t>(dout, oLevel) : nullptr; c.reco = wReco ? at<int16_t>(dout, oReco) : nullptr;
   c.deq = (nDq || nTs) ? at<int32_t>(dout, oDeq) : nullptr; c.results = at<vvcb_tu_result>(dout, oRes);
   c.rates = at<vvcb_dq_rates>(din, iRates); c.nRates = n_rates; c.states = at<const vvcb_ctx_states>(din, iStates);
@@ -1239,20 +1175,20 @@ static int tu_eval_impl(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n, const int
     if (tm) CK(cudaEventRecord(ctx->tev[0], ctx->stream));
     TuPredParams Q;
     Q.visits = at<const vvcb_rmd_visit>(din, iVis); Q.src = at<const vvcb_tu_src>(din, iSrc); Q.jobs = c.jobs; Q.n = n;
-    Q.pred = dPred; Q.resi = static_cast<int16_t*>(ctx->dTu[kTuResi]);
+    Q.pred = dPred; Q.resi = buf<int16_t>(ctx, kTuResi);
     Q.orig = ctx->bOrig; Q.reco = ctx->bReco; Q.stride = ctx->stride; Q.bd = ctx->bd; Q.ctu = ctx->ctu; Q.rom = ctx->dRom;
     const int pg = (n + kTuPredWarps - 1) / kTuPredWarps < ctx->numSms * 8 ? (n + kTuPredWarps - 1) / kTuPredWarps : ctx->numSms * 8;
     tu_pred_kernel<<<pg, kTuPredWarps * 32, 0, ctx->stream>>>(Q);
     ctx->launches++;
   } else {
-    CK(cudaMemcpyAsync(ctx->dTu[kTuResi], resi, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(buf(ctx, kTuResi), resi, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
     if (pred) CK(cudaMemcpyAsync(dPred, pred, n_samples * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->stream));
     if (tm) CK(cudaEventRecord(ctx->tev[0], ctx->stream));
   }
   if ((rc = run_tu_chain(ctx, c, L, tm ? ctx->tev : nullptr))) return rc;
   CK(cudaGetLastError());
   if (coeff) CK(cudaMemcpyAsync(coeff, c.coeff, n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (walk) CK(arena_copy(ctx, dout, ctx->hPin[kPinTuOut], outBytes));
+  if (walk) CK(arena_copy(ctx, dout, buf(ctx, kPinTuOut), outBytes));
   else {
     if (level) CK(cudaMemcpyAsync(level, c.level, n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     if (reco) CK(cudaMemcpyAsync(reco, c.reco, n_samples * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1341,10 +1277,9 @@ extern "C" int vvcb_cu_eval(vvcb_ctx* ctx, vvcb_cu_request* reqs, int n)
   const size_t iRects = in.take(nRects * sizeof(vvcb_rect)), iSmp = in.take(nRectSamples * sizeof(int16_t)), iVis = in.take((size_t)nRmd * sizeof(vvcb_rmd_visit));
   vvcb_rmd_result* hRes = nullptr; vvcb_rmd_detail* hDet = nullptr;
   if (in.size) {
-    if ((rc = pin_buf(ctx, kPinStageIn, in.size))) return rc;
-    if ((rc = tu_buf(ctx, kStageIn, in.size))) return rc;
-    void* hin = ctx->hPin[kPinStageIn];
-    void* din = ctx->dTu[kStageIn];
+    if ((rc = grow(ctx, kPinStageIn, in.size, in.size / 2 + 4096)) || (rc = grow(ctx, kStageIn, in.size))) return rc;
+    void* hin = buf(ctx, kPinStageIn);
+    void* din = buf(ctx, kStageIn);
     vvcb_rect* hr = at<vvcb_rect>(hin, iRects);
     int16_t* hs = at<int16_t>(hin, iSmp);
     vvcb_rmd_visit* hv = at<vvcb_rmd_visit>(hin, iVis);
@@ -1371,10 +1306,9 @@ extern "C" int vvcb_cu_eval(vvcb_ctx* ctx, vvcb_cu_request* reqs, int n)
     if (nRmd) {
       Arena out;
       const size_t oRes = out.take((size_t)nRmd * sizeof(vvcb_rmd_result)), oDet = out.take(anyDetail ? (size_t)nRmd * sizeof(vvcb_rmd_detail) : 0);
-      if ((rc = tu_buf(ctx, kStageOut, out.size))) return rc;
-      if ((rc = pin_buf(ctx, kPinStageOut, out.size))) return rc;
-      void* dout = ctx->dTu[kStageOut];
-      void* hout = ctx->hPin[kPinStageOut];
+      if ((rc = grow(ctx, kStageOut, out.size)) || (rc = grow(ctx, kPinStageOut, out.size, out.size / 2 + 4096))) return rc;
+      void* dout = buf(ctx, kStageOut);
+      void* hout = buf(ctx, kPinStageOut);
       hRes = at<vvcb_rmd_result>(hout, oRes);
       hDet = anyDetail ? at<vvcb_rmd_detail>(hout, oDet) : nullptr;
       if ((rc = launch_rmd(ctx, at<const vvcb_rmd_visit>(din, iVis), nRmd, at<vvcb_rmd_result>(dout, oRes),
@@ -1506,16 +1440,16 @@ extern "C" int vvcb_residual_bits(vvcb_ctx* ctx, const vvcb_tu_job* jobs, int n,
   Arena in;
   const size_t iJobs = in.take((size_t)n * sizeof(vvcb_tu_job)), iLevel = in.take(n_samples * sizeof(int32_t)), iOrder = in.take((size_t)n * sizeof(int)),
                iStates = in.take((size_t)n_states * sizeof(vvcb_ctx_states));
-  if ((rc = tu_buf(ctx, kTuIn, in.size))) return rc;
-  if ((rc = tu_buf(ctx, kTuOut, (size_t)n * sizeof(vvcb_tu_result)))) return rc;
-  void* din = ctx->dTu[kTuIn];
+  if ((rc = grow(ctx, kTuIn, in.size))) return rc;
+  if ((rc = grow(ctx, kTuOut, (size_t)n * sizeof(vvcb_tu_result)))) return rc;
+  void* din = buf(ctx, kTuIn);
   CK(cudaMemcpyAsync(at<uint8_t>(din, iJobs), jobs, (size_t)n * sizeof(vvcb_tu_job), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(at<uint8_t>(din, iLevel), levels, n_samples * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(at<uint8_t>(din, iOrder), order.data(), (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(at<uint8_t>(din, iStates), states, (size_t)n_states * sizeof(vvcb_ctx_states), cudaMemcpyHostToDevice, ctx->stream));
   RateParams R;
   R.jobs = at<const vvcb_tu_job>(din, iJobs); R.order = at<const int>(din, iOrder); R.n = n;
-  R.level = at<const int32_t>(din, iLevel); R.results = static_cast<vvcb_tu_result*>(ctx->dTu[kTuOut]);
+  R.level = at<const int32_t>(din, iLevel); R.results = buf<vvcb_tu_result>(ctx, kTuOut);
   R.states = at<const vvcb_ctx_states>(din, iStates); R.rom = ctx->dDqRom; R.rate = ctx->dRateRom; R.depQuant = ctx->depQuant;
   rate_kernel<<<std::min((n + kRateWarps - 1) / kRateWarps, 16 * ctx->numSms), kRateThreads, 0, ctx->stream>>>(R);
   ctx->launches++;
@@ -1611,25 +1545,126 @@ extern "C" int vvcb_isp_mode_param(int cu_w, int cu_h, int pred_w, int pred_h, i
   return VVCB_OK;
 }
 
+// =====================================================================================================
+// staged candidate calls: vvcb_isp_eval, vvcb_chroma_tu_eval
+// =====================================================================================================
+// A staged call runs in chunks of at most kStagedChunk candidates: their TU jobs name the candidates' carried snapshots with the 16-bit
+// rate_idx.  chunk(base, m, checkOnly) validates the m jobs from index base on and, unless checkOnly, runs them; every chunk is validated
+// before any runs.
+constexpr int kStagedChunk = 65536;
+template <class Chunk> static int run_chunks(int n, Chunk chunk)
+{
+  for (int pass = 0; pass < 2; pass++)
+    for (int b = 0; b < n; b += kStagedChunk)
+      if (const int rc = chunk(b, std::min(kStagedChunk, n - b), pass == 0)) return rc;
+  return VVCB_OK;
+}
+
+// Why the quantiser setting of a staged job may not run, nullptr when it may: its flags, the qp_per / qp_rem and lambda of each of its
+// `comps` components, and its carried snapshot (`snapshot`: states[rate_idx] exists).
+static const char* staged_job_error(const vvcb_ctx* ctx, unsigned flags, const int16_t* qpPer, const int16_t* qpRem, const double* lambda,
+                                    int comps, bool snapshot)
+{
+  if ((flags & ~(VVCB_TU_QUANT | VVCB_TU_DEPQUANT | VVCB_TU_RATE)) || !(flags & VVCB_TU_QUANT)) return "flags: VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE] only";
+  for (int c = 0; c < comps; c++) if (!qp_ok(ctx, qpPer[c], qpRem[c])) return "qp_per / qp_rem out of range";
+  const bool dq = (flags & VVCB_TU_DEPQUANT) != 0;
+  if ((dq || (flags & VVCB_TU_RATE)) && !snapshot) return "rate_idx does not name a context snapshot";
+  for (int c = 0; dq && c < comps; c++)
+    if (!lambda_ok(lambda[c])) return comps == 1 ? "dependent quantisation needs a finite lambda > 0" : "dependent quantisation needs finite lambdas > 0";
+  return nullptr;
+}
+
+// Brings device pieces back through page-locked kPinStageOut, one copy each, and waits for them.  `host` is the page-locked arena: it
+// holds each piece at its offset until the next call on the context.
+static int stage_out(vvcb_ctx* ctx, const Pieces& out, uint8_t*& host)
+{
+  const size_t size = out.layout.size;
+  int rc;
+  if ((rc = grow(ctx, kPinStageOut, size, size / 2 + 4096))) return rc;
+  host = buf<uint8_t>(ctx, kPinStageOut);
+  for (const Pieces::Piece& q : out.list)
+    if (q.bytes) CK(cudaMemcpyAsync(host + q.at, q.p, q.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(ctx_sync(ctx));
+  return VVCB_OK;
+}
+
+// One chunk of a staged call: n candidates whose blocks are coded in `steps` TU batches, step k over the TU jobs [k * n, (k + 1) * n).
+// The candidates' samples lie packed densely on the device, whatever the caller's offsets: candidate i's from dense[i] on, dense[n] in
+// all.  The inputs travel in one page-locked arena (kPinStageIn -> kStageIn, one copy).  The work arena (kStageOut) holds the steps' TU
+// results | prediction | residual | reconstruction | levels | dequantised coefficients | the prices the dependent quantiser derives per
+// candidate, then the caller's own arrays (work.take before begin).
+struct Staged {
+  const int n, steps;
+  const std::vector<size_t>& dense;
+  Pieces in;                                       // the caller's inputs, then (begin) each step's team / dq / rate lists
+  Arena work;
+  const size_t oRes, oPred, oResi, oReco, oLevel, oDeq, oRates;
+  size_t iJobs = 0, iTeam[4] = {}, iDq[4] = {}, iRate[4] = {}, oOut[3] = {};
+  uint8_t* din = nullptr; uint8_t* dw = nullptr;  // the input and work arenas on the device, from begin
+
+  Staged(int n, int steps, const std::vector<size_t>& dense)
+      : n(n), steps(steps), dense(dense), oRes(work.take((size_t)steps * n * sizeof(vvcb_tu_result))), oPred(work.take(dense[n] * sizeof(int16_t))),
+        oResi(work.take(dense[n] * sizeof(int16_t))), oReco(work.take(dense[n] * sizeof(int16_t))), oLevel(work.take(dense[n] * sizeof(int32_t))),
+        oDeq(work.take(dense[n] * sizeof(int32_t))), oRates(work.take((size_t)n * sizeof(vvcb_dq_rates))) {}
+
+  // Stages the inputs (jobs: the offset of the TU jobs among them) with the steps' lists, sizes the work arena and the quantiser scratch
+  // (once, before the first step) and zeroes the levels and dequantised coefficients, which the quantisers do not reach everywhere.
+  int begin(vvcb_ctx* ctx, size_t jobs, const TuLists* L)
+  {
+    int nDq[4], rc;
+    iJobs = jobs;
+    for (int k = 0; k < steps; k++) { iTeam[k] = in.add(L[k].team); iDq[k] = in.add(L[k].dq); iRate[k] = in.add(L[k].rate); nDq[k] = (int)L[k].dq.size(); }
+    if ((rc = stage_in(ctx, in, kStageIn, kPinStageIn)) || (rc = grow(ctx, kStageOut, work.size)) || (rc = quant_scratch(ctx, dense[n], n, nDq, steps))) return rc;
+    din = buf<uint8_t>(ctx, kStageIn); dw = buf<uint8_t>(ctx, kStageOut);
+    CK(cudaMemcpyAsync(din, buf(ctx, kPinStageIn), in.layout.size, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(dw + oLevel, 0, oRates - oLevel, ctx->stream));
+    return VVCB_OK;
+  }
+
+  // step k's TuChain with the pointers every staged call shares
+  TuChain chain(int k) const
+  {
+    TuChain c = {};
+    c.jobs = at<const vvcb_tu_job>(din, iJobs) + (size_t)k * n;
+    c.team = at<const int>(din, iTeam[k]); c.dq = at<const int>(din, iDq[k]); c.rate = at<const int>(din, iRate[k]);
+    c.resi = at<int16_t>(dw, oResi); c.pred = at<int16_t>(dw, oPred); c.level = at<int32_t>(dw, oLevel); c.reco = at<int16_t>(dw, oReco);
+    c.deq = at<int32_t>(dw, oDeq); c.results = at<vvcb_tu_result>(dw, oRes) + (size_t)k * n; c.rates = at<vvcb_dq_rates>(dw, oRates); c.nRates = n;
+    return c;
+  }
+
+  // the sample outputs the caller wants (level, reco, pred not null) as pieces of `out`, and from its page-locked copy to the caller's offsets
+  void want(Pieces& out, const int32_t* level, const int16_t* reco, const int16_t* pred)
+  {
+    oOut[0] = out.add(dw + oLevel, level ? dense[n] * sizeof(int32_t) : 0); oOut[1] = out.add(dw + oReco, reco ? dense[n] * sizeof(int16_t) : 0);
+    oOut[2] = out.add(dw + oPred, pred ? dense[n] * sizeof(int16_t) : 0);
+  }
+  template <class Job> void scatter(uint8_t* host, const Job* jobs, int32_t* level, int16_t* reco, int16_t* pred) const
+  {
+    for (int i = 0; i < n; i++) {
+      const size_t from = dense[i], m = dense[i + 1] - dense[i], to = jobs[i].offset;
+      if (level) memcpy(level + to, at<const int32_t>(host, oOut[0]) + from, m * sizeof(int32_t));
+      if (reco) memcpy(reco + to, at<const int16_t>(host, oOut[1]) + from, m * sizeof(int16_t));
+      if (pred) memcpy(pred + to, at<const int16_t>(host, oOut[2]) + from, m * sizeof(int16_t));
+    }
+  }
+};
+
 // ISP candidates (include/vvc_intra_b200.h): up to four steps, one per block index k, over the TU kernels; the blocks of every candidate
 // that has a block k run in step k: isp_pred_kernel (lines from block k-1's reconstruction, prediction, residual, cbf of block k-1 and
 // cbfDeltaBits of block k), tu_eval_kernel pass 0, the quantiser (the dependent one priced by rates_from_states_kernel from the models the
 // previous block left), pass 1 (reconstruction into the candidate's buffer), rate_kernel adapting the candidate's carried models in place.
 // A fifth isp_pred_kernel pass codes the cbf of the last block of four-block candidates.
-// One chunk of at most kIspChunk candidates (their TU jobs name the carried snapshots with the 16-bit rate_idx); base: index of the
-// chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
-constexpr int kIspChunk = 65536;
+// One chunk of a staged call (run_chunks); base: index of the chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
 static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, const vvcb_isp_job* jobs, int n, int base,
                           const vvcb_ctx_states* states, int n_states, size_t n_samples,
                           int32_t* level, int16_t* reco, int16_t* pred, vvcb_isp_result* results, bool checkOnly)
 {
-  const unsigned kFlags = VVCB_TU_QUANT | VVCB_TU_DEPQUANT | VVCB_TU_RATE;
   std::vector<IspCand> cands(n);
   std::vector<vvcb_tu_job> tj((size_t)4 * n);
   std::vector<uint8_t> trPair((size_t)4 * n, 0);
   std::vector<IspState> ist(n);
   std::vector<vvcb_ctx_states> cst(n);
-  size_t cs = 0;                                   // the chunk's own samples: candidates are packed densely on the device, whatever the caller's offsets
+  std::vector<size_t> dense(n + 1, 0);            // the candidates' samples on the device (Staged)
   for (int i = 0; i < n; i++) {
     const vvcb_isp_job& j = jobs[i];
     auto bad = [&](const char* why) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_isp_eval: job %d: %s", base + i, why); return VVCB_ERR_ARG; };
@@ -1645,17 +1680,14 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
       return bad("left / above availability is not all or nothing");
     if (j.mode >= VVCB_NUM_LUMA_MODE) return bad("mode above 66");
     if (j.lfnst_idx != 0) return bad("LFNST with ISP is not evaluated");
-    if ((j.flags & ~kFlags) || !(j.flags & VVCB_TU_QUANT)) return bad("flags: VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE] only");
-    if (j.qp_rem < 0 || j.qp_rem >= 6 || j.qp_per < 0 || 6 * j.qp_per + j.qp_rem > max_qp(ctx->bd)) return bad("qp_per / qp_rem out of range");
-    const bool dq = (j.flags & VVCB_TU_DEPQUANT) != 0, carried = dq || (j.flags & VVCB_TU_RATE);
-    if (carried && (!states || j.rate_idx >= n_states)) return bad("rate_idx does not name a context snapshot");
-    if (dq && !lambda_ok(j.lambda)) return bad("dependent quantisation needs a finite lambda > 0");
+    if (const char* why = staged_job_error(ctx, j.flags, &j.qp_per, &j.qp_rem, &j.lambda, 1, states && j.rate_idx < n_states)) return bad(why);
+    const bool carried = (j.flags & (VVCB_TU_DEPQUANT | VVCB_TU_RATE)) != 0;
     if ((size_t)j.offset + (size_t)cuW * cuH > n_samples) return bad("outputs outside n_samples");
     IspCand& c = cands[i];
     c.x = v.x; c.y = v.y; c.cuW = (int16_t)cuW; c.cuH = (int16_t)cuH; c.bw = parts[0].w; c.bh = parts[0].h;
     c.topLen = parts[0].top_ref_len; c.leftLen = parts[0].left_ref_len;
     c.hor = j.isp_mode == VVCB_ISP_HOR; c.nParts = (uint8_t)np; c.availAl = v.avail_al; c.nAbove = v.n_above; c.nAboveRight = v.n_above_right;
-    c.nLeft = v.n_left; c.nBelowLeft = v.n_below_left; c.mode = j.mode; c.offset = (uint32_t)cs;
+    c.nLeft = v.n_left; c.nBelowLeft = v.n_below_left; c.mode = j.mode; c.offset = (uint32_t)dense[i];
     c.p = make_mode_param_isp(cuW, cuH, parts[0].pred_w, parts[0].pred_h, j.mode);
     memset(&ist[i], 0, sizeof(IspState));
     ist[i].ctx[0] = j.cbf[0]; ist[i].ctx[1] = j.cbf[1];
@@ -1668,12 +1700,12 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
       t.mts_idx = 0;
       t.flags = (uint8_t)(j.flags | (carried ? VVCB_TU_RATE : 0));   // rate_kernel adapts the carried models of DEPQUANT candidates too
       t.qp_per = j.qp_per; t.qp_rem = j.qp_rem;
-      t.offset = (uint32_t)(cs + (size_t)k * parts[k].w * parts[k].h);
+      t.offset = (uint32_t)(dense[i] + (size_t)k * parts[k].w * parts[k].h);
       t.rate_idx = (uint16_t)i;                        // the candidate's own carried snapshot
       t.lambda = j.lambda;
       trPair[(size_t)k * n + i] = (uint8_t)(parts[k].tr_hor | parts[k].tr_ver << 2);
     }
-    cs += (size_t)cuW * cuH;
+    dense[i + 1] = dense[i] + (size_t)cuW * cuH;
   }
   if (checkOnly) return VVCB_OK;
   // per-step work lists (all host-known: the values change, the shapes do not)
@@ -1682,45 +1714,18 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
   for (int k = 0; k <= 4; k++)
     for (int i = 0; i < n; i++) if (cands[i].nParts > k || (k > 0 && cands[i].nParts == k)) predList[k].push_back(i);
   for (int k = 0; k < 4; k++) L[k] = tu_lists(&tj[(size_t)k * n], n, [&](int i) { return cands[i].nParts > k; });
-  // one input arena in page-locked memory: candidates, TU jobs, transform pairs, cbf state, carried models, lists
-  Arena in;
-  const size_t iCand = in.take((size_t)n * sizeof(IspCand)), iJobs = in.take(tj.size() * sizeof(vvcb_tu_job)), iTr = in.take(trPair.size()),
-               iState = in.take((size_t)n * sizeof(IspState)), iCst = in.take((size_t)n * sizeof(vvcb_ctx_states));
-  size_t iPred[5], iTeam[4], iDq[4], iRate[4];
-  for (int k = 0; k <= 4; k++) iPred[k] = in.take(predList[k].size() * sizeof(int));
-  for (int k = 0; k < 4; k++) { iTeam[k] = in.take(L[k].team.size() * sizeof(int)); iDq[k] = in.take(L[k].dq.size() * sizeof(int)); iRate[k] = in.take(L[k].rate.size() * sizeof(int)); }
-  int rc;
-  if ((rc = pin_buf(ctx, kPinStageIn, in.size))) return rc;
-  void* hin = ctx->hPin[kPinStageIn];
-  memcpy(at<IspCand>(hin, iCand), cands.data(), (size_t)n * sizeof(IspCand));
-  memcpy(at<vvcb_tu_job>(hin, iJobs), tj.data(), tj.size() * sizeof(vvcb_tu_job));
-  memcpy(at<uint8_t>(hin, iTr), trPair.data(), trPair.size());
-  memcpy(at<IspState>(hin, iState), ist.data(), (size_t)n * sizeof(IspState));
-  memcpy(at<vvcb_ctx_states>(hin, iCst), cst.data(), (size_t)n * sizeof(vvcb_ctx_states));
-  auto put = [&](size_t o, const std::vector<int>& v) { if (!v.empty()) memcpy(at<int>(hin, o), v.data(), v.size() * sizeof(int)); };
-  for (int k = 0; k <= 4; k++) put(iPred[k], predList[k]);
-  for (int k = 0; k < 4; k++) { put(iTeam[k], L[k].team); put(iDq[k], L[k].dq); put(iRate[k], L[k].rate); }
-  // work arena: per-step TU results, prediction, residual, reconstruction, levels, dequantised coefficients, derived prices
-  Arena work;
-  const size_t oRes = work.take((size_t)4 * n * sizeof(vvcb_tu_result)), oPred = work.take(cs * sizeof(int16_t)), oResi = work.take(cs * sizeof(int16_t)),
-               oReco = work.take(cs * sizeof(int16_t)), oLevel = work.take(cs * sizeof(int32_t)), oDeq = work.take(cs * sizeof(int32_t)),
-               oRates = work.take((size_t)n * sizeof(vvcb_dq_rates));
-  const int nDq[4] = { (int)L[0].dq.size(), (int)L[1].dq.size(), (int)L[2].dq.size(), (int)L[3].dq.size() };
+  // inputs: candidates, TU jobs, transform pairs, cbf state, carried models, prediction lists
+  Staged s(n, 4, dense);
+  const size_t iCand = s.in.add(cands), iJobs = s.in.add(tj), iTr = s.in.add(trPair), iState = s.in.add(ist), iCst = s.in.add(cst);
+  size_t iPred[5];
+  for (int k = 0; k <= 4; k++) iPred[k] = s.in.add(predList[k]);
   CK(cudaSetDevice(ctx->device));
-  if ((rc = tu_buf(ctx, kStageIn, in.size))) return rc;
-  if ((rc = tu_buf(ctx, kStageOut, work.size))) return rc;
-  if ((rc = quant_scratch(ctx, cs, n, nDq, 4))) return rc;
-  void* din = ctx->dTu[kStageIn];
-  void* dw = ctx->dTu[kStageOut];
-  CK(cudaMemcpyAsync(din, hin, in.size, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemsetAsync(at<uint8_t>(dw, oLevel), 0, oRates - oLevel, ctx->stream));        // levels / dequantised coefficients the quantisers do not reach stay zero
-  const IspCand* dCand = at<const IspCand>(din, iCand);
-  vvcb_tu_job* dJobs = at<vvcb_tu_job>(din, iJobs);
-  IspState* dState = at<IspState>(din, iState);
-  vvcb_ctx_states* dCst = at<vvcb_ctx_states>(din, iCst);
-  vvcb_tu_result* dRes = at<vvcb_tu_result>(dw, oRes);
-  int16_t* dPred = at<int16_t>(dw, oPred); int16_t* dResi = at<int16_t>(dw, oResi);
-  int16_t* dReco = at<int16_t>(dw, oReco); int32_t* dLevel = at<int32_t>(dw, oLevel);
+  int rc;
+  if ((rc = s.begin(ctx, iJobs, L))) return rc;
+  vvcb_tu_job* dJobs = at<vvcb_tu_job>(s.din, iJobs);
+  IspState* dState = at<IspState>(s.din, iState);
+  vvcb_ctx_states* dCst = at<vvcb_ctx_states>(s.din, iCst);
+  vvcb_tu_result* dRes = at<vvcb_tu_result>(s.dw, s.oRes);
   const bool tm = ctx->timing != 0;
   struct Events {                                    // per-stage timing of the steps (vvcb_tu_kernel_times); destroyed on every exit
     cudaEvent_t e[5 * 4] = {};
@@ -1732,44 +1737,31 @@ static int isp_eval_chunk(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_vis
     if (tm && k < 4) CK(cudaEventRecord(ev[5 * k], ctx->stream));
     if (!predList[k].empty()) {
       IspPredParams Q;
-      Q.cands = dCand; Q.list = at<const int>(din, iPred[k]); Q.n = (int)predList[k].size(); Q.k = k;
+      Q.cands = at<const IspCand>(s.din, iCand); Q.list = at<const int>(s.din, iPred[k]); Q.n = (int)predList[k].size(); Q.k = k;
       Q.jobs = dJobs + (size_t)(k < 4 ? k : 3) * n; Q.prev = dRes + (size_t)(k > 0 ? k - 1 : 0) * n; Q.state = dState;
-      Q.pred = dPred; Q.resi = dResi; Q.cuReco = dReco; Q.orig = ctx->bOrig; Q.reco = ctx->bReco; Q.stride = ctx->stride; Q.bd = ctx->bd;
+      Q.pred = at<int16_t>(s.dw, s.oPred); Q.resi = at<int16_t>(s.dw, s.oResi); Q.cuReco = at<int16_t>(s.dw, s.oReco);
+      Q.orig = ctx->bOrig; Q.reco = ctx->bReco; Q.stride = ctx->stride; Q.bd = ctx->bd;
       Q.rom = ctx->dRom; Q.frac = ctx->dRateRom->binFracBits;
       const int g = std::min((Q.n + kIspPredWarps - 1) / kIspPredWarps, ctx->numSms * 8);
       isp_pred_kernel<<<g, kIspPredWarps * 32, 0, ctx->stream>>>(Q);
       ctx->launches++;
     }
     if (k == 4 || L[k].team.empty()) continue;
-    TuChain c = {};
-    c.jobs = dJobs + (size_t)k * n; c.trPair = at<const uint8_t>(din, iTr) + (size_t)k * n;
-    c.team = at<const int>(din, iTeam[k]); c.dq = at<const int>(din, iDq[k]); c.rate = at<const int>(din, iRate[k]);
-    c.resi = dResi; c.pred = dPred; c.level = dLevel; c.reco = dReco; c.deq = at<int32_t>(dw, oDeq); c.results = dRes + (size_t)k * n;
-    c.rates = at<vvcb_dq_rates>(dw, oRates); c.nRates = n; c.priceFrom = dCst;
-    c.states = dCst; c.statesOut = dCst;                             // the block's models adapted in place for the next block
+    TuChain c = s.chain(k);
+    c.trPair = at<const uint8_t>(s.din, iTr) + (size_t)k * n;
+    c.priceFrom = dCst; c.states = dCst; c.statesOut = dCst;       // the block's models adapted in place for the next block
     if ((rc = run_tu_chain(ctx, c, L[k], tm ? ev + 5 * k : nullptr))) return rc;
   }
   CK(cudaGetLastError());
-  // page-locked output staging: per-step results, cbf state, then the wanted sample outputs of the chunk's densely packed candidates
-  Arena out;
-  const size_t hRes = out.take((size_t)4 * n * sizeof(vvcb_tu_result)), hSt = out.take((size_t)n * sizeof(IspState)),
-               hLv = out.take(level ? cs * sizeof(int32_t) : 0), hRc = out.take(reco ? cs * sizeof(int16_t) : 0), hPr = out.take(pred ? cs * sizeof(int16_t) : 0);
-  if ((rc = pin_buf(ctx, kPinStageOut, out.size))) return rc;
-  void* hout = ctx->hPin[kPinStageOut];
-  CK(cudaMemcpyAsync(at<uint8_t>(hout, hRes), dRes, (size_t)4 * n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(at<uint8_t>(hout, hSt), dState, (size_t)n * sizeof(IspState), cudaMemcpyDeviceToHost, ctx->stream));
-  if (level) CK(cudaMemcpyAsync(at<uint8_t>(hout, hLv), dLevel, cs * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (reco) CK(cudaMemcpyAsync(at<uint8_t>(hout, hRc), dReco, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (pred) CK(cudaMemcpyAsync(at<uint8_t>(hout, hPr), dPred, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(ctx_sync(ctx));
+  // outputs: per-step results, cbf state, then the wanted sample outputs
+  Pieces out;
+  const size_t hRes = out.add(dRes, (size_t)4 * n * sizeof(vvcb_tu_result)), hSt = out.add(dState, (size_t)n * sizeof(IspState));
+  s.want(out, level, reco, pred);
+  uint8_t* hout;
+  if ((rc = stage_out(ctx, out, hout))) return rc;
   const vvcb_tu_result* res = at<const vvcb_tu_result>(hout, hRes);
   memcpy(ist.data(), at<IspState>(hout, hSt), (size_t)n * sizeof(IspState));
-  for (int i = 0; i < n; i++) {                      // each candidate's samples to the caller's offset
-    const size_t from = cands[i].offset, to = jobs[i].offset, m = (size_t)cands[i].cuW * cands[i].cuH;
-    if (level) memcpy(level + to, at<const int32_t>(hout, hLv) + from, m * sizeof(int32_t));
-    if (reco) memcpy(reco + to, at<const int16_t>(hout, hRc) + from, m * sizeof(int16_t));
-    if (pred) memcpy(pred + to, at<const int16_t>(hout, hPr) + from, m * sizeof(int16_t));
-  }
+  s.scatter(hout, jobs, level, reco, pred);
   if (tm) {
     for (int k = 0; k < 4; k++) {
       if (L[k].team.empty()) continue;
@@ -1804,13 +1796,9 @@ extern "C" int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_
   if (!ctx->bOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_isp_eval: vvcb_frame_begin has not been called"); return VVCB_ERR_STATE; }
   const int rcv = check_visits(ctx, visits, n_visits);
   if (rcv) return rcv;
-  for (int pass = 0; pass < 2; pass++)                               // every job is validated before anything runs
-    for (int b = 0; b < n; b += kIspChunk) {
-      const int rc = isp_eval_chunk(ctx, visits, n_visits, jobs + b, std::min(kIspChunk, n - b), b, states, n_states, n_samples,
-                                    level, reco, pred, results + b, pass == 0);
-      if (rc) return rc;
-    }
-  return VVCB_OK;
+  return run_chunks(n, [&](int b, int m, bool checkOnly) {
+    return isp_eval_chunk(ctx, visits, n_visits, jobs + b, m, b, states, n_states, n_samples, level, reco, pred, results + b, checkOnly);
+  });
 }
 
 // =====================================================================================================
@@ -1820,7 +1808,7 @@ extern "C" int vvcb_chroma_frame_begin(vvcb_ctx* ctx, const int16_t* cb, const i
 {
   if (!ctx) return VVCB_ERR_ARG;
   REMOTE_UNAVAILABLE("vvcb_chroma_frame_begin");
-  if (!ctx->dOrig || ctx->bOrig != ctx->dOrig) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_frame_begin: vvcb_frame_begin has not been called"); return VVCB_ERR_STATE; }
+  if (!buf(ctx, kOrig) || ctx->bOrig != buf(ctx, kOrig)) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_frame_begin: vvcb_frame_begin has not been called"); return VVCB_ERR_STATE; }
   if (!cb || !cr || cw != ctx->width / 2 || ch != ctx->height / 2 || stride < cw) {
     snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_frame_begin: bad argument (4:2:0 planes of %d x %d)", ctx->width / 2, ctx->height / 2);
     return VVCB_ERR_ARG;
@@ -1828,17 +1816,14 @@ extern "C" int vvcb_chroma_frame_begin(vvcb_ctx* ctx, const int16_t* cb, const i
   CK(cudaSetDevice(ctx->device));
   const int pitch = (cw + 63) & ~63;
   const size_t plane = (size_t)pitch * ch;
-  if (4 * plane > ctx->capChroma) {
-    cudaFree(ctx->dChroma); ctx->dChroma = nullptr; ctx->capChroma = 0;
-    CK(cudaMalloc(&ctx->dChroma, 4 * plane * sizeof(int16_t)));
-    ctx->capChroma = 4 * plane;
-  }
+  int rc;
+  if ((rc = grow(ctx, kChroma, 4 * plane * sizeof(int16_t)))) return rc;
   ctx->cw = cw; ctx->ch = ch; ctx->cstride = pitch;
   const int16_t* src[2] = { cb, cr };
   for (int c = 0; c < 2; c++)
-    CK(cudaMemcpy2DAsync(ctx->dChroma + c * plane, pitch * sizeof(int16_t), src[c], stride * sizeof(int16_t), cw * sizeof(int16_t), ch,
+    CK(cudaMemcpy2DAsync(buf<int16_t>(ctx, kChroma) + c * plane, pitch * sizeof(int16_t), src[c], stride * sizeof(int16_t), cw * sizeof(int16_t), ch,
                          cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemsetAsync(ctx->dChroma + 2 * plane, 0, 2 * plane * sizeof(int16_t), ctx->stream));
+  CK(cudaMemsetAsync(buf<int16_t>(ctx, kChroma) + 2 * plane, 0, 2 * plane * sizeof(int16_t), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
@@ -1856,7 +1841,7 @@ extern "C" int vvcb_chroma_reco_update(vvcb_ctx* ctx, const int16_t* cb, const i
   const size_t plane = (size_t)ctx->cstride * ctx->ch;
   const int16_t* src[2] = { cb, cr };
   for (int c = 0; c < 2; c++)
-    CK(cudaMemcpy2DAsync(ctx->dChroma + (2 + c) * plane + (size_t)y * ctx->cstride + x, ctx->cstride * sizeof(int16_t), src[c],
+    CK(cudaMemcpy2DAsync(buf<int16_t>(ctx, kChroma) + (2 + c) * plane + (size_t)y * ctx->cstride + x, ctx->cstride * sizeof(int16_t), src[c],
                          stride * sizeof(int16_t), w * sizeof(int16_t), h, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
@@ -1899,12 +1884,9 @@ extern "C" int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, 
   Arena ar;
   const size_t oVis = ar.take(sizeof(vvcb_chroma_visit) * n), oRes = ar.take(sizeof(vvcb_chroma_result) * n);
   const size_t oOff = pred_out ? ar.take(sizeof(uint32_t) * n) : 0, oPred = pred_out ? ar.take(sizeof(int16_t) * total) : 0;
-  if (ar.size > ctx->capChromaIo) {
-    cudaFree(ctx->dChromaIo); ctx->dChromaIo = nullptr; ctx->capChromaIo = 0;
-    CK(cudaMalloc(&ctx->dChromaIo, ar.size));
-    ctx->capChromaIo = ar.size;
-  }
-  void* io = ctx->dChromaIo;
+  const int rc = grow(ctx, kChromaIo, ar.size);
+  if (rc) return rc;
+  void* io = buf(ctx, kChromaIo);
   CK(cudaMemcpyAsync(at<void>(io, oVis), visits, sizeof(vvcb_chroma_visit) * n, cudaMemcpyHostToDevice, ctx->stream));
   if (pred_out) {
     CK(cudaMemcpyAsync(at<void>(io, oOff), off.data(), sizeof(uint32_t) * n, cudaMemcpyHostToDevice, ctx->stream));
@@ -1914,7 +1896,8 @@ extern "C" int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, 
   ChromaParams P;
   P.visits = at<const vvcb_chroma_visit>(io, oVis); P.n = n; P.results = at<vvcb_chroma_result>(io, oRes);
   P.predOut = pred_out ? at<int16_t>(io, oPred) : nullptr; P.predOff = pred_out ? at<const uint32_t>(io, oOff) : nullptr;
-  P.orig[0] = ctx->dChroma; P.orig[1] = ctx->dChroma + plane; P.reco[0] = ctx->dChroma + 2 * plane; P.reco[1] = ctx->dChroma + 3 * plane;
+  const int16_t* dChroma = buf<int16_t>(ctx, kChroma);
+  P.orig[0] = dChroma; P.orig[1] = dChroma + plane; P.reco[0] = dChroma + 2 * plane; P.reco[1] = dChroma + 3 * plane;
   P.cstride = ctx->cstride; P.luma = ctx->bReco; P.lstride = ctx->stride; P.bd = ctx->bd; P.ctu = ctx->ctu; P.rom = ctx->dRom;
   const int blocks = std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16);
   chroma_eval_kernel<<<blocks, kChromaWarps * 32, 0, ctx->stream>>>(P);
@@ -1933,18 +1916,14 @@ extern "C" int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, 
 //   chroma_cbf_kernel step 1     Cb's cbf bin, Cr's cbfDeltaBits;
 //   run_tu_chain (Cr jobs)       the same kernels on the Cr plane, the quantiser on the prices of step 0, the rate on the models Cb left;
 //   chroma_cbf_kernel step 2     Cr's cbf bin.
-// One chunk of at most kChromaTuChunk candidates (their TU jobs name the carried snapshots with the 16-bit rate_idx); base: index of the
-// chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
-constexpr int kChromaTuChunk = 65536;
+// One chunk of a staged call (run_chunks); base: index of the chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
 static int chroma_tu_chunk(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_tu_job* jobs, int n, int base,
                            const vvcb_chroma_ctx_states* states, int n_states, size_t n_samples,
                            int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_tu_result* results, bool checkOnly)
 {
-  const unsigned kFlags = VVCB_TU_QUANT | VVCB_TU_DEPQUANT | VVCB_TU_RATE;
   std::vector<vvcb_tu_job> tj((size_t)2 * n);       // [Cb jobs | Cr jobs]
   std::vector<vvcb_chroma_ctx_states> cst(n);
-  std::vector<uint32_t> from(n);
-  size_t cs = 0;                                   // the chunk's own samples: candidates are packed densely on the device, whatever the caller's offsets
+  std::vector<size_t> dense(n + 1, 0);             // the candidates' samples on the device (Staged)
   for (int i = 0; i < n; i++) {
     const vvcb_chroma_tu_job& j = jobs[i];
     auto bad = [&](const char* why) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: job %d: %s", base + i, why); return VVCB_ERR_ARG; };
@@ -1953,116 +1932,75 @@ static int chroma_tu_chunk(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n
     if (j.cand >= VVCB_CHROMA_CANDS) return bad("cand above 7");
     const int code = chroma_cand_code(j.cand, v.dm_mode);
     if (code >= VVCB_LM_CHROMA && code <= VVCB_MDLM_T && !v.cclm) return bad("LM candidate of a visit without cclm");
-    if ((j.flags & ~kFlags) || !(j.flags & VVCB_TU_QUANT)) return bad("flags: VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE] only");
-    for (int c = 0; c < 2; c++)
-      if (j.qp_rem[c] < 0 || j.qp_rem[c] >= 6 || j.qp_per[c] < 0 || 6 * j.qp_per[c] + j.qp_rem[c] > max_qp(ctx->bd)) return bad("qp_per / qp_rem out of range");
-    const bool dq = (j.flags & VVCB_TU_DEPQUANT) != 0, carried = dq || (j.flags & VVCB_TU_RATE);
-    if (carried && (!states || j.rate_idx >= n_states)) return bad("rate_idx does not name a context snapshot");
-    if (dq && (!lambda_ok(j.lambda[0]) || !lambda_ok(j.lambda[1]))) return bad("dependent quantisation needs finite lambdas > 0");
+    if (const char* why = staged_job_error(ctx, j.flags, j.qp_per, j.qp_rem, j.lambda, 2, states && j.rate_idx < n_states)) return bad(why);
+    const bool carried = (j.flags & (VVCB_TU_DEPQUANT | VVCB_TU_RATE)) != 0;
     const size_t m = (size_t)1 << (v.log2w + v.log2h);
     if ((size_t)j.offset + 2 * m > n_samples) return bad("outputs outside n_samples");
     if (carried) cst[i] = states[j.rate_idx]; else memset(&cst[i], 0, sizeof(vvcb_chroma_ctx_states));
-    from[i] = (uint32_t)cs;
     for (int c = 0; c < 2; c++) {
       vvcb_tu_job& t = tj[(size_t)c * n + i];
       memset(&t, 0, sizeof(t));
       t.x = v.x; t.y = v.y; t.log2w = v.log2w; t.log2h = v.log2h;
       t.flags = j.flags; t.qp_per = j.qp_per[c]; t.qp_rem = j.qp_rem[c];
-      t.offset = (uint32_t)(cs + c * m);
+      t.offset = (uint32_t)(dense[i] + c * m);
       t.rate_idx = (uint16_t)i;                        // the candidate's own carried snapshot
       t.lambda = j.lambda[c];
     }
-    cs += 2 * m;
+    dense[i + 1] = dense[i] + 2 * m;
   }
   if (checkOnly) return VVCB_OK;
   TuLists L[2];
   for (int c = 0; c < 2; c++) L[c] = tu_lists(&tj[(size_t)c * n], n, [](int) { return true; });
-  // one input arena in page-locked memory: visits, candidates, TU jobs, carried models, lists
-  Arena in;
-  const size_t iVis = in.take((size_t)n_visits * sizeof(vvcb_chroma_visit)), iJob = in.take((size_t)n * sizeof(vvcb_chroma_tu_job)),
-               iTj = in.take(tj.size() * sizeof(vvcb_tu_job)), iCst = in.take((size_t)n * sizeof(vvcb_chroma_ctx_states));
-  size_t iTeam[2], iDq[2], iRate[2];
-  for (int c = 0; c < 2; c++) { iTeam[c] = in.take(L[c].team.size() * sizeof(int)); iDq[c] = in.take(L[c].dq.size() * sizeof(int)); iRate[c] = in.take(L[c].rate.size() * sizeof(int)); }
-  int rc;
-  if ((rc = pin_buf(ctx, kPinStageIn, in.size))) return rc;
-  void* hin = ctx->hPin[kPinStageIn];
-  memcpy(at<vvcb_chroma_visit>(hin, iVis), visits, (size_t)n_visits * sizeof(vvcb_chroma_visit));
-  memcpy(at<vvcb_chroma_tu_job>(hin, iJob), jobs, (size_t)n * sizeof(vvcb_chroma_tu_job));
-  memcpy(at<vvcb_tu_job>(hin, iTj), tj.data(), tj.size() * sizeof(vvcb_tu_job));
-  memcpy(at<vvcb_chroma_ctx_states>(hin, iCst), cst.data(), (size_t)n * sizeof(vvcb_chroma_ctx_states));
-  auto put = [&](size_t o, const std::vector<int>& v) { if (!v.empty()) memcpy(at<int>(hin, o), v.data(), v.size() * sizeof(int)); };
-  for (int c = 0; c < 2; c++) { put(iTeam[c], L[c].team); put(iDq[c], L[c].dq); put(iRate[c], L[c].rate); }
-  // work arena: TU results, prediction, residual, reconstruction, levels, dequantised coefficients, derived prices, cbf flags and bits
-  Arena work;
-  const size_t oRes = work.take((size_t)2 * n * sizeof(vvcb_tu_result)), oPred = work.take(cs * sizeof(int16_t)), oResi = work.take(cs * sizeof(int16_t)),
-               oReco = work.take(cs * sizeof(int16_t)), oLevel = work.take(cs * sizeof(int32_t)), oDeq = work.take(cs * sizeof(int32_t)),
-               oRates = work.take((size_t)n * sizeof(vvcb_dq_rates)), oCbf = work.take((size_t)2 * n), oCbfBits = work.take((size_t)2 * n * sizeof(uint32_t));
-  const int nDq[2] = { (int)L[0].dq.size(), (int)L[1].dq.size() };
+  // inputs: visits, candidates, TU jobs, carried models; work: the cbf flags and bits of both components after the common arrays
+  Staged s(n, 2, dense);
+  const size_t iVis = s.in.add(visits, (size_t)n_visits * sizeof(vvcb_chroma_visit)), iJob = s.in.add(jobs, (size_t)n * sizeof(vvcb_chroma_tu_job)),
+               iTj = s.in.add(tj), iCst = s.in.add(cst);
+  const size_t oCbf = s.work.take((size_t)2 * n), oCbfBits = s.work.take((size_t)2 * n * sizeof(uint32_t));
   CK(cudaSetDevice(ctx->device));
-  if ((rc = tu_buf(ctx, kStageIn, in.size))) return rc;
-  if ((rc = tu_buf(ctx, kStageOut, work.size))) return rc;
-  if ((rc = quant_scratch(ctx, cs, n, nDq, 2))) return rc;
-  void* din = ctx->dTu[kStageIn];
-  void* dw = ctx->dTu[kStageOut];
-  CK(cudaMemcpyAsync(din, hin, in.size, cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemsetAsync(at<uint8_t>(dw, oLevel), 0, oRates - oLevel, ctx->stream));        // levels / dequantised coefficients the quantisers do not reach stay zero
-  CK(cudaMemsetAsync(at<uint8_t>(dw, oCbf), 0, work.size - oCbf, ctx->stream));
-  vvcb_tu_job* dTj = at<vvcb_tu_job>(din, iTj);
-  vvcb_chroma_ctx_states* dCst = at<vvcb_chroma_ctx_states>(din, iCst);
-  vvcb_tu_result* dRes = at<vvcb_tu_result>(dw, oRes);
-  int16_t* dPred = at<int16_t>(dw, oPred); int16_t* dResi = at<int16_t>(dw, oResi);
-  int16_t* dReco = at<int16_t>(dw, oReco); int32_t* dLevel = at<int32_t>(dw, oLevel);
-  uint8_t* dCbf = at<uint8_t>(dw, oCbf); uint32_t* dCbfBits = at<uint32_t>(dw, oCbfBits);
+  int rc;
+  if ((rc = s.begin(ctx, iTj, L))) return rc;
+  CK(cudaMemsetAsync(s.dw + oCbf, 0, s.work.size - oCbf, ctx->stream));
+  vvcb_tu_job* dTj = at<vvcb_tu_job>(s.din, iTj);
+  vvcb_chroma_ctx_states* dCst = at<vvcb_chroma_ctx_states>(s.din, iCst);
+  uint8_t* dCbf = s.dw + oCbf; uint32_t* dCbfBits = at<uint32_t>(s.dw, oCbfBits);
+  const int16_t* dChroma = buf<int16_t>(ctx, kChroma);
   const size_t plane = (size_t)ctx->cstride * ctx->ch;
   {
     ChromaTuPredParams Q = {};
     ChromaParams& B = Q.planes;
-    B.visits = at<const vvcb_chroma_visit>(din, iVis); B.n = n_visits;
-    B.orig[0] = ctx->dChroma; B.orig[1] = ctx->dChroma + plane; B.reco[0] = ctx->dChroma + 2 * plane; B.reco[1] = ctx->dChroma + 3 * plane;
+    B.visits = at<const vvcb_chroma_visit>(s.din, iVis); B.n = n_visits;
+    B.orig[0] = dChroma; B.orig[1] = dChroma + plane; B.reco[0] = dChroma + 2 * plane; B.reco[1] = dChroma + 3 * plane;
     B.cstride = ctx->cstride; B.luma = ctx->bReco; B.lstride = ctx->stride; B.bd = ctx->bd; B.ctu = ctx->ctu; B.rom = ctx->dRom;
-    Q.jobs = at<const vvcb_chroma_tu_job>(din, iJob); Q.n = n; Q.cbJobs = dTj; Q.states = dCst;
-    Q.pred = dPred; Q.resi = dResi; Q.frac = ctx->dRateRom->binFracBits;
+    Q.jobs = at<const vvcb_chroma_tu_job>(s.din, iJob); Q.n = n; Q.cbJobs = dTj; Q.states = dCst;
+    Q.pred = at<int16_t>(s.dw, s.oPred); Q.resi = at<int16_t>(s.dw, s.oResi); Q.frac = ctx->dRateRom->binFracBits;
     chroma_tu_pred_kernel<<<std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16), kChromaWarps * 32, 0, ctx->stream>>>(Q);
     ctx->launches++;
   }
   for (int c = 0; c < 2; c++) {
-    TuChain t = {};
-    t.jobs = dTj + (size_t)c * n;
-    t.team = at<const int>(din, iTeam[c]); t.dq = at<const int>(din, iDq[c]); t.rate = at<const int>(din, iRate[c]);
-    t.resi = dResi; t.pred = dPred; t.level = dLevel; t.reco = dReco; t.deq = at<int32_t>(dw, oDeq); t.results = dRes + (size_t)c * n;
-    t.rates = at<vvcb_dq_rates>(dw, oRates); t.nRates = n;
+    TuChain t = s.chain(c);
     t.priceFrom = c == 0 ? reinterpret_cast<const vvcb_ctx_states*>(dCst) : nullptr;      // both quantisers on the starting models
     t.states = reinterpret_cast<const vvcb_ctx_states*>(dCst); t.statesOut = reinterpret_cast<vvcb_ctx_states*>(dCst);
-    t.chroma = true; t.orig = ctx->dChroma + c * plane; t.stride = ctx->cstride;
+    t.chroma = true; t.orig = dChroma + c * plane; t.stride = ctx->cstride;
     if ((rc = run_tu_chain(ctx, t, L[c], nullptr))) return rc;
     ChromaCbfParams F;
-    F.n = n; F.step = c + 1; F.res = dRes + (size_t)c * n; F.crJobs = dTj + n; F.states = dCst; F.cbf = dCbf; F.cbfBits = dCbfBits;
+    F.n = n; F.step = c + 1; F.res = t.results; F.crJobs = dTj + n; F.states = dCst; F.cbf = dCbf; F.cbfBits = dCbfBits;
     F.frac = ctx->dRateRom->binFracBits;
     chroma_cbf_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(F);
     ctx->launches++;
   }
   CK(cudaGetLastError());
-  // page-locked output staging: TU results, cbf flags and bits, then the wanted sample outputs of the chunk's densely packed candidates
-  Arena out;
-  const size_t hRes = out.take((size_t)2 * n * sizeof(vvcb_tu_result)), hCbf = out.take((size_t)2 * n), hBits = out.take((size_t)2 * n * sizeof(uint32_t)),
-               hLv = out.take(level ? cs * sizeof(int32_t) : 0), hRc = out.take(reco ? cs * sizeof(int16_t) : 0), hPr = out.take(pred ? cs * sizeof(int16_t) : 0);
-  if ((rc = pin_buf(ctx, kPinStageOut, out.size))) return rc;
-  void* hout = ctx->hPin[kPinStageOut];
-  CK(cudaMemcpyAsync(at<uint8_t>(hout, hRes), dRes, (size_t)2 * n * sizeof(vvcb_tu_result), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(at<uint8_t>(hout, hCbf), dCbf, (size_t)2 * n, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(at<uint8_t>(hout, hBits), dCbfBits, (size_t)2 * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (level) CK(cudaMemcpyAsync(at<uint8_t>(hout, hLv), dLevel, cs * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (reco) CK(cudaMemcpyAsync(at<uint8_t>(hout, hRc), dReco, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-  if (pred) CK(cudaMemcpyAsync(at<uint8_t>(hout, hPr), dPred, cs * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(ctx_sync(ctx));
+  // outputs: TU results, cbf flags and bits, then the wanted sample outputs
+  Pieces out;
+  const size_t hRes = out.add(s.dw + s.oRes, (size_t)2 * n * sizeof(vvcb_tu_result)), hCbf = out.add(dCbf, (size_t)2 * n),
+               hBits = out.add(dCbfBits, (size_t)2 * n * sizeof(uint32_t));
+  s.want(out, level, reco, pred);
+  uint8_t* hout;
+  if ((rc = stage_out(ctx, out, hout))) return rc;
   const vvcb_tu_result* res = at<const vvcb_tu_result>(hout, hRes);
-  const uint8_t* cbf = at<const uint8_t>(hout, hCbf);
+  const uint8_t* cbf = hout + hCbf;
   const uint32_t* bits = at<const uint32_t>(hout, hBits);
+  s.scatter(hout, jobs, level, reco, pred);
   for (int i = 0; i < n; i++) {
-    const size_t m = (size_t)2 << (visits[jobs[i].visit].log2w + visits[jobs[i].visit].log2h), to = jobs[i].offset;
-    if (level) memcpy(level + to, at<const int32_t>(hout, hLv) + from[i], m * sizeof(int32_t));
-    if (reco) memcpy(reco + to, at<const int16_t>(hout, hRc) + from[i], m * sizeof(int16_t));
-    if (pred) memcpy(pred + to, at<const int16_t>(hout, hPr) + from[i], m * sizeof(int16_t));
     vvcb_chroma_tu_result& r = results[i];
     memset(&r, 0, sizeof(r));
     const bool rate = (jobs[i].flags & VVCB_TU_RATE) != 0;
@@ -2092,23 +2030,9 @@ extern "C" int vvcb_chroma_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visit
   if (n == 0) return VVCB_OK;
   for (int i = 0; i < n_visits; i++)
     if (const char* why = chroma_visit_error(ctx, visits[i])) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: visit %d: %s", i, why); return VVCB_ERR_ARG; }
-  for (int pass = 0; pass < 2; pass++)                               // every job is validated before anything runs
-    for (int b = 0; b < n; b += kChromaTuChunk) {
-      const int rc = chroma_tu_chunk(ctx, visits, n_visits, jobs + b, std::min(kChromaTuChunk, n - b), b, states, n_states, n_samples,
-                                     level, reco, pred, results + b, pass == 0);
-      if (rc) return rc;
-    }
-  return VVCB_OK;
-}
-
-static int feat_buf(vvcb_ctx* ctx, int i, size_t bytes)
-{
-  if (bytes > ctx->capFeat[i]) {
-    cudaFree(ctx->dFeat[i]); ctx->dFeat[i] = nullptr; ctx->capFeat[i] = 0;
-    CK(cudaMalloc(&ctx->dFeat[i], bytes));
-    ctx->capFeat[i] = bytes;
-  }
-  return VVCB_OK;
+  return run_chunks(n, [&](int b, int m, bool checkOnly) {
+    return chroma_tu_chunk(ctx, visits, n_visits, jobs + b, m, b, states, n_states, n_samples, level, reco, pred, results + b, checkOnly);
+  });
 }
 
 extern "C" int vvcb_ctu_hads_islice(vvcb_ctx* ctx, int32_t* out, int n_ctus)
@@ -2120,8 +2044,8 @@ extern "C" int vvcb_ctu_hads_islice(vvcb_ctx* ctx, int32_t* out, int n_ctus)
   if (!out || n_ctus != perRow * rows) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_ctu_hads_islice: the frame has %d CTUs", perRow * rows); return VVCB_ERR_ARG; }
   CK(cudaSetDevice(ctx->device));
   int rc;
-  if ((rc = feat_buf(ctx, 0, (size_t)n_ctus * sizeof(int32_t)))) return rc;
-  int32_t* d = static_cast<int32_t*>(ctx->dFeat[0]);
+  if ((rc = grow(ctx, kFeatIn, (size_t)n_ctus * sizeof(int32_t)))) return rc;
+  int32_t* d = buf<int32_t>(ctx, kFeatIn);
   CK(cudaMemsetAsync(d, 0, (size_t)n_ctus * sizeof(int32_t), ctx->stream));
   const int blocks = (ctx->width >> 3) * (ctx->height >> 3);
   if (blocks > 0) {
@@ -2154,17 +2078,16 @@ extern "C" int vvcb_features_eval(vvcb_ctx* ctx, const vvcb_feat_job* jobs, int 
   }
   CK(cudaSetDevice(ctx->device));
   int rc;
-  if ((rc = feat_buf(ctx, 0, (size_t)n * sizeof(vvcb_feat_job)))) return rc;
-  if ((rc = feat_buf(ctx, 1, (size_t)n * sizeof(vvcb_feat_result)))) return rc;
-  CK(cudaMemcpyAsync(ctx->dFeat[0], jobs, (size_t)n * sizeof(vvcb_feat_job), cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = grow(ctx, kFeatIn, (size_t)n * sizeof(vvcb_feat_job))) || (rc = grow(ctx, kFeatOut, (size_t)n * sizeof(vvcb_feat_result)))) return rc;
+  CK(cudaMemcpyAsync(buf(ctx, kFeatIn), jobs, (size_t)n * sizeof(vvcb_feat_job), cudaMemcpyHostToDevice, ctx->stream));
   FeatParams P;
-  P.jobs = static_cast<const vvcb_feat_job*>(ctx->dFeat[0]); P.n = n; P.results = static_cast<vvcb_feat_result*>(ctx->dFeat[1]);
+  P.jobs = buf<const vvcb_feat_job>(ctx, kFeatIn); P.n = n; P.results = buf<vvcb_feat_result>(ctx, kFeatOut);
   P.orig = ctx->bOrig; P.stride = ctx->stride;
   const int grid = n < ctx->numSms * 16 ? n : ctx->numSms * 16;
   features_kernel<<<grid, kFeatThreads, 0, ctx->stream>>>(P);
   ctx->launches++;
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(results, ctx->dFeat[1], (size_t)n * sizeof(vvcb_feat_result), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(results, buf(ctx, kFeatOut), (size_t)n * sizeof(vvcb_feat_result), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return VVCB_OK;
 }
@@ -2172,6 +2095,7 @@ extern "C" int vvcb_features_eval(vvcb_ctx* ctx, const vvcb_feat_job* jobs, int 
 extern "C" int vvcb_dev_alloc(vvcb_ctx* ctx, size_t bytes, void** out)
 {
   if (!ctx || !out) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_dev_alloc");
   CK(cudaSetDevice(ctx->device));
   CK(cudaMalloc(out, bytes));
   return VVCB_OK;
@@ -2180,7 +2104,6 @@ extern "C" int vvcb_dev_free(vvcb_ctx* ctx, void* p)
 {
   if (!ctx) return VVCB_ERR_ARG;
   REMOTE_UNAVAILABLE("vvcb_dev_free");
-  REMOTE_UNAVAILABLE("vvcb_dev_alloc");
   CK(cudaSetDevice(ctx->device));
   CK(cudaFree(p));
   return VVCB_OK;
@@ -2188,6 +2111,7 @@ extern "C" int vvcb_dev_free(vvcb_ctx* ctx, void* p)
 extern "C" int vvcb_host_alloc(vvcb_ctx* ctx, size_t bytes, void** out)
 {
   if (!ctx || !out) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_host_alloc");
   CK(cudaSetDevice(ctx->device));
   CK(cudaHostAlloc(out, bytes, cudaHostAllocDefault));
   return VVCB_OK;
@@ -2196,7 +2120,6 @@ extern "C" int vvcb_host_free(vvcb_ctx* ctx, void* p)
 {
   if (!ctx) return VVCB_ERR_ARG;
   REMOTE_UNAVAILABLE("vvcb_host_free");
-  REMOTE_UNAVAILABLE("vvcb_host_alloc");
   CK(cudaFreeHost(p));
   return VVCB_OK;
 }
@@ -2237,6 +2160,7 @@ extern "C" int vvcb_timer_start(vvcb_ctx* ctx)
 extern "C" int vvcb_timer_stop(vvcb_ctx* ctx, float* ms)
 {
   if (!ctx || !ms) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_timer_stop");
   CK(cudaSetDevice(ctx->device));
   CK(cudaEventRecord(ctx->ev1, ctx->stream));
   CK(cudaEventSynchronize(ctx->ev1));
@@ -2247,7 +2171,6 @@ extern "C" int vvcb_measure_int_peak(vvcb_ctx* ctx, double* gops_imad, double* g
 {
   if (!ctx) return VVCB_ERR_ARG;
   REMOTE_UNAVAILABLE("vvcb_measure_int_peak");
-  REMOTE_UNAVAILABLE("vvcb_timer_stop");
   CK(cudaSetDevice(ctx->device));
   const int grid = ctx->numSms * 8, iters = 4096;
   int *dIn = nullptr, *dOut = nullptr;
