@@ -450,7 +450,8 @@ int vvcb_isp_eval(vvcb_ctx* ctx, const vvcb_rmd_visit* visits, int n_visits, con
  * modes (CL/IntraPrediction.cpp:1665-2150: xGetLumaRecPixels with the [1 2 1; 1 2 1] / 8 down-sampling of sps_cclm_colocated_chroma
  * = 0, xGetLMParameters, predIntraChromaLM) -- and measured with RdCost::xGetSAD / xGetHADs on the chroma block.  No ordering or
  * pruning of the candidates: that is the caller's.  vvcb_chroma_tu_eval (below) codes the TUs of these candidates, Cb and Cr
- * separately with DCT-II; joint Cb-Cr, chroma transform skip and the chroma QP mapping are not in the library.
+ * separately with DCT-II, and vvcb_chroma_joint_tu_eval their joint Cb-Cr tries; chroma transform skip and the chroma QP mapping are
+ * not in the library.
  * Restated from H.266 and the cited reference lines; not compared with the reference encoder's own chroma output.                   */
 #define VVCB_CHROMA_CANDS 8
 #define VVCB_LM_CHROMA   67   /* LM_CHROMA_IDX: CCLM from the above and left neighbours */
@@ -510,8 +511,8 @@ int vvcb_chroma_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n, int1
  *     (context 0), tu_cr_coded_flag (context = Cb's cbf), residual_coding of Cb, residual_coding of Cr (priced on the models Cb's
  *     residual left); each bin priced, then its model adapted.  Sign hiding is not modelled (as for luma).
  * Restated from H.266 and the cited reference lines, as the ISP and chroma-prediction entries are: parity with the reference encoder's
- * own chroma coding is unpinned.  NOT in the library: joint Cb-Cr, chroma transform skip (its transform_skip_flag bin has contexts of
- * its own and stays with the caller), LFNST for chroma, the chroma QP mapping (the caller passes QpParam per component, its mapping
+ * own chroma coding is unpinned.  Joint Cb-Cr candidates are coded by vvcb_chroma_joint_tu_eval (below).  NOT in the library: chroma
+ * transform skip (its transform_skip_flag bin has contexts of its own and stays with the caller), LFNST for chroma, the chroma QP mapping (the caller passes QpParam per component, its mapping
  * table and offsets applied), chroma distortion weighting (the caller applies m_distortionWeight to sse), 2xN blocks, 4:2:2 / 4:4:4,
  * ISP-coupled chroma.                                                                                                              */
 typedef struct vvcb_chroma_ctx_states {   /* the estimator's chroma models at the start of the chroma TU (as vvcb_ctx_states)       */
@@ -543,6 +544,60 @@ typedef struct vvcb_chroma_tu_result {
 int vvcb_chroma_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_tu_job* jobs, int n,
                         const vvcb_chroma_ctx_states* states, int n_states, size_t n_samples,
                         int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_tu_result* results);
+
+/* ---- joint Cb-Cr coding of the candidates (4:2:0, separate tree, one coded residual for both components) -----------------------
+ * The joint Cb-Cr tries of xRecurIntraChromaCodingQT for a TU that covers its chroma CU: one residual stands for Cb and Cr under
+ * TuCResMode `mode` (H.266 7.4.11.10, 8.7.2) -- 1: tu_cb_coded_flag 1, tu_cr_coded_flag 0; 2: both 1; 3: tu_cb_coded_flag 0,
+ * tu_cr_coded_flag 1 -- and CSign = `sign` = 1 - 2 * slice_joint_cbcr_sign_flag.  A job is one chroma CU, one of its 8 candidates,
+ * mode, sign and one quantiser setting (one QP, one lambda):
+ *   - prediction of Cb and Cr: exactly what vvcb_chroma_eval predicts for (visit, cand); resCb / resCr = original - prediction;
+ *   - forward combination into the coded residual.  H.266 does not specify it; this is the library's restatement of the encoder
+ *     derivation of JVET-O0105 (C division, truncating toward zero), and parity with the reference encoder's own is unpinned:
+ *     mode 2: (resCb + CSign * resCr) / 2;  mode 1: (4 * resCb + 2 * CSign * resCr) / 5;  mode 3: (4 * resCr + 2 * CSign * resCb) / 5.
+ *     It decides only which levels are chosen, never whether the reconstruction of given levels is right;
+ *   - DCT-II, Quant::quant or DepQuant::quant on the chroma contexts, dequantiser and inverse transform of that one residual, as
+ *     vvcb_chroma_tu_eval codes Cb.  cbfDeltaBits belong to the coded component (the reading of RateEstimator::xSetLastCoeffOffset
+ *     cited above): Ctx::QtCbf[Cb](0) for modes 1 and 2, Ctx::QtCbf[Cr](0) for mode 3, where tu_cb_coded_flag is 0;
+ *   - inverse mapping (normative, H.266 8.7.2), in int, with r the inverse-transformed residual after its 16-bit clip:
+ *     mode 1: resCb = r, resCr = (CSign * r) >> 1;  mode 2: resCb = r, resCr = CSign * r;  mode 3: resCr = r, resCb = (CSign * r) >> 1;
+ *     then Clip1(prediction + residual) of both components and their unweighted RdCost::xGetSSE;
+ *   - with VVCB_TU_RATE: the chroma bins of transform_unit in coding order on ONE carried copy of states[rate_idx], each priced, then
+ *     adapted -- tu_cb_coded_flag (context 0), tu_cr_coded_flag (context = tu_cb_coded_flag), tu_joint_cbcr_residual_flag = 1
+ *     (context 2 * tu_cb_coded_flag + tu_cr_coded_flag - 1), residual_coding of the coded residual on the chroma contexts.
+ * A coded residual whose levels are all zero is not a joint candidate (the syntax cannot code it): cbf = 0, the reconstruction and sse of
+ * the zero residual, no bins priced; the caller discards it.  The chroma QP mapping with the joint QP offsets, the distortion weights
+ * and the choice of modes and slice sign stay with the caller.  Restated from H.266 and the cited lines; parity unpinned.          */
+typedef struct vvcb_chroma_joint_ctx_states {
+  vvcb_chroma_ctx_states chroma;         /* the models of vvcb_chroma_tu_eval                                                      */
+  vvcb_bin_model joint[3];               /* Ctx::JointCbCrFlag                                                                     */
+} vvcb_chroma_joint_ctx_states;          /* 73 models, 438 bytes */
+typedef struct vvcb_chroma_joint_tu_job {
+  uint32_t visit;              /* index into visits[]                                                                            */
+  uint8_t  cand;               /* 0..7, as vvcb_chroma_tu_job::cand                                                              */
+  uint8_t  flags;              /* VVCB_TU_QUANT [| VVCB_TU_DEPQUANT] [| VVCB_TU_RATE]                                            */
+  uint16_t rate_idx;           /* states[rate_idx]: the models at the start of the candidate (DEPQUANT or RATE)                  */
+  uint8_t  mode;               /* TuCResMode 1..3                                                                                */
+  int8_t   sign;               /* CSign: +1 or -1                                                                                */
+  int16_t  qp_per, qp_rem;     /* QpParam of the joint residual: the caller's chroma QP mapping and joint offsets applied        */
+  uint16_t pad;
+  uint32_t offset;             /* first sample of this candidate's outputs: Cb w*h, then Cr w*h                                  */
+  uint32_t pad2;
+  double   lambda;             /* Quant::m_dLambda while the joint residual is quantised (DEPQUANT)                              */
+} vvcb_chroma_joint_tu_job;    /* 32 bytes */
+typedef struct vvcb_chroma_joint_tu_result {
+  vvcb_tu_result res;          /* the coded residual: abs sums, residual frac_bits (VVCB_TU_RATE, 0 without a level); sse unused (0) */
+  uint64_t sse[2];             /* Cb, Cr: unweighted sse of the reconstructions                                                  */
+  uint32_t cbf_bits[2];        /* VVCB_TU_RATE: fractional bits of tu_cb_coded_flag / tu_cr_coded_flag                           */
+  uint32_t joint_bits;         /* VVCB_TU_RATE: fractional bits of tu_joint_cbcr_residual_flag                                   */
+  uint8_t  cbf, pad[3];        /* 1: the coded residual has a level; 0: not a joint candidate                                    */
+} vvcb_chroma_joint_tu_result; /* 56 bytes */
+/* visits, jobs, states: HOST arrays (n_visits, n, n_states; states may be NULL when no job has DEPQUANT or RATE).  level / reco / pred:
+ * optional HOST outputs of n_samples, per candidate 2 * w*h at its offset: level the coded residual's levels, then w*h zeros; reco and
+ * pred Cb, then Cr.  VVCB_ERR_ARG for everything vvcb_chroma_tu_eval refuses and for mode outside 1..3 or sign other than +1 / -1;
+ * VVCB_ERR_STATE before vvcb_chroma_frame_begin and through the broker.                                                            */
+int vvcb_chroma_joint_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_joint_tu_job* jobs, int n,
+                              const vvcb_chroma_joint_ctx_states* states, int n_states, size_t n_samples,
+                              int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_joint_tu_result* results);
 
 /* ---- texture features (orig-only, trivially parallel) ------------------------------------------------------------
  * vvcb_ctu_hads_islice: EncCu::updateCtuDataISlice (EL/EncCu.cpp:564-675) for every CTU of the frame, as

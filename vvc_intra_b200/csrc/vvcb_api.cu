@@ -990,6 +990,7 @@ struct TuChain {
   // point at vvcb_chroma_ctx_states
   bool chroma;
   const int16_t* orig; int stride;                                  // the original plane the jobs' x / y address; nullptr: the luma plane
+  bool resiOut;                                                     // reco receives the inverse-transformed residual, no SSE (joint Cb-Cr)
 };
 
 // Launches one TU batch: tu_eval_kernel pass 0 in its two team sizes, the dependent quantiser and / or transform-skip RDOQ, pass 1 for
@@ -1002,8 +1003,20 @@ static int run_tu_chain(vvcb_ctx* ctx, const TuChain& c, const TuLists& L, const
   P.results = c.results; P.orig = c.orig ? c.orig : ctx->bOrig; P.stride = c.orig ? c.stride : ctx->stride; P.bd = ctx->bd; P.rom = ctx->dTrRom;
   P.dqCoeff = buf<int32_t>(ctx, kDqCoeff); P.dqDeq = c.deq; P.phase = 0; P.trPair = c.trPair;
   auto launch_tu = [&](TuParams Q) {
-    if (nSmall) { Q.list = c.team; Q.n = nSmall; tu_eval_kernel<32><<<std::min((nSmall + 3) / 4, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
-    if (nLarge) { Q.list = c.team + nSmall; Q.n = nLarge; tu_eval_kernel<128><<<std::min(nLarge, ctx->numSms * 8), kTuThreads, 0, ctx->stream>>>(Q); ctx->launches++; }
+    if (nSmall) {
+      Q.list = c.team; Q.n = nSmall;
+      const int g = std::min((nSmall + 3) / 4, ctx->numSms * 8);
+      if (c.resiOut) tu_eval_kernel<32, true><<<g, kTuThreads, 0, ctx->stream>>>(Q);
+      else tu_eval_kernel<32><<<g, kTuThreads, 0, ctx->stream>>>(Q);
+      ctx->launches++;
+    }
+    if (nLarge) {
+      Q.list = c.team + nSmall; Q.n = nLarge;
+      const int g = std::min(nLarge, ctx->numSms * 8);
+      if (c.resiOut) tu_eval_kernel<128, true><<<g, kTuThreads, 0, ctx->stream>>>(Q);
+      else tu_eval_kernel<128><<<g, kTuThreads, 0, ctx->stream>>>(Q);
+      ctx->launches++;
+    }
   };
   launch_tu(P);
   if (ev) CK(cudaEventRecord(ev[1], ctx->stream));
@@ -1973,7 +1986,7 @@ static int chroma_tu_chunk(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n
     B.cstride = ctx->cstride; B.luma = ctx->bReco; B.lstride = ctx->stride; B.bd = ctx->bd; B.ctu = ctx->ctu; B.rom = ctx->dRom;
     Q.jobs = at<const vvcb_chroma_tu_job>(s.din, iJob); Q.n = n; Q.cbJobs = dTj; Q.states = dCst;
     Q.pred = at<int16_t>(s.dw, s.oPred); Q.resi = at<int16_t>(s.dw, s.oResi); Q.frac = ctx->dRateRom->binFracBits;
-    chroma_tu_pred_kernel<<<std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16), kChromaWarps * 32, 0, ctx->stream>>>(Q);
+    chroma_tu_pred_kernel<false><<<std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16), kChromaWarps * 32, 0, ctx->stream>>>(Q);
     ctx->launches++;
   }
   for (int c = 0; c < 2; c++) {
@@ -2032,6 +2045,138 @@ extern "C" int vvcb_chroma_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visit
     if (const char* why = chroma_visit_error(ctx, visits[i])) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_tu_eval: visit %d: %s", i, why); return VVCB_ERR_ARG; }
   return run_chunks(n, [&](int b, int m, bool checkOnly) {
     return chroma_tu_chunk(ctx, visits, n_visits, jobs + b, m, b, states, n_states, n_samples, level, reco, pred, results + b, checkOnly);
+  });
+}
+
+// Joint Cb-Cr candidates (include/vvc_intra_b200.h): one step over the TU kernels, one coded residual per candidate.
+//   chroma_tu_pred_kernel<true>  both predictions, the combined residual, the coded component's cbfDeltaBits;
+//   run_tu_chain (resi)          pass 0, the dependent quantiser priced by chroma_rates_from_states_kernel from the candidates' starting
+//                                models, pass 1 leaving the inverse-transformed residual, rate_kernel_chroma on the carried models;
+//   chroma_joint_kernel          inverse mapping, both reconstructions and SSEs, the cbf and joint-flag bins.
+// One chunk of a staged call (run_chunks); base: index of the chunk's first job in the caller's batch.  checkOnly: validate, launch nothing.
+static int chroma_joint_tu_chunk(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_joint_tu_job* jobs, int n,
+                                 int base, const vvcb_chroma_joint_ctx_states* states, int n_states, size_t n_samples,
+                                 int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_joint_tu_result* results, bool checkOnly)
+{
+  std::vector<vvcb_tu_job> tj(n);
+  std::vector<vvcb_chroma_ctx_states> cst(n);
+  std::vector<vvcb_bin_model> jm((size_t)3 * n);
+  std::vector<size_t> dense(n + 1, 0);             // the candidates' samples on the device (Staged)
+  for (int i = 0; i < n; i++) {
+    const vvcb_chroma_joint_tu_job& j = jobs[i];
+    auto bad = [&](const char* why) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_joint_tu_eval: job %d: %s", base + i, why); return VVCB_ERR_ARG; };
+    if (j.visit >= (uint32_t)n_visits) return bad("visit index out of range");
+    const vvcb_chroma_visit& v = visits[j.visit];
+    if (j.cand >= VVCB_CHROMA_CANDS) return bad("cand above 7");
+    const int code = chroma_cand_code(j.cand, v.dm_mode);
+    if (code >= VVCB_LM_CHROMA && code <= VVCB_MDLM_T && !v.cclm) return bad("LM candidate of a visit without cclm");
+    if (j.mode < 1 || j.mode > 3) return bad("mode: TuCResMode 1..3 only");
+    if (j.sign != 1 && j.sign != -1) return bad("sign: +1 or -1 only");
+    if (const char* why = staged_job_error(ctx, j.flags, &j.qp_per, &j.qp_rem, &j.lambda, 1, states && j.rate_idx < n_states)) return bad(why);
+    const bool carried = (j.flags & (VVCB_TU_DEPQUANT | VVCB_TU_RATE)) != 0;
+    const size_t m = (size_t)1 << (v.log2w + v.log2h);
+    if ((size_t)j.offset + 2 * m > n_samples) return bad("outputs outside n_samples");
+    if (carried) {
+      cst[i] = states[j.rate_idx].chroma;
+      memcpy(&jm[(size_t)3 * i], states[j.rate_idx].joint, 3 * sizeof(vvcb_bin_model));
+    } else {
+      memset(&cst[i], 0, sizeof(vvcb_chroma_ctx_states));
+      memset(&jm[(size_t)3 * i], 0, 3 * sizeof(vvcb_bin_model));
+    }
+    vvcb_tu_job& t = tj[i];
+    memset(&t, 0, sizeof(t));
+    t.x = v.x; t.y = v.y; t.log2w = v.log2w; t.log2h = v.log2h;
+    t.flags = j.flags; t.qp_per = j.qp_per; t.qp_rem = j.qp_rem;
+    t.offset = (uint32_t)dense[i];
+    t.rate_idx = (uint16_t)i;                        // the candidate's own carried snapshot
+    t.lambda = j.lambda;
+    dense[i + 1] = dense[i] + 2 * m;
+  }
+  if (checkOnly) return VVCB_OK;
+  TuLists L = tu_lists(tj.data(), n, [](int) { return true; });
+  // inputs: visits, candidates, TU jobs, carried models; work: the SSEs, cbf flags and bits after the common arrays
+  Staged s(n, 1, dense);
+  const size_t iVis = s.in.add(visits, (size_t)n_visits * sizeof(vvcb_chroma_visit)), iJob = s.in.add(jobs, (size_t)n * sizeof(vvcb_chroma_joint_tu_job)),
+               iTj = s.in.add(tj), iCst = s.in.add(cst), iJm = s.in.add(jm);
+  const size_t oSse = s.work.take((size_t)2 * n * sizeof(uint64_t)), oBits = s.work.take((size_t)3 * n * sizeof(uint32_t)), oCbf = s.work.take((size_t)n);
+  CK(cudaSetDevice(ctx->device));
+  int rc;
+  if ((rc = s.begin(ctx, iTj, &L))) return rc;
+  CK(cudaMemsetAsync(s.dw + oSse, 0, s.work.size - oSse, ctx->stream));
+  vvcb_tu_job* dTj = at<vvcb_tu_job>(s.din, iTj);
+  vvcb_chroma_ctx_states* dCst = at<vvcb_chroma_ctx_states>(s.din, iCst);
+  const int16_t* dChroma = buf<int16_t>(ctx, kChroma);
+  const size_t plane = (size_t)ctx->cstride * ctx->ch;
+  const vvcb_chroma_visit* dVis = at<const vvcb_chroma_visit>(s.din, iVis);
+  const vvcb_chroma_joint_tu_job* dJob = at<const vvcb_chroma_joint_tu_job>(s.din, iJob);
+  {
+    ChromaTuPredParams Q = {};
+    ChromaParams& B = Q.planes;
+    B.visits = dVis; B.n = n_visits;
+    B.orig[0] = dChroma; B.orig[1] = dChroma + plane; B.reco[0] = dChroma + 2 * plane; B.reco[1] = dChroma + 3 * plane;
+    B.cstride = ctx->cstride; B.luma = ctx->bReco; B.lstride = ctx->stride; B.bd = ctx->bd; B.ctu = ctx->ctu; B.rom = ctx->dRom;
+    Q.joint = dJob; Q.n = n; Q.cbJobs = dTj; Q.states = dCst;
+    Q.pred = at<int16_t>(s.dw, s.oPred); Q.resi = at<int16_t>(s.dw, s.oResi); Q.frac = ctx->dRateRom->binFracBits;
+    chroma_tu_pred_kernel<true><<<std::min((n + kChromaWarps - 1) / kChromaWarps, ctx->numSms * 16), kChromaWarps * 32, 0, ctx->stream>>>(Q);
+    ctx->launches++;
+  }
+  TuChain t = s.chain(0);
+  t.priceFrom = reinterpret_cast<const vvcb_ctx_states*>(dCst);
+  t.states = reinterpret_cast<const vvcb_ctx_states*>(dCst); t.statesOut = reinterpret_cast<vvcb_ctx_states*>(dCst);
+  t.chroma = true; t.orig = dChroma; t.stride = ctx->cstride; t.resiOut = true;
+  if ((rc = run_tu_chain(ctx, t, L, nullptr))) return rc;
+  {
+    ChromaJointParams F;
+    F.jobs = dJob; F.n = n; F.visits = dVis; F.tuJobs = dTj; F.res = t.results; F.pred = t.pred; F.reco = t.reco;
+    F.orig[0] = dChroma; F.orig[1] = dChroma + plane; F.cstride = ctx->cstride; F.bd = ctx->bd;
+    F.states = dCst; F.joint = at<vvcb_bin_model>(s.din, iJm);
+    F.sse = at<uint64_t>(s.dw, oSse); F.cbf = s.dw + oCbf; F.bits = at<uint32_t>(s.dw, oBits); F.frac = ctx->dRateRom->binFracBits;
+    chroma_joint_kernel<<<std::min((n + 3) / 4, ctx->numSms * 16), 128, 0, ctx->stream>>>(F);
+    ctx->launches++;
+  }
+  CK(cudaGetLastError());
+  // outputs: TU results, SSEs, bits and cbf flags, then the wanted sample outputs
+  Pieces out;
+  const size_t hRes = out.add(s.dw + s.oRes, (size_t)n * sizeof(vvcb_tu_result)), hSse = out.add(s.dw + oSse, s.work.size - oSse);
+  s.want(out, level, reco, pred);
+  uint8_t* hout;
+  if ((rc = stage_out(ctx, out, hout))) return rc;
+  const vvcb_tu_result* res = at<const vvcb_tu_result>(hout, hRes);
+  const uint64_t* sse = at<const uint64_t>(hout, hSse);
+  const uint32_t* bits = at<const uint32_t>(hout, hSse + (oBits - oSse));
+  const uint8_t* cbf = hout + hSse + (oCbf - oSse);
+  s.scatter(hout, jobs, level, reco, pred);
+  for (int i = 0; i < n; i++) {
+    vvcb_chroma_joint_tu_result& r = results[i];
+    memset(&r, 0, sizeof(r));
+    const bool rate = (jobs[i].flags & VVCB_TU_RATE) != 0;
+    r.res = res[i];
+    if (!rate) r.res.frac_bits = 0;
+    r.sse[0] = sse[2 * i]; r.sse[1] = sse[2 * i + 1];
+    r.cbf = cbf[i];
+    if (rate) { r.cbf_bits[0] = bits[3 * i]; r.cbf_bits[1] = bits[3 * i + 1]; r.joint_bits = bits[3 * i + 2]; }
+  }
+  return VVCB_OK;
+}
+
+extern "C" int vvcb_chroma_joint_tu_eval(vvcb_ctx* ctx, const vvcb_chroma_visit* visits, int n_visits, const vvcb_chroma_joint_tu_job* jobs, int n,
+                                         const vvcb_chroma_joint_ctx_states* states, int n_states, size_t n_samples,
+                                         int32_t* level, int16_t* reco, int16_t* pred, vvcb_chroma_joint_tu_result* results)
+{
+  if (!ctx) return VVCB_ERR_ARG;
+  REMOTE_UNAVAILABLE("vvcb_chroma_joint_tu_eval");
+  if (n < 0 || n_states < 0 || n_visits < 0 || (n > 0 && (!jobs || !results || !visits || n_visits == 0))) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_joint_tu_eval: bad argument"); return VVCB_ERR_ARG;
+  }
+  if (!ctx->cw || ctx->cw != ctx->width / 2 || ctx->ch != ctx->height / 2 || !ctx->bReco) {
+    snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_joint_tu_eval: vvcb_chroma_frame_begin has not been called for this picture");
+    return VVCB_ERR_STATE;
+  }
+  if (n == 0) return VVCB_OK;
+  for (int i = 0; i < n_visits; i++)
+    if (const char* why = chroma_visit_error(ctx, visits[i])) { snprintf(ctx->err, sizeof(ctx->err), "vvcb_chroma_joint_tu_eval: visit %d: %s", i, why); return VVCB_ERR_ARG; }
+  return run_chunks(n, [&](int b, int m, bool checkOnly) {
+    return chroma_joint_tu_chunk(ctx, visits, n_visits, jobs + b, m, b, states, n_states, n_samples, level, reco, pred, results + b, checkOnly);
   });
 }
 

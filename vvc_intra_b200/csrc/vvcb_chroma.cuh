@@ -1,6 +1,6 @@
 // vvc_intra_b200 -- chroma intra candidates (vvcb_chroma_eval): prediction of Cb and Cr under the 8 candidates of
 // PU::getIntraChromaCandModes and their SAD / SATD, 4:2:0.  Included by vvcb_api.cu and, through the CUDA-on-pthreads shim, by
-// tests/host_emul/emul_chroma.cpp and emul_chroma_tu.cpp.
+// tests/host_emul/emul_chroma.cpp, emul_chroma_tu.cpp and emul_chroma_joint.cpp.
 //
 // One warp per visit (a chroma CU of the separate tree), warps striding over the batch:
 //   1. the Cb and Cr reference lines into shared memory -- the luma padding walk (build_line_set) with a unit of 2 samples, line 0 only,
@@ -358,7 +358,14 @@ struct ChromaTuPredParams {
   const vvcb_chroma_ctx_states* states;    // the candidate's snapshot (carried copy)
   int16_t* pred; int16_t* resi;
   const uint32_t* frac;                    // ProbModelTables::m_binFracBits
+  const vvcb_chroma_joint_tu_job* joint;   // the joint instantiation's candidates (read instead of jobs)
 };
+
+// the forward combination of joint Cb-Cr (include/vvc_intra_b200.h): C division, truncating toward zero
+__host__ __device__ __forceinline__ int chroma_joint_combine(int cb, int cr, int mode, int sign)
+{
+  return mode == 2 ? (cb + sign * cr) / 2 : mode == 1 ? (4 * cb + 2 * sign * cr) / 5 : (4 * cr + 2 * sign * cb) / 5;
+}
 
 __device__ __forceinline__ int32_t chroma_cbf_delta_bits(const vvcb_bin_model& m, const uint32_t* frac)
 {
@@ -366,6 +373,9 @@ __device__ __forceinline__ int32_t chroma_cbf_delta_bits(const vvcb_bin_model& m
   return (int32_t)frac[2 * q + 1] - (int32_t)frac[2 * q];
 }
 
+// JOINT (vvcb_chroma_joint_tu_eval): both predictions at the TU job's offset as above, the combined residual of the job's mode and sign
+// into the coded block, and the coded component's cbfDeltaBits (Ctx::QtCbf[Cr](0) for mode 3, else Ctx::QtCbf[Cb](0)).
+template <bool JOINT = false>
 __global__ void __launch_bounds__(kChromaWarps * 32) chroma_tu_pred_kernel(ChromaTuPredParams P)
 {
   __shared__ ChromaSmem smem[kChromaWarps];
@@ -375,32 +385,57 @@ __global__ void __launch_bounds__(kChromaWarps * 32) chroma_tu_pred_kernel(Chrom
   const uint32_t* filt = &rom.filt[0][0];
   const int maxv = (1 << P.planes.bd) - 1;
   for (int q = blockIdx.x * kChromaWarps + warp; q < P.n; q += gridDim.x * kChromaWarps) {
-    const vvcb_chroma_tu_job job = P.jobs[q];
-    const vvcb_chroma_visit cv = P.planes.visits[job.visit];
+    uint32_t visit; uint8_t cand;
+    if constexpr (JOINT) { visit = P.joint[q].visit; cand = P.joint[q].cand; }
+    else { const vvcb_chroma_tu_job job = P.jobs[q]; visit = job.visit; cand = job.cand; }
+    const vvcb_chroma_visit cv = P.planes.visits[visit];
     const Shape sh = chroma_visit_setup(sm, P.planes, rom, cv, lane);
     const int w = sh.w, n = sh.w * sh.h;
-    const int code = chroma_cand_code(job.cand, cv.dm_mode), mode = code == VVCB_DM_CHROMA ? cv.dm_mode : code;
+    const int code = chroma_cand_code(cand, cv.dm_mode), mode = code == VVCB_DM_CHROMA ? cv.dm_mode : code;
     const size_t off = P.cbJobs[q].offset;
-#pragma unroll 1
-    for (int comp = 0; comp < 2; comp++) {
-      const ChromaCand cd = chroma_make_cand(sm, rom, sh, mode, comp, cv.cclm);
-      int16_t* pred = P.pred + off + (size_t)comp * n;
-      int16_t* resi = P.resi + off + (size_t)comp * n;
+    if constexpr (JOINT) {
+      const int jm = P.joint[q].mode, sign = P.joint[q].sign;
+      const ChromaCand cb = chroma_make_cand(sm, rom, sh, mode, 0, cv.cclm), cr = chroma_make_cand(sm, rom, sh, mode, 1, cv.cclm);
+      int16_t* pred = P.pred + off;
+      int16_t* resi = P.resi + off;
       for (int u = lane; u < (n >> 4); u += 32) {
         const int x0 = (u & ((w >> 2) - 1)) << 2, y0 = (u >> (sh.lw - 2)) << 2;
-        int v[4][4];
-        chroma_predict_piece<4, 4>(sm, cd, sh, filt, maxv, x0, y0, v);
+        int vb[4][4], vr[4][4];
+        chroma_predict_piece<4, 4>(sm, cb, sh, filt, maxv, x0, y0, vb);
+        chroma_predict_piece<4, 4>(sm, cr, sh, filt, maxv, x0, y0, vr);
 #pragma unroll
         for (int i = 0; i < 4; i++)
 #pragma unroll
           for (int j = 0; j < 4; j++) {
             const int s = (y0 + i) * w + x0 + j;
-            pred[s] = (int16_t)v[i][j];
-            resi[s] = (int16_t)(sm.org[comp][s] - v[i][j]);
+            pred[s] = (int16_t)vb[i][j];
+            pred[n + s] = (int16_t)vr[i][j];
+            resi[s] = (int16_t)chroma_joint_combine(sm.org[0][s] - vb[i][j], sm.org[1][s] - vr[i][j], jm, sign);
           }
       }
+      if (lane == 0) P.cbJobs[q].cbf_delta_bits = chroma_cbf_delta_bits(jm == 3 ? P.states[q].cbf_cr[0] : P.states[q].cbf_cb[0], P.frac);
+    } else {
+#pragma unroll 1
+      for (int comp = 0; comp < 2; comp++) {
+        const ChromaCand cd = chroma_make_cand(sm, rom, sh, mode, comp, cv.cclm);
+        int16_t* pred = P.pred + off + (size_t)comp * n;
+        int16_t* resi = P.resi + off + (size_t)comp * n;
+        for (int u = lane; u < (n >> 4); u += 32) {
+          const int x0 = (u & ((w >> 2) - 1)) << 2, y0 = (u >> (sh.lw - 2)) << 2;
+          int v[4][4];
+          chroma_predict_piece<4, 4>(sm, cd, sh, filt, maxv, x0, y0, v);
+#pragma unroll
+          for (int i = 0; i < 4; i++)
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+              const int s = (y0 + i) * w + x0 + j;
+              pred[s] = (int16_t)v[i][j];
+              resi[s] = (int16_t)(sm.org[comp][s] - v[i][j]);
+            }
+        }
+      }
+      if (lane == 0) P.cbJobs[q].cbf_delta_bits = chroma_cbf_delta_bits(P.states[q].cbf_cb[0], P.frac);
     }
-    if (lane == 0) P.cbJobs[q].cbf_delta_bits = chroma_cbf_delta_bits(P.states[q].cbf_cb[0], P.frac);
     __syncwarp();
   }
 }
@@ -430,6 +465,71 @@ __global__ void __launch_bounds__(128) chroma_cbf_kernel(ChromaCbfParams P)
   } else {
     P.cbfBits[2 * i + 1] = isp_code_bin(st.cbf_cr[P.cbf[2 * i]], P.frac, cbf);
     P.cbf[2 * i + 1] = (uint8_t)cbf;
+  }
+}
+
+// Joint Cb-Cr after the TU chain (vvcb_chroma_joint_tu_eval), one warp per candidate: the inverse mapping of the job's mode and sign of the
+// residual r the chain's RESI pass left in the coded block, both reconstructions (Cb over r, Cr behind it) and their SSE; then, when the
+// coded residual has a level, tu_cb_coded_flag, tu_cr_coded_flag and tu_joint_cbcr_residual_flag on the candidate's carried models.
+// These models are not the residual's, so pricing them after residual_coding gives the bits of the coding order.
+struct ChromaJointParams {
+  const vvcb_chroma_joint_tu_job* jobs; int n;
+  const vvcb_chroma_visit* visits;
+  const vvcb_tu_job* tuJobs;               // the candidate's TU job (offset)
+  const vvcb_tu_result* res;               // the chain's results (the coded residual's levels)
+  const int16_t* pred; int16_t* reco;
+  const int16_t* orig[2]; int cstride, bd;
+  vvcb_chroma_ctx_states* states;          // carried models
+  vvcb_bin_model* joint;                   // carried Ctx::JointCbCrFlag models, 3 per candidate
+  uint64_t* sse;                           // [candidate][Cb, Cr]
+  uint8_t* cbf; uint32_t* bits;            // [candidate]; [candidate][cbf Cb, cbf Cr, joint flag]
+  const uint32_t* frac;
+};
+
+// H.266 8.7.2 under TuCResMode, in int: CSign * -32768 does not fit int16
+__host__ __device__ __forceinline__ void chroma_joint_inverse(int r, int mode, int sign, int& cb, int& cr)
+{
+  const int other = mode == 2 ? sign * r : (sign * r) >> 1;
+  cb = mode == 3 ? other : r;
+  cr = mode == 3 ? r : other;
+}
+
+__global__ void __launch_bounds__(128) chroma_joint_kernel(ChromaJointParams P)
+{
+  const int lane = threadIdx.x & 31;
+  const int maxv = (1 << P.bd) - 1;
+  for (int q = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); q < P.n; q += (int)((gridDim.x * blockDim.x) >> 5)) {
+    const vvcb_chroma_joint_tu_job j = P.jobs[q];
+    const vvcb_chroma_visit v = P.visits[j.visit];
+    const int w = 1 << v.log2w, n = w << v.log2h;
+    const size_t off = P.tuJobs[q].offset;
+    unsigned long long sse[2] = { 0, 0 };
+    for (int s = lane; s < n; s += 32) {
+      int res[2];
+      chroma_joint_inverse(P.reco[off + s], j.mode, j.sign, res[0], res[1]);
+#pragma unroll
+      for (int c = 0; c < 2; c++) {
+        const int rec = vmin(vmax((int)P.pred[off + c * n + s] + res[c], 0), maxv);
+        P.reco[off + c * n + s] = (int16_t)rec;
+        const int d = (int)P.orig[c][(size_t)(v.y + (s >> v.log2w)) * P.cstride + v.x + (s & (w - 1))] - rec;
+        sse[c] += (unsigned long long)(d * d);
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < 2; c++)
+      for (int o = 16; o > 0; o >>= 1) sse[c] += __shfl_xor_sync(0xffffffffu, sse[c], o);
+    if (lane == 0) {
+      const unsigned cbf = P.res[q].abs_sum_level != 0;
+      P.sse[2 * q] = sse[0]; P.sse[2 * q + 1] = sse[1];
+      P.cbf[q] = (uint8_t)cbf;
+      if (cbf) {
+        const unsigned cbfCb = j.mode != 3, cbfCr = j.mode != 1;
+        vvcb_chroma_ctx_states& st = P.states[q];
+        P.bits[3 * q] = isp_code_bin(st.cbf_cb[0], P.frac, cbfCb);
+        P.bits[3 * q + 1] = isp_code_bin(st.cbf_cr[cbfCb], P.frac, cbfCr);
+        P.bits[3 * q + 2] = isp_code_bin(P.joint[3 * q + 2 * cbfCb + cbfCr - 1], P.frac, 1);
+      }
+    }
   }
 }
 

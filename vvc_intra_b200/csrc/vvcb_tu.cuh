@@ -176,7 +176,10 @@ __device__ __forceinline__ long long team_sum(long long v, long long* red)
 constexpr int kTuSmallSamples = 256;      // blocks up to this size are worked on by one warp
 constexpr int kTuSmallB = 288;            // their transposed intermediate: kept columns x (height + 1), largest for 32x8
 
-template <int NT>
+// RESI: the reconstruction pass writes the inverse-transformed residual after its 16-bit clip into reco instead of the reconstruction, and
+// takes no SSE (joint Cb-Cr, vvcb_chroma_joint_tu_eval: the residual is mapped to both components afterwards, and cannot be recovered
+// from a clipped sample).  DCT-II jobs only.
+template <int NT, bool RESI = false>
 __global__ void __launch_bounds__(kTuThreads) tu_eval_kernel(TuParams P)
 {
   constexpr int TEAMS = kTuThreads / NT;
@@ -311,6 +314,7 @@ __global__ void __launch_bounds__(kTuThreads) tu_eval_kernel(TuParams P)
           int acc = 0;
           for (int k = 0; k < wKeep; k++) acc += (int)mh[k * w + x] * B[k * hp + y];
           const int r = clip16((acc + (1 << (shift2 - 1))) >> shift2);
+          if (RESI) { P.reco[job.offset + o] = (int16_t)r; continue; }
           const int rec = vmin(vmax((int)pred[o] + (int)(int16_t)r, 0), maxv);
           if (P.reco) P.reco[job.offset + o] = (int16_t)rec;
           const int d = (int)org[y * P.stride + x] - rec;

@@ -104,6 +104,14 @@ CHROMA_TU_JOB_DTYPE = np.dtype([('visit', '<u4'), ('cand', 'u1'), ('flags', 'u1'
                                 ('offset', '<u4'), ('pad', '<u4'), ('lambda', '<f8', 2)], align=True)
 CHROMA_TU_RESULT_DTYPE = np.dtype([('comp', TU_RESULT_DTYPE, 2), ('cbf_bits', '<u4', 2), ('cbf', 'u1', 2), ('pad', 'u1', 6)], align=True)
 assert CHROMA_CTX_STATES_DTYPE.itemsize == 420 and CHROMA_TU_JOB_DTYPE.itemsize == 40 and CHROMA_TU_RESULT_DTYPE.itemsize == 64
+# vvcb_chroma_joint_ctx_states / vvcb_chroma_joint_tu_job / vvcb_chroma_joint_tu_result (include/vvc_intra_b200.h): joint Cb-Cr candidates
+CHROMA_JOINT_CTX_STATES_DTYPE = np.dtype([('chroma', CHROMA_CTX_STATES_DTYPE), ('joint', BIN_MODEL_DTYPE, 3)])
+CHROMA_JOINT_TU_JOB_DTYPE = np.dtype([('visit', '<u4'), ('cand', 'u1'), ('flags', 'u1'), ('rate_idx', '<u2'), ('mode', 'u1'), ('sign', 'i1'),
+                                      ('qp_per', '<i2'), ('qp_rem', '<i2'), ('pad', '<u2'), ('offset', '<u4'), ('pad2', '<u4'), ('lambda', '<f8')],
+                                     align=True)
+CHROMA_JOINT_TU_RESULT_DTYPE = np.dtype([('res', TU_RESULT_DTYPE), ('sse', '<u8', 2), ('cbf_bits', '<u4', 2), ('joint_bits', '<u4'), ('cbf', 'u1'),
+                                         ('pad', 'u1', 3)], align=True)
+assert CHROMA_JOINT_CTX_STATES_DTYPE.itemsize == 438 and CHROMA_JOINT_TU_JOB_DTYPE.itemsize == 32 and CHROMA_JOINT_TU_RESULT_DTYPE.itemsize == 56
 
 
 class EngineError(RuntimeError):
@@ -168,6 +176,8 @@ def load_library():
         L.vvcb_chroma_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.vvcb_chroma_tu_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.vvcb_chroma_joint_tu_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t,
+                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.vvcb_ctu_hads_islice.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.vvcb_features_eval.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.vvcb_frame_bind_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
@@ -494,6 +504,24 @@ class IntraCostEngine:
         self._ck(self._lib.vvcb_chroma_tu_eval(self._ctx, _ptr(visits), len(visits), _ptr(jobs), len(jobs),
                                                _ptr(states) if states is not None else None, 0 if states is None else len(states), n_samples,
                                                p('level'), p('reco'), p('pred'), _ptr(out['results'])))
+        return out
+
+    def chroma_joint_tu_eval(self, visits, jobs, n_samples, states=None, want_level=False, want_reco=False, want_pred=False):
+        """vvcb_chroma_joint_tu_eval: joint Cb-Cr candidates (CHROMA_JOINT_TU_JOB_DTYPE) of the visits (CHROMA_VISIT_DTYPE).
+        states: CHROMA_JOINT_CTX_STATES_DTYPE array indexed by job['rate_idx'] (needed by DEPQUANT / RATE jobs).  Returns dict with 'results'
+        (CHROMA_JOINT_TU_RESULT_DTYPE) and the wanted flat outputs of n_samples, per candidate 2 w*h at job['offset']: level the coded
+        residual's levels then zeros, reco and pred Cb then Cr."""
+        visits = np.ascontiguousarray(visits, CHROMA_VISIT_DTYPE)
+        jobs = np.ascontiguousarray(jobs, CHROMA_JOINT_TU_JOB_DTYPE)
+        states = None if states is None else np.ascontiguousarray(states, CHROMA_JOINT_CTX_STATES_DTYPE)
+        out = dict(results=np.zeros(len(jobs), CHROMA_JOINT_TU_RESULT_DTYPE))
+        for key, want, dt in (('level', want_level, np.int32), ('reco', want_reco, np.int16), ('pred', want_pred, np.int16)):
+            if want:
+                out[key] = np.zeros(n_samples, dt)
+        p = lambda k: _ptr(out[k]) if k in out else None
+        self._ck(self._lib.vvcb_chroma_joint_tu_eval(self._ctx, _ptr(visits), len(visits), _ptr(jobs), len(jobs),
+                                                     _ptr(states) if states is not None else None, 0 if states is None else len(states),
+                                                     n_samples, p('level'), p('reco'), p('pred'), _ptr(out['results'])))
         return out
 
     def residual_bits(self, jobs, levels, states):
