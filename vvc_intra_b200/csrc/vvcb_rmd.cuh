@@ -542,7 +542,8 @@ __device__ __forceinline__ void predict_angular(const SM& sm, const int16_t* pro
   pred_angular_unit<R, C>(ml, sm.lines[s.set][ver ? 1 : 0], s.p, s.mrl, mw, mh, ver ? x0 : y0, (ver ? y0 : x0) + rOff, filt, (1 << bd) - 1, q);
 }
 
-// MIP: first interpolation pass of one slot into shared memory (CL/MatrixIntraPrediction.cpp:469-567,
+// MIP of the TU prediction kernel (the evaluation kernels predict MIP in registers, predict_mip_piece):
+// first interpolation pass of one slot into shared memory (CL/MatrixIntraPrediction.cpp:469-567,
 // shorter side first).  w >= h: plane[y * redW + rx] (vertical pass at the reduced columns);
 // h > w: plane[ry * w + x] (horizontal pass at the reduced rows).
 // When that first pass is the identity (no up-sampling along the shorter side) the plane IS the reduced prediction.
@@ -623,61 +624,155 @@ __device__ __forceinline__ void predict_mip(const SM& sm, const int16_t* plane, 
   }
 }
 
-// MIP prediction of piece k of a slot that one lane owns: the packed 4x4, 8x4, 4x8 and 8x8 shapes, one per tile class TILE 0..3
-// (4x4 matrices for 4x4, 8x8 matrices for the others; a 4 x 4 reduced block).  The reduced samples the piece needs are computed in
-// registers and up-sampled there (CL/MatrixIntraPrediction.cpp:469-567), with no plane in shared memory and no pass for an identity
-// direction.  Pieces come in order k = 0, 1 (4x4: k = 0 only): 8x4 takes reduced columns 2k, 2k + 1, 4x8 and 8x8 reduced rows 2k, 2k + 1;
-// `carry` hands piece 1 the last reduced column / row of piece 0, the sample before its first one.
-template <int TILE, int R, int C, class SM>
-__device__ __forceinline__ void predict_mip_lane(const SM& sm, const MipSlot& ms, int k, int maxv, int (&carry)[4], int (&q)[R][C])
+// MIP prediction of a 4x4 slot (one lane, 4x4 matrices): the reduced block is the prediction.
+__device__ __forceinline__ void predict_mip_4x4(const MipSlot& ms, int maxv, int (&q)[4][4])
 {
-  const int16_t* top = sm.lines[0][0];
-  const int16_t* left = sm.lines[0][1];
   // matrix row of reduced sample (ry, rx): ry * 4 + rx, transposed modes rx * 4 + ry
   const int stepY = ms.transpose ? 1 : 4, stepX = ms.transpose ? 4 : 1;
-  if constexpr (TILE == 0) {
 #pragma unroll
-    for (int i = 0; i < 4; i++)
+  for (int i = 0; i < 4; i++)
 #pragma unroll
-      for (int j = 0; j < 4; j++) q[i][j] = mip_row_sample<false>(ms, i * stepY + j * stepX, maxv);
-  } else if constexpr (TILE == 1) {
-    // 8x4: the vertical pass is the identity; horizontal up-sampling by 2 from the left boundary
+    for (int j = 0; j < 4; j++) q[i][j] = mip_row_sample<false>(ms, i * stepY + j * stepX, maxv);
+}
+
+// Matrix row of reduced sample (rx, ry) of a slot is ry * sY + rx * sX (mip_reduced_sample: the 16x4 / 4x16 row mapping and the
+// transposed modes folded into two steps)
+struct MipSteps { int sY, sX; };
+__device__ __forceinline__ MipSteps make_mip_steps(const MipGeom& mg, const Shape& sh, bool transpose)
+{
+  const int lho = sh.w == 4 && sh.h >= 16 ? 2 : 1, lvo = sh.h == 4 && sh.w >= 16 ? 2 : 1;
+  MipSteps s;
+  if (transpose) { s.sY = lvo; s.sX = lho * (mg.small ? mg.redH : 8); }
+  else           { s.sY = lvo * (mg.small ? mg.redW : 8); s.sX = lho; }
+  return s;
+}
+
+constexpr int kMipCarry = 8;                // longest reduced row / column handed from piece 0 to piece 1
+
+// MIP prediction of one piece of a unit, for every shape with MIP but 4x4, with up-sampling factors 2^LGH x 2^LGV
+// (CL/MatrixIntraPrediction.cpp:469-567, shorter side first, no pass in an identity direction).  A piece is 4 rows x C columns of the
+// block at (x0, y0): one 4x8 half of an 8x8 unit (k = 0 above k = 1), or one 4x4 unit of an 8x4 (side by side) or 4x8 (one above the
+// other) SATD tile.  e[][] holds, in registers, exactly the reduced samples the piece's up-sampling reads: those under the piece, the
+// reduced row above it when the vertical factor is > 1, the reduced column left of it when the horizontal one is, and their corner.  Where
+// that border lies outside the reduced block, the first pass reads the boundary (top[upH * (rx + 1)] / left[upV * (ry + 1)]) and the
+// second reads the boundary line itself (left[1 + y] / top[1 + x]), as build_mip_planes / predict_mip of the TU kernel do.  Every index
+// is static: the shape's factors select the instantiation (predict_mip_piece), so nothing leaves the registers.  `carry` hands piece 1
+// the border piece 0 computed for it: its last reduced column (8x4 tiles) or row, or with a vertical factor of 8 (both halves inside one
+// reduced row) the row above.
+template <int TILE, int LGH, int LGV, int C, class SM>
+__device__ __forceinline__ void mip_piece(const SM& sm, const MipSlot& ms, MipSteps st, int maxv, int x0, int y0, int k,
+                                          int (&carry)[kMipCarry], int (&q)[4][C])
+{
+  constexpr int R = 4, UH = 1 << LGH, UV = 1 << LGV;
+  constexpr bool VFIRST = TILE != 2 && TILE != 5;       // w >= h: vertical pass first (at the reduced columns)
+  constexpr bool HSPLIT = TILE == 1;                     // the pieces of a unit side by side
+  constexpr int RB = LGV > 0 ? 1 : 0, CB = LGH > 0 ? 1 : 0;
+  constexpr int ER = ((R - 1) >> LGV) + 1 + RB, EC = ((C - 1) >> LGH) + 1 + CB;
+  static_assert(ER <= 4 && EC <= 8 && (HSPLIT ? ER : EC) <= kMipCarry, "register footprint of a MIP piece");
+  const int16_t* top = sm.lines[0][0];
+  const int16_t* left = sm.lines[0][1];
+  const int ry0 = y0 >> LGV, rx0 = x0 >> LGH;
+  int e[ER][EC];
 #pragma unroll
-    for (int i = 0; i < 4; i++) {
-      const int b  = k ? carry[i] : left[1 + i];
-      const int r0 = mip_row_sample<true>(ms, i * stepY + 2 * k * stepX, maxv);
-      const int r1 = mip_row_sample<true>(ms, i * stepY + (2 * k + 1) * stepX, maxv);
-      q[i][0] = (b + r0 + 1) >> 1; q[i][1] = r0; q[i][2] = (r0 + r1 + 1) >> 1; q[i][3] = r1;
-      carry[i] = r1;
+  for (int a = 0; a < ER; a++)
+#pragma unroll
+    for (int b = 0; b < EC; b++) {
+      const int ry = ry0 - RB + a, rx = rx0 - CB + b;
+      const bool carried = HSPLIT ? CB && b == 0 : RB && a == 0;
+      if (carried && k) e[a][b] = carry[HSPLIT ? a : b];
+      else if (RB && a == 0 && ry < 0) e[a][b] = VFIRST && rx >= 0 ? top[UH * (rx + 1)] : 0;      // 0: never read
+      else if (CB && b == 0 && rx < 0) e[a][b] = !VFIRST && ry >= 0 ? left[UV * (ry + 1)] : 0;
+      else e[a][b] = mip_row_sample<true>(ms, ry * st.sY + rx * st.sX, maxv);
+    }
+  if constexpr (HSPLIT) {
+#pragma unroll
+    for (int a = 0; a < ER; a++) carry[a] = e[a][EC - 1];
+  } else if constexpr (RB) {
+#pragma unroll
+    for (int b = 0; b < EC; b++) carry[b] = e[LGV == 3 ? 0 : ER - 1][b];
+  }
+  // weight of the sample behind in output row i / column j: y0 is a multiple of 4 (of 8 for k = 0), x0 of UH
+  auto kv = [&](int i) { return LGV <= 2 ? (i & (UV - 1)) + 1 : (y0 & 7) + i + 1; };
+  if constexpr (VFIRST) {
+    int p[R][EC];                                        // first pass: output rows at the reduced columns
+#pragma unroll
+    for (int i = 0; i < R; i++)
+#pragma unroll
+      for (int b = 0; b < EC; b++) {
+        if (LGV == 0) p[i][b] = e[i][b];
+        else {
+          const int a = (i >> LGV) + 1, kk = kv(i);
+          p[i][b] = ((UV - kk) * e[a - 1][b] + kk * e[a][b] + (UV >> 1)) >> LGV;
+        }
+      }
+#pragma unroll
+    for (int i = 0; i < R; i++) {
+      const int lb = CB ? (rx0 == 0 ? left[1 + y0 + i] : p[i][0]) : 0;
+#pragma unroll
+      for (int j = 0; j < C; j++) {
+        if (LGH == 0) q[i][j] = p[i][j];
+        else {
+          const int c = (j >> LGH) + 1, kk = (j & (UH - 1)) + 1;
+          q[i][j] = ((UH - kk) * (c == 1 ? lb : p[i][c - 1]) + kk * p[i][c] + (UH >> 1)) >> LGH;
+        }
+      }
     }
   } else {
-    // 4x8, 8x8: vertical up-sampling by 2 from the top boundary (at the reduced columns), then for 8x8 horizontal by 2 from the left one
-    int v[4][4];
+    int p[ER][C];                                        // first pass: output columns at the reduced rows
 #pragma unroll
-    for (int rx = 0; rx < 4; rx++) {
-      const int b  = k ? carry[rx] : top[TILE == 3 ? 2 + 2 * rx : 1 + rx];
-      const int r0 = mip_row_sample<true>(ms, 2 * k * stepY + rx * stepX, maxv);
-      const int r1 = mip_row_sample<true>(ms, (2 * k + 1) * stepY + rx * stepX, maxv);
-      v[0][rx] = (b + r0 + 1) >> 1; v[1][rx] = r0; v[2][rx] = (r0 + r1 + 1) >> 1; v[3][rx] = r1;
-      carry[rx] = r1;
-    }
-    if constexpr (TILE == 2) {
+    for (int a = 0; a < ER; a++)
 #pragma unroll
-      for (int i = 0; i < 4; i++)
+      for (int j = 0; j < C; j++) {
+        if (LGH == 0) p[a][j] = e[a][j];
+        else {
+          const int c = (j >> LGH) + 1, kk = (j & (UH - 1)) + 1;
+          p[a][j] = ((UH - kk) * e[a][c - 1] + kk * e[a][c] + (UH >> 1)) >> LGH;
+        }
+      }
 #pragma unroll
-        for (int j = 0; j < 4; j++) q[i][j] = v[i][j];
-    } else {
+    for (int j = 0; j < C; j++) {
+      const int tb = RB ? (ry0 == 0 ? top[1 + x0 + j] : p[0][j]) : 0;
 #pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const int l = left[1 + 4 * k + i];
-#pragma unroll
-        for (int rx = 0; rx < 4; rx++) {
-          q[i][2 * rx]     = ((rx ? v[i][rx - 1] : l) + v[i][rx] + 1) >> 1;
-          q[i][2 * rx + 1] = v[i][rx];
+      for (int i = 0; i < R; i++) {
+        if (LGV == 0) q[i][j] = p[i][j];
+        else {
+          const int a = (i >> LGV) + 1, kk = kv(i);
+          q[i][j] = ((UV - kk) * (a == 1 ? tb : p[a - 1][j]) + kk * p[a][j] + (UV >> 1)) >> LGV;
         }
       }
     }
   }
+}
+
+// The factor pairs (log2 upH, log2 upV) a tile class holds: 8x4 / 16x4 (1,0); 4x8 / 4x16 (0,1); 8x8, 16x16, 32x32, 64x64 (1,1) to (3,3);
+// 16x8, 32x8, 32x16, 64x16, 64x32 (1,0), (2,0), (2,1), (3,1), (3,2); 8x16 ... 32x64 the transposes.  Packed items (MODE 1) hold only the
+// tile class's small shape: one instantiation.  The factors are uniform over a warp iteration (one visit, or one shape per packed item).
+template <int TILE, int MODE, int C, class SM>
+__device__ __forceinline__ void predict_mip_piece(const SM& sm, const MipSlot& ms, MipSteps st, const MipGeom& mg, int maxv,
+                                                  int x0, int y0, int k, int (&carry)[kMipCarry], int (&q)[4][C])
+{
+#define VVCB_MIP_PIECE(H, V) mip_piece<TILE, H, V, C>(sm, ms, st, maxv, x0, y0, k, carry, q)
+  if constexpr (TILE == 1) VVCB_MIP_PIECE(1, 0);
+  else if constexpr (TILE == 2) VVCB_MIP_PIECE(0, 1);
+  else if constexpr (MODE == 1) {
+    if constexpr (TILE == 3) VVCB_MIP_PIECE(1, 1);
+    else if constexpr (TILE == 4) VVCB_MIP_PIECE(1, 0);
+    else VVCB_MIP_PIECE(0, 1);
+  } else if constexpr (TILE == 3) {
+    if (mg.lgUpH == 1) VVCB_MIP_PIECE(1, 1);
+    else if (mg.lgUpH == 2) VVCB_MIP_PIECE(2, 2);
+    else VVCB_MIP_PIECE(3, 3);
+  } else if constexpr (TILE == 4) {
+    // plain items (MODE 0) come from calls that pack the small shapes: 16x8 is never among them
+    if (MODE == 2 && mg.lgUpH == 1) VVCB_MIP_PIECE(1, 0);
+    else if (mg.lgUpH == 2) { if (mg.lgUpV == 0) VVCB_MIP_PIECE(2, 0); else VVCB_MIP_PIECE(2, 1); }
+    else { if (mg.lgUpV == 1) VVCB_MIP_PIECE(3, 1); else VVCB_MIP_PIECE(3, 2); }
+  } else {
+    if (MODE == 2 && mg.lgUpV == 1) VVCB_MIP_PIECE(0, 1);
+    else if (mg.lgUpV == 2) { if (mg.lgUpH == 0) VVCB_MIP_PIECE(0, 2); else VVCB_MIP_PIECE(1, 2); }
+    else { if (mg.lgUpH == 1) VVCB_MIP_PIECE(1, 3); else VVCB_MIP_PIECE(2, 3); }
+  }
+#undef VVCB_MIP_PIECE
 }
 
 // =====================================================================================================
@@ -717,11 +812,17 @@ template <bool PACK> struct EvalShared {
   uint32_t sFilt[64];
 };
 
-// MIP slots that one lane owns (4x4, 8x4, 4x8, 8x8) are predicted in registers (predict_mip_lane), with the matrices of their family
-// (4x4 for the 4x4 class, 8x8 for the others) copied to shared memory: at most 1 360 bytes, which fit under the 48 KB of static shared
-// memory beside EvalShared; the slots of larger shapes read theirs from the ROM in global memory.  The lane-owned shapes come in packed
-// items, and in plain items only for the prediction-output kernels (MODE 2).
-template <int TILE, int KIND, int MODE> constexpr bool kLaneMip = KIND == KIND_MIP && TILE < 4 && MODE != 0;
+// Every MIP slot is predicted in registers (predict_mip_4x4, predict_mip_piece).  The slots that one lane owns (4x4, 8x4, 4x8, 8x8) read
+// the matrices of their family (4x4 for the 4x4 class, 8x8 for the others) from a copy in shared memory: at most 1 360 bytes, which fit
+// under the 48 KB of static shared memory beside EvalShared; the slots of larger shapes read theirs (16x16 family) from the ROM in global
+// memory, through the L1.  The lane-owned shapes come in packed items, and in plain items only for the prediction-output kernels (MODE 2).
+// Where an instantiation sees both (MODE 1 and 2 of the 8x4 / 4x8 classes, MODE 2 of the 8x8 class), the two are separate call sites, so
+// that neither reads its matrices through a generic pointer.
+constexpr int MIP_SRC_SHARED = 1, MIP_SRC_GLOBAL = 2;
+template <int TILE, int KIND, int MODE> constexpr int kMipSrc =
+    KIND != KIND_MIP ? 0 : MODE == 0 || TILE >= 4 ? MIP_SRC_GLOBAL
+                         : TILE == 0 || (TILE == 3 && MODE == 1) ? MIP_SRC_SHARED : MIP_SRC_SHARED | MIP_SRC_GLOBAL;
+template <int TILE, int KIND, int MODE> constexpr bool kLaneMip = (kMipSrc<TILE, KIND, MODE> & MIP_SRC_SHARED) != 0;
 constexpr int kMipLaneWords = 10 * 34;       // the larger of mip_family_words(0), mip_family_words(1)
 
 // sMip: kMipLaneWords of shared memory when kLaneMip<TILE, KIND, MODE>
@@ -734,7 +835,7 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
   constexpr int S = TILE < 3 ? 4 : 8;
   constexpr int V = Cfg::kVisits;
   constexpr bool LANE_MIP = kLaneMip<TILE, KIND, MODE>;
-  constexpr bool ONLY_LANE_MIP = LANE_MIP && PACK && (TILE == 0 || TILE == 3);    // the packed 4x4 and 8x8 classes hold nothing else
+  constexpr int MIP_SRC = kMipSrc<TILE, KIND, MODE>;
   constexpr int MIP_FAMILY = TILE == 0 ? 0 : 1;
   auto& smem = shm.smem;
   auto& sScratch = shm.sScratch;
@@ -845,15 +946,12 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
       const int slot = kind_slot(rom, v, KIND, (PACK ? 0 : item.slot_begin) + (tk >> sh.lgLanes));
       const SlotInfo s = make_slot_info(rom, v, sh, slot);
 
-      // ---- per-slot scratch built by the slot's lanes
-      __syncwarp();
+      // ---- per-slot scratch built by the slot's lanes (MIP slots have none)
+      if (KIND != KIND_MIP) __syncwarp();
       int dc = 0;
-      const bool laneMip = ONLY_LANE_MIP || (LANE_MIP && lanes == 1);     // uniform over the warp: one shape per item
       if (KIND == KIND_ANG) {
         if (s.p.angle < 0) build_projected_line(scratch, sm, s, s.p.is_ver ? sh.w : sh.h, s.p.is_ver ? sh.h : sh.w, gl, gsize);
-      } else if (KIND == KIND_MIP) {
-        if (!laneMip) build_mip_planes(scratch, scratch + mip_plane_offset(mg, sh), rom, sm, mg, sh, P.bd, s.mode, gl, gsize);
-      } else {
+      } else if (KIND == KIND_PDC) {
         // DC value (CL/IntraPrediction.cpp:248-285), summed by the slot's lanes
         int part = 0;
         if (s.kind == 1) {
@@ -866,13 +964,38 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
         const int denom = sh.w == sh.h ? 2 * sh.w : vmax(sh.w, sh.h);
         dc = (part + (denom >> 1)) >> vlog2(denom);
       }
-      __syncwarp();
+      if (KIND != KIND_MIP) __syncwarp();
 
       int sad = 0, satd = 0;
       const bool transposed = KIND == KIND_ANG && !s.p.is_ver;
+      // MIP: the slot's matrices from shared memory (lane-owned shapes) or global memory (the 16x16 family); mipShared is uniform over
+      // the warp (one shape per item)
       MipSlot ms = {};
-      int mipCarry[4] = {};
-      if (laneMip) ms = make_mip_slot(sMip, mg, sm.mipIn, sm.mipAux, s.mode);
+      MipSteps mst = {};
+      int mipCarry[kMipCarry] = {};
+      int mipMat = 0;                            // the mode's first word in its family
+      const bool mipShared = MIP_SRC == MIP_SRC_SHARED || (MIP_SRC != MIP_SRC_GLOBAL && mg.family != 2);
+      const uint32_t* mipGlobal = rom.mip + mip_family_base(TILE == 0 ? 0 : 2);
+      if (KIND == KIND_MIP) {
+        if (mipShared) { ms = make_mip_slot(sMip, mg, sm.mipIn, sm.mipAux, s.mode); mipMat = (int)(ms.mat - sMip); }
+        else           { ms = make_mip_slot(mipGlobal, mg, sm.mipIn, sm.mipAux, s.mode); mipMat = (int)(ms.mat - mipGlobal); }
+        mst = make_mip_steps(mg, sh, ms.transpose);
+      }
+      const int mipMax = (1 << P.bd) - 1;
+      // the MIP prediction of a piece, with the matrices read from where mipShared says (two call sites: no generic pointer)
+      auto mip_piece_at = [&](auto& q, int x0, int y0, int k) {
+        constexpr int C = sizeof(q[0]) / sizeof(q[0][0]);
+        MipSlot m = ms;
+        if (mipShared) {
+          m.mat = sMip + mipMat;
+          if constexpr (TILE == 0) predict_mip_4x4(m, mipMax, q);
+          else predict_mip_piece<TILE, MODE, C>(sm, m, mst, mg, mipMax, x0, y0, k, mipCarry, q);
+        } else {
+          m.mat = mipGlobal + mipMat;
+          if constexpr (TILE == 0) predict_mip_4x4(m, mipMax, q);
+          else predict_mip_piece<TILE, MODE, C>(sm, m, mst, mg, mipMax, x0, y0, k, mipCarry, q);
+        }
+      };
       if constexpr (S == 8) {
         // An 8x8 unit is processed as two 4x8 halves by the same loop body (kept rolled: the fully unrolled unit was
         // > 64 KB of code and instruction-fetch bound, profiles/r1m_summary.md history).  Rows and the first two column stages of the
@@ -890,8 +1013,7 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
           int q[4][8], d[4][8];
           const int hx = transposed ? x0 + 4 * k : x0, hy = transposed ? y0 : y0 + 4 * k;   // picture origin of the half
           if (KIND == KIND_ANG)      predict_angular<4, 8>(sm, scratch, s, sh, sFilt, P.bd, x0, y0, 4 * k, q);
-          else if (KIND == KIND_MIP && laneMip) predict_mip_lane<TILE, 4, 8>(sm, ms, k, (1 << P.bd) - 1, mipCarry, q);
-          else if (KIND == KIND_MIP) predict_mip<4, 8>(sm, scratch + mip_plane_offset(mg, sh), mg, sh, hx, hy, q);
+          else if (KIND == KIND_MIP) mip_piece_at(q, hx, hy, k);
           else pred_planar_dc_unit<4, 8>(sm.lines[s.set][0], sm.lines[s.set][1], s.kind, s.p.pdpc, dc, sh.lw, sh.lh, hx, hy, q);
           if (WITH_PRED && P.predOut && act) store_pred<4, 8>(P.predOut + (size_t)slot * sh.w * sh.h, sh.w, hx, hy, transposed, q);
           if (transposed) residual_unit<4, 8, true>(org + hy * P.stride + hx, P.stride, q, d, sad);
@@ -935,8 +1057,7 @@ __device__ __forceinline__ void rmd_eval_body(const EvalParams& P, EvalShared<MO
           const int y0 = ty * (TILE == 2 ? 8 : 4) + (TILE == 2 ? 4 * k : 0);
           int q[4][4], d[4][4];
           if (KIND == KIND_ANG)      predict_angular<4, 4>(sm, scratch, s, sh, sFilt, P.bd, x0, y0, 0, q);
-          else if (KIND == KIND_MIP && laneMip) predict_mip_lane<TILE, 4, 4>(sm, ms, k, (1 << P.bd) - 1, mipCarry, q);
-          else if (KIND == KIND_MIP) predict_mip<4, 4>(sm, scratch + mip_plane_offset(mg, sh), mg, sh, x0, y0, q);
+          else if (KIND == KIND_MIP) mip_piece_at(q, x0, y0, k);
           else pred_planar_dc_unit<4, 4>(sm.lines[s.set][0], sm.lines[s.set][1], s.kind, s.p.pdpc, dc, sh.lw, sh.lh, x0, y0, q);
           if (WITH_PRED && P.predOut && act) store_pred<4, 4>(P.predOut + (size_t)slot * sh.w * sh.h, sh.w, x0, y0, transposed, q);
           if (transposed) residual_unit<4, 4, true>(org + y0 * P.stride + x0, P.stride, q, d, sad);
